@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: HMC chain-steps/s on BASELINE config c2.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1], SURVEY.md section 8(d) c2): HMCDiag, L=10
 leapfrog steps, 65,536 chains PER GPU on the 1000-dim dense-precision Gaussian
@@ -16,6 +16,11 @@ HOST buffers (pinned host -> device copy of the chain state and device -> host
 copy of every draw + log density inside the timed region, every step).
 `config.secondary` carries the other BASELINE configs (c1, c3, c4 strong / weak
 over the N ranks, c5, MALA on c2), each with its own roofline fraction.
+
+`--dump-outputs DIR` writes what the last timed sample_n call of rank 0
+returned, for comparing two builds output for output: DIR/draws.npy and
+DIR/logp.npy (fp32, [draws, chains, ...]) for a fixed, seeded sample of chains.
+The inputs depend only on the arguments, so equal arguments give equal inputs.
 """
 from __future__ import annotations
 
@@ -171,6 +176,20 @@ class ClockSampler:
 
 # --------------------------------------------------------------------------------
 DRAWS_PER_STEP = 16   # one step = one sample_n(16) call for every chain: 20 steps ~ 1 s of device time
+DUMP_BYTES = 32 << 20  # --dump-outputs budget: a whole step's draws are 4 GB at the default size
+
+
+def dump_outputs(out_dir, draws, logp):
+    """Save draws [n, C, D] and logp [n, C] of one sample_n call, restricted to a seeded sample of chains."""
+    import numpy as np
+    import torch
+    n, C, D = draws.shape
+    k = min(C, max(1, DUMP_BYTES // (n * (D + 1) * 4)))
+    idx = np.sort(np.random.default_rng(0).choice(C, size=k, replace=False))
+    sel = torch.as_tensor(idx, device=draws.device)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "draws.npy"), draws[:, sel].cpu().numpy())
+    np.save(os.path.join(out_dir, "logp.npy"), logp[:, sel].cpu().numpy())
 
 
 def bind_to_gpu_numa(local):
@@ -200,7 +219,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-secondary", action="store_true", help="skip the c1 / c3 / c4 / c5 / MALA legs")
     ap.add_argument("--e2e-chunk", type=int, default=0, help="chains per sample_host chunk (0: library default)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's draws and log densities here")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs records the CUDA path; the reference arm has nothing to dump")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":
@@ -261,8 +285,10 @@ def main():
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     ev0.record()
     for _ in range(args.steps):
-        # every draw streams ~1.6 GB of chain state (>> L2) and a step writes a fresh 16 x 262 MB draw block
-        sampler.sample_n(n)
+        # every draw streams ~1.6 GB of chain state (>> L2) and a step writes a fresh 16 x 262 MB draw block;
+        # the previous step's block is released first, so every step reuses the same cached allocation
+        last = None
+        last = sampler.sample_n(n)
     ev1.record()
     barrier()
     ms = ev0.elapsed_time(ev1)
@@ -274,6 +300,9 @@ def main():
     lib.bk_profile_read(_lib.PROF_STEP, sms_, sn)
     accept = float(sampler.last_accept.float().mean())
     clk = clocks.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *last)
+    del last
     ms_max = rank_max(ms)
     value = world * C * n * args.steps / (ms_max * 1e-3)
     stage(f"device-resident done: {ms:.1f} ms")
@@ -285,7 +314,7 @@ def main():
     host_draws = torch.empty(n, C, D, dtype=torch.float32, pin_memory=True)
     host_lp = torch.empty(n, C, dtype=torch.float32, pin_memory=True)
     host_draws[n - 1].copy_(sampler.theta)
-    e2e_steps = max(3, min(args.steps, 10))
+    e2e_steps = args.steps
 
     def e2e_step():
         # next step's input = this step's last draw, read in place from the pinned result buffer (a chunk's
