@@ -13,7 +13,7 @@ LIB_PATH = os.environ.get("BK_LIB") or os.path.join(_HERE, "libbk_b200.so")   # 
 
 BK_OK, BK_E_INVALID, BK_E_UNSUPPORTED, BK_E_CUDA, BK_E_WORKSPACE, BK_E_HANDLE = 0, -1, -2, -3, -4, -5
 BK_F32, BK_F64 = 0, 1
-MODEL_ISO, MODEL_DIAG, MODEL_DENSE, MODEL_HLR, MODEL_GPL, MODEL_BINOM = range(6)
+MODEL_ISO, MODEL_DIAG, MODEL_DENSE, MODEL_HLR, MODEL_GPL, MODEL_BINOM, MODEL_USER = range(7)
 SMC_KERNEL_RW, SMC_KERNEL_MALA, SMC_KERNEL_HMC = 0, 1, 2
 SMC_MAX_WORLD, SMC_MAILBOX_BYTES = 16, 4096
 RNG_PHILOX, RNG_INJECTED = 0, 1
@@ -76,6 +76,7 @@ _SIGNATURES = {
     "bk_model_log_density_gradient": (C.c_int, [u64, vp, i64, vp, vp, vp, sz, vp]),
     "bk_model_log_density_gradient_fast": (C.c_int, [u64, vp, i64, vp, vp, vp, sz, vp]),
     "bk_model_log_prior_likelihood": (C.c_int, [u64, vp, i64, vp, vp, vp]),
+    "bk_model_create_cuda": (C.c_int, [C.c_char_p, i64, i32, vp, i64, C.POINTER(u64), C.c_char_p, sz]),
     "bk_init_normal": (C.c_int, [vp, i64, i64, i32, u64, u64, C.c_uint32, vp]),
     "bk_hmc_diag_workspace_bytes": (sz, [u64, i64]),
     "bk_hmc_diag_sample": (C.c_int, [u64, vp, vp, vp, C.POINTER(i32), i64, f64, i32, vp, i64,

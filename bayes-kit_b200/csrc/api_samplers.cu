@@ -5,6 +5,7 @@
 
 #include "dense_tc.h"
 #include "sampler_generic.h"
+#include "user_kernels.cuh"
 
 using namespace bk;
 
@@ -39,6 +40,29 @@ bool force_generic() {
 
 template <typename T>
 bool use_fused(const Model& m) { return m.separable() && m.d.dims <= SEP_MAX_D && !force_generic(); }
+
+// user-written CUDA model with D <= USER_FUSED_MAX_D: one register-resident kernel per call (user_model.cu)
+bool use_user_fused(const Model& m) { return user_fused(m) && !force_generic(); }
+
+UserRunArgs user_args(const Model& m, void* theta, int64_t C, int64_t n, const bk_rng* rng, const bk_draw_out& out) {
+    UserRunArgs a;
+    memset(&a, 0, sizeof(a));
+    a.theta = theta;
+    a.params = m.user_params;
+    a.normals = rng->normals;
+    a.uniforms = rng->uniforms;
+    a.draws = out.draws;
+    a.logp = out.logp;
+    a.accept = out.accept;
+    a.C = C;
+    a.n_draws = n;
+    a.seed = rng->seed;
+    a.draw_offset = rng->draw_offset;
+    a.chain_offset = rng->chain_offset;
+    a.rng_mode = rng->mode;
+    a.n_uniform = rng->n_uniform;
+    return a;
+}
 
 template <typename T>
 void fill_sep(SepArgs<T>& a, const Model& m, void* theta, int64_t C, const void* metric, int64_t n,
@@ -96,6 +120,14 @@ int hmc_t(const Model& m, void* theta, void* lp, void* grad, int32_t* valid, int
         a.L = L;
         return launch_sep_sampler<T>(a, st);
     }
+    if (use_user_fused(m)) {
+        UserRunArgs a = user_args(m, theta, C, n, rng, out);
+        a.metric = metric;
+        a.eps = eps;
+        a.half_eps = 0.5 * eps;
+        a.L = L;
+        return user_fused_sample(m, ALGO_HMC, a, valid, st);
+    }
     BK_CHECK_ARG(lp && grad, "bk_hmc_diag_sample: lp_cache/grad_cache are required for this model");
     if constexpr (sizeof(T) == 4) {
         // tensor-core pipeline: L-1 fused bf16 steps + one split-precision endpoint gradient
@@ -124,6 +156,13 @@ int mala_t(const Model& m, void* theta, void* lp, void* grad, int32_t* valid, in
         a.sd = (T)sd;
         a.coef = (T)coef;
         return launch_sep_sampler<T>(a, st);
+    }
+    if (use_user_fused(m)) {
+        UserRunArgs a = user_args(m, theta, C, n, rng, out);
+        a.eps = eps;
+        a.sd = sd;
+        a.coef = coef;
+        return user_fused_sample(m, ALGO_MALA, a, valid, st);
     }
     BK_CHECK_ARG(lp && grad, "bk_mala_sample: lp_cache/grad_cache are required for this model");
     if constexpr (sizeof(T) == 4) {
@@ -154,6 +193,13 @@ int mh_t(const Model& m, void* theta, void* lp, int32_t* valid, int64_t C, doubl
         a.hastings = hastings;
         return launch_sep_sampler<T>(a, st);
     }
+    if (use_user_fused(m)) {
+        UserRunArgs a = user_args(m, theta, C, n, rng, out);
+        a.scale = scale;
+        a.s2 = scale * scale;
+        a.hastings = hastings;
+        return user_fused_sample(m, ALGO_MHRW, a, valid, st);
+    }
     BK_CHECK_ARG(lp, "bk_mh_rw_sample: lp_cache is required for this model");
     GenArgs<T> p;
     fill_gen(p, m, theta, lp, nullptr, C, nullptr, n, rng, out);
@@ -167,6 +213,7 @@ size_t sampler_ws(uint64_t h, int64_t C) {
     const Model* m = get_model(h);
     if (!m || C <= 0) return 0;
     if (m->separable() && m->d.dims <= SEP_MAX_D && !force_generic()) return 0;
+    if (use_user_fused(*m)) return 0;
     if (dense_tc_enabled(*m)) {
         size_t a = dense_tc_hmc_ws_bytes(*m, C), b = generic_ws_bytes<float>(*m, C);
         return a > b ? a : b;

@@ -27,6 +27,14 @@ const Model* get_model(uint64_t h) {
     return &it->second;
 }
 
+int register_model(const Model& m, uint64_t* handle_out) {
+    std::lock_guard<std::mutex> lk(g_mu);
+    uint64_t h = g_next++;
+    g_models[h] = m;
+    *handle_out = h;
+    return BK_OK;
+}
+
 // ---- elementwise models: one warp per chain --------------------------------
 // kind ISO / DIAG / GAUSS_PRIOR_LIK (as a density: lik + prior)
 template <typename T>
@@ -255,6 +263,8 @@ static int eval_t(const Model& m, const T* theta, int64_t C, T* lp, T* grad, voi
             BK_LAUNCH_CHECK();
             return BK_OK;
         }
+        case BK_MODEL_USER_CUDA:
+            return user_eval(m, theta, C, lp, grad, ws, ws_bytes, st);
         default:
             set_error("model kind %d has no device evaluator", m.d.kind);
             return BK_E_UNSUPPORTED;
@@ -270,6 +280,8 @@ size_t model_eval_ws_bytes(const Model& m, int64_t C) {
         if (dense_tc_enabled(m)) n += 2 * align_up(align_up((size_t)C, 256) * m.Dp * 2, 256) + 512;  // bf16 hi/lo
         return n;
     }
+    if (m.d.kind == BK_MODEL_USER_CUDA)   // gradient scratch of a density-only evaluation
+        return align_up((size_t)C * m.d.dims * (m.d.dtype == BK_F64 ? 8 : 4), 256) + 256;
     return 0;
 }
 
@@ -321,6 +333,9 @@ int bk_model_create(const bk_model_desc* desc, void* ws, size_t ws_bytes, void* 
             BK_CHECK_ARG(desc->scalars[0] > 0 && desc->scalars[1] > 0, "BINOMIAL_LOGIT: alpha, beta must be > 0");
             BK_CHECK_ARG(desc->scalars[3] >= desc->scalars[2] && desc->scalars[2] >= 0, "BINOMIAL_LOGIT: need 0 <= x <= N");
             break;
+        case BK_MODEL_USER_CUDA:
+            set_error("bk_model_create: USER_CUDA models are created by bk_model_create_cuda");
+            return BK_E_INVALID;
         default:
             set_error("bk_model_create: unknown kind %d", desc->kind);
             return BK_E_INVALID;
@@ -336,11 +351,7 @@ int bk_model_create(const bk_model_desc* desc, void* ws, size_t ws_bytes, void* 
         int rc = hlr_tc_prepare(m, ws, ws_bytes, (cudaStream_t)stream);
         if (rc) return rc;
     }
-    std::lock_guard<std::mutex> lk(g_mu);
-    uint64_t h = g_next++;
-    g_models[h] = m;
-    *handle_out = h;
-    return BK_OK;
+    return register_model(m, handle_out);
 }
 
 int bk_model_destroy(uint64_t handle) {

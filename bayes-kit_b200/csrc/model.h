@@ -17,6 +17,8 @@ struct Model {
     __nv_bfloat16* Xlo = nullptr;   // [Np, 128] bf16(X - Xb): split-precision logits
     float* yp = nullptr;            // [Np] responses, zero padded
     float* yh = nullptr;            // [Np] responses - 1/2 (0 on padded rows)
+    const struct UserLib* user = nullptr;   // USER_CUDA: the runtime-compiled kernels (user_model.cu)
+    const void* user_params = nullptr;      // USER_CUDA: [n_params] caller array, dtype
     bool separable() const {
         return d.kind == BK_MODEL_ISO_GAUSS || d.kind == BK_MODEL_DIAG_GAUSS;
     }
@@ -24,6 +26,21 @@ struct Model {
 
 // returns nullptr (and sets the error) for an unknown handle
 const Model* get_model(uint64_t handle);
+// adds m to the registry
+int register_model(const Model& m, uint64_t* handle_out);
+
+// user-written CUDA models (user_model.cu).  The fused register-resident samplers serve D <= USER_FUSED_MAX_D: up to
+// there both measured models gain more than 10x over the generic engine (DESIGN.md 4.4a).  Defining
+// BK_USER_FUSED_MAX_D at build time moves the threshold (scripts/time_user_model.py measures beyond it that way).
+#ifndef BK_USER_FUSED_MAX_D
+#define BK_USER_FUSED_MAX_D 32
+#endif
+constexpr int USER_FUSED_MAX_D = BK_USER_FUSED_MAX_D;
+struct UserRunArgs;
+int user_eval(const Model& m, const void* theta, int64_t C, void* lp, void* grad, void* ws, size_t ws_bytes,
+              cudaStream_t st);
+bool user_fused(const Model& m);
+int user_fused_sample(const Model& m, int algo, const UserRunArgs& a, int32_t* cache_valid, cudaStream_t st);
 
 size_t model_eval_ws_bytes(const Model& m, int64_t C);
 // true when model_eval(..., precise=false) is a genuinely cheaper (tensor-core) evaluation

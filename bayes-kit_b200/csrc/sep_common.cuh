@@ -128,12 +128,6 @@ struct Lanes {
     }
 };
 
-// log(u) with numpy semantics for u == 0 (-inf: always accepts)
-template <typename T>
-__device__ __forceinline__ T log_u(T u) {
-    return u > T(0) ? Ar<T>::log_(u) : neg_inf<T>();
-}
-
 // Per-lane view of a diagonal Gaussian (MK_ISO keeps nothing per element).
 template <typename T, int G, int J, int MK>
 struct SepGauss {

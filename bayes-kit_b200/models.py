@@ -219,11 +219,82 @@ class HierLogReg(DeviceModel):
         self._register(X=self.X, y=self.y, n_obs=Xt.shape[0])
 
 
+_NVRTC_LOADED = False
+
+
+def _load_nvrtc() -> None:
+    """Make ``libnvrtc.so.12`` loadable by soname for the library's ``dlopen``: the system copy when the
+    loader finds one, else the copy bundled with torch (nvidia-cuda-nvrtc), loaded ``RTLD_GLOBAL``."""
+    global _NVRTC_LOADED
+    if _NVRTC_LOADED:
+        return
+    try:
+        C.CDLL("libnvrtc.so.12", mode=C.RTLD_GLOBAL)
+    except OSError:
+        import glob
+        import os
+        import sys
+        for base in sys.path:
+            for cand in glob.glob(os.path.join(base, "nvidia", "cuda_nvrtc", "lib", "libnvrtc.so.12")):
+                try:
+                    C.CDLL(cand, mode=C.RTLD_GLOBAL)
+                    _NVRTC_LOADED = True
+                    return
+                except OSError:
+                    pass
+        return          # bk_model_create_cuda reports BK_E_UNSUPPORTED
+    _NVRTC_LOADED = True
+
+
+class CudaModel(DeviceModel):
+    """A model written by the user as one CUDA C++ function, compiled at run time (NVRTC) for the GPU::
+
+        __device__ bk_real log_density_gradient(const bk_real* theta, bk_real* grad, const bk_real* params);
+
+    It returns ``log p(theta)`` and writes the gradient into ``grad[0 .. BK_DIMS)``; ``bk_real`` is the model's
+    dtype and ``BK_DIMS == dims`` a compile-time constant.  Helper functions, structs and constants may precede
+    it; no header can be included (math builtins need none).  ``params``: the model's data and
+    hyper-parameters as one flat array, passed to the function on the device.
+
+    Every sampler except ``TemperedLikelihoodSMC`` accepts it.  ``HMCDiag``, ``MALA`` and the random-walk
+    ``Metropolis`` / ``MetropolisHastings`` run one fused kernel per call (one thread per chain, state in
+    registers) for ``dims <= 32``, the generic engine above.  A compile error raises ``ValueError`` with
+    NVRTC's log; ``compile_log`` holds the log of a successful compile, with the registers and spills of
+    every kernel."""
+
+    _kind = L.MODEL_USER
+
+    def __init__(self, source: str, dims: int, params=None, dtype=torch.float32, device="cuda"):
+        if not isinstance(source, str):
+            raise TypeError("source must be a str of CUDA C++")
+        if isinstance(dims, bool) or not isinstance(dims, (int, np.integer)):
+            raise TypeError(f"dims must be an int, not {type(dims)}")
+        super().__init__(dims, dtype, device)
+        self.source = source
+        self.params = None
+        if params is not None:
+            self.params = to_dev(params, dtype, self.device).reshape(-1)
+            if self.params.numel() == 0:
+                self.params = None
+        n_params = 0 if self.params is None else self.params.numel()
+        _load_nvrtc()
+        log = C.create_string_buffer(1 << 20)
+        h = L.u64(0)
+        with torch.cuda.device(self.device):
+            rc = L.lib().bk_model_create_cuda(source.encode(), self._dims, dtype_id(dtype), ptr(self.params),
+                                              n_params, C.byref(h), log, len(log))
+        self.compile_log = log.value.decode(errors="replace")
+        if rc == L.BK_E_INVALID and self.compile_log:
+            raise ValueError(f"CudaModel: NVRTC compilation failed:\n{self.compile_log}")
+        L.check(rc)
+        self._handle = h.value
+
+
 def require_plugin(model) -> DeviceModel:
     if not isinstance(model, DeviceModel):
         raise TypeError(
             "bayes_kit_b200 samplers evaluate the model inside CUDA kernels: `model` must be a "
             "registered device plugin (bayes_kit_b200.models.IsoGauss / DiagGauss / DensePrecGauss / "
-            "HierLogReg / GaussPriorLik / Binomial), not an arbitrary Python object. Python callbacks cannot "
+            "HierLogReg / GaussPriorLik / Binomial, or your own CUDA source as CudaModel), not an arbitrary Python object. Python callbacks cannot "
             f"run per step on the device and there is no CPU fallback (got {type(model).__name__}).")
     return model

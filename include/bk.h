@@ -16,7 +16,8 @@
  *   - the CALLER owns every buffer.  All pointers are DEVICE pointers unless
  *     a name ends in _host.  The library never frees caller memory and
  *     allocates no device memory: scratch is passed in (`ws`, sized by the
- *     matching *_workspace_bytes()).
+ *     matching *_workspace_bytes()).  One exception: bk_model_create_cuda loads
+ *     the module it compiles (kept for the life of the process).
  *   - all work is enqueued asynchronously on `stream`; no hidden syncs.
  *   - tensors are dense row-major: theta [C, D], draws [n, C, D].
  *   - `dtype`: BK_F32 (timed mode) or BK_F64 (parity mode: separate
@@ -53,9 +54,10 @@ enum { BK_MODEL_ISO_GAUSS = 0,        /* -0.5 |theta|^2 / sigma^2               
        BK_MODEL_DENSE_PREC_GAUSS = 2, /* -0.5 (theta-mu)^T P (theta-mu)                    */
        BK_MODEL_HIER_LOGREG = 3,      /* hierarchical logistic regression (DESIGN.md)      */
        BK_MODEL_GAUSS_PRIOR_LIK = 4,  /* prior N(m0, 1/p0) x likelihood N(mu, 1/pl) (SMC)  */
-       BK_MODEL_BINOMIAL_LOGIT = 5    /* beta-binomial on the logit scale, D = 1: the reference's own
+       BK_MODEL_BINOMIAL_LOGIT = 5,   /* beta-binomial on the logit scale, D = 1: the reference's own
                                          test target (test/models/binomial.py:11-74), with
-                                         log_prior / log_likelihood for the SMC                */ };
+                                         log_prior / log_likelihood for the SMC                */
+       BK_MODEL_USER_CUDA = 6         /* user-written CUDA source, bk_model_create_cuda        */ };
 
 enum { BK_RNG_PHILOX = 0,   /* device Philox4x32-10, counter = (block, tag, chain, draw) */
        BK_RNG_INJECTED = 1  /* pre-drawn streams in the reference's consumption order */ };
@@ -151,6 +153,32 @@ BK_API int bk_model_log_density_gradient_fast(uint64_t handle, const void* theta
 /* log_prior / log_likelihood (smc.py:29-33): GAUSS_PRIOR_LIK, BINOMIAL_LOGIT */
 BK_API int bk_model_log_prior_likelihood(uint64_t handle, const void* theta, int64_t C,
                                   void* log_prior_out, void* log_lik_out, void* stream);
+
+/* User-written model (BK_MODEL_USER_CUDA): any log density the caller can write as one CUDA C++ function
+ *
+ *     __device__ bk_real log_density_gradient(const bk_real* theta, bk_real* grad, const bk_real* params);
+ *
+ * returning log p(theta) and writing d log p / d theta into grad[0 .. BK_DIMS).  bk_real is float (BK_F32) or
+ * double (BK_F64), BK_DIMS the model's dimension as a compile-time constant; helper functions, structs and
+ * constants may precede it in `source`.  No header can be included: math builtins (exp, log1p, lgamma, ...)
+ * are available without one.  `params` [n_params] (device, dtype; NULL exactly when n_params == 0) holds the
+ * model's data and hyper-parameters and must outlive the handle.
+ *
+ * The source is compiled at run time by NVRTC (libnvrtc.so.12, loaded on first use) for sm_100a with
+ * -std=c++17, plus --fmad=false in fp64 (the parity mode forbids contraction).  Compiled modules are cached for
+ * the life of the process by (source, dims, dtype) and never unloaded.  The handle works everywhere a model
+ * handle does except the SMC (no log_prior / log_likelihood split): HMCDiag, MALA and RW-Metropolis run one
+ * fused register-resident kernel per call for dims <= 32 (one thread per chain; otherwise the generic
+ * engine), DrGhmcDiag and the Stretcher run their generic engines.  The fused kernels draw the same Philox
+ * words as every other engine and leave *cache_valid_host = 0.
+ *
+ * log_out [log_bytes] (may be NULL) receives NVRTC's log, truncated and NUL terminated; it includes ptxas's
+ * register / spill report of every kernel.  Returns BK_E_INVALID on a bad argument or a compile error (the
+ * first line of the log goes to bk_last_error), BK_E_UNSUPPORTED when NVRTC cannot be loaded, BK_E_CUDA when
+ * the compiled module cannot be loaded (e.g. no device).  Arguments are checked before any device call. */
+#define BK_USER_MAX_DIMS 65536
+BK_API int bk_model_create_cuda(const char* source, int64_t dims, int32_t dtype, const void* params,
+                                int64_t n_params, uint64_t* handle_out, char* log_out, size_t log_bytes);
 
 /* Initial states theta0 ~ N(0, I) (hmc.py:24-28, mala.py:26-30, metropolis.py:94-98; DrGhmcDiag's rho0,
  * drghmc.py:77): out [C, D] filled with device-Philox standard normals keyed by the GLOBAL chain id
