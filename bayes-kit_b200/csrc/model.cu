@@ -393,9 +393,12 @@ int bk_model_log_prior_likelihood(uint64_t handle, const void* theta, int64_t C,
                                   void* log_prior_out, void* log_lik_out, void* stream) {
     const Model* m = get_model(handle);
     if (!m) return BK_E_HANDLE;
-    BK_CHECK_ARG(m->d.kind == BK_MODEL_GAUSS_PRIOR_LIK || m->d.kind == BK_MODEL_BINOMIAL_LOGIT,
-                 "log_prior/log_likelihood need a GAUSS_PRIOR_LIK or BINOMIAL_LOGIT model");
+    BK_CHECK_ARG(m->d.kind == BK_MODEL_GAUSS_PRIOR_LIK || m->d.kind == BK_MODEL_BINOMIAL_LOGIT || user_prior_lik(*m),
+                 "log_prior/log_likelihood need a GAUSS_PRIOR_LIK or BINOMIAL_LOGIT model, or a user model created by "
+                 "bk_model_create_cuda_prior_lik");
     if (C == 0) return BK_OK;
+    if (m->d.kind == BK_MODEL_USER_CUDA)
+        return user_log_prior_likelihood(*m, theta, C, log_prior_out, log_lik_out, (cudaStream_t)stream);
     const int D = (int)m->d.dims;
     const unsigned blocks = (unsigned)((C * 32 + 255) / 256);
     cudaStream_t st = (cudaStream_t)stream;

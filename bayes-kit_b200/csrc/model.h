@@ -41,6 +41,12 @@ int user_eval(const Model& m, const void* theta, int64_t C, void* lp, void* grad
               cudaStream_t st);
 bool user_fused(const Model& m);
 int user_fused_sample(const Model& m, int algo, const UserRunArgs& a, int32_t* cache_valid, cudaStream_t st);
+// prior/likelihood user models (bk_model_create_cuda_prior_lik): log_prior / log_likelihood of theta [C, D] (each
+// output nullable) and TemperedLikelihoodSMC's move + weight kernel (move: BK_SMC_KERNEL_*)
+struct UserSmcArgs;
+bool user_prior_lik(const Model& m);
+int user_log_prior_likelihood(const Model& m, const void* theta, int64_t C, void* lprior, void* llik, cudaStream_t st);
+int user_smc_move(const Model& m, int move, const UserSmcArgs& a, cudaStream_t st);
 
 size_t model_eval_ws_bytes(const Model& m, int64_t C);
 // true when model_eval(..., precise=false) is a genuinely cheaper (tensor-core) evaluation

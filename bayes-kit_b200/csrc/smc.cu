@@ -10,10 +10,9 @@
 #include "model.h"
 #include "sep_common.cuh"
 #include "smc_shard.cuh"
+#include "user_kernels.cuh"
 
 namespace bk {
-
-constexpr int SMC_MAXPART = 2048;   // per-CTA partials of the move kernel's statistics epilogue
 
 enum { SMC_MODEL_GPL = 0, SMC_MODEL_BINOM = 1 };
 
@@ -371,9 +370,49 @@ static int launch_smc(const SmcArgs<T>& a, int move, cudaStream_t st) {
     return BK_E_INVALID;
 }
 
+// a prior/likelihood user model: the same arguments, as the plain fields of its runtime-compiled kernel
+template <typename T>
+static int smc_user(const Model& m, const SmcArgs<T>& a, const bk_smc_kernel& kn, cudaStream_t st) {
+    UserSmcArgs u;
+    memset(&u, 0, sizeof(u));
+    u.thetas = a.thetas;
+    u.src = a.src;
+    u.src_idx = a.src_idx;
+    u.M = a.M;
+    u.t0 = (double)a.t0;
+    u.t1 = (double)a.t1;
+    u.scale = kn.scale;
+    u.steps = kn.steps;
+    u.rng_mode = a.rng.mode;
+    u.n_uniform = a.rng.n_uniform;
+    u.seed = a.rng.seed;
+    u.draw_offset = a.rng.draw_offset;
+    u.chain_offset = a.rng.chain_offset;
+    u.normals = a.rng.normals;
+    u.uniforms = a.rng.uniforms;
+    u.logw = a.logw;
+    u.logw_prev = a.logw_prev;
+    u.accept = a.accept;
+    u.sh = a.sh;
+    for (int r = 0; r < BK_SMC_MAX_WORLD; ++r) {
+        u.src_tab[r] = a.src_tab[r];
+        u.llpr_tab[r] = a.llpr_tab[r];
+        u.mail_tab[r] = a.mail_tab[r];
+    }
+    u.llpr_out = a.llpr_out;
+    u.carry = a.carry;
+    u.epoch = a.epoch;
+    u.wait_done = a.wait_done;
+    u.maxpart = a.maxpart;
+    u.ticket = a.ticket;
+    u.params = m.user_params;
+    return user_smc_move(m, kn.kind, u, st);
+}
+
 // fills the model / geometry part of the arguments and picks the lane layout
 template <typename T>
 static int smc_dispatch(const Model& m, SmcArgs<T>& a, const bk_smc_kernel& kn, cudaStream_t st) {
+    if (m.d.kind == BK_MODEL_USER_CUDA) return smc_user<T>(m, a, kn, st);
     a.D = (int)m.d.dims;
     a.scale = (T)kn.scale;
     a.steps = kn.steps;
@@ -422,8 +461,12 @@ static int smc_dispatch(const Model& m, SmcArgs<T>& a, const bk_smc_kernel& kn, 
 }
 
 static int check_smc_model(const Model& m, const bk_smc_kernel& kn) {
-    BK_CHECK_ARG(m.d.kind == BK_MODEL_GAUSS_PRIOR_LIK || m.d.kind == BK_MODEL_BINOMIAL_LOGIT,
-                 "bk_smc_move_weight: the model must expose log_prior / log_likelihood (GAUSS_PRIOR_LIK, BINOMIAL_LOGIT)");
+    BK_CHECK_ARG(m.d.kind == BK_MODEL_GAUSS_PRIOR_LIK || m.d.kind == BK_MODEL_BINOMIAL_LOGIT || user_prior_lik(m),
+                 "bk_smc_move_weight: the model must expose log_prior / log_likelihood (GAUSS_PRIOR_LIK, BINOMIAL_LOGIT, "
+                 "or a user model created by bk_model_create_cuda_prior_lik)");
+    BK_CHECK_ARG(m.d.kind != BK_MODEL_USER_CUDA || m.d.dims <= BK_USER_PRIOR_LIK_MAX_DIMS,
+                 "bk_smc_move_weight: user models support dims <= %d (got %lld)", BK_USER_PRIOR_LIK_MAX_DIMS,
+                 (long long)m.d.dims);
     BK_CHECK_ARG(kn.kind >= BK_SMC_KERNEL_RW && kn.kind <= BK_SMC_KERNEL_HMC, "bk_smc: unknown kernel kind %d", kn.kind);
     BK_CHECK_ARG(kn.scale > 0, "bk_smc: kernel scale / step size must be positive (got %g)", kn.scale);
     BK_CHECK_ARG(kn.kind != BK_SMC_KERNEL_HMC || kn.steps >= 0, "bk_smc: HMC kernel needs steps >= 0");

@@ -10,108 +10,9 @@
 //     into the idx array of the rank that owns the slot;
 //   * the particle ROWS, read from their owner's array by the next move kernel.
 // With world == 1 the same kernels run; every wait is already satisfied by stream order.
+//
+// The device side of the protocol (geometry, mailbox layout, waits and posts) lives in smc_mailbox.cuh, which the
+// SMC kernels of runtime-compiled user models share.
 #pragma once
 #include "common.cuh"
-
-namespace bk {
-
-struct ShardGeom {
-    int32_t world, rank;   // world == 0: not a sharded call
-    int32_t extra, small;  // first `extra` ranks hold base + 1 items; small: every id fits 32 bits
-    int64_t M, base;       // global item count, floor(M / world)
-};
-
-__host__ __device__ __forceinline__ int64_t shard_lo(const ShardGeom& g, int r) {
-    return (int64_t)r * g.base + (r < g.extra ? r : g.extra);
-}
-__host__ __device__ __forceinline__ int64_t shard_n(const ShardGeom& g, int r) { return g.base + (r < g.extra ? 1 : 0); }
-
-// owner rank and local row of global id gid
-__device__ __forceinline__ void shard_locate(const ShardGeom& g, int64_t gid, int& r, int64_t& loc) {
-    const int64_t cut = (int64_t)g.extra * (g.base + 1);
-    if (g.small) {
-        const uint32_t u = (uint32_t)gid, c = (uint32_t)cut;
-        if (u < c) { const uint32_t q = u / (uint32_t)(g.base + 1); r = (int)q; loc = u - q * (uint32_t)(g.base + 1); }
-        else { const uint32_t q = (u - c) / (uint32_t)g.base; r = g.extra + (int)q; loc = (u - c) - q * (uint32_t)g.base; }
-    } else {
-        if (gid < cut) { const int64_t q = gid / (g.base + 1); r = (int)q; loc = gid - q * (g.base + 1); }
-        else { const int64_t q = (gid - cut) / g.base; r = g.extra + (int)q; loc = (gid - cut) - q * g.base; }
-    }
-}
-
-// ---- mailbox layout (64-bit words; one mailbox per rank, written by every rank) -----------------
-// word 0: error word (0 = fine; 1 = a wait timed out; 2 = all weights vanished)
-// slots are indexed [parity of the step][source rank]
-enum : int {
-    MB_ERR = 0,
-    MB_MAX = 8,                                   // {max (double bits), step}
-    MB_MASS = MB_MAX + 2 * BK_SMC_MAX_WORLD * 2,  // {W (int64), Q (double bits), n_local, step}
-    MB_DONE = MB_MASS + 2 * BK_SMC_MAX_WORLD * 4, // {step}
-    MB_WORDS = MB_DONE + 2 * BK_SMC_MAX_WORLD
-};
-static_assert(MB_WORDS * 8 <= BK_SMC_MAILBOX_BYTES, "mailbox size");
-
-__device__ __forceinline__ void st_release_sys(uint64_t* p, uint64_t v) {
-    asm volatile("st.release.sys.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
-}
-__device__ __forceinline__ void st_relaxed_sys(uint64_t* p, uint64_t v) {
-    asm volatile("st.relaxed.sys.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
-}
-__device__ __forceinline__ uint64_t ld_acquire_sys(const uint64_t* p) {
-    uint64_t v;
-    asm volatile("ld.acquire.sys.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
-    return v;
-}
-__device__ __forceinline__ uint64_t ld_relaxed_sys(const uint64_t* p) {
-    uint64_t v;
-    asm volatile("ld.relaxed.sys.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
-    return v;
-}
-__device__ __forceinline__ uint64_t ld_relaxed_gpu(const uint64_t* p) {
-    uint64_t v;
-    asm volatile("ld.relaxed.gpu.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
-    return v;
-}
-__device__ __forceinline__ void st_relaxed_gpu(uint64_t* p, uint64_t v) {
-    asm volatile("st.relaxed.gpu.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
-}
-__device__ __forceinline__ double ld_relaxed_gpu_f64(const double* p) {
-    return __longlong_as_double((long long)ld_relaxed_gpu(reinterpret_cast<const uint64_t*>(p)));
-}
-__device__ __forceinline__ uint64_t global_ns() {
-    uint64_t t;
-    asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
-    return t;
-}
-
-// Wait until the step word at `flag` (in OUR mailbox) reaches `step`.  Bounded: a rank that never
-// arrives (crashed peer) makes the wait give up after BK_SMC_WAIT_NS, flags the error word and lets the
-// kernel run to completion on garbage -- the host raises when it next looks at the mailbox.
-constexpr uint64_t BK_SMC_WAIT_NS = 20ull * 1000 * 1000 * 1000;
-__device__ __forceinline__ bool mail_wait(const uint64_t* flag, uint64_t step, uint64_t* mailbox) {
-    if (ld_acquire_sys(flag) >= step) return true;
-    if (ld_relaxed_sys(mailbox + MB_ERR) == 1ull) return false;   // a wait already timed out: the run is lost, do not wait again
-    const uint64_t t0 = global_ns();
-    unsigned it = 0;
-    while (ld_acquire_sys(flag) < step) {
-        __nanosleep(64);
-        if ((++it & 1023u) == 0 && global_ns() - t0 > BK_SMC_WAIT_NS) {
-            st_relaxed_sys(mailbox + MB_ERR, 1ull);
-            return false;
-        }
-    }
-    return true;
-}
-// post {payload, step} / {p0, p1, p2, step}: payload first, then a release store of the step number
-__device__ __forceinline__ void mail_post1(uint64_t* slot, uint64_t payload, uint64_t step) {
-    st_relaxed_sys(slot, payload);
-    st_release_sys(slot + 1, step);
-}
-__device__ __forceinline__ void mail_post3(uint64_t* slot, uint64_t p0, uint64_t p1, uint64_t p2, uint64_t step) {
-    st_relaxed_sys(slot, p0);
-    st_relaxed_sys(slot + 1, p1);
-    st_relaxed_sys(slot + 2, p2);
-    st_release_sys(slot + 3, step);
-}
-
-}  // namespace bk
+#include "smc_mailbox.cuh"

@@ -1,8 +1,14 @@
-// Kernels of a user-written CUDA model (BK_MODEL_USER_CUDA, bk.h).  The host side (user_model.cu) includes this file
-// for UserRunArgs only; the kernels are compiled at run time by NVRTC, one library per (source, D, dtype), from
-//   integer typedefs + device_rng.cuh + `typedef float|double bk_real;` + the user's source + this file
-// with -DBK_DIMS=D.  The user's source defines
+// Kernels of a user-written CUDA model (BK_MODEL_USER_CUDA, bk.h).  The host side (user_model.cu, smc.cu) includes
+// this file for the launch-argument structs only; the kernels are compiled at run time by NVRTC, one library per
+// (source, D, dtype, prior_lik), from
+//   integer typedefs + device_rng.cuh + `typedef float|double bk_real;` [+ smc_mailbox.cuh] + the user's source
+//   + this file
+// with -DBK_DIMS=D.  The user's source defines either
 //   __device__ bk_real log_density_gradient(const bk_real* theta, bk_real* grad, const bk_real* params);
+// or (bk_model_create_cuda_prior_lik: compiled with -DBK_PRIOR_LIK=1 and the shared SMC protocol header) the pair
+//   __device__ bk_real log_prior_gradient(const bk_real* theta, bk_real* grad, const bk_real* params);
+//   __device__ bk_real log_likelihood_gradient(const bk_real* theta, bk_real* grad, const bk_real* params);
+// from which this file derives log_density_gradient = likelihood + prior.
 //
 // bk_user_eval      one thread per chain on global rows: model_eval's case for this kind, through which the
 //                   generic HMC / MALA / RW-Metropolis engine, the lockstep DrGHMC engine and the Stretcher run.
@@ -12,7 +18,16 @@
 //                   (Row<T> and k_hmc_* / k_mala_* / k_mh_* in sampler_generic.cu): philox_normal4 per block of 4
 //                   elements, philox_accept_uniform at block ceil(D / 4), the same sequence of Ar<T> operations;
 //                   in fp64 only the summation order of the kinetic / proposal-energy sums differs.
+// bk_user_eval_pl   (prior/likelihood models) log_prior and log_likelihood of global rows, one thread per row.
+// bk_user_smc_rw/mala/hmc
+//                   (prior/likelihood models) TemperedLikelihoodSMC's move + importance-weight kernel, one thread
+//                   per particle: k_smc_move_weight (smc.cu) step for step with one lane per particle, on the same
+//                   Philox words, the same resample-index / peer-row / (ll, prior)-carry rules and the same mailbox
+//                   posts (smc_mailbox.cuh).
 #pragma once
+#ifndef __CUDACC_RTC__
+#include "smc_mailbox.cuh"
+#endif
 
 namespace bk {
 
@@ -36,9 +51,55 @@ struct UserRunArgs {
     double scale, s2;         // RW-Metropolis
 };
 
+#if !defined(__CUDACC_RTC__) || defined(BK_PRIOR_LIK)
+// Launch arguments of bk_user_smc_rw / _mala / _hmc: SmcArgs<T> of smc.cu with plain fields (the host (nvcc) and the
+// kernels (NVRTC) must agree on the layout).  Pointers are in the model's dtype unless typed.
+struct UserSmcArgs {
+    void* thetas;                          // [M, D] moved particles (out)
+    const void* src;                       // particles to move: row src_idx[m] (the pending resample) or row m
+    const int64_t* src_idx;                // [M] or NULL
+    int64_t M;
+    double t0, t1;                         // temperatures, already rounded to the dtype
+    double scale;                          // RW: proposal sd; MALA: epsilon; HMC: stepsize
+    int32_t steps;                         // HMC: leapfrog steps
+    int32_t rng_mode, n_uniform;           // bk_rng
+    uint64_t seed, draw_offset, chain_offset;
+    const void* normals;                   // injected [M, D]
+    const void* uniforms;                  // injected [M, n_uniform]
+    void* logw;                            // [M] out
+    const void* logw_prev;                 // [M] carried log-weights or NULL
+    int32_t* accept;                       // [M] or NULL
+    // ---- sharded particle system (smc_mailbox.cuh); sh.world == 0: plain single-array call ----
+    ShardGeom sh;                          // src_idx holds GLOBAL particle ids, row gid lives on rank owner(gid)
+    const void* src_tab[BK_SMC_MAX_WORLD];
+    const void* llpr_tab[BK_SMC_MAX_WORLD];
+    uint64_t* mail_tab[BK_SMC_MAX_WORLD];
+    void* llpr_out;                        // [M, 2] (log_likelihood, log_prior) of the moved particles, or NULL
+    int32_t carry;                         // read the parent's pair from llpr_tab instead of evaluating the model
+    uint64_t epoch, wait_done;
+    double* maxpart;                       // [gridDim.x] per-CTA maxima (NULL: no statistics epilogue)
+    unsigned* ticket;
+    const void* params;                    // [n_params] or NULL
+};
+#endif
+
 }  // namespace bk
 
 #ifdef __CUDACC_RTC__
+
+#ifdef BK_PRIOR_LIK
+// The posterior's density from the pair, in the order of the built-in GAUSS_PRIOR_LIK evaluator (k_sep_eval):
+// lp = ll + prior, grad = gll + gpr.
+__device__ __forceinline__ bk_real log_density_gradient(const bk_real* theta, bk_real* grad, const bk_real* params) {
+    using A = bk::Ar<bk_real>;
+    bk_real gpr[BK_DIMS];
+    const bk_real pr = log_prior_gradient(theta, gpr, params);
+    const bk_real ll = log_likelihood_gradient(theta, grad, params);
+#pragma unroll
+    for (int e = 0; e < BK_DIMS; ++e) grad[e] = A::add(grad[e], gpr[e]);
+    return A::add(ll, pr);
+}
+#endif
 
 namespace bk {
 namespace user {
@@ -267,4 +328,181 @@ extern "C" __global__ void __launch_bounds__(128) bk_user_mh(const bk::UserRunAr
 }
 
 #endif  // BK_DIMS <= BK_USER_FUSED_MAX_D
+
+// The prior / likelihood kernels are compiled only for models created by bk_model_create_cuda_prior_lik.
+#ifdef BK_PRIOR_LIK
+
+// theta [C, D] -> log_prior [C], log_likelihood [C] (each nullable)
+extern "C" __global__ void __launch_bounds__(128) bk_user_eval_pl(const bk_real* __restrict__ theta, long long C,
+                                                                  const bk_real* __restrict__ params,
+                                                                  bk_real* __restrict__ lprior,
+                                                                  bk_real* __restrict__ llik) {
+    const long long c = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= C) return;
+    bk_real g[BK_DIMS];
+    const bk_real* x = theta + c * BK_DIMS;
+    if (lprior) lprior[c] = log_prior_gradient(x, g, params);
+    if (llik) llik[c] = log_likelihood_gradient(x, g, params);
+}
+
+namespace bk {
+namespace user {
+
+// (ll, prior) of x and the gradient of the tempered density lp_t = ll * t + prior: g = gll * t + gpr (smc.cu's tgrad)
+__device__ __forceinline__ void tempered(const T (&x)[D], T t, const T* params, T& ll, T& pr, T (&g)[D]) {
+    T gp[D];
+    pr = log_prior_gradient(x, gp, params);
+    ll = log_likelihood_gradient(x, g, params);
+#pragma unroll
+    for (int e = 0; e < D; ++e) g[e] = A::add(A::mul(g[e], t), gp[e]);
+}
+
+// k_smc_move_weight with one lane per particle.  MOVE: BK_SMC_KERNEL_RW / _MALA / _HMC (bk.h: 0 / 1 / 2).
+template <int MOVE>
+__device__ __forceinline__ void smc_move(const UserSmcArgs& a) {
+    const T* params = reinterpret_cast<const T*>(a.params);
+    const T t0 = (T)a.t0, t1 = (T)a.t1;
+    const bool carry = a.carry != 0;
+    // sharded source: the resample indices are global particle ids; the row is read from its owner's array
+    const bool sharded = a.sh.world > 1 && a.src_idx != nullptr;
+    if (a.wait_done) {   // the indices (and the rows they point at) of the previous step are final on every rank
+        if ((int)threadIdx.x < a.sh.world)
+            mail_wait(a.mail_tab[a.sh.rank] + MB_DONE + (a.wait_done & 1) * BK_SMC_MAX_WORLD + threadIdx.x, a.wait_done,
+                      a.mail_tab[a.sh.rank]);
+        __syncthreads();
+    }
+    double lw_max = (double)neg_inf<float>();
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t m = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; m < a.M; m += stride) {
+        const int64_t gid = a.src_idx ? a.src_idx[m] : m;
+        const T* row;
+        const T* llpr;
+        if (sharded) {
+            int r;
+            int64_t loc;
+            shard_locate(a.sh, gid, r, loc);
+            row = reinterpret_cast<const T*>(a.src_tab[r]) + loc * (int64_t)D;
+            llpr = reinterpret_cast<const T*>(a.llpr_tab[r]) + 2 * loc;
+        } else {
+            row = reinterpret_cast<const T*>(a.src) + gid * (int64_t)D;
+            llpr = reinterpret_cast<const T*>(a.llpr_tab[a.sh.world > 0 ? a.sh.rank : 0]) + 2 * gid;
+        }
+        T th[D], st[D], z[D];
+        load_row(row, th);
+        // proposal normals: the words Lanes<T, G, J>::normals consumes for blocks 0 .. ceil(D / 4) - 1
+#pragma unroll
+        for (int b = 0; b < NB; ++b) {
+            T z4[4];
+            if (a.rng_mode == 1) {   // BK_RNG_INJECTED: [M, D]
+                const T* p = reinterpret_cast<const T*>(a.normals) + m * (int64_t)D;
+#pragma unroll
+                for (int i = 0; i < 4; ++i) z4[i] = (4 * b + i < D) ? p[4 * b + i] : T(0);
+            } else {
+                philox_normal4<T>(a.seed, (uint32_t)b, (uint32_t)(a.chain_offset + (uint64_t)m), (uint32_t)a.draw_offset,
+                                  z4);
+            }
+#pragma unroll
+            for (int i = 0; i < 4; ++i)
+                if (4 * b + i < D) z[4 * b + i] = z4[i];
+        }
+        const T lu = log_u(a.rng_mode == 1
+                               ? reinterpret_cast<const T*>(a.uniforms)[m * a.n_uniform]
+                               : philox_accept_uniform<T>(a.seed, (uint32_t)(a.chain_offset + (uint64_t)m),
+                                                          (uint32_t)a.draw_offset, D));
+        T ll_c, pr_c, ll_s, pr_s;
+        if (carry) { ll_c = llpr[0]; pr_c = llpr[1]; }
+        bool acc;
+        if constexpr (MOVE == 0) {   // RW (smc.py:79-89); the gradients are dead code after inlining
+            T unused[D];
+            if (!carry) tempered(th, t0, params, ll_c, pr_c, unused);
+            const T lp_c = A::add(A::mul(ll_c, t0), pr_c);
+#pragma unroll
+            for (int e = 0; e < D; ++e) st[e] = A::add(th[e], A::mul((T)a.scale, z[e]));   // smc.py:81
+            tempered(st, t0, params, ll_s, pr_s, unused);
+            const T lp_s = A::add(A::mul(ll_s, t0), pr_s);
+            acc = lu < A::sub(lp_s, lp_c);   // smc.py:85
+        } else if constexpr (MOVE == 1) {   // one MALA transition on the tempered density (mala.py:40-66)
+            const T eps = (T)a.scale, sd = A::sqrt_(A::mul(T(2), eps)), coef = T(-0.25) / eps;
+            T g[D], gs[D], ll_e, pr_e;
+            tempered(th, t0, params, ll_e, pr_e, g);
+            if (!carry) { ll_c = ll_e; pr_c = pr_e; }
+            const T lp_c = A::add(A::mul(ll_c, t0), pr_c);
+#pragma unroll
+            for (int e = 0; e < D; ++e) st[e] = A::add(A::add(th[e], A::mul(eps, g[e])), A::mul(sd, z[e]));
+            tempered(st, t0, params, ll_s, pr_s, gs);
+            const T lp_s = A::add(A::mul(ll_s, t0), pr_s);
+            T sf = T(0), sr = T(0);
+#pragma unroll
+            for (int e = 0; e < D; ++e) {
+                const T df = A::sub(A::sub(st[e], th[e]), A::mul(eps, g[e]));
+                const T dr = A::sub(A::sub(th[e], st[e]), A::mul(eps, gs[e]));
+                sf = A::add(sf, A::mul(df, df));
+                sr = A::add(sr, A::mul(dr, dr));
+            }
+            const T fwd = A::mul(coef, sf), rev = A::mul(coef, sr);
+            acc = lu < A::add(A::sub(lp_s, lp_c), A::sub(rev, fwd));   // metropolis.py:41-76
+        } else {   // one HMCDiag transition, identity metric, on the tempered density (hmc.py:40-63)
+            const T eps = (T)a.scale, heps = A::mul(T(0.5), eps);
+            T g[D];
+            tempered(th, t0, params, ll_s, pr_s, g);   // (ll_s, pr_s): the terms at st, which starts at th
+            if (!carry) { ll_c = ll_s; pr_c = pr_s; }
+            const T lp_c = A::add(A::mul(ll_c, t0), pr_c);
+            T kin = T(0);
+#pragma unroll
+            for (int e = 0; e < D; ++e) kin = A::add(kin, A::mul(z[e], z[e]));
+            const T h0 = A::sub(lp_c, A::mul(T(0.5), kin));
+#pragma unroll
+            for (int e = 0; e < D; ++e) {   // backward half kick (hmc.py:46)
+                st[e] = th[e];
+                z[e] = A::sub(z[e], A::mul(heps, g[e]));
+            }
+            for (int s = 0; s < a.steps; ++s) {   // hmc.py:47-50
+#pragma unroll
+                for (int e = 0; e < D; ++e) {
+                    z[e] = A::add(z[e], A::mul(eps, g[e]));
+                    st[e] = A::add(st[e], A::mul(eps, z[e]));
+                }
+                tempered(st, t0, params, ll_s, pr_s, g);
+            }
+            kin = T(0);
+#pragma unroll
+            for (int e = 0; e < D; ++e) {   // forward half kick (hmc.py:52)
+                z[e] = A::add(z[e], A::mul(heps, g[e]));
+                kin = A::add(kin, A::mul(z[e], z[e]));
+            }
+            const T h1 = A::sub(A::add(A::mul(ll_s, t0), pr_s), A::mul(T(0.5), kin));
+            acc = lu < A::sub(h1, h0);   // hmc.py:60
+        }
+        if (acc) {
+#pragma unroll
+            for (int e = 0; e < D; ++e) th[e] = st[e];
+            ll_c = ll_s;
+            pr_c = pr_s;
+        }
+        // importance log-weight, both tempered densities in full (smc.py:67-70)
+        const T lw = A::sub(A::add(A::mul(ll_c, t1), pr_c), A::add(A::mul(ll_c, t0), pr_c));
+        T* out = reinterpret_cast<T*>(a.thetas) + m * (int64_t)D;
+#pragma unroll
+        for (int e = 0; e < D; ++e) out[e] = th[e];
+        if (a.llpr_out) {
+            T* lo = reinterpret_cast<T*>(a.llpr_out) + 2 * m;
+            lo[0] = ll_c;
+            lo[1] = pr_c;
+        }
+        const T lw_tot = a.logw_prev ? A::add(reinterpret_cast<const T*>(a.logw_prev)[m], lw) : lw;
+        reinterpret_cast<T*>(a.logw)[m] = lw_tot;
+        lw_max = fmax(lw_max, (double)lw_tot);
+        if (a.accept) a.accept[m] = acc ? 1 : 0;
+    }
+    if (a.maxpart) smc_post_max(lw_max, a.maxpart, a.ticket, a.sh, a.mail_tab, a.epoch);
+}
+
+}  // namespace user
+}  // namespace bk
+
+extern "C" __global__ void __launch_bounds__(128) bk_user_smc_rw(const bk::UserSmcArgs a) { bk::user::smc_move<0>(a); }
+extern "C" __global__ void __launch_bounds__(128) bk_user_smc_mala(const bk::UserSmcArgs a) { bk::user::smc_move<1>(a); }
+extern "C" __global__ void __launch_bounds__(128) bk_user_smc_hmc(const bk::UserSmcArgs a) { bk::user::smc_move<2>(a); }
+
+#endif  // BK_PRIOR_LIK
 #endif  // __CUDACC_RTC__

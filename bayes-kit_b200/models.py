@@ -256,13 +256,15 @@ class CudaModel(DeviceModel):
     it; no header can be included (math builtins need none).  ``params``: the model's data and
     hyper-parameters as one flat array, passed to the function on the device.
 
-    Every sampler except ``TemperedLikelihoodSMC`` accepts it.  ``HMCDiag``, ``MALA`` and the random-walk
+    Every sampler except ``TemperedLikelihoodSMC`` accepts it; for the SMC, write the log prior and the log
+    likelihood separately as a ``CudaPriorLikModel``.  ``HMCDiag``, ``MALA`` and the random-walk
     ``Metropolis`` / ``MetropolisHastings`` run one fused kernel per call (one thread per chain, state in
     registers) for ``dims <= 32``, the generic engine above.  A compile error raises ``ValueError`` with
     NVRTC's log; ``compile_log`` holds the log of a successful compile, with the registers and spills of
     every kernel."""
 
     _kind = L.MODEL_USER
+    _create = "bk_model_create_cuda"
 
     def __init__(self, source: str, dims: int, params=None, dtype=torch.float32, device="cuda"):
         if not isinstance(source, str):
@@ -281,13 +283,34 @@ class CudaModel(DeviceModel):
         log = C.create_string_buffer(1 << 20)
         h = L.u64(0)
         with torch.cuda.device(self.device):
-            rc = L.lib().bk_model_create_cuda(source.encode(), self._dims, dtype_id(dtype), ptr(self.params),
-                                              n_params, C.byref(h), log, len(log))
+            rc = getattr(L.lib(), self._create)(source.encode(), self._dims, dtype_id(dtype), ptr(self.params),
+                                                n_params, C.byref(h), log, len(log))
         self.compile_log = log.value.decode(errors="replace")
         if rc == L.BK_E_INVALID and self.compile_log:
-            raise ValueError(f"CudaModel: NVRTC compilation failed:\n{self.compile_log}")
+            raise ValueError(f"{type(self).__name__}: NVRTC compilation failed:\n{self.compile_log}")
         L.check(rc)
         self._handle = h.value
+
+
+class CudaPriorLikModel(CudaModel):
+    """A model written by the user as a log prior and a log likelihood, compiled at run time (NVRTC), for
+    ``TemperedLikelihoodSMC`` (the reference's ``LogPriorLikelihoodModel``, typing.py:37-42)::
+
+        __device__ bk_real log_prior_gradient(const bk_real* theta, bk_real* grad, const bk_real* params);
+        __device__ bk_real log_likelihood_gradient(const bk_real* theta, bk_real* grad, const bk_real* params);
+
+    Each returns its log term and writes that term's gradient into ``grad[0 .. BK_DIMS)``; ``bk_real``,
+    ``BK_DIMS``, ``params`` and helper code are as for ``CudaModel``.  ``dims <= 256`` (the SMC's limit;
+    ``ValueError`` above).  The library derives ``log_density_gradient`` = likelihood + prior from the pair, so the
+    same object also runs on every MCMC sampler, targeting the posterior.  The SMC moves its particles with one
+    thread per particle (RW / MALA / HMC kernels, sharded or not).  ``log_prior`` / ``log_likelihood`` are batched
+    on the device like ``GaussPriorLik``'s."""
+
+    _create = "bk_model_create_cuda_prior_lik"
+
+    _pl = GaussPriorLik._pl
+    log_prior = GaussPriorLik.log_prior
+    log_likelihood = GaussPriorLik.log_likelihood
 
 
 def require_plugin(model) -> DeviceModel:
@@ -295,6 +318,6 @@ def require_plugin(model) -> DeviceModel:
         raise TypeError(
             "bayes_kit_b200 samplers evaluate the model inside CUDA kernels: `model` must be a "
             "registered device plugin (bayes_kit_b200.models.IsoGauss / DiagGauss / DensePrecGauss / "
-            "HierLogReg / GaussPriorLik / Binomial, or your own CUDA source as CudaModel), not an arbitrary Python object. Python callbacks cannot "
+            "HierLogReg / GaussPriorLik / Binomial, or your own CUDA source as CudaModel / CudaPriorLikModel), not an arbitrary Python object. Python callbacks cannot "
             f"run per step on the device and there is no CPU fallback (got {type(model).__name__}).")
     return model

@@ -11,6 +11,11 @@ three small messages per step into each other's mailboxes (local max of the
 log-weights, local weight mass, "indices final"), store the resample indices of the
 offspring they resolve straight into the owner's index array, and the next move
 reads the selected rows from their owners over NVLink peer memory (peer.py, bk.h).
+
+The model is a built-in plugin with a log_prior / log_likelihood split (GaussPriorLik,
+Binomial: lane-grouped move kernel) or the user's own CUDA source as a
+CudaPriorLikModel (runtime-compiled move kernel, one thread per particle, same
+random streams, resampling and cross-rank messages).
 """
 from __future__ import annotations
 
@@ -25,7 +30,7 @@ from . import _lib as L
 from . import dist as D_
 from . import peer as P_
 from ._util import make_rng, resolve_seed, stream_ptr, to_dev
-from .models import Binomial, GaussPriorLik, require_plugin
+from .models import Binomial, CudaPriorLikModel, GaussPriorLik, require_plugin
 
 
 class _Kernel:
@@ -83,7 +88,8 @@ def hmc_kernel(stepsize: float, steps: int) -> HMCKernel:
 class TemperedLikelihoodSMC:
     """``TemperedLikelihoodSMC(model, M, N, sample_initial, kernel)`` (smc.py:13-27).
 
-    * ``model``: a plugin with ``log_prior`` / ``log_likelihood`` (``GaussPriorLik``, ``Binomial``).
+    * ``model``: a plugin with ``log_prior`` / ``log_likelihood``: ``GaussPriorLik``, ``Binomial``, or the user's
+      own CUDA source as a ``CudaPriorLikModel`` (dims <= 256).
     * ``sample_initial``: the reference's callable ``m -> theta0[m]`` (evaluated
       once per particle on the host, as smc.py:23 does), or directly an [M, D]
       array / tensor.
@@ -103,9 +109,9 @@ class TemperedLikelihoodSMC:
     def __init__(self, model, M: int, N: int, sample_initial, kernel, *, resample: str = "multinomial",
                  ess_threshold: Optional[float] = None, seed=None, group=None):
         self._model = require_plugin(model)
-        if not isinstance(self._model, (GaussPriorLik, Binomial)):
+        if not isinstance(self._model, (GaussPriorLik, Binomial, CudaPriorLikModel)):
             raise TypeError("TemperedLikelihoodSMC needs a model plugin with log_prior/log_likelihood "
-                            "(bayes_kit_b200.models.GaussPriorLik / Binomial)")
+                            "(bayes_kit_b200.models.GaussPriorLik / Binomial / CudaPriorLikModel)")
         if not isinstance(kernel, _Kernel):
             raise TypeError("kernel must be bayes_kit_b200.metropolis_kernel(scale) (or mala_kernel / hmc_kernel): "
                             "arbitrary Python kernels cannot run per particle on the GPU and there is no CPU fallback")

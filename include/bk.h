@@ -150,7 +150,8 @@ BK_API int bk_model_log_density_gradient(uint64_t handle, const void* theta, int
 BK_API int bk_model_log_density_gradient_fast(uint64_t handle, const void* theta, int64_t C,
                                        void* lp_out, void* grad_out, void* ws, size_t ws_bytes,
                                        void* stream);
-/* log_prior / log_likelihood (smc.py:29-33): GAUSS_PRIOR_LIK, BINOMIAL_LOGIT */
+/* log_prior / log_likelihood (smc.py:29-33): GAUSS_PRIOR_LIK, BINOMIAL_LOGIT, and user models created by
+ * bk_model_create_cuda_prior_lik.  Either output may be NULL. */
 BK_API int bk_model_log_prior_likelihood(uint64_t handle, const void* theta, int64_t C,
                                   void* log_prior_out, void* log_lik_out, void* stream);
 
@@ -166,19 +167,36 @@ BK_API int bk_model_log_prior_likelihood(uint64_t handle, const void* theta, int
  *
  * The source is compiled at run time by NVRTC (libnvrtc.so.12, loaded on first use) for sm_100a with
  * -std=c++17, plus --fmad=false in fp64 (the parity mode forbids contraction).  Compiled modules are cached for
- * the life of the process by (source, dims, dtype) and never unloaded.  The handle works everywhere a model
- * handle does except the SMC (no log_prior / log_likelihood split): HMCDiag, MALA and RW-Metropolis run one
- * fused register-resident kernel per call for dims <= 32 (one thread per chain; otherwise the generic
- * engine), DrGhmcDiag and the Stretcher run their generic engines.  The fused kernels draw the same Philox
- * words as every other engine and leave *cache_valid_host = 0.
+ * the life of the process by (source, dims, dtype, prior/likelihood split) and never unloaded.  The handle works
+ * everywhere a model handle does except the SMC, which needs the split (bk_model_create_cuda_prior_lik below):
+ * HMCDiag, MALA and RW-Metropolis run one fused register-resident kernel per call for dims <= 32 (one thread per
+ * chain; otherwise the generic engine), DrGhmcDiag and the Stretcher run their generic engines.  The fused kernels
+ * draw the same Philox words as every other engine and leave *cache_valid_host = 0.
  *
  * log_out [log_bytes] (may be NULL) receives NVRTC's log, truncated and NUL terminated; it includes ptxas's
  * register / spill report of every kernel.  Returns BK_E_INVALID on a bad argument or a compile error (the
  * first line of the log goes to bk_last_error), BK_E_UNSUPPORTED when NVRTC cannot be loaded, BK_E_CUDA when
  * the compiled module cannot be loaded (e.g. no device).  Arguments are checked before any device call. */
 #define BK_USER_MAX_DIMS 65536
+#define BK_USER_PRIOR_LIK_MAX_DIMS 256   /* bk_model_create_cuda_prior_lik */
 BK_API int bk_model_create_cuda(const char* source, int64_t dims, int32_t dtype, const void* params,
                                 int64_t n_params, uint64_t* handle_out, char* log_out, size_t log_bytes);
+
+/* User-written model with a log_prior / log_likelihood split, for TemperedLikelihoodSMC: `source` defines the pair
+ *
+ *     __device__ bk_real log_prior_gradient(const bk_real* theta, bk_real* grad, const bk_real* params);
+ *     __device__ bk_real log_likelihood_gradient(const bk_real* theta, bk_real* grad, const bk_real* params);
+ *
+ * each returning its log term and writing that term's gradient into grad[0 .. BK_DIMS).  The library derives
+ * log_density_gradient = likelihood + prior (gradients likewise) after the source, so the handle (kind
+ * BK_MODEL_USER_CUDA) also works everywhere a bk_model_create_cuda handle does.  In addition
+ * bk_model_log_prior_likelihood accepts it, and the SMC entry points (bk_smc_move_weight, bk_smc_shard_move / _run,
+ * ...) move its particles with one thread per particle: the same Philox words, resample indices, peer row reads and
+ * mailbox messages as the built-in plugins, RW / MALA / HMC moves alike.  Same arguments, checks, log and return codes
+ * as bk_model_create_cuda, with dims <= BK_USER_PRIOR_LIK_MAX_DIMS (the SMC's limit; each thread keeps a few
+ * dims-element arrays). */
+BK_API int bk_model_create_cuda_prior_lik(const char* source, int64_t dims, int32_t dtype, const void* params,
+                                          int64_t n_params, uint64_t* handle_out, char* log_out, size_t log_bytes);
 
 /* Initial states theta0 ~ N(0, I) (hmc.py:24-28, mala.py:26-30, metropolis.py:94-98; DrGhmcDiag's rho0,
  * drghmc.py:77): out [C, D] filled with device-Philox standard normals keyed by the GLOBAL chain id
