@@ -27,7 +27,7 @@ def _as_metric(metric, dim):
 # --------------------------------------------------------------------------
 # HMCDiag  -- bayes_kit/hmc.py
 # --------------------------------------------------------------------------
-def hmc_diag(model, theta0, normals, uniforms, stepsize, steps, metric=None):
+def hmc_diag(model, theta0, normals, uniforms, stepsize, steps, metric=None, with_ratio=False):
     """n draws of diagonal-metric HMC for one chain.
 
     Follows ``HMCDiag.sample`` (hmc.py:55-63), ``joint_logp`` (hmc.py:36-38)
@@ -36,11 +36,13 @@ def hmc_diag(model, theta0, normals, uniforms, stepsize, steps, metric=None):
     ``log(u) < H1 - H0`` (strict); returns the *joint* log density.
 
     normals: [n, D] momentum draws; uniforms: [n] accept uniforms.
-    Returns (draws [n, D], logp [n], accepted [n] bool).
+    Returns (draws [n, D], logp [n], accepted [n] bool), and with ``with_ratio``
+    the log acceptance ratio H1 - H0 [n] the accept test compared ``log(u)`` with.
     """
     theta = np.array(theta0, dtype=np.float64, copy=True)
     n, dim = normals.shape
     m = _as_metric(metric, dim)
+    ratio = np.empty(n)
     half = 0.5 * stepsize
     draws = np.empty((n, dim))
     logps = np.empty(n)
@@ -59,6 +61,7 @@ def hmc_diag(model, theta0, normals, uniforms, stepsize, steps, metric=None):
             g = np.asarray(g)
         r = r + half * (m * g)
         h1 = model.log_density(q) - 0.5 * np.dot(r, m * r)
+        ratio[t] = h1 - h0
         if _log_u(uniforms[t]) < h1 - h0:
             theta = q
             logps[t] = h1
@@ -66,19 +69,20 @@ def hmc_diag(model, theta0, normals, uniforms, stepsize, steps, metric=None):
         else:
             logps[t] = h0
         draws[t] = theta
-    return draws, logps, acc
+    return (draws, logps, acc, ratio) if with_ratio else (draws, logps, acc)
 
 
 # --------------------------------------------------------------------------
 # MALA  -- bayes_kit/mala.py
 # --------------------------------------------------------------------------
-def mala(model, theta0, normals, uniforms, epsilon):
+def mala(model, theta0, normals, uniforms, epsilon, with_ratio=False):
     """n MALA draws for one chain.
 
     Follows ``MALA.sample`` (mala.py:40-66) with the cached (lp, grad) of the
     current point (mala.py:31-32, 62-64), the proposal density
     ``q(a|b) = -(1/4eps) |a - b - eps grad_b|^2`` (mala.py:68-79) and the
-    Metropolis-Hastings test of metropolis.py:41-76.
+    Metropolis-Hastings test of metropolis.py:41-76.  ``with_ratio``: also
+    return the log acceptance ratio [n] (as hmc_diag).
     """
     theta = np.array(theta0, dtype=np.float64, copy=True)
     n, dim = normals.shape
@@ -86,6 +90,7 @@ def mala(model, theta0, normals, uniforms, epsilon):
     g = np.asarray(g)
     sd = np.sqrt(2 * epsilon)
     coef = -0.25 / epsilon
+    ratio = np.empty(n)
     draws = np.empty((n, dim))
     logps = np.empty(n)
     acc = np.zeros(n, dtype=bool)
@@ -98,12 +103,13 @@ def mala(model, theta0, normals, uniforms, epsilon):
         fwd = coef * d_f.dot(d_f)
         rev = coef * d_r.dot(d_r)
         log_ratio = (lp_p - lp) + (rev - fwd)
+        ratio[t] = log_ratio
         if _log_u(uniforms[t]) < log_ratio:
             theta, lp, g = prop, lp_p, g_p
             acc[t] = True
         draws[t] = theta
         logps[t] = lp
-    return draws, logps, acc
+    return (draws, logps, acc, ratio) if with_ratio else (draws, logps, acc)
 
 
 def _log_u(u):
@@ -115,18 +121,20 @@ def _log_u(u):
 # Metropolis / MetropolisHastings with a Gaussian random-walk proposal
 # -- bayes_kit/metropolis.py
 # --------------------------------------------------------------------------
-def metropolis_rw(model, theta0, normals, uniforms, scale, hastings=False):
+def metropolis_rw(model, theta0, normals, uniforms, scale, hastings=False, with_ratio=False):
     """Random-walk Metropolis: proposal ``theta + scale * z``.
 
     Follows ``MetropolisHastings.sample/_propose/_accept_test``
     (metropolis.py:107-135) with ``proposal_fn = normal(loc=theta, scale)`` and
     the accept rules of metropolis.py:12-38 / 41-76.  With ``hastings=True`` the
     (exactly cancelling) symmetric transition terms are included, as
-    ``MetropolisHastings`` would compute them.
+    ``MetropolisHastings`` would compute them.  ``with_ratio``: also return the
+    log acceptance ratio [n] (as hmc_diag).
     """
     theta = np.array(theta0, dtype=np.float64, copy=True)
     n, dim = normals.shape
     lp = model.log_density(theta)
+    ratios = np.empty(n)
     draws = np.empty((n, dim))
     logps = np.empty(n)
     acc = np.zeros(n, dtype=bool)
@@ -140,12 +148,13 @@ def metropolis_rw(model, theta0, normals, uniforms, scale, hastings=False):
             d2 = theta - prop
             rev = -0.5 * np.dot(d2, d2) / (scale * scale)
             ratio = ratio + (rev - fwd)
+        ratios[t] = ratio
         if _log_u(uniforms[t]) < ratio:
             theta, lp = prop, lp_p
             acc[t] = True
         draws[t] = theta
         logps[t] = lp
-    return draws, logps, acc
+    return (draws, logps, acc, ratios) if with_ratio else (draws, logps, acc)
 
 
 # --------------------------------------------------------------------------
@@ -377,30 +386,28 @@ def smc_tempered(model, thetas0, prop_normals, acc_uniforms, res_uniforms,
 # --------------------------------------------------------------------------
 # batch helpers (leading chain axis)
 # --------------------------------------------------------------------------
-def hmc_diag_batch(model, theta0, normals, uniforms, stepsize, steps, metric=None):
+def _stack_chains(out):
+    return tuple(np.stack([o[i] for o in out], 1) for i in range(len(out[0])))
+
+
+def hmc_diag_batch(model, theta0, normals, uniforms, stepsize, steps, metric=None, with_ratio=False):
     """theta0 [C, D], normals [n, C, D], uniforms [n, C] ->
-    draws [n, C, D], logp [n, C], acc [n, C]."""
+    draws [n, C, D], logp [n, C], acc [n, C] (, log ratio [n, C])."""
     C = theta0.shape[0]
-    out = [hmc_diag(model, theta0[c], normals[:, c], uniforms[:, c], stepsize,
-                    steps, metric) for c in range(C)]
-    return (np.stack([o[0] for o in out], 1), np.stack([o[1] for o in out], 1),
-            np.stack([o[2] for o in out], 1))
+    return _stack_chains([hmc_diag(model, theta0[c], normals[:, c], uniforms[:, c], stepsize,
+                                   steps, metric, with_ratio) for c in range(C)])
 
 
-def mala_batch(model, theta0, normals, uniforms, epsilon):
+def mala_batch(model, theta0, normals, uniforms, epsilon, with_ratio=False):
     C = theta0.shape[0]
-    out = [mala(model, theta0[c], normals[:, c], uniforms[:, c], epsilon)
-           for c in range(C)]
-    return (np.stack([o[0] for o in out], 1), np.stack([o[1] for o in out], 1),
-            np.stack([o[2] for o in out], 1))
+    return _stack_chains([mala(model, theta0[c], normals[:, c], uniforms[:, c], epsilon, with_ratio)
+                          for c in range(C)])
 
 
-def metropolis_rw_batch(model, theta0, normals, uniforms, scale, hastings=False):
+def metropolis_rw_batch(model, theta0, normals, uniforms, scale, hastings=False, with_ratio=False):
     C = theta0.shape[0]
-    out = [metropolis_rw(model, theta0[c], normals[:, c], uniforms[:, c], scale,
-                         hastings) for c in range(C)]
-    return (np.stack([o[0] for o in out], 1), np.stack([o[1] for o in out], 1),
-            np.stack([o[2] for o in out], 1))
+    return _stack_chains([metropolis_rw(model, theta0[c], normals[:, c], uniforms[:, c], scale,
+                                        hastings, with_ratio) for c in range(C)])
 
 
 def drghmc_batch(model, theta0, rho0, normals, uniforms, max_proposals,
