@@ -15,7 +15,7 @@ from .ess import ess, ess_imse, ess_ipse
 from .hmc import HMCDiag
 from .iat import iat, iat_imse, iat_ipse
 from .mala import MALA
-from .metropolis import (GaussianRW, Metropolis, MetropolisHastings, metropolis_accept_test,
+from .metropolis import (CudaProposal, GaussianRW, Metropolis, MetropolisHastings, metropolis_accept_test,
                          metropolis_hastings_accept_test)
 from .models import Binomial, CudaModel, CudaPriorLikModel, DensePrecGauss, DiagGauss, GaussPriorLik, HierLogReg, IsoGauss, StdNormal
 from .rhat import (chain_moments, rank_chains, rank_normalize_chains, rank_normalized_rhat, rhat,
@@ -27,6 +27,7 @@ __all__ = [
     "Stretcher", "ess", "ess_imse", "ess_ipse", "iat", "iat_imse", "iat_ipse", "rhat", "autocorr",
     # device-side additions
     "GaussianRW", "metropolis_kernel", "mala_kernel", "hmc_kernel", "models", "dist", "peer", "Binomial", "IsoGauss", "StdNormal", "DiagGauss", "CudaModel", "CudaPriorLikModel",
+    "CudaProposal",
     "DensePrecGauss", "GaussPriorLik", "HierLogReg", "chain_moments",
     # rhat.py's split / rank-normalised family (not re-exported by the reference's __init__)
     "split_chains", "split_rhat", "rank_chains", "rank_normalize_chains", "rank_normalized_rhat",

@@ -78,6 +78,13 @@ _SIGNATURES = {
     "bk_model_log_prior_likelihood": (C.c_int, [u64, vp, i64, vp, vp, vp]),
     "bk_model_create_cuda": (C.c_int, [C.c_char_p, i64, i32, vp, i64, C.POINTER(u64), C.c_char_p, sz]),
     "bk_model_create_cuda_prior_lik": (C.c_int, [C.c_char_p, i64, i32, vp, i64, C.POINTER(u64), C.c_char_p, sz]),
+    "bk_proposal_create_cuda": (C.c_int, [C.c_char_p, i64, i32, vp, i64, i32, i32, i32, C.POINTER(u64), C.c_char_p,
+                                          sz]),
+    "bk_proposal_destroy": (C.c_int, [u64]),
+    "bk_mh_cuda_workspace_bytes": (sz, [u64, u64, i64]),
+    "bk_mh_cuda_prepare": (C.c_int, [u64, u64, C.c_char_p, sz]),
+    "bk_mh_cuda_sample": (C.c_int, [u64, u64, vp, vp, C.POINTER(i32), i64, i32, i64, C.POINTER(Rng), C.POINTER(DrawOut),
+                                    vp, sz, vp]),
     "bk_init_normal": (C.c_int, [vp, i64, i64, i32, u64, u64, C.c_uint32, vp]),
     "bk_hmc_diag_workspace_bytes": (sz, [u64, i64]),
     "bk_hmc_diag_sample": (C.c_int, [u64, vp, vp, vp, C.POINTER(i32), i64, f64, i32, vp, i64,

@@ -33,6 +33,7 @@ class ChainSampler:
     def __init__(self, model, init, seed, chains: Optional[int], chain_offset: int = 0):
         self._model = require_plugin(model)
         self._dim = self._model.dims()
+        self._n_normal = self._dim   # injected normals per (draw, chain)
         self.device, self.dtype = self._model.device, self._model.dtype
         self._seed = resolve_seed(seed)
         self._chain_offset = int(chain_offset)
@@ -127,7 +128,7 @@ class ChainSampler:
         logp = torch.empty(n, C_, dtype=self.dtype, device=self.device)
         acc = torch.empty(n, C_, dtype=torch.int32, device=self.device)
         if normals is not None:
-            normals = to_dev(normals, self.dtype, self.device).reshape(n, C_, D)
+            normals = to_dev(normals, self.dtype, self.device).reshape(n, C_, self._n_normal)
             uniforms = to_dev(uniforms, self.dtype, self.device).reshape(n, C_, self._n_uniform)
         rng = make_rng(self._seed, self._t, self._chain_offset, normals, uniforms, self._n_uniform)
         out = L.DrawOut(ptr(draws), logp.data_ptr(), acc.data_ptr())

@@ -209,6 +209,83 @@ int mh_t(const Model& m, void* theta, void* lp, int32_t* valid, int64_t C, doubl
     return run_generic<T>(m, p, ALGO_MHRW, valid, ws, wsb, st);
 }
 
+// ---- Metropolis / MetropolisHastings with a user proposal (bk_mh_cuda_*) ---------------------------------------------
+// fused: one bk_user_mhp launch per call (user model, dims and n_normals <= USER_FUSED_MAX_D); otherwise the generic
+// engine's ALGO_MHRW loop with bk_user_propose in place of k_mh_propose and its Hastings term in GenArgs::dh
+bool use_mhp_fused(const Model& m, const UserProposal& p) { return user_mhp_fusable(m, p) && !force_generic(); }
+
+// workspace of the three-launch path: [dh [C] | z, u scratch | generic engine]
+size_t proposal_scratch_bytes(const Model& m, const UserProposal& p, int64_t C) {
+    return align_up((size_t)C * (m.d.dtype == BK_F64 ? 8 : 4), 256) + user_propose_ws_bytes(p, C);
+}
+
+size_t mh_cuda_ws(const Model& m, const UserProposal& p, int64_t C) {
+    if (C <= 0 || use_mhp_fused(m, p)) return 0;
+    return proposal_scratch_bytes(m, p, C) +
+           (m.d.dtype == BK_F64 ? generic_ws_bytes<double>(m, C) : generic_ws_bytes<float>(m, C));
+}
+
+struct ProposeCtx {
+    const UserProposal* p;
+    UserProposeArgs a;   // everything but theta, q, dh and t
+};
+
+int propose_hook(const void* ctx, const void* theta, void* q, void* dh, int64_t t, cudaStream_t st) {
+    const ProposeCtx* h = static_cast<const ProposeCtx*>(ctx);
+    UserProposeArgs a = h->a;
+    a.theta = theta;
+    a.q = q;
+    a.dh = dh;
+    a.t = t;
+    return user_propose(*h->p, a, st);
+}
+
+template <typename T>
+int mh_cuda_t(const Model& m, const UserProposal& pr, void* theta, void* lp, int32_t* valid, int64_t C, int hastings,
+              int64_t n, const bk_rng* rng, const bk_draw_out& out, void* ws, size_t wsb, cudaStream_t st) {
+    // Philox mode: the accept uniform is the single-uniform samplers' rule (philox_accept_uniform), which Row<T> and
+    // user::accept_uniform apply only when n_uniform == 1; the proposal's own uniforms are TAG_UNIFORM words 0, 1, ...
+    bk_rng r = *rng;
+    if (r.mode == BK_RNG_PHILOX) r.n_uniform = 1;
+    if (use_mhp_fused(m, pr)) {
+        UserRunArgs a = user_args(m, theta, C, n, &r, out);
+        a.hastings = hastings;
+        a.prop_params = pr.params;
+        return user_mhp_sample(m, pr, a, valid, st);
+    }
+    BK_CHECK_ARG(lp, "bk_mh_cuda_sample: lp_cache is required for this model");
+    Arena ar(ws, wsb);
+    T* dh = ar.take<T>(C);
+    void* zbuf = ar.take<T>((size_t)C * pr.n_normals);
+    void* ubuf = ar.take<T>((size_t)C * pr.n_uniforms);
+    ar.off = align_up(ar.off, 256);
+    const size_t gbytes = generic_ws_bytes<T>(m, C);
+    if (!ar.ok() || wsb - ar.off < gbytes) {
+        set_error("bk_mh_cuda_sample: workspace too small: need %zu bytes, got %zu", mh_cuda_ws(m, pr, C), wsb);
+        return BK_E_WORKSPACE;
+    }
+    ProposeCtx ctx;
+    memset(&ctx.a, 0, sizeof(ctx.a));
+    ctx.p = &pr;
+    ctx.a.params = pr.params;
+    ctx.a.normals = r.normals;
+    ctx.a.uniforms = r.uniforms;
+    ctx.a.zbuf = zbuf;
+    ctx.a.ubuf = ubuf;
+    ctx.a.C = C;
+    ctx.a.seed = r.seed;
+    ctx.a.draw_offset = r.draw_offset;
+    ctx.a.chain_offset = r.chain_offset;
+    ctx.a.rng_mode = r.mode;
+    ctx.a.n_uniform = r.n_uniform;
+    const MhProposeHook hook{propose_hook, &ctx};
+    GenArgs<T> p;
+    fill_gen(p, m, theta, lp, nullptr, C, nullptr, n, &r, out);
+    p.hastings = hastings;
+    p.dh = hastings ? dh : nullptr;
+    return run_generic<T>(m, p, ALGO_MHRW, valid, ar.base + ar.off, wsb - ar.off, st, &hook);
+}
+
 size_t sampler_ws(uint64_t h, int64_t C) {
     const Model* m = get_model(h);
     if (!m || C <= 0) return 0;
@@ -226,17 +303,25 @@ size_t sampler_ws(uint64_t h, int64_t C) {
 // fused_extras: true when this call's engine handles bk_draw_out's extras itself.
 bool fused_extras(const Model& m) { return m.d.dtype == BK_F32 && use_fused<float>(m); }
 
-int check_extras(const Model& m, const bk_draw_out& o, const char* who) {
-    if (fused_extras(m)) return BK_OK;
+// the extras of an engine that writes [n, C, D] draws and folds the moments from them (check_folded / fold_extras)
+int check_folded(const bk_draw_out& o, const char* who) {
     BK_CHECK_ARG(o.layout == BK_DRAWS_NCD || !o.draws,
                  "%s: the series-major draw layout is written by the fused fp32 separable samplers only", who);
     BK_CHECK_ARG(!o.mom_mean || o.draws, "%s: streaming moments on this engine fold the stored draws -- pass draws", who);
     return BK_OK;
 }
 
-int finish_extras(const Model& m, const bk_draw_out& o, int64_t C, int64_t n, void* stream) {
-    if (fused_extras(m) || !o.mom_mean) return BK_OK;
+int fold_extras(const Model& m, const bk_draw_out& o, int64_t C, int64_t n, void* stream) {
+    if (!o.mom_mean) return BK_OK;
     return bk_moments_accumulate(o.draws, m.d.dtype, n, C * m.d.dims, o.mom_n0, o.mom_mean, o.mom_m2, stream);
+}
+
+int check_extras(const Model& m, const bk_draw_out& o, const char* who) {
+    return fused_extras(m) ? BK_OK : check_folded(o, who);
+}
+
+int finish_extras(const Model& m, const bk_draw_out& o, int64_t C, int64_t n, void* stream) {
+    return fused_extras(m) ? BK_OK : fold_extras(m, o, C, n, stream);
 }
 
 }  // namespace
@@ -342,6 +427,56 @@ int bk_mh_rw_sample(uint64_t handle, void* theta, void* lp_cache, int32_t* cache
         rc = mh_t<float>(*m, theta, lp_cache, cache_valid_host, C, scale, hastings, n_draws, rng, o, ws,
                        ws_bytes, (cudaStream_t)stream);
     return rc ? rc : finish_extras(*m, o, C, n_draws, stream);
+}
+
+size_t bk_mh_cuda_workspace_bytes(uint64_t model, uint64_t proposal, int64_t C) {
+    const Model* m = get_model(model);
+    const UserProposal* p = get_proposal(proposal);
+    return m && p ? mh_cuda_ws(*m, *p, C) : 0;
+}
+
+int bk_mh_cuda_prepare(uint64_t model, uint64_t proposal, char* log_out, size_t log_bytes) {
+    if (log_out && log_bytes) log_out[0] = '\0';
+    const Model* m = get_model(model);
+    if (!m) return BK_E_HANDLE;
+    const UserProposal* p = get_proposal(proposal);
+    if (!p) return BK_E_HANDLE;
+    BK_CHECK_ARG(m->d.dims == p->dims && m->d.dtype == p->dtype,
+                 "bk_mh_cuda_prepare: the proposal (dims %lld, dtype %d) does not match the model (dims %lld, dtype %d)",
+                 (long long)p->dims, p->dtype, (long long)m->d.dims, m->d.dtype);
+    return use_mhp_fused(*m, *p) ? user_mhp_prepare(*m, *p, log_out, log_bytes) : BK_OK;
+}
+
+int bk_mh_cuda_sample(uint64_t model, uint64_t proposal, void* theta, void* lp_cache, int32_t* cache_valid_host,
+                      int64_t C, int32_t hastings, int64_t n_draws, const bk_rng* rng, const bk_draw_out* out, void* ws,
+                      size_t ws_bytes, void* stream) {
+    const char* who = "bk_mh_cuda_sample";
+    const Model* m = get_model(model);
+    if (!m) return BK_E_HANDLE;
+    const UserProposal* p = get_proposal(proposal);
+    if (!p) return BK_E_HANDLE;
+    BK_CHECK_ARG(theta && C >= 0 && n_draws >= 0, "%s: bad theta/C/n_draws", who);
+    BK_CHECK_ARG(m->d.dims == p->dims && m->d.dtype == p->dtype,
+                 "%s: the proposal (dims %lld, dtype %d) does not match the model (dims %lld, dtype %d)", who,
+                 (long long)p->dims, p->dtype, (long long)m->d.dims, m->d.dtype);
+    BK_CHECK_ARG(!hastings || p->has_transition,
+                 "%s: hastings needs a proposal created with has_transition = 1 (transition_log_density)", who);
+    int rc = check_rng(rng, who);
+    if (rc) return rc;
+    if (rng->mode == BK_RNG_INJECTED)
+        BK_CHECK_ARG(rng->n_uniform == 1 + p->n_uniforms,
+                     "%s: injected rng needs n_uniform = 1 + the proposal's n_uniforms = %d (got %d)", who,
+                     1 + p->n_uniforms, rng->n_uniform);
+    bk_draw_out o = out ? *out : bk_draw_out{nullptr, nullptr, nullptr};
+    if (C == 0 || n_draws == 0) return BK_OK;
+    if ((rc = check_folded(o, who))) return rc;   // no engine of a user proposal fuses the extras
+    if (m->d.dtype == BK_F64)
+        rc = mh_cuda_t<double>(*m, *p, theta, lp_cache, cache_valid_host, C, hastings, n_draws, rng, o, ws, ws_bytes,
+                               (cudaStream_t)stream);
+    else
+        rc = mh_cuda_t<float>(*m, *p, theta, lp_cache, cache_valid_host, C, hastings, n_draws, rng, o, ws, ws_bytes,
+                              (cudaStream_t)stream);
+    return rc ? rc : fold_extras(*m, o, C, n_draws, stream);
 }
 
 }  // extern "C"

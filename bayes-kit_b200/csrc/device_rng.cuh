@@ -137,18 +137,18 @@ __device__ __forceinline__ void philox_normal4<double>(uint64_t seed, uint32_t b
 
 // k-th uniform of (chain, draw)
 template <typename T>
-__device__ __forceinline__ T philox_uniform(uint64_t seed, uint32_t k, uint32_t chain, uint32_t draw,
-                                            uint32_t tag = TAG_UNIFORM);
+__host__ __device__ __forceinline__ T philox_uniform(uint64_t seed, uint32_t k, uint32_t chain, uint32_t draw,
+                                                     uint32_t tag = TAG_UNIFORM);
 template <>
-__device__ __forceinline__ float philox_uniform<float>(uint64_t seed, uint32_t k, uint32_t chain,
-                                                       uint32_t draw, uint32_t tag) {
+__host__ __device__ __forceinline__ float philox_uniform<float>(uint64_t seed, uint32_t k, uint32_t chain,
+                                                                uint32_t draw, uint32_t tag) {
     uint32_t r[4];
     Philox::gen(seed, k >> 2, tag, chain, draw, r);
     return u01(r[k & 3]);
 }
 template <>
-__device__ __forceinline__ double philox_uniform<double>(uint64_t seed, uint32_t k, uint32_t chain,
-                                                         uint32_t draw, uint32_t tag) {
+__host__ __device__ __forceinline__ double philox_uniform<double>(uint64_t seed, uint32_t k, uint32_t chain,
+                                                                  uint32_t draw, uint32_t tag) {
     uint32_t r[4];
     Philox::gen(seed, k >> 1, tag, chain, draw, r);
     return (k & 1) ? u01d(r[2], r[3]) : u01d(r[0], r[1]);
@@ -170,6 +170,14 @@ __device__ __forceinline__ T philox_accept_uniform(uint64_t seed, uint32_t chain
     uint32_t r[4];
     Philox::gen(seed, (uint32_t)accept_block(D), TAG_NORMAL, chain, draw, r);
     return uniform_of_words<T>(r[0], r[1]);
+}
+
+// Normals of a user proposal (bk_proposal_create_cuda): normal k is element k % 4 of philox_normal4 on element block
+// proposal_normal_block(k, D) -- the blocks 0, 1, ... with accept_block(D) skipped, so the accept uniform never shares
+// its words with a proposal normal, and a proposal with at most D normals reads exactly the random walk's normals.
+__host__ __device__ __forceinline__ int proposal_normal_block(int k, int D) {
+    const int b = k >> 2;
+    return b < accept_block(D) ? b : b + 1;
 }
 
 // log(u) with numpy semantics for u == 0 (-inf: always accepts)

@@ -48,6 +48,25 @@ bool user_prior_lik(const Model& m);
 int user_log_prior_likelihood(const Model& m, const void* theta, int64_t C, void* lprior, void* llik, cudaStream_t st);
 int user_smc_move(const Model& m, int move, const UserSmcArgs& a, cudaStream_t st);
 
+// user-written CUDA proposals (bk_proposal_create_cuda, user_model.cu)
+struct UserProposal {
+    const struct PropLib* lib;   // the compiled proposal-only program (bk_user_propose)
+    int64_t dims;
+    int32_t dtype, n_normals, n_uniforms, has_transition;
+    const void* params;          // [n_params] caller array, dtype, or NULL
+};
+// returns nullptr (and sets the error) for an unknown handle
+const UserProposal* get_proposal(uint64_t handle);
+// the fused bk_user_mhp serves (m, p): a user model with dims <= USER_FUSED_MAX_D and n_normals <= USER_FUSED_MAX_D
+bool user_mhp_fusable(const Model& m, const UserProposal& p);
+// compiles (once per process) and loads the fused program of (m, p); log_out as bk_model_create_cuda's
+int user_mhp_prepare(const Model& m, const UserProposal& p, char* log_out, size_t log_bytes);
+int user_mhp_sample(const Model& m, const UserProposal& p, const UserRunArgs& a, int32_t* cache_valid, cudaStream_t st);
+// three-launch path: Philox scratch of bk_user_propose ([C, n_normals] and [C, n_uniforms]) and its launch
+struct UserProposeArgs;
+size_t user_propose_ws_bytes(const UserProposal& p, int64_t C);
+int user_propose(const UserProposal& p, const UserProposeArgs& a, cudaStream_t st);
+
 size_t model_eval_ws_bytes(const Model& m, int64_t C);
 // true when model_eval(..., precise=false) is a genuinely cheaper (tensor-core) evaluation
 bool model_has_fast_path(const Model& m);

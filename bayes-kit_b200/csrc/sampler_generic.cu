@@ -206,7 +206,9 @@ __global__ void k_mh_accept(GenArgs<T> p, int64_t t) {
     Row<T> row{p.rng, p.C, c, t, D, lane};
     const T lp = p.lp[c], lpq = p.lp_q[c];
     T ratio = A::sub(lpq, lp);
-    if (p.hastings) {
+    if (p.dh) {
+        ratio = A::add(ratio, p.dh[c]);
+    } else if (p.hastings) {
         T sf = T(0), sr = T(0);
         for (int e = lane; e < D; e += 32) {
             T df = A::sub(p.q[off + e], p.theta[off + e]), dr = A::sub(p.theta[off + e], p.q[off + e]);
@@ -267,7 +269,7 @@ static int carve(const Model& m, GenArgs<T>& p, void* ws, size_t ws_bytes, void*
 
 template <typename T>
 int run_generic(const Model& m, GenArgs<T> p, int algo, int* cache_valid, void* ws, size_t ws_bytes,
-                cudaStream_t st) {
+                cudaStream_t st, const MhProposeHook* propose) {
     if (p.C == 0 || p.n_draws == 0) return BK_OK;
     void* ews;
     size_t ebytes;
@@ -331,8 +333,13 @@ int run_generic(const Model& m, GenArgs<T> p, int algo, int* cache_valid, void* 
             k_mala_accept<T><<<blocks, 256, 0, st>>>(p, t);
             BK_LAUNCH_CHECK();
         } else {
-            k_mh_propose<T><<<blocks, 256, 0, st>>>(p, t);
-            BK_LAUNCH_CHECK();
+            if (propose) {
+                rc = propose->fn(propose->ctx, p.theta, p.q, p.dh, t, st);
+                if (rc) return rc;
+            } else {
+                k_mh_propose<T><<<blocks, 256, 0, st>>>(p, t);
+                BK_LAUNCH_CHECK();
+            }
             rc = model_eval(m, p.q, p.C, p.lp_q, nullptr, ews, ebytes, st);
             if (rc) return rc;
             k_mh_accept<T><<<blocks, 256, 0, st>>>(p, t);
@@ -342,7 +349,9 @@ int run_generic(const Model& m, GenArgs<T> p, int algo, int* cache_valid, void* 
     return BK_OK;
 }
 
-template int run_generic<float>(const Model&, GenArgs<float>, int, int*, void*, size_t, cudaStream_t);
-template int run_generic<double>(const Model&, GenArgs<double>, int, int*, void*, size_t, cudaStream_t);
+template int run_generic<float>(const Model&, GenArgs<float>, int, int*, void*, size_t, cudaStream_t,
+                                const MhProposeHook*);
+template int run_generic<double>(const Model&, GenArgs<double>, int, int*, void*, size_t, cudaStream_t,
+                                 const MhProposeHook*);
 
 }  // namespace bk

@@ -25,12 +25,21 @@ struct GenArgs {
     T* draws;
     T* logp;
     int32_t* accept;
+    T* dh;      // [C] Hastings term of a user proposal (log q(theta | q) - log q(q | theta)), added by k_mh_accept in
+                // place of the Gaussian random walk's; NULL: the built-in term (when hastings)
+};
+
+// Replaces k_mh_propose in run_generic's ALGO_MHRW loop (user proposals): writes q [C, D] from theta [C, D] for draw t
+// of the call, and dh [C] when dh is not NULL.
+struct MhProposeHook {
+    int (*fn)(const void* ctx, const void* theta, void* q, void* dh, int64_t t, cudaStream_t st);
+    const void* ctx;
 };
 
 template <typename T>
 size_t generic_ws_bytes(const Model& m, int64_t C);
 template <typename T>
 int run_generic(const Model& m, GenArgs<T> p, int algo, int* cache_valid, void* ws, size_t ws_bytes,
-                cudaStream_t st);
+                cudaStream_t st, const MhProposeHook* propose = nullptr);
 
 }  // namespace bk

@@ -24,6 +24,10 @@
 //                   per particle: k_smc_move_weight (smc.cu) step for step with one lane per particle, on the same
 //                   Philox words, the same resample-index / peer-row / (ll, prior)-carry rules and the same mailbox
 //                   posts (smc_mailbox.cuh).
+// bk_user_propose   (proposal programs, bk_proposal_create_cuda) one draw of a user proposal for global rows, one
+//                   thread per chain: the propose step of the three-launch Metropolis(-Hastings) path.
+// bk_user_mhp       (model + proposal programs) Metropolis / MetropolisHastings with a user proposal fused with a
+//                   user model, one thread per chain: bk_user_mh with propose() in place of the random walk.
 #pragma once
 #ifndef __CUDACC_RTC__
 #include "smc_mailbox.cuh"
@@ -49,6 +53,25 @@ struct UserRunArgs {
     double eps, half_eps;     // HMC; MALA: eps
     double sd, coef;          // MALA: sqrt(2 eps), -0.25 / eps
     double scale, s2;         // RW-Metropolis
+    const void* prop_params;  // bk_user_mhp: the proposal's [n_params] or NULL
+};
+
+// Launch arguments of bk_user_propose (one draw of a user proposal for C chains, three-launch path).  Streams: injected
+// normals [n, C, BK_PROPOSAL_NORMALS] and uniforms [n, C, n_uniform] (column 0: the accept uniform, columns 1 + k:
+// u[k]); in Philox mode the kernel writes this draw's z / u into zbuf [C, BK_PROPOSAL_NORMALS] / ubuf
+// [C, BK_PROPOSAL_UNIFORMS] and hands the proposal those rows.
+struct UserProposeArgs {
+    const void* theta;        // [C, D]
+    void* q;                  // [C, D] out
+    void* dh;                 // [C] out: log q(theta | q) - log q(q | theta), or NULL (no Hastings term)
+    const void* params;       // [n_params] or NULL
+    const void* normals;
+    const void* uniforms;
+    void* zbuf;
+    void* ubuf;
+    int64_t C, t;             // t: draw of this call
+    uint64_t seed, draw_offset, chain_offset;
+    int32_t rng_mode, n_uniform;
 };
 
 #if !defined(__CUDACC_RTC__) || defined(BK_PRIOR_LIK)
@@ -160,6 +183,9 @@ __device__ __forceinline__ void emit(const UserRunArgs& a, int64_t c, int64_t t,
 
 }  // namespace user
 }  // namespace bk
+
+// Model programs compile the kernels below; proposal programs (BK_PROPOSAL, further down) only their own.
+#ifndef BK_PROPOSAL
 
 // theta [C, D] -> lp [C] (nullable), grad [C, D]
 extern "C" __global__ void __launch_bounds__(128) bk_user_eval(const bk_real* __restrict__ theta, long long C,
@@ -505,4 +531,120 @@ extern "C" __global__ void __launch_bounds__(128) bk_user_smc_mala(const bk::Use
 extern "C" __global__ void __launch_bounds__(128) bk_user_smc_hmc(const bk::UserSmcArgs a) { bk::user::smc_move<2>(a); }
 
 #endif  // BK_PRIOR_LIK
+#endif  // !BK_PROPOSAL
+
+// ---- user proposals (bk_proposal_create_cuda) ----------------------------------------------------------------------
+// A proposal program holds the user's proposal source inside namespace bk_proposal and is compiled with
+// -DBK_PROPOSAL=1 -DBK_PROPOSAL_NORMALS=.. -DBK_PROPOSAL_UNIFORMS=.. -DBK_PROPOSAL_TRANSITION=0|1, either alone
+// (-DBK_PROPOSAL_ONLY=1: bk_user_propose) or after a model's source (bk_user_mhp, the fused sampler).
+#ifdef BK_PROPOSAL
+
+namespace bk {
+namespace user {
+
+constexpr int NZ = BK_PROPOSAL_NORMALS, NU = BK_PROPOSAL_UNIFORMS;
+constexpr int NZ1 = NZ > 0 ? NZ : 1, NU1 = NU > 0 ? NU : 1;   // array extents
+
+// the proposal's Philox streams of (global chain, draw): z[k] from block proposal_normal_block(k, D), u[k] the k-th
+// TAG_UNIFORM uniform
+__device__ __forceinline__ void proposal_philox(uint64_t seed, uint32_t chain, uint32_t draw, T* z, T* u) {
+#pragma unroll
+    for (int b = 0; 4 * b < NZ; ++b) {
+        T z4[4];
+        philox_normal4<T>(seed, (uint32_t)proposal_normal_block(4 * b, D), chain, draw, z4);
+#pragma unroll
+        for (int i = 0; i < 4; ++i)
+            if (4 * b + i < NZ) z[4 * b + i] = z4[i];
+    }
+#pragma unroll
+    for (int k = 0; k < NU; ++k) u[k] = philox_uniform<T>(seed, (uint32_t)k, chain, draw);
+}
+
+// log q(theta | q) - log q(q | theta), in MetropolisHastings's order: fwd = q(proposal | theta), rev = q(theta | proposal)
+__device__ __forceinline__ T proposal_dh(const T* th, const T* q, const T* pp) {
+#if BK_PROPOSAL_TRANSITION
+    const T fwd = bk_proposal::transition_log_density(q, th, pp);
+    const T rev = bk_proposal::transition_log_density(th, q, pp);
+    return A::sub(rev, fwd);
+#else
+    return T(0);
+#endif
+}
+
+}  // namespace user
+}  // namespace bk
+
+#ifdef BK_PROPOSAL_ONLY
+
+// One draw of the proposal for every chain: q = propose(theta, z, u) and, when dh is given, the Hastings term.
+extern "C" __global__ void __launch_bounds__(128) bk_user_propose(const bk::UserProposeArgs a) {
+    using namespace bk::user;
+    const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= a.C) return;
+    const T* pp = reinterpret_cast<const T*>(a.params);
+    const T* th = reinterpret_cast<const T*>(a.theta) + c * (int64_t)D;
+    T* q = reinterpret_cast<T*>(a.q) + c * (int64_t)D;
+    const T *z, *u;
+    if (a.rng_mode == 1) {   // BK_RNG_INJECTED
+        const int64_t r = a.t * a.C + c;
+        z = reinterpret_cast<const T*>(a.normals) + r * NZ;
+        u = reinterpret_cast<const T*>(a.uniforms) + r * a.n_uniform + 1;
+    } else {
+        T* zw = reinterpret_cast<T*>(a.zbuf) + c * NZ;
+        T* uw = reinterpret_cast<T*>(a.ubuf) + c * NU;
+        proposal_philox(a.seed, (uint32_t)(a.chain_offset + (uint64_t)c), (uint32_t)(a.draw_offset + (uint64_t)a.t),
+                        zw, uw);
+        z = zw;
+        u = uw;
+    }
+    bk_proposal::propose(th, q, z, u, pp);
+    if (a.dh) reinterpret_cast<T*>(a.dh)[c] = proposal_dh(th, q, pp);
+}
+
+#else
+
+// Metropolis / MetropolisHastings with a user proposal, fused with the user's model: bk_user_mh with the random walk
+// replaced by propose() and its Gaussian Hastings sum by transition_log_density.  The model's gradient is dead code.
+extern "C" __global__ void __launch_bounds__(128) bk_user_mhp(const bk::UserRunArgs a) {
+    using namespace bk::user;
+    const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= a.C) return;
+    const T* params = reinterpret_cast<const T*>(a.params);
+    const T* pp = reinterpret_cast<const T*>(a.prop_params);
+    T* row = reinterpret_cast<T*>(a.theta) + c * (int64_t)D;
+    T th[D], unused[D];
+    load_row(row, th);
+    T lp = log_density_gradient(th, unused, params);
+    for (int64_t t = 0; t < a.n_draws; ++t) {
+        T q[D], z[NZ1], u[NU1];
+        if (a.rng_mode == 1) {   // BK_RNG_INJECTED
+            const int64_t r = t * a.C + c;
+            const T* zi = reinterpret_cast<const T*>(a.normals) + r * NZ;
+            const T* ui = reinterpret_cast<const T*>(a.uniforms) + r * a.n_uniform + 1;
+#pragma unroll
+            for (int k = 0; k < NZ; ++k) z[k] = zi[k];
+#pragma unroll
+            for (int k = 0; k < NU; ++k) u[k] = ui[k];
+        } else {
+            proposal_philox(a.seed, (uint32_t)(a.chain_offset + (uint64_t)c), (uint32_t)(a.draw_offset + (uint64_t)t),
+                            z, u);
+        }
+        bk_proposal::propose(th, q, z, u, pp);
+        const T lpq = log_density_gradient(q, unused, params);
+        T ratio = A::sub(lpq, lp);
+        if (a.hastings) ratio = A::add(ratio, proposal_dh(th, q, pp));
+        const bool acc = bk::log_u(accept_uniform(a, c, t)) < ratio;
+        if (acc) {
+#pragma unroll
+            for (int e = 0; e < D; ++e) th[e] = q[e];
+            lp = lpq;
+        }
+        emit(a, c, t, th, lp, acc);
+    }
+#pragma unroll
+    for (int e = 0; e < D; ++e) row[e] = th[e];
+}
+
+#endif  // BK_PROPOSAL_ONLY
+#endif  // BK_PROPOSAL
 #endif  // __CUDACC_RTC__

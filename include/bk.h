@@ -92,6 +92,11 @@ typedef struct bk_rng {
     const void* normals;    /* INJECTED: [n_draws, C, D] standard normals (dtype)        */
     const void* uniforms;   /* INJECTED: [n_draws, C, n_uniform] uniforms in [0,1)       */
 } bk_rng;
+/* bk_mh_cuda_sample (user proposals) reads INJECTED streams as normals [n_draws, C, n_normals] and uniforms
+ * [n_draws, C, 1 + n_uniforms] (n_uniform = 1 + n_uniforms): column 0 is the accept uniform, column 1 + k the
+ * proposal's u[k].  In PHILOX mode z[k] is element k % 4 of the normals of element block b(k) = k / 4, or k / 4 + 1
+ * from block ceil(D / 4) on (that block holds the accept uniform of the single-uniform samplers, which is unchanged;
+ * with n_normals <= D, z is exactly the random walk's normal vector), and u[k] is the k-th TAG_UNIFORM uniform. */
 
 enum { BK_DRAWS_NCD = 0,  /* draws [n_draws, C, D]: one draw of every chain after the other      */
        BK_DRAWS_CDN = 1   /* draws [C, D, n_draws]: every (chain, dim) SERIES contiguous over the
@@ -233,6 +238,46 @@ BK_API int bk_mh_rw_sample(uint64_t handle, void* theta, void* lp_cache, int32_t
                     int64_t C, double scale, int32_t hastings, int64_t n_draws,
                     const bk_rng* rng, const bk_draw_out* out, void* ws, size_t ws_bytes,
                     void* stream);
+
+/* ---- Metropolis / MetropolisHastings with a user-written proposal (metropolis.py:79-135: proposal_fn and
+ * transition_lp_fn written in CUDA C++).  `source` defines
+ *
+ *     __device__ void propose(const bk_real* theta, bk_real* proposal, const bk_real* z, const bk_real* u,
+ *                             const bk_real* params);
+ *     __device__ bk_real transition_log_density(const bk_real* to, const bk_real* from, const bk_real* params);
+ *
+ * propose writes theta' into proposal[0 .. BK_DIMS) from z [BK_PROPOSAL_NORMALS] standard normals and u
+ * [BK_PROPOSAL_UNIFORMS] uniforms in (0, 1) of this (chain, draw) -- the library draws all of them before every
+ * call (streams: see bk_rng) -- and transition_log_density returns log q(to | from) up to a constant; it is required
+ * only with has_transition = 1.  bk_real, BK_DIMS, the compile options, the absence of headers and the log are those
+ * of bk_model_create_cuda; the source is compiled inside namespace bk_proposal, so its helpers may share names with a
+ * model's.  BK_PROPOSAL_NORMALS = n_normals and BK_PROPOSAL_UNIFORMS = n_uniforms are compile-time constants.
+ * `params` [n_params] (device, dtype; NULL exactly when n_params == 0) must outlive the handle.  Compiled programs
+ * are cached for the life of the process and never unloaded.  Arguments are checked before any compilation or device
+ * call: source and handle_out required, dims in [1, BK_USER_MAX_DIMS], n_normals in [0, BK_PROPOSAL_MAX_NORMALS],
+ * n_uniforms in [0, BK_PROPOSAL_MAX_UNIFORMS].  Returns BK_E_INVALID on a bad argument or a compile error,
+ * BK_E_UNSUPPORTED without NVRTC, BK_E_CUDA when the compiled module cannot be loaded.  Proposal handles have a
+ * registry of their own: no model entry point accepts one. */
+#define BK_PROPOSAL_MAX_NORMALS BK_USER_MAX_DIMS
+#define BK_PROPOSAL_MAX_UNIFORMS 64
+BK_API int bk_proposal_create_cuda(const char* source, int64_t dims, int32_t dtype, const void* params,
+                                   int64_t n_params, int32_t n_normals, int32_t n_uniforms, int32_t has_transition,
+                                   uint64_t* handle_out, char* log_out, size_t log_bytes);
+BK_API int bk_proposal_destroy(uint64_t handle);
+/* Engines: a user model (bk_model_create_cuda*) with dims <= 32 and a proposal with n_normals <= 32 run one fused
+ * kernel per call (bk_user_mhp: one thread per chain, theta and log p(theta) in registers across the draws; leaves
+ * *cache_valid_host = 0; compiled from the model's and the proposal's sources together, once per process, by
+ * bk_mh_cuda_prepare or on the first call).  Every other model runs three launches per draw: the proposal
+ * (bk_user_propose), the model's evaluation of the proposals and the accept test of bk_mh_rw_sample, with
+ * lp_cache / cache_valid_host as there.  hastings != 0 adds transition_log_density(theta, theta') -
+ * transition_log_density(theta', theta).  BK_E_INVALID when the model's and the proposal's dims or dtype differ,
+ * when hastings != 0 and the proposal has no transition, or when INJECTED n_uniform != 1 + n_uniforms.  Draws are
+ * [n_draws, C, D] only; streaming moments are folded from them. */
+BK_API size_t bk_mh_cuda_workspace_bytes(uint64_t model, uint64_t proposal, int64_t C);
+BK_API int bk_mh_cuda_prepare(uint64_t model, uint64_t proposal, char* log_out, size_t log_bytes);
+BK_API int bk_mh_cuda_sample(uint64_t model, uint64_t proposal, void* theta, void* lp_cache,
+                             int32_t* cache_valid_host, int64_t C, int32_t hastings, int64_t n_draws,
+                             const bk_rng* rng, const bk_draw_out* out, void* ws, size_t ws_bytes, void* stream);
 
 /* ---- DrGhmcDiag (drghmc.py:37-446) --------------------------------------
  * theta, rho [C,D] in/out; step_sizes_host[K], step_counts_host[K].
