@@ -20,14 +20,14 @@ from .metropolis import (CudaProposal, GaussianRW, Metropolis, MetropolisHasting
 from .models import Binomial, CudaModel, CudaPriorLikModel, DensePrecGauss, DiagGauss, GaussPriorLik, HierLogReg, IsoGauss, StdNormal
 from .rhat import (chain_moments, rank_chains, rank_normalize_chains, rank_normalized_rhat, rhat,
                    split_chains, split_rhat)
-from .smc import TemperedLikelihoodSMC, hmc_kernel, mala_kernel, metropolis_kernel
+from .smc import TemperedLikelihoodSMC, hmc_kernel, mala_kernel, metropolis_kernel, proposal_kernel
 
 __all__ = [
     "DrGhmcDiag", "HMCDiag", "MALA", "Metropolis", "MetropolisHastings", "TemperedLikelihoodSMC",
     "Stretcher", "ess", "ess_imse", "ess_ipse", "iat", "iat_imse", "iat_ipse", "rhat", "autocorr",
     # device-side additions
     "GaussianRW", "metropolis_kernel", "mala_kernel", "hmc_kernel", "models", "dist", "peer", "Binomial", "IsoGauss", "StdNormal", "DiagGauss", "CudaModel", "CudaPriorLikModel",
-    "CudaProposal",
+    "CudaProposal", "proposal_kernel",
     "DensePrecGauss", "GaussPriorLik", "HierLogReg", "chain_moments",
     # rhat.py's split / rank-normalised family (not re-exported by the reference's __init__)
     "split_chains", "split_rhat", "rank_chains", "rank_normalize_chains", "rank_normalized_rhat",

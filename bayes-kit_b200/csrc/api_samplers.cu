@@ -444,7 +444,7 @@ int bk_mh_cuda_prepare(uint64_t model, uint64_t proposal, char* log_out, size_t 
     BK_CHECK_ARG(m->d.dims == p->dims && m->d.dtype == p->dtype,
                  "bk_mh_cuda_prepare: the proposal (dims %lld, dtype %d) does not match the model (dims %lld, dtype %d)",
                  (long long)p->dims, p->dtype, (long long)m->d.dims, m->d.dtype);
-    return use_mhp_fused(*m, *p) ? user_mhp_prepare(*m, *p, log_out, log_bytes) : BK_OK;
+    return use_mhp_fused(*m, *p) ? user_mhp_prepare(*m, *p, "bk_mh_cuda_prepare", log_out, log_bytes) : BK_OK;
 }
 
 int bk_mh_cuda_sample(uint64_t model, uint64_t proposal, void* theta, void* lp_cache, int32_t* cache_valid_host,

@@ -59,9 +59,12 @@ struct UserProposal {
 const UserProposal* get_proposal(uint64_t handle);
 // the fused bk_user_mhp serves (m, p): a user model with dims <= USER_FUSED_MAX_D and n_normals <= USER_FUSED_MAX_D
 bool user_mhp_fusable(const Model& m, const UserProposal& p);
-// compiles (once per process) and loads the fused program of (m, p); log_out as bk_model_create_cuda's
-int user_mhp_prepare(const Model& m, const UserProposal& p, char* log_out, size_t log_bytes);
+// compiles (once per process) and loads the fused program of (m, p) -- bk_user_mhp and, for a prior/likelihood model,
+// bk_user_smc_mhp; log_out as bk_model_create_cuda's, `who` names the caller in errors
+int user_mhp_prepare(const Model& m, const UserProposal& p, const char* who, char* log_out, size_t log_bytes);
 int user_mhp_sample(const Model& m, const UserProposal& p, const UserRunArgs& a, int32_t* cache_valid, cudaStream_t st);
+// the SMC's proposal move (BK_SMC_KERNEL_PROPOSAL): bk_user_smc_mhp of the fused program of (m, p), prior_lik models
+int user_smc_mhp(const Model& m, const UserProposal& p, const UserSmcArgs& a, cudaStream_t st);
 // three-launch path: Philox scratch of bk_user_propose ([C, n_normals] and [C, n_uniforms]) and its launch
 struct UserProposeArgs;
 size_t user_propose_ws_bytes(const UserProposal& p, int64_t C);

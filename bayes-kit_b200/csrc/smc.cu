@@ -406,6 +406,12 @@ static int smc_user(const Model& m, const SmcArgs<T>& a, const bk_smc_kernel& kn
     u.maxpart = a.maxpart;
     u.ticket = a.ticket;
     u.params = m.user_params;
+    if (kn.kind == BK_SMC_KERNEL_PROPOSAL) {   // check_smc_model resolved the handle
+        const UserProposal* p = get_proposal(kn.proposal);
+        if (!p) return BK_E_HANDLE;
+        u.prop_params = p->params;
+        return user_smc_mhp(m, *p, u, st);
+    }
     return user_smc_move(m, kn.kind, u, st);
 }
 
@@ -460,14 +466,38 @@ static int smc_dispatch(const Model& m, SmcArgs<T>& a, const bk_smc_kernel& kn, 
     return BK_E_UNSUPPORTED;
 }
 
-static int check_smc_model(const Model& m, const bk_smc_kernel& kn) {
+// the PROPOSAL kind: a user prior/likelihood model and a proposal of its dims and dtype; rng (may be NULL): the
+// injected uniforms carry the accept uniform and the proposal's
+static int check_smc_proposal(const Model& m, const bk_smc_kernel& kn, const bk_rng* rng) {
+    if (!user_prior_lik(m)) {
+        set_error("bk_smc: the proposal move runs on user models created by bk_model_create_cuda_prior_lik only "
+                  "(restate a built-in GAUSS_PRIOR_LIK / BINOMIAL_LOGIT model as one)");
+        return BK_E_UNSUPPORTED;
+    }
+    const UserProposal* p = get_proposal(kn.proposal);
+    if (!p) return BK_E_HANDLE;
+    BK_CHECK_ARG(m.d.dims == p->dims && m.d.dtype == p->dtype,
+                 "bk_smc: the proposal (dims %lld, dtype %d) does not match the model (dims %lld, dtype %d)",
+                 (long long)p->dims, p->dtype, (long long)m.d.dims, m.d.dtype);
+    BK_CHECK_ARG(p->n_normals <= BK_SMC_PROPOSAL_MAX_NORMALS,
+                 "bk_smc: the proposal move supports n_normals <= %d (got %d)", BK_SMC_PROPOSAL_MAX_NORMALS,
+                 p->n_normals);
+    BK_CHECK_ARG(!rng || rng->mode != BK_RNG_INJECTED || rng->n_uniform == 1 + p->n_uniforms,
+                 "bk_smc: injected rng needs n_uniform = 1 + the proposal's n_uniforms = %d (got %d)",
+                 1 + p->n_uniforms, rng ? rng->n_uniform : 0);
+    return BK_OK;
+}
+
+static int check_smc_model(const Model& m, const bk_smc_kernel& kn, const bk_rng* rng = nullptr) {
     BK_CHECK_ARG(m.d.kind == BK_MODEL_GAUSS_PRIOR_LIK || m.d.kind == BK_MODEL_BINOMIAL_LOGIT || user_prior_lik(m),
                  "bk_smc_move_weight: the model must expose log_prior / log_likelihood (GAUSS_PRIOR_LIK, BINOMIAL_LOGIT, "
                  "or a user model created by bk_model_create_cuda_prior_lik)");
     BK_CHECK_ARG(m.d.kind != BK_MODEL_USER_CUDA || m.d.dims <= BK_USER_PRIOR_LIK_MAX_DIMS,
                  "bk_smc_move_weight: user models support dims <= %d (got %lld)", BK_USER_PRIOR_LIK_MAX_DIMS,
                  (long long)m.d.dims);
-    BK_CHECK_ARG(kn.kind >= BK_SMC_KERNEL_RW && kn.kind <= BK_SMC_KERNEL_HMC, "bk_smc: unknown kernel kind %d", kn.kind);
+    BK_CHECK_ARG(kn.kind >= BK_SMC_KERNEL_RW && kn.kind <= BK_SMC_KERNEL_PROPOSAL, "bk_smc: unknown kernel kind %d",
+                 kn.kind);
+    if (kn.kind == BK_SMC_KERNEL_PROPOSAL) return check_smc_proposal(m, kn, rng);
     BK_CHECK_ARG(kn.scale > 0, "bk_smc: kernel scale / step size must be positive (got %g)", kn.scale);
     BK_CHECK_ARG(kn.kind != BK_SMC_KERNEL_HMC || kn.steps >= 0, "bk_smc: HMC kernel needs steps >= 0");
     return BK_OK;
@@ -1331,7 +1361,7 @@ int bk_smc_shard_move(uint64_t handle, const bk_smc_shard* sh, const void* src_l
     const Model* m = get_model(handle);
     if (!m) return BK_E_HANDLE;
     BK_CHECK_ARG(kernel && rng, "bk_smc_shard_move: null argument");
-    if (int rc = check_smc_model(*m, *kernel)) return rc;
+    if (int rc = check_smc_model(*m, *kernel, rng)) return rc;
     ShardGeom g;
     if (int rc = make_geom(sh, &g)) return rc;
     BK_CHECK_ARG(T >= 1 && n >= 1 && n <= T, "bk_smc_shard_move: need 1 <= n <= T (n=%d, T=%d)", n, T);
@@ -1486,6 +1516,17 @@ int bk_smc_shard_run(uint64_t handle, const bk_smc_shard* sh, const void* src_lo
         s.epoch += 1;
     }
     return BK_OK;
+}
+
+int bk_smc_cuda_prepare(uint64_t model, uint64_t proposal, char* log_out, size_t log_bytes) {
+    if (log_out && log_bytes) log_out[0] = '\0';
+    const Model* m = get_model(model);
+    if (!m) return BK_E_HANDLE;
+    const UserProposal* p = get_proposal(proposal);
+    if (!p) return BK_E_HANDLE;
+    bk_smc_kernel kn = {BK_SMC_KERNEL_PROPOSAL, 0, 0.0, proposal};
+    if (int rc = check_smc_model(*m, kn)) return rc;
+    return user_mhp_prepare(*m, *p, "bk_smc_cuda_prepare", log_out, log_bytes);
 }
 
 int bk_smc_shard_gather(const bk_smc_shard* sh, int64_t D, int32_t dtype, void* out, void* stream) {

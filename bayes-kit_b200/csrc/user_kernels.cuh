@@ -28,6 +28,9 @@
 //                   thread per chain: the propose step of the three-launch Metropolis(-Hastings) path.
 // bk_user_mhp       (model + proposal programs) Metropolis / MetropolisHastings with a user proposal fused with a
 //                   user model, one thread per chain: bk_user_mh with propose() in place of the random walk.
+// bk_user_smc_mhp   (prior/likelihood model + proposal programs) TemperedLikelihoodSMC's move + weight kernel with
+//                   one Metropolis(-Hastings) step of the user's proposal as the move: bk_user_smc_rw with propose()
+//                   in place of the random walk (BK_SMC_KERNEL_PROPOSAL).
 #pragma once
 #ifndef __CUDACC_RTC__
 #include "smc_mailbox.cuh"
@@ -103,6 +106,7 @@ struct UserSmcArgs {
     double* maxpart;                       // [gridDim.x] per-CTA maxima (NULL: no statistics epilogue)
     unsigned* ticket;
     const void* params;                    // [n_params] or NULL
+    const void* prop_params;               // bk_user_smc_mhp: the proposal's [n_params] or NULL
 };
 #endif
 
@@ -184,7 +188,51 @@ __device__ __forceinline__ void emit(const UserRunArgs& a, int64_t c, int64_t t,
 }  // namespace user
 }  // namespace bk
 
-// Model programs compile the kernels below; proposal programs (BK_PROPOSAL, further down) only their own.
+// ---- user proposals (bk_proposal_create_cuda) ----------------------------------------------------------------------
+// A proposal program holds the user's proposal source inside namespace bk_proposal and is compiled with
+// -DBK_PROPOSAL=1 -DBK_PROPOSAL_NORMALS=.. -DBK_PROPOSAL_UNIFORMS=.. -DBK_PROPOSAL_TRANSITION=0|1, either alone
+// (-DBK_PROPOSAL_ONLY=1: bk_user_propose) or after a model's source (bk_user_mhp, the fused sampler; prior/likelihood
+// models also bk_user_smc_mhp).
+#ifdef BK_PROPOSAL
+
+namespace bk {
+namespace user {
+
+constexpr int NZ = BK_PROPOSAL_NORMALS, NU = BK_PROPOSAL_UNIFORMS;
+constexpr int NZ1 = NZ > 0 ? NZ : 1, NU1 = NU > 0 ? NU : 1;   // array extents
+
+// the proposal's Philox streams of (global chain, draw): z[k] from block proposal_normal_block(k, D), u[k] the k-th
+// TAG_UNIFORM uniform
+__device__ __forceinline__ void proposal_philox(uint64_t seed, uint32_t chain, uint32_t draw, T* z, T* u) {
+#pragma unroll
+    for (int b = 0; 4 * b < NZ; ++b) {
+        T z4[4];
+        philox_normal4<T>(seed, (uint32_t)proposal_normal_block(4 * b, D), chain, draw, z4);
+#pragma unroll
+        for (int i = 0; i < 4; ++i)
+            if (4 * b + i < NZ) z[4 * b + i] = z4[i];
+    }
+#pragma unroll
+    for (int k = 0; k < NU; ++k) u[k] = philox_uniform<T>(seed, (uint32_t)k, chain, draw);
+}
+
+// log q(theta | q) - log q(q | theta), in MetropolisHastings's order: fwd = q(proposal | theta), rev = q(theta | proposal)
+__device__ __forceinline__ T proposal_dh(const T* th, const T* q, const T* pp) {
+#if BK_PROPOSAL_TRANSITION
+    const T fwd = bk_proposal::transition_log_density(q, th, pp);
+    const T rev = bk_proposal::transition_log_density(th, q, pp);
+    return A::sub(rev, fwd);
+#else
+    return T(0);
+#endif
+}
+
+}  // namespace user
+}  // namespace bk
+
+#endif  // BK_PROPOSAL
+
+// Model programs compile the kernels below; proposal programs only bk_user_propose / bk_user_mhp / bk_user_smc_mhp.
 #ifndef BK_PROPOSAL
 
 // theta [C, D] -> lp [C] (nullable), grad [C, D]
@@ -354,9 +402,11 @@ extern "C" __global__ void __launch_bounds__(128) bk_user_mh(const bk::UserRunAr
 }
 
 #endif  // BK_DIMS <= BK_USER_FUSED_MAX_D
+#endif  // !BK_PROPOSAL
 
 // The prior / likelihood kernels are compiled only for models created by bk_model_create_cuda_prior_lik.
 #ifdef BK_PRIOR_LIK
+#ifndef BK_PROPOSAL
 
 // theta [C, D] -> log_prior [C], log_likelihood [C] (each nullable)
 extern "C" __global__ void __launch_bounds__(128) bk_user_eval_pl(const bk_real* __restrict__ theta, long long C,
@@ -371,6 +421,8 @@ extern "C" __global__ void __launch_bounds__(128) bk_user_eval_pl(const bk_real*
     if (llik) llik[c] = log_likelihood_gradient(x, g, params);
 }
 
+#endif  // !BK_PROPOSAL
+
 namespace bk {
 namespace user {
 
@@ -383,7 +435,7 @@ __device__ __forceinline__ void tempered(const T (&x)[D], T t, const T* params, 
     for (int e = 0; e < D; ++e) g[e] = A::add(A::mul(g[e], t), gp[e]);
 }
 
-// k_smc_move_weight with one lane per particle.  MOVE: BK_SMC_KERNEL_RW / _MALA / _HMC (bk.h: 0 / 1 / 2).
+// k_smc_move_weight with one lane per particle.  MOVE: BK_SMC_KERNEL_RW / _MALA / _HMC / _PROPOSAL (bk.h: 0 .. 3).
 template <int MOVE>
 __device__ __forceinline__ void smc_move(const UserSmcArgs& a) {
     const T* params = reinterpret_cast<const T*>(a.params);
@@ -415,9 +467,10 @@ __device__ __forceinline__ void smc_move(const UserSmcArgs& a) {
         }
         T th[D], st[D], z[D];
         load_row(row, th);
-        // proposal normals: the words Lanes<T, G, J>::normals consumes for blocks 0 .. ceil(D / 4) - 1
+        // proposal normals: the words Lanes<T, G, J>::normals consumes for blocks 0 .. ceil(D / 4) - 1 (the user's
+        // proposal draws its own streams below)
 #pragma unroll
-        for (int b = 0; b < NB; ++b) {
+        for (int b = 0; b < (MOVE == 3 ? 0 : NB); ++b) {
             T z4[4];
             if (a.rng_mode == 1) {   // BK_RNG_INJECTED: [M, D]
                 const T* p = reinterpret_cast<const T*>(a.normals) + m * (int64_t)D;
@@ -467,6 +520,31 @@ __device__ __forceinline__ void smc_move(const UserSmcArgs& a) {
             }
             const T fwd = A::mul(coef, sf), rev = A::mul(coef, sr);
             acc = lu < A::add(A::sub(lp_s, lp_c), A::sub(rev, fwd));   // metropolis.py:41-76
+#ifdef BK_PROPOSAL
+        } else if constexpr (MOVE == 3) {   // the RW branch with the user's proposal: bk_user_mhp's step
+            const T* pp = reinterpret_cast<const T*>(a.prop_params);
+            T zp[NZ1], up[NU1], unused[D];
+            if (a.rng_mode == 1) {   // BK_RNG_INJECTED: normals [M, NZ], uniforms [M, 1 + NU] (column 0: accept)
+                const T* zi = reinterpret_cast<const T*>(a.normals) + m * NZ;
+                const T* ui = reinterpret_cast<const T*>(a.uniforms) + m * a.n_uniform + 1;
+#pragma unroll
+                for (int k = 0; k < NZ; ++k) zp[k] = zi[k];
+#pragma unroll
+                for (int k = 0; k < NU; ++k) up[k] = ui[k];
+            } else {
+                proposal_philox(a.seed, (uint32_t)(a.chain_offset + (uint64_t)m), (uint32_t)a.draw_offset, zp, up);
+            }
+            if (!carry) tempered(th, t0, params, ll_c, pr_c, unused);
+            const T lp_c = A::add(A::mul(ll_c, t0), pr_c);
+            bk_proposal::propose(th, st, zp, up, pp);
+            tempered(st, t0, params, ll_s, pr_s, unused);
+            const T lp_s = A::add(A::mul(ll_s, t0), pr_s);
+            T ratio = A::sub(lp_s, lp_c);
+#if BK_PROPOSAL_TRANSITION
+            ratio = A::add(ratio, proposal_dh(th, st, pp));
+#endif
+            acc = lu < ratio;
+#endif
         } else {   // one HMCDiag transition, identity metric, on the tempered density (hmc.py:40-63)
             const T eps = (T)a.scale, heps = A::mul(T(0.5), eps);
             T g[D];
@@ -526,53 +604,17 @@ __device__ __forceinline__ void smc_move(const UserSmcArgs& a) {
 }  // namespace user
 }  // namespace bk
 
+#ifndef BK_PROPOSAL
 extern "C" __global__ void __launch_bounds__(128) bk_user_smc_rw(const bk::UserSmcArgs a) { bk::user::smc_move<0>(a); }
 extern "C" __global__ void __launch_bounds__(128) bk_user_smc_mala(const bk::UserSmcArgs a) { bk::user::smc_move<1>(a); }
 extern "C" __global__ void __launch_bounds__(128) bk_user_smc_hmc(const bk::UserSmcArgs a) { bk::user::smc_move<2>(a); }
+#elif !defined(BK_PROPOSAL_ONLY)
+extern "C" __global__ void __launch_bounds__(128) bk_user_smc_mhp(const bk::UserSmcArgs a) { bk::user::smc_move<3>(a); }
+#endif
 
 #endif  // BK_PRIOR_LIK
-#endif  // !BK_PROPOSAL
 
-// ---- user proposals (bk_proposal_create_cuda) ----------------------------------------------------------------------
-// A proposal program holds the user's proposal source inside namespace bk_proposal and is compiled with
-// -DBK_PROPOSAL=1 -DBK_PROPOSAL_NORMALS=.. -DBK_PROPOSAL_UNIFORMS=.. -DBK_PROPOSAL_TRANSITION=0|1, either alone
-// (-DBK_PROPOSAL_ONLY=1: bk_user_propose) or after a model's source (bk_user_mhp, the fused sampler).
 #ifdef BK_PROPOSAL
-
-namespace bk {
-namespace user {
-
-constexpr int NZ = BK_PROPOSAL_NORMALS, NU = BK_PROPOSAL_UNIFORMS;
-constexpr int NZ1 = NZ > 0 ? NZ : 1, NU1 = NU > 0 ? NU : 1;   // array extents
-
-// the proposal's Philox streams of (global chain, draw): z[k] from block proposal_normal_block(k, D), u[k] the k-th
-// TAG_UNIFORM uniform
-__device__ __forceinline__ void proposal_philox(uint64_t seed, uint32_t chain, uint32_t draw, T* z, T* u) {
-#pragma unroll
-    for (int b = 0; 4 * b < NZ; ++b) {
-        T z4[4];
-        philox_normal4<T>(seed, (uint32_t)proposal_normal_block(4 * b, D), chain, draw, z4);
-#pragma unroll
-        for (int i = 0; i < 4; ++i)
-            if (4 * b + i < NZ) z[4 * b + i] = z4[i];
-    }
-#pragma unroll
-    for (int k = 0; k < NU; ++k) u[k] = philox_uniform<T>(seed, (uint32_t)k, chain, draw);
-}
-
-// log q(theta | q) - log q(q | theta), in MetropolisHastings's order: fwd = q(proposal | theta), rev = q(theta | proposal)
-__device__ __forceinline__ T proposal_dh(const T* th, const T* q, const T* pp) {
-#if BK_PROPOSAL_TRANSITION
-    const T fwd = bk_proposal::transition_log_density(q, th, pp);
-    const T rev = bk_proposal::transition_log_density(th, q, pp);
-    return A::sub(rev, fwd);
-#else
-    return T(0);
-#endif
-}
-
-}  // namespace user
-}  // namespace bk
 
 #ifdef BK_PROPOSAL_ONLY
 

@@ -15,7 +15,9 @@ reads the selected rows from their owners over NVLink peer memory (peer.py, bk.h
 The model is a built-in plugin with a log_prior / log_likelihood split (GaussPriorLik,
 Binomial: lane-grouped move kernel) or the user's own CUDA source as a
 CudaPriorLikModel (runtime-compiled move kernel, one thread per particle, same
-random streams, resampling and cross-rank messages).
+random streams, resampling and cross-rank messages).  On a CudaPriorLikModel the
+move may also be one Metropolis(-Hastings) step of a user-written CudaProposal
+(``proposal_kernel``), compiled together with the model into one kernel.
 """
 from __future__ import annotations
 
@@ -30,6 +32,7 @@ from . import _lib as L
 from . import dist as D_
 from . import peer as P_
 from ._util import make_rng, resolve_seed, stream_ptr, to_dev
+from .metropolis import CudaProposal
 from .models import Binomial, CudaPriorLikModel, GaussPriorLik, require_plugin
 
 
@@ -44,6 +47,10 @@ class _Kernel:
 
     def desc(self) -> L.SmcKernel:
         return L.SmcKernel(self.kind, self.steps, self.scale)
+
+    def stream_widths(self, D: int):
+        """(normals, uniforms) per particle of the injected streams."""
+        return D, 1
 
 
 class RWMetropolisKernel(_Kernel):
@@ -71,6 +78,27 @@ class HMCKernel(_Kernel):
             raise ValueError(f"steps must be >= 0, got {steps}")
 
 
+class ProposalKernel(_Kernel):
+    """One Metropolis(-Hastings) step of a user-written ``CudaProposal`` on the tempered density
+    ``lp_t = ll * t + prior``: ``theta* = propose(theta, z, u)``, accepted iff ``log(u_acc) < lp_t(theta*) -
+    lp_t(theta)`` plus, for a proposal created with ``transition=True``, ``log q(theta | theta*) - log q(theta* |
+    theta)`` (the reference's ``kernel`` argument with any Markov kernel, smc.py:54-57).  Runs on a
+    ``CudaPriorLikModel`` of the proposal's dims and dtype, compiled together with it into one kernel."""
+    kind = L.SMC_KERNEL_PROPOSAL
+
+    def __init__(self, proposal):
+        if not isinstance(proposal, CudaProposal):
+            raise TypeError("proposal_kernel needs a bayes_kit_b200.CudaProposal written in CUDA C++ "
+                            f"(got {type(proposal).__name__})")
+        self.proposal = proposal          # keeps the handle alive as long as the kernel
+
+    def desc(self) -> L.SmcKernel:
+        return L.SmcKernel(self.kind, 0, 0.0, self.proposal.handle)
+
+    def stream_widths(self, D: int):
+        return self.proposal.normals, 1 + self.proposal.uniforms
+
+
 def metropolis_kernel(scale: float) -> RWMetropolisKernel:
     return RWMetropolisKernel(scale)
 
@@ -85,6 +113,11 @@ def hmc_kernel(stepsize: float, steps: int) -> HMCKernel:
     return HMCKernel(stepsize, steps)
 
 
+def proposal_kernel(proposal: CudaProposal) -> ProposalKernel:
+    """MCMC-kernel plug-in for the SMC: one Metropolis(-Hastings) step of a user-written ``CudaProposal``."""
+    return ProposalKernel(proposal)
+
+
 class TemperedLikelihoodSMC:
     """``TemperedLikelihoodSMC(model, M, N, sample_initial, kernel)`` (smc.py:13-27).
 
@@ -93,7 +126,9 @@ class TemperedLikelihoodSMC:
     * ``sample_initial``: the reference's callable ``m -> theta0[m]`` (evaluated
       once per particle on the host, as smc.py:23 does), or directly an [M, D]
       array / tensor.
-    * ``kernel``: ``metropolis_kernel(scale)`` (the reference's), ``mala_kernel(eps)``, ``hmc_kernel(eps, L)``.
+    * ``kernel``: ``metropolis_kernel(scale)`` (the reference's), ``mala_kernel(eps)``, ``hmc_kernel(eps, L)``,
+      or, on a ``CudaPriorLikModel``, ``proposal_kernel(CudaProposal(...))``.  The fused program of the model and
+      the proposal is compiled at construction (``compile_log``: ptxas's report, else "").
     * ``resample``: ``"multinomial"`` (reference semantics: no max-shift, legacy
       ``np.random.choice`` indices) or ``"systematic"`` (log-sum-exp normalised,
       stratified points, exact fixed-point CDF: the indices do not depend on how the
@@ -113,8 +148,12 @@ class TemperedLikelihoodSMC:
             raise TypeError("TemperedLikelihoodSMC needs a model plugin with log_prior/log_likelihood "
                             "(bayes_kit_b200.models.GaussPriorLik / Binomial / CudaPriorLikModel)")
         if not isinstance(kernel, _Kernel):
-            raise TypeError("kernel must be bayes_kit_b200.metropolis_kernel(scale) (or mala_kernel / hmc_kernel): "
-                            "arbitrary Python kernels cannot run per particle on the GPU and there is no CPU fallback")
+            raise TypeError("kernel must be bayes_kit_b200.metropolis_kernel(scale) (or mala_kernel / hmc_kernel / "
+                            "proposal_kernel): arbitrary Python kernels cannot run per particle on the GPU and there is "
+                            "no CPU fallback")
+        self.compile_log = ""
+        if isinstance(kernel, ProposalKernel):
+            self._prepare(kernel.proposal)
         if resample not in ("multinomial", "systematic"):
             raise ValueError("resample must be 'multinomial' or 'systematic'")
         if ess_threshold is not None and not 0 < ess_threshold <= 1:
@@ -171,6 +210,23 @@ class TemperedLikelihoodSMC:
         self._steps_taken = []
         self._shard = None
         self.last_accept = None
+
+    def _prepare(self, prop: CudaProposal) -> None:
+        """Check (model, proposal) and compile their fused program now, not in the first move."""
+        if not isinstance(self._model, CudaPriorLikModel):
+            raise NotImplementedError("proposal_kernel runs on a CudaPriorLikModel only: restate the built-in "
+                                      f"{type(self._model).__name__} as a CudaPriorLikModel")
+        if prop.dims != self._model.dims() or prop.dtype != self._model.dtype:
+            raise ValueError(f"the proposal (dims {prop.dims}, {prop.dtype}) does not match the model "
+                             f"(dims {self._model.dims()}, {self._model.dtype})")
+        log = C.create_string_buffer(1 << 20)
+        with torch.cuda.device(self._model.device):
+            rc = L.lib().bk_smc_cuda_prepare(self._model.handle, prop.handle, log, len(log))
+        if rc == L.BK_E_INVALID and log.value:
+            raise ValueError("TemperedLikelihoodSMC: NVRTC compilation of the model with the proposal failed:\n"
+                             + log.value.decode(errors="replace"))
+        L.check(rc)
+        self.compile_log = log.value.decode(errors="replace")
 
     # ---- plumbing --------------------------------------------------------------------
     def _sh(self) -> L.SmcShard:
@@ -289,7 +345,9 @@ class TemperedLikelihoodSMC:
     def transition(self, n: int, normals=None, acc_uniforms=None, res_uniforms=None) -> None:
         """One temperature step (smc.py:46-60).  The optional arrays inject the
         reference's recorded legacy-RNG streams (parity mode): proposal normals
-        [M_local, D], accept uniforms [M_local], resampling uniforms [M_local] (systematic: [1])."""
+        [M_local, D], accept uniforms [M_local], resampling uniforms [M_local] (systematic: [1]).
+        With ``proposal_kernel``: normals [M_local, normals] and acc_uniforms [M_local, 1 + uniforms] (column 0 the
+        accept uniform, columns 1.. the proposal's u; [M_local] when it draws no uniforms)."""
         self._move(n, normals, acc_uniforms)
         self._resample(n, res_uniforms, 0)
 
@@ -300,11 +358,19 @@ class TemperedLikelihoodSMC:
         Ml = self._hi - self._lo
         self._epoch += 1
         self._acc = torch.empty(Ml, dtype=torch.int32, device=self.device)
-        if normals is not None:
+        nz, nu = self.kernel.stream_widths(self.D)
+        if normals is not None and isinstance(self.kernel, ProposalKernel):
+            normals = to_dev(normals, self.dtype, self.device)
+            acc_uniforms = to_dev(acc_uniforms, self.dtype, self.device)
+            if normals.numel() != Ml * nz or acc_uniforms.numel() != Ml * nu:
+                raise ValueError(f"injected streams of the proposal move: normals [{Ml}, {nz}] and acc_uniforms "
+                                 f"[{Ml}, {nu}] (got {tuple(normals.shape)} and {tuple(acc_uniforms.shape)})")
+            normals, acc_uniforms = normals.reshape(Ml, nz), acc_uniforms.reshape(Ml, nu)
+        elif normals is not None:
             normals = to_dev(normals, self.dtype, self.device).reshape(Ml, self.D)
             acc_uniforms = to_dev(acc_uniforms, self.dtype, self.device).reshape(Ml)
         self._inj = (normals, acc_uniforms)     # keep the injected streams alive until the kernel ran
-        rng = make_rng(self._seed, n, self._lo, normals, acc_uniforms, 1)
+        rng = make_rng(self._seed, n, self._lo, normals, acc_uniforms, nu)
         kn = self.kernel.desc()
         src = None if self._pending else self._src_local.data_ptr()
         accumulate = 1 if (self.ess_threshold is not None and self._epoch > 1) else 0

@@ -96,7 +96,11 @@ typedef struct bk_rng {
  * [n_draws, C, 1 + n_uniforms] (n_uniform = 1 + n_uniforms): column 0 is the accept uniform, column 1 + k the
  * proposal's u[k].  In PHILOX mode z[k] is element k % 4 of the normals of element block b(k) = k / 4, or k / 4 + 1
  * from block ceil(D / 4) on (that block holds the accept uniform of the single-uniform samplers, which is unchanged;
- * with n_normals <= D, z is exactly the random walk's normal vector), and u[k] is the k-th TAG_UNIFORM uniform. */
+ * with n_normals <= D, z is exactly the random walk's normal vector), and u[k] is the k-th TAG_UNIFORM uniform.
+ * The SMC's proposal move (BK_SMC_KERNEL_PROPOSAL) uses the same layout with the particle in place of the chain and
+ * the temperature step n in place of the draw: INJECTED normals [M_local, n_normals] and uniforms
+ * [M_local, 1 + n_uniforms]; PHILOX z and u of (chain_offset + m, n) by the rule above, the accept uniform of
+ * (chain_offset + m, n) by the random-walk move's rule. */
 
 enum { BK_DRAWS_NCD = 0,  /* draws [n_draws, C, D]: one draw of every chain after the other      */
        BK_DRAWS_CDN = 1   /* draws [C, D, n_draws]: every (chain, dim) SERIES contiguous over the
@@ -378,11 +382,27 @@ BK_API int bk_gather_rows(const void* src, const int64_t* idx, int64_t M, int64_
  * ONCE before the first step.  A wait that is not satisfied within 20 s (dead peer) sets mailbox word
  * 0 to 1 and the kernels finish on garbage instead of hanging; 2 = every weight vanished. */
 /* the Markov kernel that moves a particle at temperature time(n-1) (smc.py:54-57):
- *   RW    theta* = theta + scale z, Metropolis test                       (metropolis_kernel, smc.py:79-89)
- *   MALA  one Langevin proposal with step `scale` on the tempered density (mala.py:40-66; smc.py:78 TODO)
- *   HMC   `steps` leapfrog steps of size `scale`, identity metric          (hmc.py:40-63;  smc.py:78 TODO) */
-enum { BK_SMC_KERNEL_RW = 0, BK_SMC_KERNEL_MALA = 1, BK_SMC_KERNEL_HMC = 2 };
-typedef struct bk_smc_kernel { int32_t kind; int32_t steps; double scale; } bk_smc_kernel;
+ *   RW        theta* = theta + scale z, Metropolis test                       (metropolis_kernel, smc.py:79-89)
+ *   MALA      one Langevin proposal with step `scale` on the tempered density (mala.py:40-66; smc.py:78 TODO)
+ *   HMC       `steps` leapfrog steps of size `scale`, identity metric          (hmc.py:40-63;  smc.py:78 TODO)
+ *   PROPOSAL  theta* = propose(theta, z, u) of the user proposal `proposal` (bk_proposal_create_cuda), then the
+ *             Metropolis test on the tempered density plus, when the proposal was created with has_transition,
+ *             the Hastings term transition_log_density(theta, theta*) - transition_log_density(theta*, theta)
+ *             (smc.py:54-57 with any kernel).  User prior/likelihood models only (bk_model_create_cuda_prior_lik;
+ *             restate GAUSS_PRIOR_LIK / BINOMIAL_LOGIT as one): BK_E_UNSUPPORTED otherwise.  The proposal's dims
+ *             and dtype must be the model's and n_normals <= BK_SMC_PROPOSAL_MAX_NORMALS; INJECTED streams need
+ *             n_uniform = 1 + n_uniforms (layout: the note after bk_rng).  `scale` and `steps` are not read.
+ * `proposal` is read only by the PROPOSAL kind: initialisers such as {BK_SMC_KERNEL_RW, 0, scale} leave it 0. */
+enum { BK_SMC_KERNEL_RW = 0, BK_SMC_KERNEL_MALA = 1, BK_SMC_KERNEL_HMC = 2, BK_SMC_KERNEL_PROPOSAL = 3 };
+typedef struct bk_smc_kernel { int32_t kind; int32_t steps; double scale; uint64_t proposal; } bk_smc_kernel;
+/* one thread per particle keeps the proposal's normals in local memory: the bound keeps that array small */
+#define BK_SMC_PROPOSAL_MAX_NORMALS 512
+/* Checks (model, proposal) as bk_smc_shard_move does for the PROPOSAL kind and compiles their fused program
+ * (bk_user_smc_mhp; once per process and pair, shared with bk_mh_cuda_prepare), so that the first move does not
+ * pay the NVRTC compile.  log_out as bk_model_create_cuda's.  BK_E_HANDLE for an unknown handle, BK_E_INVALID
+ * on a bad argument or a compile error (with the log), BK_E_UNSUPPORTED for a model the proposal move does not
+ * serve. */
+BK_API int bk_smc_cuda_prepare(uint64_t model, uint64_t proposal, char* log_out, size_t log_bytes);
 #define BK_SMC_MAX_WORLD 16
 #define BK_SMC_MAILBOX_BYTES 4096
 typedef struct bk_smc_shard {
