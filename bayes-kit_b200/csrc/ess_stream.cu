@@ -244,11 +244,15 @@ __global__ void __launch_bounds__(ES_WARPS * 32, 2) k_ess_stream(SeriesView v, i
 // a whole row apart).  32 x 32 tiles through shared memory: reads coalesced along the series axis,
 // writes along the draw axis.  A warp walking ONE such series would use 4 bytes of every 32-byte
 // sector it touches and a new page per draw.
+// grid.x: 32-series tiles; grid.y: 32-draw tiles tt0, tt0 + 1, ... (gridDim.y is at most 65,535: longer series take
+// several launches, see ess_stream_launch).
+constexpr int64_t ES_GATHER_MAX_TY = 65535;
 template <typename TI>
-__global__ void __launch_bounds__(256) k_gather_series(SeriesView v, int64_t s0, int64_t ns, TI* __restrict__ out) {
+__global__ void __launch_bounds__(256) k_gather_series(SeriesView v, int64_t s0, int64_t ns, int64_t tt0,
+                                                       TI* __restrict__ out) {
     __shared__ TI tile[32][33];
     const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
-    const int64_t sb = (int64_t)blockIdx.x * 32, tb = (int64_t)blockIdx.y * 32;
+    const int64_t sb = (int64_t)blockIdx.x * 32, tb = (tt0 + blockIdx.y) * 32;
     const TI* x = reinterpret_cast<const TI*>(v.x);
     {
         const int64_t s = s0 + sb + tx;
@@ -289,10 +293,14 @@ int ess_stream_launch(const SeriesView& v, int estimator, double* iat, double* e
     void* buf = reinterpret_cast<void*>((reinterpret_cast<uintptr_t>(ws) + 255) & ~(uintptr_t)255);
     for (int64_t s0 = 0; s0 < v.n_series; s0 += chunk) {
         const int64_t ns = v.n_series - s0 < chunk ? v.n_series - s0 : chunk;
-        dim3 grid((unsigned)((ns + 31) / 32), (unsigned)((v.N + 31) / 32));
-        if (v.dtype == BK_F64) k_gather_series<double><<<grid, 256, 0, st>>>(v, s0, ns, (double*)buf);
-        else k_gather_series<float><<<grid, 256, 0, st>>>(v, s0, ns, (float*)buf);
-        BK_LAUNCH_CHECK();
+        const int64_t n_tt = (v.N + 31) / 32;
+        for (int64_t tt0 = 0; tt0 < n_tt; tt0 += ES_GATHER_MAX_TY) {
+            const int64_t ny = n_tt - tt0 < ES_GATHER_MAX_TY ? n_tt - tt0 : ES_GATHER_MAX_TY;
+            dim3 grid((unsigned)((ns + 31) / 32), (unsigned)ny);
+            if (v.dtype == BK_F64) k_gather_series<double><<<grid, 256, 0, st>>>(v, s0, ns, tt0, (double*)buf);
+            else k_gather_series<float><<<grid, 256, 0, st>>>(v, s0, ns, tt0, (float*)buf);
+            BK_LAUNCH_CHECK();
+        }
         const SeriesView sv{buf, v.dtype, ns, v.N, 1, v.N, 0, 1};
         int rc = ess_stream_launch_direct(sv, estimator, iat ? iat + s0 : nullptr, ess ? ess + s0 : nullptr, st);
         if (rc) return rc;
