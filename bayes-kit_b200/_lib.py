@@ -97,6 +97,7 @@ _SIGNATURES = {
     "bk_mh_rw_sample": (C.c_int, [u64, vp, vp, C.POINTER(i32), i64, f64, i32, i64, C.POINTER(Rng),
                                   C.POINTER(DrawOut), vp, sz, vp]),
     "bk_drghmc_workspace_bytes": (sz, [u64, i64, i32]),
+    "bk_drghmc_cuda_prepare": (C.c_int, [u64, C.c_char_p, sz]),
     "bk_drghmc_sample": (C.c_int, [u64, vp, vp, i64, i32, C.POINTER(f64), C.POINTER(i32), f64, i32,
                                    vp, i64, C.POINTER(Rng), C.POINTER(DrawOut), vp, vp, sz, vp]),
     "bk_stretch_workspace_bytes": (sz, [u64, i64]),

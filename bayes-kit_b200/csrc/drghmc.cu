@@ -295,18 +295,27 @@ using namespace bk;
 
 extern "C" {
 
-// the fused register-resident kernel serves iso / diagonal Gaussian plugins up to 256 dims; everything else
-// (dense precision, logistic regression, binomial, D > 256) runs on the lockstep engine of drghmc_generic.cu
-static bool drghmc_fused(const Model& m) {
+static bool force_generic() {
     const char* e = getenv("BK_FORCE_GENERIC");   // test hook: both engines must produce the same chains
-    const bool force = e && e[0] == '1';
-    return !force && m.separable() && m.d.dims <= 256;
+    return e && e[0] == '1';
 }
+// the fused register-resident kernel serves iso / diagonal Gaussian plugins up to 256 dims, the runtime-compiled
+// bk_user_drghmc (user_model.cu) user models up to USER_FUSED_MAX_D; everything else (dense precision, logistic
+// regression, binomial, D > 256, larger user models) runs on the lockstep engine of drghmc_generic.cu
+static bool drghmc_fused(const Model& m) { return !force_generic() && m.separable() && m.d.dims <= 256; }
+static bool drghmc_user_fused(const Model& m) { return !force_generic() && user_fused(m); }
 
 size_t bk_drghmc_workspace_bytes(uint64_t handle, int64_t C, int32_t max_proposals) {
     const Model* m = get_model(handle);
-    if (!m || drghmc_fused(*m)) return 0;
+    if (!m || drghmc_fused(*m) || drghmc_user_fused(*m)) return 0;
     return drghmc_generic_ws_bytes(*m, C, max_proposals);
+}
+
+int bk_drghmc_cuda_prepare(uint64_t handle, char* log_out, size_t log_bytes) {
+    if (log_out && log_bytes) log_out[0] = '\0';
+    const Model* m = get_model(handle);
+    if (!m) return BK_E_HANDLE;
+    return drghmc_user_fused(*m) ? user_drghmc_prepare(*m, log_out, log_bytes) : BK_OK;
 }
 
 int bk_drghmc_sample(uint64_t handle, void* theta, void* rho, int64_t C, int32_t max_proposals,
@@ -337,6 +346,9 @@ int bk_drghmc_sample(uint64_t handle, void* theta, void* rho, int64_t C, int32_t
     }
     bk_draw_out o = out ? *out : bk_draw_out{nullptr, nullptr, nullptr};
     if (C == 0 || n_draws == 0) return BK_OK;
+    if (drghmc_user_fused(*m))
+        return user_drghmc_sample(*m, theta, rho, C, max_proposals, step_sizes_host, step_counts_host, damping,
+                                  prob_retry, metric, n_draws, rng, o, n_uniform_used_out, (cudaStream_t)stream);
     if (!drghmc_fused(*m))
         return drghmc_generic(*m, theta, rho, C, max_proposals, step_sizes_host, step_counts_host, damping, prob_retry,
                               metric, n_draws, rng, o, n_uniform_used_out, ws, ws_bytes, (cudaStream_t)stream);

@@ -48,6 +48,14 @@ bool user_prior_lik(const Model& m);
 int user_log_prior_likelihood(const Model& m, const void* theta, int64_t C, void* lprior, void* llik, cudaStream_t st);
 int user_smc_move(const Model& m, int move, const UserSmcArgs& a, cudaStream_t st);
 
+// DrGhmcDiag on a user model with dims <= USER_FUSED_MAX_D: bk_user_drghmc, from a program of its own per model library
+// compiled (once per process) by user_drghmc_prepare or on the first user_drghmc_sample; log_out as
+// bk_model_create_cuda's.  K <= DR_KMAX (drghmc.cu).
+int user_drghmc_prepare(const Model& m, char* log_out, size_t log_bytes);
+int user_drghmc_sample(const Model& m, void* theta, void* rho, int64_t C, int K, const double* sizes,
+                       const int32_t* counts, double damping, int prob_retry, const void* metric, int64_t n,
+                       const bk_rng* rng, const bk_draw_out& out, int32_t* n_used, cudaStream_t st);
+
 // user-written CUDA proposals (bk_proposal_create_cuda, user_model.cu)
 struct UserProposal {
     const struct PropLib* lib;   // the compiled proposal-only program (bk_user_propose)

@@ -31,6 +31,9 @@
 // bk_user_smc_mhp   (prior/likelihood model + proposal programs) TemperedLikelihoodSMC's move + weight kernel with
 //                   one Metropolis(-Hastings) step of the user's proposal as the move: bk_user_smc_rw with propose()
 //                   in place of the random walk (BK_SMC_KERNEL_PROPOSAL).
+// bk_user_drghmc    (DrGHMC programs: a model's source compiled with -DBK_DRGHMC=1, which compiles this kernel and no
+//                   other) DrGhmcDiag, one thread per chain: k_drghmc (drghmc.cu) on the arithmetic and streams of
+//                   the lockstep engine (drghmc_generic.cu).
 #pragma once
 #ifndef __CUDACC_RTC__
 #include "smc_mailbox.cuh"
@@ -59,6 +62,22 @@ struct UserRunArgs {
     const void* prop_params;  // bk_user_mhp: the proposal's [n_params] or NULL
 };
 
+#if !defined(__CUDACC_RTC__) || defined(BK_DRGHMC)
+// Launch arguments of bk_user_drghmc.  `run` holds what bk_user_hmc reads (theta, params, metric, the streams with
+// n_uniform = 2K when injected, draws / logp / accept); step sizes and the damping terms are rounded to the dtype in
+// the kernel, as the lockstep engine rounds them on the host.
+constexpr int USER_DR_KMAX = 6;   // drghmc.cu's DR_KMAX: bk_drghmc_sample refuses a larger K before dispatching
+struct UserDrArgs {
+    UserRunArgs run;
+    void* rho;                        // [C, D] in/out: the persistent momentum
+    int32_t* n_used;                  // [n, C] uniforms consumed per draw, or NULL
+    int32_t K, prob_retry;
+    int32_t cnt[USER_DR_KMAX];        // leapfrog steps of proposal k
+    double eps[USER_DR_KMAX], half_eps[USER_DR_KMAX];
+    double s_keep, s_new;             // sqrt(1 - damping), sqrt(damping)
+};
+#endif
+
 // Launch arguments of bk_user_propose (one draw of a user proposal for C chains, three-launch path).  Streams: injected
 // normals [n, C, BK_PROPOSAL_NORMALS] and uniforms [n, C, n_uniform] (column 0: the accept uniform, columns 1 + k:
 // u[k]); in Philox mode the kernel writes this draw's z / u into zbuf [C, BK_PROPOSAL_NORMALS] / ubuf
@@ -77,7 +96,7 @@ struct UserProposeArgs {
     int32_t rng_mode, n_uniform;
 };
 
-#if !defined(__CUDACC_RTC__) || defined(BK_PRIOR_LIK)
+#if !defined(__CUDACC_RTC__) || (defined(BK_PRIOR_LIK) && !defined(BK_DRGHMC))
 // Launch arguments of bk_user_smc_rw / _mala / _hmc: SmcArgs<T> of smc.cu with plain fields (the host (nvcc) and the
 // kernels (NVRTC) must agree on the layout).  Pointers are in the model's dtype unless typed.
 struct UserSmcArgs {
@@ -232,8 +251,9 @@ __device__ __forceinline__ T proposal_dh(const T* th, const T* q, const T* pp) {
 
 #endif  // BK_PROPOSAL
 
-// Model programs compile the kernels below; proposal programs only bk_user_propose / bk_user_mhp / bk_user_smc_mhp.
-#ifndef BK_PROPOSAL
+// Model programs compile the kernels below; proposal programs only bk_user_propose / bk_user_mhp / bk_user_smc_mhp,
+// DrGHMC programs only bk_user_drghmc.
+#if !defined(BK_PROPOSAL) && !defined(BK_DRGHMC)
 
 // theta [C, D] -> lp [C] (nullable), grad [C, D]
 extern "C" __global__ void __launch_bounds__(128) bk_user_eval(const bk_real* __restrict__ theta, long long C,
@@ -404,8 +424,9 @@ extern "C" __global__ void __launch_bounds__(128) bk_user_mh(const bk::UserRunAr
 #endif  // BK_DIMS <= BK_USER_FUSED_MAX_D
 #endif  // !BK_PROPOSAL
 
-// The prior / likelihood kernels are compiled only for models created by bk_model_create_cuda_prior_lik.
-#ifdef BK_PRIOR_LIK
+// The prior / likelihood kernels are compiled only for models created by bk_model_create_cuda_prior_lik (DrGHMC
+// programs of such models: only the derived log_density_gradient above, without the SMC protocol header).
+#if defined(BK_PRIOR_LIK) && !defined(BK_DRGHMC)
 #ifndef BK_PROPOSAL
 
 // theta [C, D] -> log_prior [C], log_likelihood [C] (each nullable)
@@ -612,7 +633,7 @@ extern "C" __global__ void __launch_bounds__(128) bk_user_smc_hmc(const bk::User
 extern "C" __global__ void __launch_bounds__(128) bk_user_smc_mhp(const bk::UserSmcArgs a) { bk::user::smc_move<3>(a); }
 #endif
 
-#endif  // BK_PRIOR_LIK
+#endif  // BK_PRIOR_LIK && !BK_DRGHMC
 
 #ifdef BK_PROPOSAL
 
@@ -689,4 +710,190 @@ extern "C" __global__ void __launch_bounds__(128) bk_user_mhp(const bk::UserRunA
 
 #endif  // BK_PROPOSAL_ONLY
 #endif  // BK_PROPOSAL
+
+// ---- DrGhmcDiag (DrGHMC programs, -DBK_DRGHMC=1) -------------------------------------------------------------------
+// One chain per thread follows its own retry / accept / ghost schedule (drghmc.py:348-446) and integrates only the
+// trajectories that schedule reaches; the lockstep engine integrates every trajectory a chain could need.  Every point
+// carries its own (log p, grad log p), as the lockstep engine's levels do: theta's pair across attempts and draws, a
+// proposal's from the last evaluation of its trajectory, so a trajectory of cnt steps costs cnt evaluations.
+// The proposal recursion is compile-time (DrAccept<k>, the shape of drghmc.cu's Accept<k>) with a __noinline__ run()
+// per level, and every trajectory goes through one __noinline__ trajectory(): the user's function is inlined twice
+// (at entry and in trajectory()) whatever K is, which bounds NVRTC's work for a heavy model.
+#ifdef BK_DRGHMC
+
+namespace bk {
+namespace user {
+
+struct DrCtx {
+    const T* params;
+    const T* metric;   // [D] or NULL (identity)
+    T eps[USER_DR_KMAX], half[USER_DR_KMAX];
+    int cnt[USER_DR_KMAX];
+    int prob_retry;
+};
+
+// drghmc.py:317: bool * float (False * -inf = nan on purpose)
+__device__ __forceinline__ T dr_retry(const DrCtx& c, T reject_logp) {
+    return c.prob_retry ? reject_logp : A::mul(T(0), reject_logp);
+}
+__device__ __forceinline__ T dr_log1m_exp(T a) { return A::log1p_(-A::exp_(a)); }   // np.log1p(-np.exp(a))
+__device__ __forceinline__ T dr_mg(const DrCtx& c, int e, T g) { return c.metric ? A::mul(c.metric[e], g) : g; }
+
+// the k-th uniform of (chain c, draw t): drg_uniform (drghmc_generic.cu)
+__device__ __forceinline__ T dr_uniform(const UserRunArgs& a, int64_t c, int64_t t, int k) {
+    if (a.rng_mode == 1) return reinterpret_cast<const T*>(a.uniforms)[(t * a.C + c) * a.n_uniform + k];   // INJECTED
+    return philox_uniform<T>(a.seed, (uint32_t)k, (uint32_t)(a.chain_offset + (uint64_t)c),
+                             (uint32_t)(a.draw_offset + (uint64_t)t));
+}
+
+// proposal_map (drghmc.py:319-346) of proposal i from (q0, r0, g0): k_drg_first, then cnt - 1 times (evaluate,
+// k_drg_step), evaluate, k_drg_last.  Leaves the end point's pair in (lp, g) and returns its joint log density
+// lp - kinetic(r).
+__device__ __noinline__ T trajectory(const DrCtx& c, int i, const T (&q0)[D], const T (&r0)[D], const T (&g0)[D],
+                                     T (&q)[D], T (&r)[D], T (&g)[D], T& lp) {
+    const T eps = c.eps[i], half = c.half[i];
+    T qq[D], rr[D], gg[D];
+#pragma unroll
+    for (int e = 0; e < D; ++e) {
+        rr[e] = A::add(r0[e], A::mul(half, dr_mg(c, e, g0[e])));
+        qq[e] = A::add(q0[e], A::mul(eps, rr[e]));
+    }
+    T l;
+    for (int s = 1;; ++s) {
+        l = log_density_gradient(qq, gg, c.params);
+        if (s == c.cnt[i]) break;
+#pragma unroll
+        for (int e = 0; e < D; ++e) {
+            rr[e] = A::add(rr[e], A::mul(eps, dr_mg(c, e, gg[e])));
+            qq[e] = A::add(qq[e], A::mul(eps, rr[e]));
+        }
+    }
+    T kin = T(0);
+#pragma unroll
+    for (int e = 0; e < D; ++e) {
+        const T re = -A::add(rr[e], A::mul(half, dr_mg(c, e, gg[e])));
+        kin = A::add(kin, A::mul(re, dr_mg(c, e, re)));
+        q[e] = qq[e];
+        r[e] = re;
+        g[e] = gg[e];
+    }
+    lp = l;
+    return A::sub(l, A::mul(T(0.5), kin));
+}
+
+// log acceptance probability of proposal K, the point (qp, rp, gp) with joint log density prop_logp, made from a state
+// with (cur_hastings, cur_logp): drghmc.py:391-446
+template <int K>
+struct DrAccept {
+    // ghosts I .. K - 1 of the point (drghmc.py:424-436); true on the early exit at accept_logp == 0
+    template <int I>
+    static __device__ __forceinline__ bool ghosts(const DrCtx& c, const T (&qp)[D], const T (&rp)[D],
+                                                  const T (&gp)[D], T prop_logp, T& prop_hastings) {
+        if constexpr (I < K) {
+            T qg[D], rg[D], gg[D], lg;
+            const T jg = trajectory(c, I, qp, rp, gp, qg, rg, gg, lg);
+            const T ai = DrAccept<I>::run(c, qg, rg, gg, jg, prop_hastings, prop_logp);
+            if (ai == T(0)) return true;
+            prop_hastings = A::add(prop_hastings, dr_log1m_exp(ai));
+            return ghosts<I + 1>(c, qp, rp, gp, prop_logp, prop_hastings);
+        } else {
+            return false;
+        }
+    }
+
+    static __device__ __noinline__ T run(const DrCtx& c, const T (&qp)[D], const T (&rp)[D], const T (&gp)[D],
+                                         T prop_logp, T cur_hastings, T cur_logp) {
+        T prop_hastings = T(0);
+        if (ghosts<0>(c, qp, rp, gp, prop_logp, prop_hastings)) return neg_inf<T>();
+        const T frac = A::add(A::add(A::sub(prop_logp, cur_logp), A::sub(prop_hastings, cur_hastings)),
+                              A::sub(dr_retry(c, prop_hastings), dr_retry(c, cur_hastings)));
+        return frac < T(0) ? frac : T(0);   // python min(0, frac): nan -> 0
+    }
+};
+
+// DrAccept<k>::run for a run-time k < K <= USER_DR_KMAX
+template <int K>
+__device__ __forceinline__ T dr_accept(int k, const DrCtx& c, const T (&qp)[D], const T (&rp)[D], const T (&gp)[D],
+                                       T prop_logp, T cur_hastings, T cur_logp) {
+    if constexpr (K < USER_DR_KMAX) {
+        if (k == K) return DrAccept<K>::run(c, qp, rp, gp, prop_logp, cur_hastings, cur_logp);
+        return dr_accept<K + 1>(k, c, qp, rp, gp, prop_logp, cur_hastings, cur_logp);
+    } else {
+        return neg_inf<T>();
+    }
+}
+
+}  // namespace user
+}  // namespace bk
+
+// theta, rho [C, D] in/out; per draw (drghmc.py:348-389): partial momentum refresh, up to K attempts (retry test,
+// proposal, accept test), unconditional momentum flip
+extern "C" __global__ void __launch_bounds__(128) bk_user_drghmc(const bk::UserDrArgs a) {
+    using namespace bk::user;
+    const bk::UserRunArgs& ra = a.run;
+    const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= ra.C) return;
+    DrCtx ctx;
+    ctx.params = reinterpret_cast<const T*>(ra.params);
+    ctx.metric = reinterpret_cast<const T*>(ra.metric);
+#pragma unroll
+    for (int k = 0; k < bk::USER_DR_KMAX; ++k) {
+        ctx.eps[k] = (T)a.eps[k];
+        ctx.half[k] = (T)a.half_eps[k];
+        ctx.cnt[k] = a.cnt[k];
+    }
+    ctx.prob_retry = a.prob_retry;
+    const T s_keep = (T)a.s_keep, s_new = (T)a.s_new;
+    T* row = reinterpret_cast<T*>(ra.theta) + c * (int64_t)D;
+    T* rrow = reinterpret_cast<T*>(a.rho) + c * (int64_t)D;
+    T th[D], rho[D], g[D];
+    load_row(row, th);
+    load_row(rrow, rho);
+    T lp = log_density_gradient(th, g, ctx.params);
+    for (int64_t t = 0; t < ra.n_draws; ++t) {
+        T z[D];
+        normals(ra, c, t, z);
+        T kin = T(0);
+#pragma unroll
+        for (int e = 0; e < D; ++e) {   // k_drg_refresh
+            rho[e] = A::add(A::mul(rho[e], s_keep), A::mul(s_new, z[e]));
+            kin = A::add(kin, A::mul(rho[e], dr_mg(ctx, e, rho[e])));
+        }
+        T cur_logp = A::sub(lp, A::mul(T(0.5), kin));
+        T cur_hastings = T(0), reject_logp = T(0);
+        int ui = 0;
+        bool moved = false;
+        for (int k = 0; k < a.K; ++k) {
+            if (!(bk::log_u(dr_uniform(ra, c, t, ui++)) < dr_retry(ctx, reject_logp))) break;   // drghmc.py:369-371
+            T qp[D], rp[D], gp[D], lpp;
+            const T jp = trajectory(ctx, k, th, rho, g, qp, rp, gp, lpp);
+            const T acc_lp = dr_accept<0>(k, ctx, qp, rp, gp, jp, cur_hastings, cur_logp);
+            if (bk::log_u(dr_uniform(ra, c, t, ui++)) < acc_lp) {   // drghmc.py:378-381
+#pragma unroll
+                for (int e = 0; e < D; ++e) {
+                    th[e] = qp[e];
+                    rho[e] = rp[e];
+                    g[e] = gp[e];
+                }
+                lp = lpp;
+                cur_logp = jp;
+                moved = true;
+                break;
+            }
+            reject_logp = dr_log1m_exp(acc_lp);
+            cur_hastings = A::add(cur_hastings, reject_logp);
+        }
+#pragma unroll
+        for (int e = 0; e < D; ++e) rho[e] = -rho[e];   // drghmc.py:388
+        emit(ra, c, t, th, cur_logp, moved);
+        if (a.n_used) a.n_used[t * ra.C + c] = ui;
+    }
+#pragma unroll
+    for (int e = 0; e < D; ++e) {
+        row[e] = th[e];
+        rrow[e] = rho[e];
+    }
+}
+
+#endif  // BK_DRGHMC
 #endif  // __CUDACC_RTC__

@@ -12,6 +12,7 @@ import torch
 from . import _lib as L
 from ._sampler import ChainSampler, _is_empty_init
 from ._util import ptr, stream_ptr, to_dev
+from .models import CudaModel
 
 
 class DrGhmcDiag(ChainSampler):
@@ -26,7 +27,12 @@ class DrGhmcDiag(ChainSampler):
     (drghmc.py:391-446), unconditional momentum flip.  ``sample()`` returns
     ``(theta, joint_logp)``.  Every chain follows its own data-dependent
     proposal schedule inside one fused kernel (explicit recursion on the
-    proposal index instead of Python recursion).
+    proposal index instead of Python recursion) on iso / diagonal Gaussians
+    and on a ``CudaModel`` / ``CudaPriorLikModel`` with ``dims <= 32``; the
+    latter's kernel is compiled from the model's source at construction
+    (``compile_log``: ptxas's report, ``""`` on every other engine; a compile
+    error raises ``ValueError`` with NVRTC's log).  Every other model runs
+    the lockstep engine.
     """
 
     def __init__(self, model, max_proposals, leapfrog_step_sizes, leapfrog_step_counts, damping,
@@ -54,6 +60,16 @@ class DrGhmcDiag(ChainSampler):
         self._sizes = (C.c_double * int(max_proposals))(*[float(s) for s in leapfrog_step_sizes])
         self._counts = (C.c_int32 * int(max_proposals))(*[int(c) for c in leapfrog_step_counts])
         self.last_n_uniform = None
+        self.compile_log = ""
+        if isinstance(self._model, CudaModel):
+            log = C.create_string_buffer(1 << 20)
+            with torch.cuda.device(self.device):     # compile the fused kernel now, not in the first sample()
+                rc = L.lib().bk_drghmc_cuda_prepare(self._model.handle, log, len(log))
+            if rc == L.BK_E_INVALID and log.value:
+                raise ValueError("DrGhmcDiag: NVRTC compilation of the model's DrGHMC kernel failed:\n"
+                                 + log.value.decode(errors="replace"))
+            L.check(rc)
+            self.compile_log = log.value.decode(errors="replace")   # the fused kernel's, or "" (lockstep engine)
 
     @property
     def rho(self) -> torch.Tensor:

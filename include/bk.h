@@ -286,8 +286,19 @@ BK_API int bk_mh_cuda_sample(uint64_t model, uint64_t proposal, void* theta, voi
 /* ---- DrGhmcDiag (drghmc.py:37-446) --------------------------------------
  * theta, rho [C,D] in/out; step_sizes_host[K], step_counts_host[K].
  * uniforms are consumed retry-test then accept-test per attempt
- * (drghmc.py:370,378): rng->n_uniform must be 2K in INJECTED mode. */
+ * (drghmc.py:370,378): rng->n_uniform must be 2K in INJECTED mode.
+ * Engines: iso / diagonal Gaussian plugins up to 256 dims run one fused kernel; a user model
+ * (bk_model_create_cuda*) with dims <= 32 runs one fused kernel per call too (bk_user_drghmc: one
+ * thread per chain, theta, rho, the gradient and log p(theta) in registers across the draws; compiled
+ * from the model's source in a program of its own, once per process, by bk_drghmc_cuda_prepare or on
+ * the first call); every other model runs the lockstep engine, with scratch from
+ * bk_drghmc_workspace_bytes (0 on the fused engines). */
 BK_API size_t bk_drghmc_workspace_bytes(uint64_t handle, int64_t C, int32_t max_proposals);
+/* Compiles and loads the fused DrGHMC program of a user model that takes that engine, so that the first
+ * bk_drghmc_sample does not pay the NVRTC compile; log_out as bk_model_create_cuda's (ptxas's report of
+ * bk_user_drghmc).  BK_OK with an empty log for any other model, BK_E_HANDLE for an unknown handle,
+ * BK_E_INVALID on a compile error (with the log), BK_E_UNSUPPORTED without NVRTC. */
+BK_API int bk_drghmc_cuda_prepare(uint64_t handle, char* log_out, size_t log_bytes);
 BK_API int bk_drghmc_sample(uint64_t handle, void* theta, void* rho, int64_t C, int32_t max_proposals,
                      const double* step_sizes_host, const int32_t* step_counts_host,
                      double damping, int32_t prob_retry, const void* metric, int64_t n_draws,
