@@ -2,6 +2,8 @@
 streams and torch.distributed; never the compute path)."""
 from __future__ import annotations
 
+import ctypes as C
+
 import numpy as np
 import torch
 
@@ -57,6 +59,20 @@ class Workspace:
         if self.buf is None or self.buf.numel() < nbytes:
             self.buf = torch.empty(nbytes, dtype=torch.uint8, device=self.device)
         return self.buf.data_ptr(), self.buf.numel()
+
+
+def compile_log(call, prefix: str, device) -> str:
+    """Run ``call(log, log_bytes)``, a library entry point that compiles a user program (NVRTC) and fills its log, on
+    ``device``; return the decoded log.  A compile error (``BK_E_INVALID`` with a log) raises ``ValueError(prefix +
+    log)``, any other failure ``L.check``'s error."""
+    log = C.create_string_buffer(1 << 20)
+    with torch.cuda.device(device):
+        rc = call(log, len(log))
+    text = log.value.decode(errors="replace")
+    if rc == L.BK_E_INVALID and text:
+        raise ValueError(prefix + text)
+    L.check(rc)
+    return text
 
 
 def make_rng(seed, draw_offset, chain_offset, normals=None, uniforms=None, n_uniform=1) -> L.Rng:

@@ -9,6 +9,11 @@
 
 using namespace bk;
 
+bool bk::force_generic() {
+    const char* e = getenv("BK_FORCE_GENERIC");
+    return e && e[0] == '1';
+}
+
 namespace {
 
 bool ptr_aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
@@ -31,38 +36,11 @@ struct Common {
     bk_draw_out out;
 };
 
-// BK_FORCE_GENERIC=1 routes separable plugins through the generic engine too
-// (test hook: both engines must produce the same chains).
-bool force_generic() {
-    const char* e = getenv("BK_FORCE_GENERIC");
-    return e && e[0] == '1';
-}
-
 template <typename T>
 bool use_fused(const Model& m) { return m.separable() && m.d.dims <= SEP_MAX_D && !force_generic(); }
 
 // user-written CUDA model with D <= USER_FUSED_MAX_D: one register-resident kernel per call (user_model.cu)
 bool use_user_fused(const Model& m) { return user_fused(m) && !force_generic(); }
-
-UserRunArgs user_args(const Model& m, void* theta, int64_t C, int64_t n, const bk_rng* rng, const bk_draw_out& out) {
-    UserRunArgs a;
-    memset(&a, 0, sizeof(a));
-    a.theta = theta;
-    a.params = m.user_params;
-    a.normals = rng->normals;
-    a.uniforms = rng->uniforms;
-    a.draws = out.draws;
-    a.logp = out.logp;
-    a.accept = out.accept;
-    a.C = C;
-    a.n_draws = n;
-    a.seed = rng->seed;
-    a.draw_offset = rng->draw_offset;
-    a.chain_offset = rng->chain_offset;
-    a.rng_mode = rng->mode;
-    a.n_uniform = rng->n_uniform;
-    return a;
-}
 
 template <typename T>
 void fill_sep(SepArgs<T>& a, const Model& m, void* theta, int64_t C, const void* metric, int64_t n,
@@ -126,7 +104,7 @@ int hmc_t(const Model& m, void* theta, void* lp, void* grad, int32_t* valid, int
         a.eps = eps;
         a.half_eps = 0.5 * eps;
         a.L = L;
-        return user_fused_sample(m, ALGO_HMC, a, valid, st);
+        return user_fused_sample(m, nullptr, ALGO_HMC, a, valid, st);
     }
     BK_CHECK_ARG(lp && grad, "bk_hmc_diag_sample: lp_cache/grad_cache are required for this model");
     if constexpr (sizeof(T) == 4) {
@@ -162,7 +140,7 @@ int mala_t(const Model& m, void* theta, void* lp, void* grad, int32_t* valid, in
         a.eps = eps;
         a.sd = sd;
         a.coef = coef;
-        return user_fused_sample(m, ALGO_MALA, a, valid, st);
+        return user_fused_sample(m, nullptr, ALGO_MALA, a, valid, st);
     }
     BK_CHECK_ARG(lp && grad, "bk_mala_sample: lp_cache/grad_cache are required for this model");
     if constexpr (sizeof(T) == 4) {
@@ -198,7 +176,7 @@ int mh_t(const Model& m, void* theta, void* lp, int32_t* valid, int64_t C, doubl
         a.scale = scale;
         a.s2 = scale * scale;
         a.hastings = hastings;
-        return user_fused_sample(m, ALGO_MHRW, a, valid, st);
+        return user_fused_sample(m, nullptr, ALGO_MHRW, a, valid, st);
     }
     BK_CHECK_ARG(lp, "bk_mh_rw_sample: lp_cache is required for this model");
     GenArgs<T> p;
@@ -251,7 +229,7 @@ int mh_cuda_t(const Model& m, const UserProposal& pr, void* theta, void* lp, int
         UserRunArgs a = user_args(m, theta, C, n, &r, out);
         a.hastings = hastings;
         a.prop_params = pr.params;
-        return user_mhp_sample(m, pr, a, valid, st);
+        return user_fused_sample(m, &pr, ALGO_MHRW, a, valid, st);
     }
     BK_CHECK_ARG(lp, "bk_mh_cuda_sample: lp_cache is required for this model");
     Arena ar(ws, wsb);

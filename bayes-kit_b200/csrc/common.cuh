@@ -51,6 +51,10 @@ inline void count_launch(uint64_t n = 1) { g_launches.fetch_add(n, std::memory_o
 void prof_begin(int tag, cudaStream_t st);
 void prof_end(int tag, cudaStream_t st);
 
+// BK_FORCE_GENERIC=1 routes every model through the generic engines (test hook: both engines must produce the same
+// chains)
+bool force_generic();
+
 inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
 // bump allocator over the caller-provided workspace

@@ -295,10 +295,6 @@ using namespace bk;
 
 extern "C" {
 
-static bool force_generic() {
-    const char* e = getenv("BK_FORCE_GENERIC");   // test hook: both engines must produce the same chains
-    return e && e[0] == '1';
-}
 // the fused register-resident kernel serves iso / diagonal Gaussian plugins up to 256 dims, the runtime-compiled
 // bk_user_drghmc (user_model.cu) user models up to USER_FUSED_MAX_D; everything else (dense precision, logistic
 // regression, binomial, D > 256, larger user models) runs on the lockstep engine of drghmc_generic.cu

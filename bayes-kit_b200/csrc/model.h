@@ -17,7 +17,7 @@ struct Model {
     __nv_bfloat16* Xlo = nullptr;   // [Np, 128] bf16(X - Xb): split-precision logits
     float* yp = nullptr;            // [Np] responses, zero padded
     float* yh = nullptr;            // [Np] responses - 1/2 (0 on padded rows)
-    const struct UserLib* user = nullptr;   // USER_CUDA: the runtime-compiled kernels (user_model.cu)
+    const struct Program* user = nullptr;   // USER_CUDA: the model's runtime-compiled program (user_model.cu)
     const void* user_params = nullptr;      // USER_CUDA: [n_params] caller array, dtype
     bool separable() const {
         return d.kind == BK_MODEL_ISO_GAUSS || d.kind == BK_MODEL_DIAG_GAUSS;
@@ -37,44 +37,42 @@ int register_model(const Model& m, uint64_t* handle_out);
 #endif
 constexpr int USER_FUSED_MAX_D = BK_USER_FUSED_MAX_D;
 struct UserRunArgs;
-int user_eval(const Model& m, const void* theta, int64_t C, void* lp, void* grad, void* ws, size_t ws_bytes,
-              cudaStream_t st);
-bool user_fused(const Model& m);
-int user_fused_sample(const Model& m, int algo, const UserRunArgs& a, int32_t* cache_valid, cudaStream_t st);
-// prior/likelihood user models (bk_model_create_cuda_prior_lik): log_prior / log_likelihood of theta [C, D] (each
-// output nullable) and TemperedLikelihoodSMC's move + weight kernel (move: BK_SMC_KERNEL_*)
 struct UserSmcArgs;
-bool user_prior_lik(const Model& m);
-int user_log_prior_likelihood(const Model& m, const void* theta, int64_t C, void* lprior, void* llik, cudaStream_t st);
-int user_smc_move(const Model& m, int move, const UserSmcArgs& a, cudaStream_t st);
-
-// DrGhmcDiag on a user model with dims <= USER_FUSED_MAX_D: bk_user_drghmc, from a program of its own per model library
-// compiled (once per process) by user_drghmc_prepare or on the first user_drghmc_sample; log_out as
-// bk_model_create_cuda's.  K <= DR_KMAX (drghmc.cu).
-int user_drghmc_prepare(const Model& m, char* log_out, size_t log_bytes);
-int user_drghmc_sample(const Model& m, void* theta, void* rho, int64_t C, int K, const double* sizes,
-                       const int32_t* counts, double damping, int prob_retry, const void* metric, int64_t n,
-                       const bk_rng* rng, const bk_draw_out& out, int32_t* n_used, cudaStream_t st);
-
-// user-written CUDA proposals (bk_proposal_create_cuda, user_model.cu)
+struct UserProposeArgs;
+// user-written CUDA proposals (bk_proposal_create_cuda)
 struct UserProposal {
-    const struct PropLib* lib;   // the compiled proposal-only program (bk_user_propose)
+    const struct Program* lib;   // the proposal's own program (bk_user_propose)
     int64_t dims;
     int32_t dtype, n_normals, n_uniforms, has_transition;
     const void* params;          // [n_params] caller array, dtype, or NULL
 };
 // returns nullptr (and sets the error) for an unknown handle
 const UserProposal* get_proposal(uint64_t handle);
+
+int user_eval(const Model& m, const void* theta, int64_t C, void* lp, void* grad, void* ws, size_t ws_bytes,
+              cudaStream_t st);
+bool user_fused(const Model& m);
+// theta, the model's params, the streams and the outputs of a fused launch; the caller sets the sampler's fields
+UserRunArgs user_args(const Model& m, void* theta, int64_t C, int64_t n, const bk_rng* rng, const bk_draw_out& out);
+// bk_user_hmc / mala / mh (algo: ALGO_*), or with a proposal p bk_user_mhp of the program of (m, p)
+int user_fused_sample(const Model& m, const UserProposal* p, int algo, const UserRunArgs& a, int32_t* cache_valid,
+                      cudaStream_t st);
+// prior/likelihood user models (bk_model_create_cuda_prior_lik): log_prior / log_likelihood of theta [C, D] (each
+// output nullable) and TemperedLikelihoodSMC's move + weight kernel (move: BK_SMC_KERNEL_*; the PROPOSAL move runs
+// bk_user_smc_mhp of the program of (m, p))
+bool user_prior_lik(const Model& m);
+int user_log_prior_likelihood(const Model& m, const void* theta, int64_t C, void* lprior, void* llik, cudaStream_t st);
+int user_smc_move(const Model& m, const UserProposal* p, int move, const UserSmcArgs& a, cudaStream_t st);
 // the fused bk_user_mhp serves (m, p): a user model with dims <= USER_FUSED_MAX_D and n_normals <= USER_FUSED_MAX_D
 bool user_mhp_fusable(const Model& m, const UserProposal& p);
-// compiles (once per process) and loads the fused program of (m, p) -- bk_user_mhp and, for a prior/likelihood model,
-// bk_user_smc_mhp; log_out as bk_model_create_cuda's, `who` names the caller in errors
+// The programs of (m, p) and of m's DrGHMC kernel are compiled (once per process) by these or on their first launch;
+// log_out as bk_model_create_cuda's, `who` names the caller in errors.  K <= DR_KMAX (drghmc.cu).
 int user_mhp_prepare(const Model& m, const UserProposal& p, const char* who, char* log_out, size_t log_bytes);
-int user_mhp_sample(const Model& m, const UserProposal& p, const UserRunArgs& a, int32_t* cache_valid, cudaStream_t st);
-// the SMC's proposal move (BK_SMC_KERNEL_PROPOSAL): bk_user_smc_mhp of the fused program of (m, p), prior_lik models
-int user_smc_mhp(const Model& m, const UserProposal& p, const UserSmcArgs& a, cudaStream_t st);
+int user_drghmc_prepare(const Model& m, char* log_out, size_t log_bytes);
+int user_drghmc_sample(const Model& m, void* theta, void* rho, int64_t C, int K, const double* sizes,
+                       const int32_t* counts, double damping, int prob_retry, const void* metric, int64_t n,
+                       const bk_rng* rng, const bk_draw_out& out, int32_t* n_used, cudaStream_t st);
 // three-launch path: Philox scratch of bk_user_propose ([C, n_normals] and [C, n_uniforms]) and its launch
-struct UserProposeArgs;
 size_t user_propose_ws_bytes(const UserProposal& p, int64_t C);
 int user_propose(const UserProposal& p, const UserProposeArgs& a, cudaStream_t st);
 

@@ -406,13 +406,13 @@ static int smc_user(const Model& m, const SmcArgs<T>& a, const bk_smc_kernel& kn
     u.maxpart = a.maxpart;
     u.ticket = a.ticket;
     u.params = m.user_params;
+    const UserProposal* p = nullptr;
     if (kn.kind == BK_SMC_KERNEL_PROPOSAL) {   // check_smc_model resolved the handle
-        const UserProposal* p = get_proposal(kn.proposal);
+        p = get_proposal(kn.proposal);
         if (!p) return BK_E_HANDLE;
         u.prop_params = p->params;
-        return user_smc_mhp(m, *p, u, st);
     }
-    return user_smc_move(m, kn.kind, u, st);
+    return user_smc_move(m, p, kn.kind, u, st);
 }
 
 // fills the model / geometry part of the arguments and picks the lane layout

@@ -1,14 +1,23 @@
-// Kernels of a user-written CUDA model (BK_MODEL_USER_CUDA, bk.h).  The host side (user_model.cu, smc.cu) includes
-// this file for the launch-argument structs only; the kernels are compiled at run time by NVRTC, one library per
-// (source, D, dtype, prior_lik), from
-//   integer typedefs + device_rng.cuh + `typedef float|double bk_real;` [+ smc_mailbox.cuh] + the user's source
-//   + this file
-// with -DBK_DIMS=D.  The user's source defines either
+// Kernels of user-written CUDA programs (BK_MODEL_USER_CUDA models and user proposals, bk.h).  The host side
+// (user_model.cu, smc.cu) includes this file for the launch-argument structs and the program kinds only; the kernels
+// are compiled at run time by NVRTC, one program per kind and key (user_model.cu), from
+//   integer typedefs + device_rng.cuh + `typedef float|double bk_real;` [+ the model's source [+ smc_mailbox.cuh]]
+//   [+ the proposal's source inside namespace bk_proposal] + this file
+// with -DBK_DIMS=D and -DBK_PROGRAM=<kind>, which selects one of the sections at the end of this file:
+//   BK_PROGRAM_MODEL            bk_user_eval; bk_user_hmc / mala / mh (D <= BK_USER_FUSED_MAX_D); prior/likelihood
+//                               models also bk_user_eval_pl and bk_user_smc_rw / mala / hmc
+//   BK_PROGRAM_PROPOSAL         bk_user_propose
+//   BK_PROGRAM_MODEL_PROPOSAL   bk_user_mhp; prior/likelihood models also bk_user_smc_mhp
+//   BK_PROGRAM_DRGHMC           bk_user_drghmc (also compiled with -DBK_DRGHMC=1, which the model's source may test)
+// -DBK_SMC_KERNELS=1 marks the programs that carry SMC kernels (prior/likelihood models, kinds MODEL and
+// MODEL_PROPOSAL): exactly those into which smc_mailbox.cuh is spliced.
+// A model's source defines either
 //   __device__ bk_real log_density_gradient(const bk_real* theta, bk_real* grad, const bk_real* params);
-// or (bk_model_create_cuda_prior_lik: compiled with -DBK_PRIOR_LIK=1 and the shared SMC protocol header) the pair
+// or (bk_model_create_cuda_prior_lik: compiled with -DBK_PRIOR_LIK=1) the pair
 //   __device__ bk_real log_prior_gradient(const bk_real* theta, bk_real* grad, const bk_real* params);
 //   __device__ bk_real log_likelihood_gradient(const bk_real* theta, bk_real* grad, const bk_real* params);
-// from which this file derives log_density_gradient = likelihood + prior.
+// from which this file derives log_density_gradient = likelihood + prior.  A proposal's source defines propose() and,
+// with -DBK_PROPOSAL_TRANSITION=1, transition_log_density() (bk.h), for -DBK_PROPOSAL_NORMALS / _UNIFORMS streams.
 //
 // bk_user_eval      one thread per chain on global rows: model_eval's case for this kind, through which the
 //                   generic HMC / MALA / RW-Metropolis engine, the lockstep DrGHMC engine and the Stretcher run.
@@ -24,20 +33,24 @@
 //                   per particle: k_smc_move_weight (smc.cu) step for step with one lane per particle, on the same
 //                   Philox words, the same resample-index / peer-row / (ll, prior)-carry rules and the same mailbox
 //                   posts (smc_mailbox.cuh).
-// bk_user_propose   (proposal programs, bk_proposal_create_cuda) one draw of a user proposal for global rows, one
-//                   thread per chain: the propose step of the three-launch Metropolis(-Hastings) path.
-// bk_user_mhp       (model + proposal programs) Metropolis / MetropolisHastings with a user proposal fused with a
-//                   user model, one thread per chain: bk_user_mh with propose() in place of the random walk.
-// bk_user_smc_mhp   (prior/likelihood model + proposal programs) TemperedLikelihoodSMC's move + weight kernel with
-//                   one Metropolis(-Hastings) step of the user's proposal as the move: bk_user_smc_rw with propose()
-//                   in place of the random walk (BK_SMC_KERNEL_PROPOSAL).
-// bk_user_drghmc    (DrGHMC programs: a model's source compiled with -DBK_DRGHMC=1, which compiles this kernel and no
-//                   other) DrGhmcDiag, one thread per chain: k_drghmc (drghmc.cu) on the arithmetic and streams of
-//                   the lockstep engine (drghmc_generic.cu).
+// bk_user_propose   one draw of a user proposal for global rows, one thread per chain: the propose step of the
+//                   three-launch Metropolis(-Hastings) path.
+// bk_user_mhp       Metropolis / MetropolisHastings with a user proposal fused with a user model, one thread per
+//                   chain: bk_user_mh with propose() in place of the random walk.
+// bk_user_smc_mhp   (prior/likelihood models) TemperedLikelihoodSMC's move + weight kernel with one
+//                   Metropolis(-Hastings) step of the user's proposal as the move: bk_user_smc_rw with propose() in
+//                   place of the random walk (BK_SMC_KERNEL_PROPOSAL).
+// bk_user_drghmc    DrGhmcDiag, one thread per chain: k_drghmc (drghmc.cu) on the arithmetic and streams of the
+//                   lockstep engine (drghmc_generic.cu).
 #pragma once
 #ifndef __CUDACC_RTC__
 #include "smc_mailbox.cuh"
 #endif
+
+#define BK_PROGRAM_MODEL 1
+#define BK_PROGRAM_PROPOSAL 2
+#define BK_PROGRAM_MODEL_PROPOSAL 3
+#define BK_PROGRAM_DRGHMC 4
 
 namespace bk {
 
@@ -62,7 +75,7 @@ struct UserRunArgs {
     const void* prop_params;  // bk_user_mhp: the proposal's [n_params] or NULL
 };
 
-#if !defined(__CUDACC_RTC__) || defined(BK_DRGHMC)
+#if !defined(__CUDACC_RTC__) || BK_PROGRAM == BK_PROGRAM_DRGHMC
 // Launch arguments of bk_user_drghmc.  `run` holds what bk_user_hmc reads (theta, params, metric, the streams with
 // n_uniform = 2K when injected, draws / logp / accept); step sizes and the damping terms are rounded to the dtype in
 // the kernel, as the lockstep engine rounds them on the host.
@@ -96,9 +109,9 @@ struct UserProposeArgs {
     int32_t rng_mode, n_uniform;
 };
 
-#if !defined(__CUDACC_RTC__) || (defined(BK_PRIOR_LIK) && !defined(BK_DRGHMC))
-// Launch arguments of bk_user_smc_rw / _mala / _hmc: SmcArgs<T> of smc.cu with plain fields (the host (nvcc) and the
-// kernels (NVRTC) must agree on the layout).  Pointers are in the model's dtype unless typed.
+#if !defined(__CUDACC_RTC__) || defined(BK_SMC_KERNELS)
+// Launch arguments of bk_user_smc_rw / _mala / _hmc / _mhp: SmcArgs<T> of smc.cu with plain fields (the host (nvcc) and
+// the kernels (NVRTC) must agree on the layout).  Pointers are in the model's dtype unless typed.
 struct UserSmcArgs {
     void* thetas;                          // [M, D] moved particles (out)
     const void* src;                       // particles to move: row src_idx[m] (the pending resample) or row m
@@ -155,38 +168,60 @@ constexpr int NB = (D + 3) / 4;   // element blocks of 4
 using T = bk_real;
 using A = Ar<T>;
 
-// normals of element block b of (chain c, draw t): the rule of Row<T>::normal4
-__device__ __forceinline__ void normal4(const UserRunArgs& a, int64_t c, int64_t t, int b, T (&z)[4]) {
-    if (a.rng_mode == 1) {   // BK_RNG_INJECTED
-        const T* p = reinterpret_cast<const T*>(a.normals) + (t * a.C + c) * (int64_t)D;
+// ---- the random streams ---------------------------------------------------------------------------------------------
+// S is a launch-argument struct (its bk_rng fields).  A launch reads draw t of chain c: injected streams are
+// [n, C, width] arrays read at row t * C + c, Philox words are keyed by the global chain chain_offset + c and the
+// global draw draw_offset + t.  The SMC's move is one draw (t = 0) of C = M particles.  C is taken by reference so
+// that it is loaded, and the row formed, in the injected branch only: passed by value, its load moves ahead of the
+// branch and ptxas schedules the fused samplers differently.
+template <class S>
+__device__ __forceinline__ uint32_t chain_word(const S& s, int64_t c) {
+    return (uint32_t)(s.chain_offset + (uint64_t)c);
+}
+template <class S>
+__device__ __forceinline__ uint32_t draw_word(const S& s, int64_t t) {
+    return (uint32_t)(s.draw_offset + (uint64_t)t);
+}
+
+// normals of element block b: the rule of Row<T>::normal4
+template <class S>
+__device__ __forceinline__ void normal4(const S& s, const int64_t& C, int64_t c, int64_t t, int b, T (&z)[4]) {
+    if (s.rng_mode == 1) {   // BK_RNG_INJECTED
+        const T* p = reinterpret_cast<const T*>(s.normals) + (t * C + c) * (int64_t)D;
 #pragma unroll
         for (int i = 0; i < 4; ++i) z[i] = (4 * b + i < D) ? p[4 * b + i] : T(0);
     } else {
-        philox_normal4<T>(a.seed, (uint32_t)b, (uint32_t)(a.chain_offset + (uint64_t)c),
-                          (uint32_t)(a.draw_offset + (uint64_t)t), z);
+        philox_normal4<T>(s.seed, (uint32_t)b, chain_word(s, c), draw_word(s, t), z);
     }
 }
 
-// the accept uniform: Row<T>::uniform(0)
-__device__ __forceinline__ T accept_uniform(const UserRunArgs& a, int64_t c, int64_t t) {
-    if (a.rng_mode == 1) return reinterpret_cast<const T*>(a.uniforms)[(t * a.C + c) * a.n_uniform];
-    if (a.n_uniform == 1)
-        return philox_accept_uniform<T>(a.seed, (uint32_t)(a.chain_offset + (uint64_t)c),
-                                        (uint32_t)(a.draw_offset + (uint64_t)t), D);
-    return philox_uniform<T>(a.seed, 0u, (uint32_t)(a.chain_offset + (uint64_t)c),
-                             (uint32_t)(a.draw_offset + (uint64_t)t));
-}
-
-// all D normals of (c, t)
-__device__ __forceinline__ void normals(const UserRunArgs& a, int64_t c, int64_t t, T (&z)[D]) {
+// all D normals
+template <class S>
+__device__ __forceinline__ void normals(const S& s, const int64_t& C, int64_t c, int64_t t, T (&z)[D]) {
 #pragma unroll
     for (int b = 0; b < NB; ++b) {
         T z4[4];
-        normal4(a, c, t, b, z4);
+        normal4(s, C, c, t, b, z4);
 #pragma unroll
         for (int i = 0; i < 4; ++i)
             if (4 * b + i < D) z[4 * b + i] = z4[i];
     }
+}
+
+// the accept uniform: column 0 of the injected row, else the Philox accept block or, with `streams` (Row<T>::uniform(0)
+// of a draw of several uniforms), TAG_UNIFORM word 0
+template <class S>
+__device__ __forceinline__ T accept_uniform(const S& s, const int64_t& C, int64_t c, int64_t t, bool streams = false) {
+    if (s.rng_mode == 1) return reinterpret_cast<const T*>(s.uniforms)[(t * C + c) * s.n_uniform];
+    if (!streams) return philox_accept_uniform<T>(s.seed, chain_word(s, c), draw_word(s, t), D);
+    return philox_uniform<T>(s.seed, 0u, chain_word(s, c), draw_word(s, t));
+}
+
+// the k-th uniform: column k of the injected row, else TAG_UNIFORM word k (drg_uniform, drghmc_generic.cu)
+template <class S>
+__device__ __forceinline__ T uniform(const S& s, const int64_t& C, int64_t c, int64_t t, int k) {
+    if (s.rng_mode == 1) return reinterpret_cast<const T*>(s.uniforms)[(t * C + c) * s.n_uniform + k];
+    return philox_uniform<T>(s.seed, (uint32_t)k, chain_word(s, c), draw_word(s, t));
 }
 
 __device__ __forceinline__ void load_row(const T* p, T (&v)[D]) {
@@ -207,18 +242,24 @@ __device__ __forceinline__ void emit(const UserRunArgs& a, int64_t c, int64_t t,
 }  // namespace user
 }  // namespace bk
 
-// ---- user proposals (bk_proposal_create_cuda) ----------------------------------------------------------------------
-// A proposal program holds the user's proposal source inside namespace bk_proposal and is compiled with
-// -DBK_PROPOSAL=1 -DBK_PROPOSAL_NORMALS=.. -DBK_PROPOSAL_UNIFORMS=.. -DBK_PROPOSAL_TRANSITION=0|1, either alone
-// (-DBK_PROPOSAL_ONLY=1: bk_user_propose) or after a model's source (bk_user_mhp, the fused sampler; prior/likelihood
-// models also bk_user_smc_mhp).
-#ifdef BK_PROPOSAL
+// ---- what a proposal's programs share -------------------------------------------------------------------------------
+#if BK_PROGRAM == BK_PROGRAM_PROPOSAL || BK_PROGRAM == BK_PROGRAM_MODEL_PROPOSAL
 
 namespace bk {
 namespace user {
 
 constexpr int NZ = BK_PROPOSAL_NORMALS, NU = BK_PROPOSAL_UNIFORMS;
 constexpr int NZ1 = NZ > 0 ? NZ : 1, NU1 = NU > 0 ? NU : 1;   // array extents
+
+// the proposal's injected rows: normals [row, NZ]; uniforms [row, n_uniform], whose column 0 is the accept uniform
+template <class S>
+__device__ __forceinline__ const T* proposal_z(const S& s, int64_t row) {
+    return reinterpret_cast<const T*>(s.normals) + row * NZ;
+}
+template <class S>
+__device__ __forceinline__ const T* proposal_u(const S& s, int64_t row) {
+    return reinterpret_cast<const T*>(s.uniforms) + row * s.n_uniform + 1;
+}
 
 // the proposal's Philox streams of (global chain, draw): z[k] from block proposal_normal_block(k, D), u[k] the k-th
 // TAG_UNIFORM uniform
@@ -235,6 +276,23 @@ __device__ __forceinline__ void proposal_philox(uint64_t seed, uint32_t chain, u
     for (int k = 0; k < NU; ++k) u[k] = philox_uniform<T>(seed, (uint32_t)k, chain, draw);
 }
 
+// the proposal's z / u into local arrays: copied from the injected rows or drawn from Philox
+template <class S>
+__device__ __forceinline__ void proposal_streams(const S& s, const int64_t& C, int64_t c, int64_t t, T (&z)[NZ1],
+                                                 T (&u)[NU1]) {
+    if (s.rng_mode == 1) {   // BK_RNG_INJECTED
+        const int64_t r = t * C + c;
+        const T* zi = proposal_z(s, r);
+        const T* ui = proposal_u(s, r);
+#pragma unroll
+        for (int k = 0; k < NZ; ++k) z[k] = zi[k];
+#pragma unroll
+        for (int k = 0; k < NU; ++k) u[k] = ui[k];
+    } else {
+        proposal_philox(s.seed, chain_word(s, c), draw_word(s, t), z, u);
+    }
+}
+
 // log q(theta | q) - log q(q | theta), in MetropolisHastings's order: fwd = q(proposal | theta), rev = q(theta | proposal)
 __device__ __forceinline__ T proposal_dh(const T* th, const T* q, const T* pp) {
 #if BK_PROPOSAL_TRANSITION
@@ -249,200 +307,10 @@ __device__ __forceinline__ T proposal_dh(const T* th, const T* q, const T* pp) {
 }  // namespace user
 }  // namespace bk
 
-#endif  // BK_PROPOSAL
+#endif  // proposal programs
 
-// Model programs compile the kernels below; proposal programs only bk_user_propose / bk_user_mhp / bk_user_smc_mhp,
-// DrGHMC programs only bk_user_drghmc.
-#if !defined(BK_PROPOSAL) && !defined(BK_DRGHMC)
-
-// theta [C, D] -> lp [C] (nullable), grad [C, D]
-extern "C" __global__ void __launch_bounds__(128) bk_user_eval(const bk_real* __restrict__ theta, long long C,
-                                                               const bk_real* __restrict__ params,
-                                                               bk_real* __restrict__ lp, bk_real* __restrict__ grad) {
-    const long long c = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (c >= C) return;
-    const bk_real v = log_density_gradient(theta + c * BK_DIMS, grad + c * BK_DIMS, params);
-    if (lp) lp[c] = v;
-}
-
-// The fused samplers are compiled only where the library dispatches to them (D <= BK_USER_FUSED_MAX_D).
-#if BK_DIMS <= BK_USER_FUSED_MAX_D
-
-// HMCDiag: k_hmc_begin / k_hmc_step / k_hmc_end with the state in registers
-extern "C" __global__ void __launch_bounds__(128) bk_user_hmc(const bk::UserRunArgs a) {
-    using namespace bk::user;
-    const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (c >= a.C) return;
-    const T* params = reinterpret_cast<const T*>(a.params);
-    const T* metric = reinterpret_cast<const T*>(a.metric);
-    const T eps = (T)a.eps, half_eps = (T)a.half_eps;
-    T* row = reinterpret_cast<T*>(a.theta) + c * (int64_t)D;
-    T th[D], g[D];
-    load_row(row, th);
-    T lp = log_density_gradient(th, g, params);
-    for (int64_t t = 0; t < a.n_draws; ++t) {
-        T q[D], r[D], gq[D];
-        normals(a, c, t, r);
-        T kin = T(0);
-#pragma unroll
-        for (int e = 0; e < D; ++e) {
-            const T z = r[e];
-            const T m = metric ? metric[e] : T(1);
-            const T mg = metric ? A::mul(m, g[e]) : g[e];
-            kin = A::add(kin, A::mul(z, metric ? A::mul(m, z) : z));
-            T re = A::sub(z, A::mul(half_eps, mg));
-            T qe = th[e];
-            if (a.L > 0) {
-                re = A::add(re, A::mul(eps, mg));
-                qe = A::add(qe, A::mul(eps, re));
-            }
-            r[e] = re;
-            q[e] = qe;
-        }
-        const T h0 = A::sub(lp, A::mul(T(0.5), kin));
-        T lpq = lp;
-#pragma unroll
-        for (int e = 0; e < D; ++e) gq[e] = g[e];
-        for (int s = 0; s < a.L; ++s) {
-            lpq = log_density_gradient(q, gq, params);
-            if (s + 1 < a.L) {
-#pragma unroll
-                for (int e = 0; e < D; ++e) {
-                    const T mg = metric ? A::mul(metric[e], gq[e]) : gq[e];
-                    r[e] = A::add(r[e], A::mul(eps, mg));
-                    q[e] = A::add(q[e], A::mul(eps, r[e]));
-                }
-            }
-        }
-        kin = T(0);
-#pragma unroll
-        for (int e = 0; e < D; ++e) {
-            const T m = metric ? metric[e] : T(1);
-            const T mg = metric ? A::mul(m, gq[e]) : gq[e];
-            const T re = A::add(r[e], A::mul(half_eps, mg));
-            kin = A::add(kin, A::mul(re, metric ? A::mul(m, re) : re));
-        }
-        const T h1 = A::sub(lpq, A::mul(T(0.5), kin));
-        const bool acc = bk::log_u(accept_uniform(a, c, t)) < A::sub(h1, h0);
-        if (acc) {
-#pragma unroll
-            for (int e = 0; e < D; ++e) {
-                th[e] = q[e];
-                g[e] = gq[e];
-            }
-            lp = lpq;
-        }
-        emit(a, c, t, th, acc ? h1 : h0, acc);
-    }
-#pragma unroll
-    for (int e = 0; e < D; ++e) row[e] = th[e];
-}
-
-// MALA: k_mala_propose / k_mala_accept
-extern "C" __global__ void __launch_bounds__(128) bk_user_mala(const bk::UserRunArgs a) {
-    using namespace bk::user;
-    const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (c >= a.C) return;
-    const T* params = reinterpret_cast<const T*>(a.params);
-    const T eps = (T)a.eps, sd = (T)a.sd, coef = (T)a.coef;
-    T* row = reinterpret_cast<T*>(a.theta) + c * (int64_t)D;
-    T th[D], g[D];
-    load_row(row, th);
-    T lp = log_density_gradient(th, g, params);
-    for (int64_t t = 0; t < a.n_draws; ++t) {
-        T q[D], gq[D];
-        normals(a, c, t, q);
-#pragma unroll
-        for (int e = 0; e < D; ++e) q[e] = A::add(A::add(th[e], A::mul(eps, g[e])), A::mul(sd, q[e]));
-        const T lpq = log_density_gradient(q, gq, params);
-        T sf = T(0), sr = T(0);
-#pragma unroll
-        for (int e = 0; e < D; ++e) {
-            const T df = A::sub(A::sub(q[e], th[e]), A::mul(eps, g[e]));
-            const T dr = A::sub(A::sub(th[e], q[e]), A::mul(eps, gq[e]));
-            sf = A::add(sf, A::mul(df, df));
-            sr = A::add(sr, A::mul(dr, dr));
-        }
-        const T fwd = A::mul(coef, sf), rev = A::mul(coef, sr);
-        const bool acc = bk::log_u(accept_uniform(a, c, t)) < A::add(A::sub(lpq, lp), A::sub(rev, fwd));
-        if (acc) {
-#pragma unroll
-            for (int e = 0; e < D; ++e) {
-                th[e] = q[e];
-                g[e] = gq[e];
-            }
-            lp = lpq;
-        }
-        emit(a, c, t, th, lp, acc);
-    }
-#pragma unroll
-    for (int e = 0; e < D; ++e) row[e] = th[e];
-}
-
-// Metropolis / MetropolisHastings with the Gaussian random walk: k_mh_propose / k_mh_accept.  The gradient the
-// user's function writes is never read: after inlining its computation is dead code.
-extern "C" __global__ void __launch_bounds__(128) bk_user_mh(const bk::UserRunArgs a) {
-    using namespace bk::user;
-    const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (c >= a.C) return;
-    const T* params = reinterpret_cast<const T*>(a.params);
-    const T scale = (T)a.scale, s2 = (T)a.s2;
-    T* row = reinterpret_cast<T*>(a.theta) + c * (int64_t)D;
-    T th[D], unused[D];
-    load_row(row, th);
-    T lp = log_density_gradient(th, unused, params);
-    for (int64_t t = 0; t < a.n_draws; ++t) {
-        T q[D];
-        normals(a, c, t, q);
-#pragma unroll
-        for (int e = 0; e < D; ++e) q[e] = A::add(th[e], A::mul(scale, q[e]));
-        const T lpq = log_density_gradient(q, unused, params);
-        T ratio = A::sub(lpq, lp);
-        if (a.hastings) {
-            T sf = T(0), sr = T(0);
-#pragma unroll
-            for (int e = 0; e < D; ++e) {
-                const T df = A::sub(q[e], th[e]), dr = A::sub(th[e], q[e]);
-                sf = A::add(sf, A::mul(df, df));
-                sr = A::add(sr, A::mul(dr, dr));
-            }
-            const T fwd = A::mul(T(-0.5), sf) / s2, rev = A::mul(T(-0.5), sr) / s2;
-            ratio = A::add(ratio, A::sub(rev, fwd));
-        }
-        const bool acc = bk::log_u(accept_uniform(a, c, t)) < ratio;
-        if (acc) {
-#pragma unroll
-            for (int e = 0; e < D; ++e) th[e] = q[e];
-            lp = lpq;
-        }
-        emit(a, c, t, th, lp, acc);
-    }
-#pragma unroll
-    for (int e = 0; e < D; ++e) row[e] = th[e];
-}
-
-#endif  // BK_DIMS <= BK_USER_FUSED_MAX_D
-#endif  // !BK_PROPOSAL
-
-// The prior / likelihood kernels are compiled only for models created by bk_model_create_cuda_prior_lik (DrGHMC
-// programs of such models: only the derived log_density_gradient above, without the SMC protocol header).
-#if defined(BK_PRIOR_LIK) && !defined(BK_DRGHMC)
-#ifndef BK_PROPOSAL
-
-// theta [C, D] -> log_prior [C], log_likelihood [C] (each nullable)
-extern "C" __global__ void __launch_bounds__(128) bk_user_eval_pl(const bk_real* __restrict__ theta, long long C,
-                                                                  const bk_real* __restrict__ params,
-                                                                  bk_real* __restrict__ lprior,
-                                                                  bk_real* __restrict__ llik) {
-    const long long c = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (c >= C) return;
-    bk_real g[BK_DIMS];
-    const bk_real* x = theta + c * BK_DIMS;
-    if (lprior) lprior[c] = log_prior_gradient(x, g, params);
-    if (llik) llik[c] = log_likelihood_gradient(x, g, params);
-}
-
-#endif  // !BK_PROPOSAL
+// ---- what the SMC kernels share -------------------------------------------------------------------------------------
+#ifdef BK_SMC_KERNELS
 
 namespace bk {
 namespace user {
@@ -489,26 +357,17 @@ __device__ __forceinline__ void smc_move(const UserSmcArgs& a) {
         T th[D], st[D], z[D];
         load_row(row, th);
         // proposal normals: the words Lanes<T, G, J>::normals consumes for blocks 0 .. ceil(D / 4) - 1 (the user's
-        // proposal draws its own streams below)
+        // proposal draws its own streams below).  The loop is normals()'s, spelled out: through normals() ptxas
+        // allocates the fp64 RW kernel's registers differently.
 #pragma unroll
         for (int b = 0; b < (MOVE == 3 ? 0 : NB); ++b) {
             T z4[4];
-            if (a.rng_mode == 1) {   // BK_RNG_INJECTED: [M, D]
-                const T* p = reinterpret_cast<const T*>(a.normals) + m * (int64_t)D;
-#pragma unroll
-                for (int i = 0; i < 4; ++i) z4[i] = (4 * b + i < D) ? p[4 * b + i] : T(0);
-            } else {
-                philox_normal4<T>(a.seed, (uint32_t)b, (uint32_t)(a.chain_offset + (uint64_t)m), (uint32_t)a.draw_offset,
-                                  z4);
-            }
+            normal4(a, a.M, m, 0, b, z4);
 #pragma unroll
             for (int i = 0; i < 4; ++i)
                 if (4 * b + i < D) z[4 * b + i] = z4[i];
         }
-        const T lu = log_u(a.rng_mode == 1
-                               ? reinterpret_cast<const T*>(a.uniforms)[m * a.n_uniform]
-                               : philox_accept_uniform<T>(a.seed, (uint32_t)(a.chain_offset + (uint64_t)m),
-                                                          (uint32_t)a.draw_offset, D));
+        const T lu = log_u(accept_uniform(a, a.M, m, 0));
         T ll_c, pr_c, ll_s, pr_s;
         if (carry) { ll_c = llpr[0]; pr_c = llpr[1]; }
         bool acc;
@@ -541,20 +400,11 @@ __device__ __forceinline__ void smc_move(const UserSmcArgs& a) {
             }
             const T fwd = A::mul(coef, sf), rev = A::mul(coef, sr);
             acc = lu < A::add(A::sub(lp_s, lp_c), A::sub(rev, fwd));   // metropolis.py:41-76
-#ifdef BK_PROPOSAL
+#if BK_PROGRAM == BK_PROGRAM_MODEL_PROPOSAL
         } else if constexpr (MOVE == 3) {   // the RW branch with the user's proposal: bk_user_mhp's step
             const T* pp = reinterpret_cast<const T*>(a.prop_params);
             T zp[NZ1], up[NU1], unused[D];
-            if (a.rng_mode == 1) {   // BK_RNG_INJECTED: normals [M, NZ], uniforms [M, 1 + NU] (column 0: accept)
-                const T* zi = reinterpret_cast<const T*>(a.normals) + m * NZ;
-                const T* ui = reinterpret_cast<const T*>(a.uniforms) + m * a.n_uniform + 1;
-#pragma unroll
-                for (int k = 0; k < NZ; ++k) zp[k] = zi[k];
-#pragma unroll
-                for (int k = 0; k < NU; ++k) up[k] = ui[k];
-            } else {
-                proposal_philox(a.seed, (uint32_t)(a.chain_offset + (uint64_t)m), (uint32_t)a.draw_offset, zp, up);
-            }
+            proposal_streams(a, a.M, m, 0, zp, up);   // injected: normals [M, NZ], uniforms [M, 1 + NU]
             if (!carry) tempered(th, t0, params, ll_c, pr_c, unused);
             const T lp_c = A::add(A::mul(ll_c, t0), pr_c);
             bk_proposal::propose(th, st, zp, up, pp);
@@ -625,19 +475,203 @@ __device__ __forceinline__ void smc_move(const UserSmcArgs& a) {
 }  // namespace user
 }  // namespace bk
 
-#ifndef BK_PROPOSAL
+#endif  // BK_SMC_KERNELS
+
+// =====================================================================================================================
+// ---- BK_PROGRAM_MODEL: a model's own program (bk_model_create_cuda / _prior_lik) -----------------------------------
+#if BK_PROGRAM == BK_PROGRAM_MODEL
+
+// theta [C, D] -> lp [C] (nullable), grad [C, D]
+extern "C" __global__ void __launch_bounds__(128) bk_user_eval(const bk_real* __restrict__ theta, long long C,
+                                                               const bk_real* __restrict__ params,
+                                                               bk_real* __restrict__ lp, bk_real* __restrict__ grad) {
+    const long long c = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= C) return;
+    const bk_real v = log_density_gradient(theta + c * BK_DIMS, grad + c * BK_DIMS, params);
+    if (lp) lp[c] = v;
+}
+
+// The fused samplers are compiled only where the library dispatches to them (D <= BK_USER_FUSED_MAX_D).
+#if BK_DIMS <= BK_USER_FUSED_MAX_D
+
+// HMCDiag: k_hmc_begin / k_hmc_step / k_hmc_end with the state in registers
+extern "C" __global__ void __launch_bounds__(128) bk_user_hmc(const bk::UserRunArgs a) {
+    using namespace bk::user;
+    const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= a.C) return;
+    const T* params = reinterpret_cast<const T*>(a.params);
+    const T* metric = reinterpret_cast<const T*>(a.metric);
+    const T eps = (T)a.eps, half_eps = (T)a.half_eps;
+    T* row = reinterpret_cast<T*>(a.theta) + c * (int64_t)D;
+    T th[D], g[D];
+    load_row(row, th);
+    T lp = log_density_gradient(th, g, params);
+    for (int64_t t = 0; t < a.n_draws; ++t) {
+        T q[D], r[D], gq[D];
+        normals(a, a.C, c, t, r);
+        T kin = T(0);
+#pragma unroll
+        for (int e = 0; e < D; ++e) {
+            const T z = r[e];
+            const T m = metric ? metric[e] : T(1);
+            const T mg = metric ? A::mul(m, g[e]) : g[e];
+            kin = A::add(kin, A::mul(z, metric ? A::mul(m, z) : z));
+            T re = A::sub(z, A::mul(half_eps, mg));
+            T qe = th[e];
+            if (a.L > 0) {
+                re = A::add(re, A::mul(eps, mg));
+                qe = A::add(qe, A::mul(eps, re));
+            }
+            r[e] = re;
+            q[e] = qe;
+        }
+        const T h0 = A::sub(lp, A::mul(T(0.5), kin));
+        T lpq = lp;
+#pragma unroll
+        for (int e = 0; e < D; ++e) gq[e] = g[e];
+        for (int s = 0; s < a.L; ++s) {
+            lpq = log_density_gradient(q, gq, params);
+            if (s + 1 < a.L) {
+#pragma unroll
+                for (int e = 0; e < D; ++e) {
+                    const T mg = metric ? A::mul(metric[e], gq[e]) : gq[e];
+                    r[e] = A::add(r[e], A::mul(eps, mg));
+                    q[e] = A::add(q[e], A::mul(eps, r[e]));
+                }
+            }
+        }
+        kin = T(0);
+#pragma unroll
+        for (int e = 0; e < D; ++e) {
+            const T m = metric ? metric[e] : T(1);
+            const T mg = metric ? A::mul(m, gq[e]) : gq[e];
+            const T re = A::add(r[e], A::mul(half_eps, mg));
+            kin = A::add(kin, A::mul(re, metric ? A::mul(m, re) : re));
+        }
+        const T h1 = A::sub(lpq, A::mul(T(0.5), kin));
+        const bool acc = bk::log_u(accept_uniform(a, a.C, c, t, a.n_uniform != 1)) < A::sub(h1, h0);
+        if (acc) {
+#pragma unroll
+            for (int e = 0; e < D; ++e) {
+                th[e] = q[e];
+                g[e] = gq[e];
+            }
+            lp = lpq;
+        }
+        emit(a, c, t, th, acc ? h1 : h0, acc);
+    }
+#pragma unroll
+    for (int e = 0; e < D; ++e) row[e] = th[e];
+}
+
+// MALA: k_mala_propose / k_mala_accept
+extern "C" __global__ void __launch_bounds__(128) bk_user_mala(const bk::UserRunArgs a) {
+    using namespace bk::user;
+    const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= a.C) return;
+    const T* params = reinterpret_cast<const T*>(a.params);
+    const T eps = (T)a.eps, sd = (T)a.sd, coef = (T)a.coef;
+    T* row = reinterpret_cast<T*>(a.theta) + c * (int64_t)D;
+    T th[D], g[D];
+    load_row(row, th);
+    T lp = log_density_gradient(th, g, params);
+    for (int64_t t = 0; t < a.n_draws; ++t) {
+        T q[D], gq[D];
+        normals(a, a.C, c, t, q);
+#pragma unroll
+        for (int e = 0; e < D; ++e) q[e] = A::add(A::add(th[e], A::mul(eps, g[e])), A::mul(sd, q[e]));
+        const T lpq = log_density_gradient(q, gq, params);
+        T sf = T(0), sr = T(0);
+#pragma unroll
+        for (int e = 0; e < D; ++e) {
+            const T df = A::sub(A::sub(q[e], th[e]), A::mul(eps, g[e]));
+            const T dr = A::sub(A::sub(th[e], q[e]), A::mul(eps, gq[e]));
+            sf = A::add(sf, A::mul(df, df));
+            sr = A::add(sr, A::mul(dr, dr));
+        }
+        const T fwd = A::mul(coef, sf), rev = A::mul(coef, sr);
+        const bool acc = bk::log_u(accept_uniform(a, a.C, c, t, a.n_uniform != 1)) < A::add(A::sub(lpq, lp), A::sub(rev, fwd));
+        if (acc) {
+#pragma unroll
+            for (int e = 0; e < D; ++e) {
+                th[e] = q[e];
+                g[e] = gq[e];
+            }
+            lp = lpq;
+        }
+        emit(a, c, t, th, lp, acc);
+    }
+#pragma unroll
+    for (int e = 0; e < D; ++e) row[e] = th[e];
+}
+
+// Metropolis / MetropolisHastings with the Gaussian random walk: k_mh_propose / k_mh_accept.  The gradient the
+// user's function writes is never read: after inlining its computation is dead code.
+extern "C" __global__ void __launch_bounds__(128) bk_user_mh(const bk::UserRunArgs a) {
+    using namespace bk::user;
+    const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= a.C) return;
+    const T* params = reinterpret_cast<const T*>(a.params);
+    const T scale = (T)a.scale, s2 = (T)a.s2;
+    T* row = reinterpret_cast<T*>(a.theta) + c * (int64_t)D;
+    T th[D], unused[D];
+    load_row(row, th);
+    T lp = log_density_gradient(th, unused, params);
+    for (int64_t t = 0; t < a.n_draws; ++t) {
+        T q[D];
+        normals(a, a.C, c, t, q);
+#pragma unroll
+        for (int e = 0; e < D; ++e) q[e] = A::add(th[e], A::mul(scale, q[e]));
+        const T lpq = log_density_gradient(q, unused, params);
+        T ratio = A::sub(lpq, lp);
+        if (a.hastings) {
+            T sf = T(0), sr = T(0);
+#pragma unroll
+            for (int e = 0; e < D; ++e) {
+                const T df = A::sub(q[e], th[e]), dr = A::sub(th[e], q[e]);
+                sf = A::add(sf, A::mul(df, df));
+                sr = A::add(sr, A::mul(dr, dr));
+            }
+            const T fwd = A::mul(T(-0.5), sf) / s2, rev = A::mul(T(-0.5), sr) / s2;
+            ratio = A::add(ratio, A::sub(rev, fwd));
+        }
+        const bool acc = bk::log_u(accept_uniform(a, a.C, c, t, a.n_uniform != 1)) < ratio;
+        if (acc) {
+#pragma unroll
+            for (int e = 0; e < D; ++e) th[e] = q[e];
+            lp = lpq;
+        }
+        emit(a, c, t, th, lp, acc);
+    }
+#pragma unroll
+    for (int e = 0; e < D; ++e) row[e] = th[e];
+}
+
+#endif  // BK_DIMS <= BK_USER_FUSED_MAX_D
+
+#ifdef BK_SMC_KERNELS
+
+// theta [C, D] -> log_prior [C], log_likelihood [C] (each nullable)
+extern "C" __global__ void __launch_bounds__(128) bk_user_eval_pl(const bk_real* __restrict__ theta, long long C,
+                                                                  const bk_real* __restrict__ params,
+                                                                  bk_real* __restrict__ lprior,
+                                                                  bk_real* __restrict__ llik) {
+    const long long c = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= C) return;
+    bk_real g[BK_DIMS];
+    const bk_real* x = theta + c * BK_DIMS;
+    if (lprior) lprior[c] = log_prior_gradient(x, g, params);
+    if (llik) llik[c] = log_likelihood_gradient(x, g, params);
+}
+
 extern "C" __global__ void __launch_bounds__(128) bk_user_smc_rw(const bk::UserSmcArgs a) { bk::user::smc_move<0>(a); }
 extern "C" __global__ void __launch_bounds__(128) bk_user_smc_mala(const bk::UserSmcArgs a) { bk::user::smc_move<1>(a); }
 extern "C" __global__ void __launch_bounds__(128) bk_user_smc_hmc(const bk::UserSmcArgs a) { bk::user::smc_move<2>(a); }
-#elif !defined(BK_PROPOSAL_ONLY)
-extern "C" __global__ void __launch_bounds__(128) bk_user_smc_mhp(const bk::UserSmcArgs a) { bk::user::smc_move<3>(a); }
-#endif
 
-#endif  // BK_PRIOR_LIK && !BK_DRGHMC
+#endif  // BK_SMC_KERNELS
 
-#ifdef BK_PROPOSAL
-
-#ifdef BK_PROPOSAL_ONLY
+// ---- BK_PROGRAM_PROPOSAL: a proposal's own program (bk_proposal_create_cuda) ----------------------------------------
+#elif BK_PROGRAM == BK_PROGRAM_PROPOSAL
 
 // One draw of the proposal for every chain: q = propose(theta, z, u) and, when dh is given, the Hastings term.
 extern "C" __global__ void __launch_bounds__(128) bk_user_propose(const bk::UserProposeArgs a) {
@@ -648,15 +682,14 @@ extern "C" __global__ void __launch_bounds__(128) bk_user_propose(const bk::User
     const T* th = reinterpret_cast<const T*>(a.theta) + c * (int64_t)D;
     T* q = reinterpret_cast<T*>(a.q) + c * (int64_t)D;
     const T *z, *u;
-    if (a.rng_mode == 1) {   // BK_RNG_INJECTED
+    if (a.rng_mode == 1) {   // BK_RNG_INJECTED: the proposal reads the rows in place
         const int64_t r = a.t * a.C + c;
-        z = reinterpret_cast<const T*>(a.normals) + r * NZ;
-        u = reinterpret_cast<const T*>(a.uniforms) + r * a.n_uniform + 1;
-    } else {
+        z = proposal_z(a, r);
+        u = proposal_u(a, r);
+    } else {   // Philox: through the scratch rows, so that a proposal of any size runs
         T* zw = reinterpret_cast<T*>(a.zbuf) + c * NZ;
         T* uw = reinterpret_cast<T*>(a.ubuf) + c * NU;
-        proposal_philox(a.seed, (uint32_t)(a.chain_offset + (uint64_t)c), (uint32_t)(a.draw_offset + (uint64_t)a.t),
-                        zw, uw);
+        proposal_philox(a.seed, chain_word(a, c), draw_word(a, a.t), zw, uw);
         z = zw;
         u = uw;
     }
@@ -664,7 +697,13 @@ extern "C" __global__ void __launch_bounds__(128) bk_user_propose(const bk::User
     if (a.dh) reinterpret_cast<T*>(a.dh)[c] = proposal_dh(th, q, pp);
 }
 
-#else
+// ---- BK_PROGRAM_MODEL_PROPOSAL: a model's and a proposal's sources in one program, compiled on first use -----------
+#elif BK_PROGRAM == BK_PROGRAM_MODEL_PROPOSAL
+
+// (defined first: ptxas then reports the two kernels in the order it always has)
+#ifdef BK_SMC_KERNELS
+extern "C" __global__ void __launch_bounds__(128) bk_user_smc_mhp(const bk::UserSmcArgs a) { bk::user::smc_move<3>(a); }
+#endif
 
 // Metropolis / MetropolisHastings with a user proposal, fused with the user's model: bk_user_mh with the random walk
 // replaced by propose() and its Gaussian Hastings sum by transition_log_density.  The model's gradient is dead code.
@@ -680,23 +719,12 @@ extern "C" __global__ void __launch_bounds__(128) bk_user_mhp(const bk::UserRunA
     T lp = log_density_gradient(th, unused, params);
     for (int64_t t = 0; t < a.n_draws; ++t) {
         T q[D], z[NZ1], u[NU1];
-        if (a.rng_mode == 1) {   // BK_RNG_INJECTED
-            const int64_t r = t * a.C + c;
-            const T* zi = reinterpret_cast<const T*>(a.normals) + r * NZ;
-            const T* ui = reinterpret_cast<const T*>(a.uniforms) + r * a.n_uniform + 1;
-#pragma unroll
-            for (int k = 0; k < NZ; ++k) z[k] = zi[k];
-#pragma unroll
-            for (int k = 0; k < NU; ++k) u[k] = ui[k];
-        } else {
-            proposal_philox(a.seed, (uint32_t)(a.chain_offset + (uint64_t)c), (uint32_t)(a.draw_offset + (uint64_t)t),
-                            z, u);
-        }
+        proposal_streams(a, a.C, c, t, z, u);
         bk_proposal::propose(th, q, z, u, pp);
         const T lpq = log_density_gradient(q, unused, params);
         T ratio = A::sub(lpq, lp);
         if (a.hastings) ratio = A::add(ratio, proposal_dh(th, q, pp));
-        const bool acc = bk::log_u(accept_uniform(a, c, t)) < ratio;
+        const bool acc = bk::log_u(accept_uniform(a, a.C, c, t, a.n_uniform != 1)) < ratio;
         if (acc) {
 #pragma unroll
             for (int e = 0; e < D; ++e) th[e] = q[e];
@@ -708,10 +736,7 @@ extern "C" __global__ void __launch_bounds__(128) bk_user_mhp(const bk::UserRunA
     for (int e = 0; e < D; ++e) row[e] = th[e];
 }
 
-#endif  // BK_PROPOSAL_ONLY
-#endif  // BK_PROPOSAL
-
-// ---- DrGhmcDiag (DrGHMC programs, -DBK_DRGHMC=1) -------------------------------------------------------------------
+// ---- BK_PROGRAM_DRGHMC: DrGhmcDiag on a model, compiled on first use ------------------------------------------------
 // One chain per thread follows its own retry / accept / ghost schedule (drghmc.py:348-446) and integrates only the
 // trajectories that schedule reaches; the lockstep engine integrates every trajectory a chain could need.  Every point
 // carries its own (log p, grad log p), as the lockstep engine's levels do: theta's pair across attempts and draws, a
@@ -719,7 +744,7 @@ extern "C" __global__ void __launch_bounds__(128) bk_user_mhp(const bk::UserRunA
 // The proposal recursion is compile-time (DrAccept<k>, the shape of drghmc.cu's Accept<k>) with a __noinline__ run()
 // per level, and every trajectory goes through one __noinline__ trajectory(): the user's function is inlined twice
 // (at entry and in trajectory()) whatever K is, which bounds NVRTC's work for a heavy model.
-#ifdef BK_DRGHMC
+#elif BK_PROGRAM == BK_PROGRAM_DRGHMC
 
 namespace bk {
 namespace user {
@@ -738,13 +763,6 @@ __device__ __forceinline__ T dr_retry(const DrCtx& c, T reject_logp) {
 }
 __device__ __forceinline__ T dr_log1m_exp(T a) { return A::log1p_(-A::exp_(a)); }   // np.log1p(-np.exp(a))
 __device__ __forceinline__ T dr_mg(const DrCtx& c, int e, T g) { return c.metric ? A::mul(c.metric[e], g) : g; }
-
-// the k-th uniform of (chain c, draw t): drg_uniform (drghmc_generic.cu)
-__device__ __forceinline__ T dr_uniform(const UserRunArgs& a, int64_t c, int64_t t, int k) {
-    if (a.rng_mode == 1) return reinterpret_cast<const T*>(a.uniforms)[(t * a.C + c) * a.n_uniform + k];   // INJECTED
-    return philox_uniform<T>(a.seed, (uint32_t)k, (uint32_t)(a.chain_offset + (uint64_t)c),
-                             (uint32_t)(a.draw_offset + (uint64_t)t));
-}
 
 // proposal_map (drghmc.py:319-346) of proposal i from (q0, r0, g0): k_drg_first, then cnt - 1 times (evaluate,
 // k_drg_step), evaluate, k_drg_last.  Leaves the end point's pair in (lp, g) and returns its joint log density
@@ -852,7 +870,7 @@ extern "C" __global__ void __launch_bounds__(128) bk_user_drghmc(const bk::UserD
     T lp = log_density_gradient(th, g, ctx.params);
     for (int64_t t = 0; t < ra.n_draws; ++t) {
         T z[D];
-        normals(ra, c, t, z);
+        normals(ra, ra.C, c, t, z);
         T kin = T(0);
 #pragma unroll
         for (int e = 0; e < D; ++e) {   // k_drg_refresh
@@ -864,11 +882,11 @@ extern "C" __global__ void __launch_bounds__(128) bk_user_drghmc(const bk::UserD
         int ui = 0;
         bool moved = false;
         for (int k = 0; k < a.K; ++k) {
-            if (!(bk::log_u(dr_uniform(ra, c, t, ui++)) < dr_retry(ctx, reject_logp))) break;   // drghmc.py:369-371
+            if (!(bk::log_u(uniform(ra, ra.C, c, t, ui++)) < dr_retry(ctx, reject_logp))) break;   // drghmc.py:369-371
             T qp[D], rp[D], gp[D], lpp;
             const T jp = trajectory(ctx, k, th, rho, g, qp, rp, gp, lpp);
             const T acc_lp = dr_accept<0>(k, ctx, qp, rp, gp, jp, cur_hastings, cur_logp);
-            if (bk::log_u(dr_uniform(ra, c, t, ui++)) < acc_lp) {   // drghmc.py:378-381
+            if (bk::log_u(uniform(ra, ra.C, c, t, ui++)) < acc_lp) {   // drghmc.py:378-381
 #pragma unroll
                 for (int e = 0; e < D; ++e) {
                     th[e] = qp[e];
@@ -895,5 +913,5 @@ extern "C" __global__ void __launch_bounds__(128) bk_user_drghmc(const bk::UserD
     }
 }
 
-#endif  // BK_DRGHMC
+#endif  // BK_PROGRAM
 #endif  // __CUDACC_RTC__

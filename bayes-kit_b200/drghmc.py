@@ -11,7 +11,7 @@ import torch
 
 from . import _lib as L
 from ._sampler import ChainSampler, _is_empty_init
-from ._util import ptr, stream_ptr, to_dev
+from ._util import compile_log, ptr, stream_ptr, to_dev
 from .models import CudaModel
 
 
@@ -62,14 +62,10 @@ class DrGhmcDiag(ChainSampler):
         self.last_n_uniform = None
         self.compile_log = ""
         if isinstance(self._model, CudaModel):
-            log = C.create_string_buffer(1 << 20)
-            with torch.cuda.device(self.device):     # compile the fused kernel now, not in the first sample()
-                rc = L.lib().bk_drghmc_cuda_prepare(self._model.handle, log, len(log))
-            if rc == L.BK_E_INVALID and log.value:
-                raise ValueError("DrGhmcDiag: NVRTC compilation of the model's DrGHMC kernel failed:\n"
-                                 + log.value.decode(errors="replace"))
-            L.check(rc)
-            self.compile_log = log.value.decode(errors="replace")   # the fused kernel's, or "" (lockstep engine)
+            # compile the fused kernel now, not in the first sample(); its log, or "" (lockstep engine)
+            self.compile_log = compile_log(
+                lambda log, n: L.lib().bk_drghmc_cuda_prepare(self._model.handle, log, n),
+                "DrGhmcDiag: NVRTC compilation of the model's DrGHMC kernel failed:\n", self.device)
 
     @property
     def rho(self) -> torch.Tensor:

@@ -19,7 +19,7 @@ import torch
 
 from . import _lib as L
 from ._sampler import ChainSampler
-from ._util import dtype_id, ptr, require_cuda, stream_ptr, to_dev
+from ._util import compile_log, dtype_id, ptr, require_cuda, stream_ptr, to_dev
 
 
 def metropolis_accept_test(lp_proposal: float, lp_current: float, rng) -> bool:
@@ -92,16 +92,12 @@ class CudaProposal:
                 self.params = None
         n_params = 0 if self.params is None else self.params.numel()
         _load_nvrtc()
-        log = C.create_string_buffer(1 << 20)
         h = L.u64(0)
-        with torch.cuda.device(self.device):
-            rc = L.lib().bk_proposal_create_cuda(source.encode(), self.dims, dtype_id(dtype), ptr(self.params), n_params,
-                                                 self.normals, self.uniforms, int(self.transition), C.byref(h), log,
-                                                 len(log))
-        self.compile_log = log.value.decode(errors="replace")
-        if rc == L.BK_E_INVALID and self.compile_log:
-            raise ValueError(f"CudaProposal: NVRTC compilation failed:\n{self.compile_log}")
-        L.check(rc)
+        self.compile_log = compile_log(
+            lambda log, n: L.lib().bk_proposal_create_cuda(source.encode(), self.dims, dtype_id(dtype), ptr(self.params),
+                                                           n_params, self.normals, self.uniforms, int(self.transition),
+                                                           C.byref(h), log, n),
+            "CudaProposal: NVRTC compilation failed:\n", self.device)
         self._handle = h.value
 
     @property
@@ -153,14 +149,10 @@ class MetropolisHastings(ChainSampler):
                 raise ValueError(f"the proposal (dims {prop.dims}, {prop.dtype}) does not match the model "
                                  f"(dims {self._dim}, {self.dtype})")
             self._n_normal, self._n_uniform = prop.normals, 1 + prop.uniforms
-            log = C.create_string_buffer(1 << 20)
-            with torch.cuda.device(self.device):     # compile the fused kernel now, not in the first sample()
-                rc = L.lib().bk_mh_cuda_prepare(self._model.handle, prop.handle, log, len(log))
-            if rc == L.BK_E_INVALID and log.value:
-                raise ValueError("MetropolisHastings: NVRTC compilation of the model with the proposal failed:\n"
-                                 + log.value.decode(errors="replace"))
-            L.check(rc)
-            self.compile_log = log.value.decode(errors="replace")   # the fused kernel's, or "" (three launches)
+            # compile the fused kernel now, not in the first sample(); its log, or "" (three launches)
+            self.compile_log = compile_log(
+                lambda log, n: L.lib().bk_mh_cuda_prepare(self._model.handle, prop.handle, log, n),
+                "MetropolisHastings: NVRTC compilation of the model with the proposal failed:\n", self.device)
 
     def _fuses_extras(self) -> bool:
         return not isinstance(self._proposal_fn, CudaProposal) and super()._fuses_extras()

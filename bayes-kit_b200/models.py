@@ -17,7 +17,7 @@ import numpy as np
 import torch
 
 from . import _lib as L
-from ._util import Workspace, dtype_id, ptr, require_cuda, stream_ptr, to_dev
+from ._util import Workspace, compile_log, dtype_id, ptr, require_cuda, stream_ptr, to_dev
 
 
 class DeviceModel:
@@ -280,15 +280,12 @@ class CudaModel(DeviceModel):
                 self.params = None
         n_params = 0 if self.params is None else self.params.numel()
         _load_nvrtc()
-        log = C.create_string_buffer(1 << 20)
         h = L.u64(0)
-        with torch.cuda.device(self.device):
-            rc = getattr(L.lib(), self._create)(source.encode(), self._dims, dtype_id(dtype), ptr(self.params),
-                                                n_params, C.byref(h), log, len(log))
-        self.compile_log = log.value.decode(errors="replace")
-        if rc == L.BK_E_INVALID and self.compile_log:
-            raise ValueError(f"{type(self).__name__}: NVRTC compilation failed:\n{self.compile_log}")
-        L.check(rc)
+        create = getattr(L.lib(), self._create)
+        self.compile_log = compile_log(
+            lambda log, n: create(source.encode(), self._dims, dtype_id(dtype), ptr(self.params), n_params,
+                                  C.byref(h), log, n),
+            f"{type(self).__name__}: NVRTC compilation failed:\n", self.device)
         self._handle = h.value
 
 

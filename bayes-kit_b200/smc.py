@@ -31,7 +31,7 @@ import torch.distributed as dist
 from . import _lib as L
 from . import dist as D_
 from . import peer as P_
-from ._util import make_rng, resolve_seed, stream_ptr, to_dev
+from ._util import compile_log, make_rng, resolve_seed, stream_ptr, to_dev
 from .metropolis import CudaProposal
 from .models import Binomial, CudaPriorLikModel, GaussPriorLik, require_plugin
 
@@ -219,14 +219,9 @@ class TemperedLikelihoodSMC:
         if prop.dims != self._model.dims() or prop.dtype != self._model.dtype:
             raise ValueError(f"the proposal (dims {prop.dims}, {prop.dtype}) does not match the model "
                              f"(dims {self._model.dims()}, {self._model.dtype})")
-        log = C.create_string_buffer(1 << 20)
-        with torch.cuda.device(self._model.device):
-            rc = L.lib().bk_smc_cuda_prepare(self._model.handle, prop.handle, log, len(log))
-        if rc == L.BK_E_INVALID and log.value:
-            raise ValueError("TemperedLikelihoodSMC: NVRTC compilation of the model with the proposal failed:\n"
-                             + log.value.decode(errors="replace"))
-        L.check(rc)
-        self.compile_log = log.value.decode(errors="replace")
+        self.compile_log = compile_log(
+            lambda log, n: L.lib().bk_smc_cuda_prepare(self._model.handle, prop.handle, log, n),
+            "TemperedLikelihoodSMC: NVRTC compilation of the model with the proposal failed:\n", self._model.device)
 
     # ---- plumbing --------------------------------------------------------------------
     def _sh(self) -> L.SmcShard:
