@@ -101,6 +101,7 @@ _SIGNATURES = {
     "bk_drghmc_sample": (C.c_int, [u64, vp, vp, i64, i32, C.POINTER(f64), C.POINTER(i32), f64, i32,
                                    vp, i64, C.POINTER(Rng), C.POINTER(DrawOut), vp, vp, sz, vp]),
     "bk_stretch_workspace_bytes": (sz, [u64, i64]),
+    "bk_stretch_cuda_prepare": (C.c_int, [u64, C.c_char_p, sz]),
     "bk_stretch_move": (C.c_int, [u64, vp, vp, C.POINTER(i32), vp, i64, i64, f64, C.POINTER(Rng), vp, vp, sz, vp]),
     "bk_smc_move_weight": (C.c_int, [u64, vp, i64, i32, i32, f64, C.POINTER(Rng), vp, vp, vp]),
     "bk_smc_gather_move_weight": (C.c_int, [u64, vp, vp, vp, i64, i32, i32, f64, C.POINTER(Rng), vp, vp, vp]),

@@ -7,7 +7,9 @@
 //   accept iff log u < (D-1) log z + log p(theta*) - log p(theta_k) (:51-53)
 // Every active walker moves in parallel -- that is the point of splitting the ensemble.  Three
 // launches: propose (warp per walker), the plugin's batched density (tensor cores where it has
-// them), accept.  The current walkers' log densities are cached (the reference's TODO, :69).
+// them), accept.  A user model (bk_model_create_cuda*) with dims <= USER_FUSED_MAX_D runs all three
+// in one launch of the runtime-compiled bk_user_stretch (user_model.cu, one thread per walker).  The
+// current walkers' log densities are cached (the reference's TODO, :69); both engines keep the cache.
 #include "model.h"
 #include "sep_common.cuh"
 
@@ -109,14 +111,25 @@ static int stretch_t(const Model& m, void* active, void* lp, int32_t* lp_valid, 
 
 using namespace bk;
 
+// the runtime-compiled bk_user_stretch serves user models up to USER_FUSED_MAX_D dims; every other model runs stretch_t
+static bool stretch_user_fused(const Model& m) { return !force_generic() && user_fused(m); }
+
 extern "C" {
 
 size_t bk_stretch_workspace_bytes(uint64_t handle, int64_t n_active) {
     const Model* m = get_model(handle);
     if (!m || n_active <= 0) return 256;
+    if (stretch_user_fused(*m)) return 0;
     const size_t es = m->d.dtype == BK_F64 ? 8 : 4;
     return align_up((size_t)n_active * m->d.dims * es, 256) + 2 * align_up((size_t)n_active * es, 256) +
            model_eval_ws_bytes(*m, n_active) + 1024;
+}
+
+int bk_stretch_cuda_prepare(uint64_t handle, char* log_out, size_t log_bytes) {
+    if (log_out && log_bytes) log_out[0] = '\0';
+    const Model* m = get_model(handle);
+    if (!m) return BK_E_HANDLE;
+    return stretch_user_fused(*m) ? user_stretch_prepare(*m, log_out, log_bytes) : BK_OK;
 }
 
 int bk_stretch_move(uint64_t handle, void* active, void* lp_active, int32_t* lp_valid_host, const void* other,
@@ -130,6 +143,14 @@ int bk_stretch_move(uint64_t handle, void* active, void* lp_active, int32_t* lp_
     BK_CHECK_ARG(rng->mode == BK_RNG_PHILOX || (rng->mode == BK_RNG_INJECTED && rng->uniforms),
                  "bk_stretch_move: injected rng needs uniforms [n_active, 3]");
     if (n_active == 0) return BK_OK;
+    if (stretch_user_fused(*m)) {
+        const bool eval_lp = !lp_valid_host || !*lp_valid_host;
+        if (int rc = user_stretch_move(*m, active, lp_active, eval_lp, other, n_active, n_other, a, rng, accept_out,
+                                       (cudaStream_t)stream))
+            return rc;
+        if (lp_valid_host) *lp_valid_host = 1;
+        return BK_OK;
+    }
     if (m->d.dtype == BK_F64)
         return stretch_t<double>(*m, active, lp_active, lp_valid_host, other, n_active, n_other, a, rng, accept_out,
                                  ws, ws_bytes, (cudaStream_t)stream);

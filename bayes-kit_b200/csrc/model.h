@@ -72,6 +72,12 @@ int user_drghmc_prepare(const Model& m, char* log_out, size_t log_bytes);
 int user_drghmc_sample(const Model& m, void* theta, void* rho, int64_t C, int K, const double* sizes,
                        const int32_t* counts, double damping, int prob_retry, const void* metric, int64_t n,
                        const bk_rng* rng, const bk_draw_out& out, int32_t* n_used, cudaStream_t st);
+// The Stretcher on a user model with dims <= USER_FUSED_MAX_D: the program of bk_user_stretch, compiled (once per
+// process) by the prepare or on the first move, and one half-step of bk_stretch_move in one launch.  eval_lp: lp [n]
+// is not valid and the kernel evaluates it first.
+int user_stretch_prepare(const Model& m, char* log_out, size_t log_bytes);
+int user_stretch_move(const Model& m, void* active, void* lp, bool eval_lp, const void* other, int64_t n, int64_t mo,
+                      double a, const bk_rng* rng, int32_t* accept, cudaStream_t st);
 // three-launch path: Philox scratch of bk_user_propose ([C, n_normals] and [C, n_uniforms]) and its launch
 size_t user_propose_ws_bytes(const UserProposal& p, int64_t C);
 int user_propose(const UserProposal& p, const UserProposeArgs& a, cudaStream_t st);

@@ -9,6 +9,7 @@
 //   BK_PROGRAM_PROPOSAL         bk_user_propose
 //   BK_PROGRAM_MODEL_PROPOSAL   bk_user_mhp; prior/likelihood models also bk_user_smc_mhp
 //   BK_PROGRAM_DRGHMC           bk_user_drghmc (also compiled with -DBK_DRGHMC=1, which the model's source may test)
+//   BK_PROGRAM_STRETCH          bk_user_stretch (also compiled with -DBK_STRETCH=1, which the model's source may test)
 // -DBK_SMC_KERNELS=1 marks the programs that carry SMC kernels (prior/likelihood models, kinds MODEL and
 // MODEL_PROPOSAL): exactly those into which smc_mailbox.cuh is spliced.
 // A model's source defines either
@@ -20,7 +21,8 @@
 // with -DBK_PROPOSAL_TRANSITION=1, transition_log_density() (bk.h), for -DBK_PROPOSAL_NORMALS / _UNIFORMS streams.
 //
 // bk_user_eval      one thread per chain on global rows: model_eval's case for this kind, through which the
-//                   generic HMC / MALA / RW-Metropolis engine, the lockstep DrGHMC engine and the Stretcher run.
+//                   generic HMC / MALA / RW-Metropolis engine, the lockstep DrGHMC engine and the Stretcher's
+//                   three-launch engine run.
 // bk_user_hmc/mala/mh
 //                   fused samplers, one thread per chain: theta, its gradient and log density stay in registers
 //                   across all n_draws of a call.  Randomness and arithmetic follow the generic engine exactly
@@ -42,6 +44,8 @@
 //                   place of the random walk (BK_SMC_KERNEL_PROPOSAL).
 // bk_user_drghmc    DrGhmcDiag, one thread per chain: k_drghmc (drghmc.cu) on the arithmetic and streams of the
 //                   lockstep engine (drghmc_generic.cu).
+// bk_user_stretch   one half-step of the Stretcher, one thread per active walker: k_stretch_propose, the density of
+//                   the proposal and k_stretch_accept (ensemble.cu) in one launch, on the same uniforms and arithmetic.
 #pragma once
 #ifndef __CUDACC_RTC__
 #include "smc_mailbox.cuh"
@@ -51,6 +55,7 @@
 #define BK_PROGRAM_PROPOSAL 2
 #define BK_PROGRAM_MODEL_PROPOSAL 3
 #define BK_PROGRAM_DRGHMC 4
+#define BK_PROGRAM_STRETCH 5
 
 namespace bk {
 
@@ -88,6 +93,24 @@ struct UserDrArgs {
     int32_t cnt[USER_DR_KMAX];        // leapfrog steps of proposal k
     double eps[USER_DR_KMAX], half_eps[USER_DR_KMAX];
     double s_keep, s_new;             // sqrt(1 - damping), sqrt(damping)
+};
+#endif
+
+#if !defined(__CUDACC_RTC__) || BK_PROGRAM == BK_PROGRAM_STRETCH
+// Launch arguments of bk_user_stretch: one half-step of the Stretcher (bk_stretch_move).  lo / width are rounded to
+// the dtype in the kernel, as stretch_t (ensemble.cu) rounds them on the host.
+struct UserStretchArgs {
+    void* active;             // [n, D] in/out: the walkers that move
+    void* lp;                 // [n] in/out: their cached log densities
+    const void* other;        // [m, D] the complementary walkers
+    int32_t* accept;          // [n] or NULL
+    const void* params;       // [n_params] or NULL
+    const void* uniforms;     // injected [n, 3]: partner, stretch, accept
+    int64_t n, m;
+    double lo, width;         // u_z = lo + width * u1: 1 / sqrt(a), sqrt(a) - 1 / sqrt(a)
+    uint64_t seed, draw_offset, chain_offset;
+    int32_t rng_mode, n_uniform;   // n_uniform = 3
+    int32_t eval_lp;          // evaluate log p(active) first (the cache is invalid) and store it
 };
 #endif
 
@@ -911,6 +934,56 @@ extern "C" __global__ void __launch_bounds__(128) bk_user_drghmc(const bk::UserD
         row[e] = th[e];
         rrow[e] = rho[e];
     }
+}
+
+// ---- BK_PROGRAM_STRETCH: the Stretcher on a model, compiled on first use --------------------------------------------
+#elif BK_PROGRAM == BK_PROGRAM_STRETCH
+
+namespace bk {
+namespace user {
+
+// The generic engine stores (D - 1) log z, log p(q) and log p(theta) to memory before k_stretch_accept sums them.  Kept
+// in registers, an fp32 sum with a product (the user's function may end in one) could be contracted into an FMA:
+// these round every operation, as those stores do.  In fp64 they are Ar<double>'s.
+__device__ __forceinline__ float rn_mul(float a, float b) { return __fmul_rn(a, b); }
+__device__ __forceinline__ float rn_add(float a, float b) { return __fadd_rn(a, b); }
+__device__ __forceinline__ float rn_sub(float a, float b) { return __fsub_rn(a, b); }
+__device__ __forceinline__ double rn_mul(double a, double b) { return __dmul_rn(a, b); }
+__device__ __forceinline__ double rn_add(double a, double b) { return __dadd_rn(a, b); }
+__device__ __forceinline__ double rn_sub(double a, double b) { return __dsub_rn(a, b); }
+
+}  // namespace user
+}  // namespace bk
+
+// One half-step, one thread per active walker k: k_stretch_propose, the model's density of the proposal and
+// k_stretch_accept (ensemble.cu) on the same uniforms and the same sequence of Ar<T> operations, with the proposal in
+// registers.  Only the log density is used: the gradient the user's function writes is dead code after inlining.
+extern "C" __global__ void __launch_bounds__(128) bk_user_stretch(const bk::UserStretchArgs a) {
+    using namespace bk::user;
+    const int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= a.n) return;
+    const T* params = reinterpret_cast<const T*>(a.params);
+    T* row = reinterpret_cast<T*>(a.active) + k * (int64_t)D;
+    T* lpk = reinterpret_cast<T*>(a.lp) + k;
+    T th[D], q[D], unused[D];
+    load_row(row, th);
+    const T lp = a.eval_lp ? log_density_gradient(th, unused, params) : *lpk;
+    int64_t j = (int64_t)(uniform(a, a.n, k, 0, 0) * (T)a.m);
+    j = j < a.m ? j : a.m - 1;
+    const T uz = A::add((T)a.lo, A::mul((T)a.width, uniform(a, a.n, k, 0, 1)));
+    const T z = A::mul(uz, uz);
+    const T* oj = reinterpret_cast<const T*>(a.other) + j * (int64_t)D;
+#pragma unroll
+    for (int e = 0; e < D; ++e) q[e] = A::add(oj[e], A::mul(z, A::sub(th[e], oj[e])));
+    const T lpq = log_density_gradient(q, unused, params);
+    const T log_q = rn_sub(rn_add(rn_mul((T)(D - 1), A::log_(z)), lpq), lp);
+    const bool acc = bk::log_u(uniform(a, a.n, k, 0, 2)) < log_q;
+    if (acc) {
+#pragma unroll
+        for (int e = 0; e < D; ++e) row[e] = q[e];
+    }
+    if (acc || a.eval_lp) *lpk = acc ? lpq : lp;
+    if (a.accept) a.accept[k] = acc ? 1 : 0;
 }
 
 #endif  // BK_PROGRAM

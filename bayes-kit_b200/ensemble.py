@@ -4,7 +4,9 @@ Upstream the class body is a docstring only: the Goodman & Weare stretch-move
 implementation is commented out (ensemble.py:16-66).  This is that algorithm, with
 the constructor the comments sketch, running on device: the walkers of one half
 move in parallel against the complementary half (three launches per half-step,
-the density through the model plugin -- tensor cores where it has them).  With
+the density through the model plugin -- tensor cores where it has them; one
+fused launch, compiled from the model's source, for a ``CudaModel`` /
+``CudaPriorLikModel`` with ``dims <= 32``).  With
 torch.distributed initialised each rank owns a slice of both halves and the
 complementary half is all-gathered before each half-step (the one collective).
 Parity is pinned by oracle/samplers.py::stretch only (no executable reference).
@@ -20,8 +22,8 @@ import torch
 from . import _lib as L
 from . import dist as D_
 from . import peer as P_
-from ._util import Workspace, make_rng, resolve_seed, stream_ptr, to_dev
-from .models import require_plugin
+from ._util import Workspace, compile_log, make_rng, resolve_seed, stream_ptr, to_dev
+from .models import CudaModel, require_plugin
 
 
 class Stretcher:
@@ -33,6 +35,10 @@ class Stretcher:
     ``sample()`` performs one sweep (first half against the second, then the second
     against the updated first, ensemble.py:55-63) and returns the walkers
     ``[walkers, dims]`` (this rank's walkers under torch.distributed).
+    On a ``CudaModel`` / ``CudaPriorLikModel`` with ``dims <= 32`` each half-step
+    is one fused kernel compiled from the model's source at construction
+    (``compile_log``: ptxas's report, ``""`` on every other engine; a compile
+    error raises ``ValueError`` with NVRTC's log).
     """
 
     def __init__(self, model, a: Optional[float] = None, walkers: Optional[int] = None, init=None, *,
@@ -69,6 +75,12 @@ class Stretcher:
         self._ws = Workspace(self.device)
         self._t = 0
         self.last_accept = None
+        self.compile_log = ""
+        if isinstance(self._model, CudaModel):
+            # compile the fused kernel now, not in the first sample(); its log, or "" (three-launch engine)
+            self.compile_log = compile_log(
+                lambda log, n: L.lib().bk_stretch_cuda_prepare(self._model.handle, log, n),
+                "Stretcher: NVRTC compilation of the model's stretch kernel failed:\n", self.device)
         if isinstance(group, P_.FakeRank):      # single-GPU fake world: the other ranks' halves live on this device
             group.fake._regions.setdefault("stretch", [None] * self._world)[self._rank] = self._halves
 

@@ -257,11 +257,12 @@ class CudaModel(DeviceModel):
     hyper-parameters as one flat array, passed to the function on the device.
 
     Every sampler except ``TemperedLikelihoodSMC`` accepts it; for the SMC, write the log prior and the log
-    likelihood separately as a ``CudaPriorLikModel``.  ``HMCDiag``, ``MALA`` and the random-walk
-    ``Metropolis`` / ``MetropolisHastings`` run one fused kernel per call (one thread per chain, state in
-    registers) for ``dims <= 32``, the generic engine above.  A compile error raises ``ValueError`` with
-    NVRTC's log; ``compile_log`` holds the log of a successful compile, with the registers and spills of
-    every kernel."""
+    likelihood separately as a ``CudaPriorLikModel``.  ``HMCDiag``, ``MALA``, the random-walk
+    ``Metropolis`` / ``MetropolisHastings``, ``DrGhmcDiag`` and the ``Stretcher`` run one fused kernel per call
+    (one thread per chain or walker, state in registers) for ``dims <= 32``, the generic engines above; the
+    kernels of ``DrGhmcDiag`` and the ``Stretcher`` are compiled when the sampler is constructed.  A compile
+    error raises ``ValueError`` with NVRTC's log; ``compile_log`` holds the log of a successful compile, with
+    the registers and spills of every kernel."""
 
     _kind = L.MODEL_USER
     _create = "bk_model_create_cuda"

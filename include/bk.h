@@ -179,8 +179,9 @@ BK_API int bk_model_log_prior_likelihood(uint64_t handle, const void* theta, int
  * the life of the process by (source, dims, dtype, prior/likelihood split) and never unloaded.  The handle works
  * everywhere a model handle does except the SMC, which needs the split (bk_model_create_cuda_prior_lik below):
  * HMCDiag, MALA and RW-Metropolis run one fused register-resident kernel per call for dims <= 32 (one thread per
- * chain; otherwise the generic engine), DrGhmcDiag and the Stretcher run their generic engines.  The fused kernels
- * draw the same Philox words as every other engine and leave *cache_valid_host = 0.
+ * chain; otherwise the generic engine), as do DrGhmcDiag and the Stretcher (see bk_drghmc_sample and
+ * bk_stretch_move).  The fused kernels draw the same Philox words as every other engine; those of HMCDiag, MALA and
+ * RW-Metropolis leave *cache_valid_host = 0.
  *
  * log_out [log_bytes] (may be NULL) receives NVRTC's log, truncated and NUL terminated; it includes ptxas's
  * register / spill report of every kernel.  Returns BK_E_INVALID on a bad argument or a compile error (the
@@ -473,8 +474,18 @@ BK_API int bk_smc_shard_gather(const bk_smc_shard* sh, int64_t D, int32_t dtype,
  *   theta* = other[j] + z (theta_k - other[j])
  *   accept iff log(u2) < (D - 1) log z + log p(theta*) - log p(theta_k)
  * u0..u2: Philox keyed by (seed, chain_offset + k, draw_offset) or INJECTED
- * uniforms [n_active, 3].  accept_out [n_active] or NULL. */
+ * uniforms [n_active, 3].  accept_out [n_active] or NULL.
+ * Engines: a user model (bk_model_create_cuda*) with dims <= 32 runs one fused kernel per call
+ * (bk_user_stretch: one thread per walker, the proposal in registers, lp_active kept as on the
+ * other engine; compiled from the model's source in a program of its own, once per process, by
+ * bk_stretch_cuda_prepare or on the first call); every other model runs three launches (propose,
+ * the model's density, accept) with scratch from bk_stretch_workspace_bytes (0 on the fused engine). */
 BK_API size_t bk_stretch_workspace_bytes(uint64_t handle, int64_t n_active);
+/* Compiles and loads the fused Stretcher program of a user model that takes that engine, so that the
+ * first bk_stretch_move does not pay the NVRTC compile; log_out as bk_model_create_cuda's (ptxas's
+ * report of bk_user_stretch).  BK_OK with an empty log for any other model, BK_E_HANDLE for an
+ * unknown handle, BK_E_INVALID on a compile error (with the log), BK_E_UNSUPPORTED without NVRTC. */
+BK_API int bk_stretch_cuda_prepare(uint64_t handle, char* log_out, size_t log_bytes);
 BK_API int bk_stretch_move(uint64_t handle, void* active, void* lp_active, int32_t* lp_valid_host,
                     const void* other, int64_t n_active, int64_t n_other, double a,
                     const bk_rng* rng, int32_t* accept_out, void* ws, size_t ws_bytes, void* stream);
