@@ -82,6 +82,7 @@ _SIGNATURES = {
     "bk_proposal_create_cuda": (C.c_int, [C.c_char_p, i64, i32, vp, i64, i32, i32, i32, C.POINTER(u64), C.c_char_p,
                                           sz]),
     "bk_proposal_destroy": (C.c_int, [u64]),
+    "bk_user_wide_prepare": (C.c_int, [u64, C.c_char_p, sz]),
     "bk_mh_cuda_workspace_bytes": (sz, [u64, u64, i64]),
     "bk_mh_cuda_prepare": (C.c_int, [u64, u64, C.c_char_p, sz]),
     "bk_mh_cuda_sample": (C.c_int, [u64, u64, vp, vp, C.POINTER(i32), i64, i32, i64, C.POINTER(Rng), C.POINTER(DrawOut),

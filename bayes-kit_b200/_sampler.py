@@ -374,6 +374,18 @@ class ChainSampler:
     def _launch(self, n, rng, out, c0=0, cn=None, cache_valid=None):  # pragma: no cover - overridden
         raise NotImplementedError
 
+    def _prepare_wide(self, who: str) -> None:
+        """HMCDiag / MALA / Metropolis(-Hastings) with the Gaussian random walk: compile the wide kernel of a
+        ``CudaModel`` with 32 < dims <= 192 now, not in the first sample().  ``compile_log``: ptxas's report, or ``""``
+        on every other engine."""
+        from ._util import compile_log
+        from .models import CudaModel
+        self.compile_log = ""
+        if isinstance(self._model, CudaModel):
+            self.compile_log = compile_log(
+                lambda log, n: L.lib().bk_user_wide_prepare(self._model.handle, log, n),
+                f"{who}: NVRTC compilation of the model's wide kernels failed:\n", self.device)
+
     def _need_grad_cache(self):
         if self._grad is None:
             self._grad = torch.empty_like(self._theta)

@@ -42,6 +42,19 @@ bool use_fused(const Model& m) { return m.separable() && m.d.dims <= SEP_MAX_D &
 // user-written CUDA model with D <= USER_FUSED_MAX_D: one register-resident kernel per call (user_model.cu)
 bool use_user_fused(const Model& m) { return user_fused(m) && !force_generic(); }
 
+// user-written CUDA model with USER_FUSED_MAX_D < D <= USER_WIDE_MAX_D: one kernel per call with the trajectory in
+// shared memory and the state in the generic engine's (lp, grad) cache (user_model.cu)
+bool use_user_wide(const Model& m) { return user_wide(m) && !force_generic(); }
+
+UserWideArgs wide_args(const UserRunArgs& run, void* lp, void* grad) {
+    UserWideArgs a;
+    memset(&a, 0, sizeof(a));
+    a.run = run;
+    a.lp = lp;
+    a.grad = grad;
+    return a;
+}
+
 template <typename T>
 void fill_sep(SepArgs<T>& a, const Model& m, void* theta, int64_t C, const void* metric, int64_t n,
               const bk_rng* rng, const bk_draw_out& out) {
@@ -107,6 +120,15 @@ int hmc_t(const Model& m, void* theta, void* lp, void* grad, int32_t* valid, int
         return user_fused_sample(m, nullptr, ALGO_HMC, a, valid, st);
     }
     BK_CHECK_ARG(lp && grad, "bk_hmc_diag_sample: lp_cache/grad_cache are required for this model");
+    if (use_user_wide(m)) {
+        UserRunArgs r = user_args(m, theta, C, n, rng, out);
+        r.metric = metric;
+        r.eps = eps;
+        r.half_eps = 0.5 * eps;
+        r.L = L;
+        UserWideArgs a = wide_args(r, lp, grad);
+        return user_wide_sample(m, ALGO_HMC, a, valid, st);
+    }
     if constexpr (sizeof(T) == 4) {
         // tensor-core pipeline: L-1 fused bf16 steps + one split-precision endpoint gradient
         if (dense_tc_enabled(m) && L >= 1)
@@ -143,6 +165,14 @@ int mala_t(const Model& m, void* theta, void* lp, void* grad, int32_t* valid, in
         return user_fused_sample(m, nullptr, ALGO_MALA, a, valid, st);
     }
     BK_CHECK_ARG(lp && grad, "bk_mala_sample: lp_cache/grad_cache are required for this model");
+    if (use_user_wide(m)) {
+        UserRunArgs r = user_args(m, theta, C, n, rng, out);
+        r.eps = eps;
+        r.sd = sd;
+        r.coef = coef;
+        UserWideArgs a = wide_args(r, lp, grad);
+        return user_wide_sample(m, ALGO_MALA, a, valid, st);
+    }
     if constexpr (sizeof(T) == 4) {
         // theta + eps g + sqrt(2 eps) z is one leapfrog step of size h = sqrt(2 eps) from momentum z,
         // and the Hastings ratio equals the Hamiltonian difference: begin -> split-precision
@@ -179,6 +209,14 @@ int mh_t(const Model& m, void* theta, void* lp, int32_t* valid, int64_t C, doubl
         return user_fused_sample(m, nullptr, ALGO_MHRW, a, valid, st);
     }
     BK_CHECK_ARG(lp, "bk_mh_rw_sample: lp_cache is required for this model");
+    if (use_user_wide(m)) {
+        UserRunArgs r = user_args(m, theta, C, n, rng, out);
+        r.scale = scale;
+        r.s2 = scale * scale;
+        r.hastings = hastings;
+        UserWideArgs a = wide_args(r, lp, nullptr);
+        return user_wide_sample(m, ALGO_MHRW, a, valid, st);
+    }
     GenArgs<T> p;
     fill_gen(p, m, theta, lp, nullptr, C, nullptr, n, rng, out);
     p.scale = (T)scale;
@@ -268,7 +306,7 @@ size_t sampler_ws(uint64_t h, int64_t C) {
     const Model* m = get_model(h);
     if (!m || C <= 0) return 0;
     if (m->separable() && m->d.dims <= SEP_MAX_D && !force_generic()) return 0;
-    if (use_user_fused(*m)) return 0;
+    if (use_user_fused(*m) || use_user_wide(*m)) return 0;
     if (dense_tc_enabled(*m)) {
         size_t a = dense_tc_hmc_ws_bytes(*m, C), b = generic_ws_bytes<float>(*m, C);
         return a > b ? a : b;
@@ -405,6 +443,13 @@ int bk_mh_rw_sample(uint64_t handle, void* theta, void* lp_cache, int32_t* cache
         rc = mh_t<float>(*m, theta, lp_cache, cache_valid_host, C, scale, hastings, n_draws, rng, o, ws,
                        ws_bytes, (cudaStream_t)stream);
     return rc ? rc : finish_extras(*m, o, C, n_draws, stream);
+}
+
+int bk_user_wide_prepare(uint64_t model, char* log_out, size_t log_bytes) {
+    if (log_out && log_bytes) log_out[0] = '\0';
+    const Model* m = get_model(model);
+    if (!m) return BK_E_HANDLE;
+    return use_user_wide(*m) ? user_wide_prepare(*m, log_out, log_bytes) : BK_OK;
 }
 
 size_t bk_mh_cuda_workspace_bytes(uint64_t model, uint64_t proposal, int64_t C) {

@@ -36,7 +36,15 @@ int register_model(const Model& m, uint64_t* handle_out);
 #define BK_USER_FUSED_MAX_D 32
 #endif
 constexpr int USER_FUSED_MAX_D = BK_USER_FUSED_MAX_D;
+// Above it, up to USER_WIDE_MAX_D, HMCDiag / MALA / RW-Metropolis run the wide kernels (trajectory in shared memory):
+// up to there they beat the generic engine on both measured models and all three samplers (DESIGN.md 4.4a).
+// Defining BK_USER_WIDE_MAX_D at build time moves this threshold too.
+#ifndef BK_USER_WIDE_MAX_D
+#define BK_USER_WIDE_MAX_D 192
+#endif
+constexpr int USER_WIDE_MAX_D = BK_USER_WIDE_MAX_D;
 struct UserRunArgs;
+struct UserWideArgs;
 struct UserSmcArgs;
 struct UserProposeArgs;
 // user-written CUDA proposals (bk_proposal_create_cuda)
@@ -57,6 +65,13 @@ UserRunArgs user_args(const Model& m, void* theta, int64_t C, int64_t n, const b
 // bk_user_hmc / mala / mh (algo: ALGO_*), or with a proposal p bk_user_mhp of the program of (m, p)
 int user_fused_sample(const Model& m, const UserProposal* p, int algo, const UserRunArgs& a, int32_t* cache_valid,
                       cudaStream_t st);
+// user model with USER_FUSED_MAX_D < dims <= USER_WIDE_MAX_D: the program of bk_user_wide_hmc / mala / mh, compiled
+// (once per process) by the prepare or on the first call, and one launch of its kernel for algo (ALGO_*).  The kernels
+// keep the generic engine's (lp, grad) cache valid: they evaluate it first when *cache_valid is 0 (or cache_valid is
+// NULL) and set *cache_valid.
+bool user_wide(const Model& m);
+int user_wide_prepare(const Model& m, char* log_out, size_t log_bytes);
+int user_wide_sample(const Model& m, int algo, UserWideArgs& a, int32_t* cache_valid, cudaStream_t st);
 // prior/likelihood user models (bk_model_create_cuda_prior_lik): log_prior / log_likelihood of theta [C, D] (each
 // output nullable) and TemperedLikelihoodSMC's move + weight kernel (move: BK_SMC_KERNEL_*; the PROPOSAL move runs
 // bk_user_smc_mhp of the program of (m, p))

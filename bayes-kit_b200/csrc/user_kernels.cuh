@@ -10,6 +10,8 @@
 //   BK_PROGRAM_MODEL_PROPOSAL   bk_user_mhp; prior/likelihood models also bk_user_smc_mhp
 //   BK_PROGRAM_DRGHMC           bk_user_drghmc (also compiled with -DBK_DRGHMC=1, which the model's source may test)
 //   BK_PROGRAM_STRETCH          bk_user_stretch (also compiled with -DBK_STRETCH=1, which the model's source may test)
+//   BK_PROGRAM_WIDE             bk_user_wide_hmc / mala / mh (BK_USER_FUSED_MAX_D < D <= BK_USER_WIDE_MAX_D; also
+//                               compiled with -DBK_WIDE=1, which the model's source may test)
 // -DBK_SMC_KERNELS=1 marks the programs that carry SMC kernels (prior/likelihood models, kinds MODEL and
 // MODEL_PROPOSAL): exactly those into which smc_mailbox.cuh is spliced.
 // A model's source defines either
@@ -46,6 +48,10 @@
 //                   lockstep engine (drghmc_generic.cu).
 // bk_user_stretch   one half-step of the Stretcher, one thread per active walker: k_stretch_propose, the density of
 //                   the proposal and k_stretch_accept (ensemble.cu) in one launch, on the same uniforms and arithmetic.
+// bk_user_wide_hmc/mala/mh
+//                   the fused samplers of bk_user_hmc / mala / mh for models too wide for registers: one thread per
+//                   chain, one warp of 32 consecutive chains per CTA, the trajectory in shared memory and the chain's
+//                   state (theta, log p, grad log p) in the generic engine's global cache, staged by the warp.
 #pragma once
 #ifndef __CUDACC_RTC__
 #include "smc_mailbox.cuh"
@@ -56,6 +62,7 @@
 #define BK_PROGRAM_MODEL_PROPOSAL 3
 #define BK_PROGRAM_DRGHMC 4
 #define BK_PROGRAM_STRETCH 5
+#define BK_PROGRAM_WIDE 6
 
 namespace bk {
 
@@ -112,6 +119,24 @@ struct UserStretchArgs {
     int32_t rng_mode, n_uniform;   // n_uniform = 3
     int32_t eval_lp;          // evaluate log p(active) first (the cache is invalid) and store it
 };
+#endif
+
+#if !defined(__CUDACC_RTC__) || BK_PROGRAM == BK_PROGRAM_WIDE
+// Launch arguments of bk_user_wide_hmc / _mala / _mh: `run` as for bk_user_hmc / _mala / _mh, and the generic engine's
+// cache of the chains' state, which the kernels keep valid: lp [C] = log p(theta), grad [C, D] = its gradient (HMC and
+// MALA only).
+struct UserWideArgs {
+    UserRunArgs run;
+    void* lp;                 // [C] in/out
+    void* grad;               // [C, D] in/out, or NULL (RW-Metropolis)
+    int32_t eval;             // the cache is stale: evaluate it at theta first
+};
+// Every CTA of a wide kernel is one warp of USER_WIDE_CHAINS chains with `vectors` [32, D] arrays in dynamic shared
+// memory, each row at an odd stride D | 1 (HMC: 3, MALA: 3, RW-Metropolis: 2).
+constexpr int USER_WIDE_CHAINS = 32;
+__host__ __device__ constexpr size_t user_wide_smem_bytes(int vectors, int64_t D, size_t elem) {
+    return (size_t)vectors * USER_WIDE_CHAINS * (size_t)(D | 1) * elem;
+}
 #endif
 
 // Launch arguments of bk_user_propose (one draw of a user proposal for C chains, three-launch path).  Streams: injected
@@ -984,6 +1009,321 @@ extern "C" __global__ void __launch_bounds__(128) bk_user_stretch(const bk::User
     }
     if (acc || a.eval_lp) *lpk = acc ? lpq : lp;
     if (a.accept) a.accept[k] = acc ? 1 : 0;
+}
+
+// ---- BK_PROGRAM_WIDE: HMCDiag / MALA / RW-Metropolis on a model wider than the registers, compiled on first use ---
+// One thread per chain, one warp of 32 consecutive chains per CTA, so that the warp's rows of every [C, D] array form
+// one contiguous block.  The vectors handed to the user's function are per-thread rows in dynamic shared memory at
+// the odd stride S = D | 1: when the 32 threads read element e together they hit 32 different banks, in fp32 and in
+// fp64.  The chain's state lives in the generic engine's cache in global memory: theta [C, D], lp [C] and grad [C, D].
+// The warp stages it in and out with coalesced copies (the element i of the block goes to lane i % 32), only where it
+// is needed: at the start of a call, and for the chains that rejected, whose shared rows hold the proposal.  After a
+// rejection nothing is written back.  The draws leave coalesced from shared memory.  Randomness and arithmetic are
+// those of bk_user_hmc / mala / mh: the same Philox words and the same sequence of Ar<T> operations.
+#elif BK_PROGRAM == BK_PROGRAM_WIDE
+
+namespace bk {
+namespace user {
+
+constexpr int W = USER_WIDE_CHAINS;
+constexpr int S = D | 1;
+
+// shared rows (stride S) of chains 0 .. n - 1 <-> their global block g [n, D]
+__device__ __forceinline__ void stage_in(T* s, const T* g, int n, int lane) {
+#pragma unroll 4
+    for (int i = lane; i < n * D; i += W) {
+        const int j = i / D;
+        s[j * S + i - j * D] = g[i];
+    }
+}
+__device__ __forceinline__ void stage_out(T* g, const T* s, int n, int lane) {
+#pragma unroll 4
+    for (int i = lane; i < n * D; i += W) {
+        const int j = i / D;
+        g[i] = s[j * S + i - j * D];
+    }
+}
+
+// After the accept tests of a draw (bit j of acc: chain j accepted), the shared rows x (and g, when given) of an
+// accepted chain hold its new state: they go to its global rows xg (and gg).  A rejected chain's shared rows that
+// the draw overwrote (g, and x when X_MOVED) are staged in from its global rows again.
+template <bool X_MOVED>
+__device__ __forceinline__ void commit(unsigned acc, T* x, T* xg, T* g, T* gg, int n, int lane) {
+#pragma unroll 4
+    for (int i = lane; i < n * D; i += W) {
+        const int j = i / D, k = j * S + i - j * D;
+        if ((acc >> j) & 1) {
+            xg[i] = x[k];
+            if (g) gg[i] = g[k];
+        } else {
+            if (X_MOVED) x[k] = xg[i];
+            if (g) g[k] = gg[i];
+        }
+    }
+}
+
+// the warp's geometry: first chain c0, chains present n (1 .. 32; fewer in the last CTA), this thread's chain c
+struct WideCta {
+    int lane, n;
+    int64_t c0, c;
+    bool live;
+    __device__ __forceinline__ WideCta(int64_t C) {
+        lane = (int)threadIdx.x;
+        c0 = (int64_t)blockIdx.x * W;
+        c = c0 + lane;
+        n = C - c0 < W ? (int)(C - c0) : W;
+        live = lane < n;
+    }
+};
+
+// draw t's outputs: the state rows x of every chain (coalesced), this thread's log density and accept flag
+__device__ __forceinline__ void wide_emit(const UserRunArgs& a, const WideCta& w, int64_t t, const T* x, T lp,
+                                          bool acc) {
+    if (w.live) {
+        if (a.logp) reinterpret_cast<T*>(a.logp)[t * a.C + w.c] = lp;
+        if (a.accept) a.accept[t * a.C + w.c] = acc ? 1 : 0;
+    }
+    if (a.draws) stage_out(reinterpret_cast<T*>(a.draws) + (t * a.C + w.c0) * (int64_t)D, x, w.n, w.lane);
+}
+
+}  // namespace user
+}  // namespace bk
+
+// HMCDiag: bk_user_hmc with q and its gradient in shared rows, the momentum element-major in shared memory.  At the
+// start of a draw the rows hold theta and grad log p(theta).
+extern "C" __global__ void __launch_bounds__(32) bk_user_wide_hmc(const bk::UserWideArgs wa) {
+    using namespace bk::user;
+    extern __shared__ __align__(16) unsigned char bk_smem[];
+    const bk::UserRunArgs& a = wa.run;
+    const WideCta w(a.C);
+    const T* params = reinterpret_cast<const T*>(a.params);
+    const T* metric = reinterpret_cast<const T*>(a.metric);
+    const T eps = (T)a.eps, half_eps = (T)a.half_eps;
+    T* sq = reinterpret_cast<T*>(bk_smem);
+    T* sg = sq + W * S;
+    T* r = sg + W * S + w.lane;   // element e at r[e * W]
+    T* q = sq + w.lane * S;
+    T* g = sg + w.lane * S;
+    T* th_g = reinterpret_cast<T*>(a.theta) + w.c0 * D;
+    T* gr_g = reinterpret_cast<T*>(wa.grad) + w.c0 * D;
+    T* lp_g = reinterpret_cast<T*>(wa.lp);
+    stage_in(sq, th_g, w.n, w.lane);
+    if (!wa.eval) stage_in(sg, gr_g, w.n, w.lane);
+    __syncwarp();
+    T lp = T(0);
+    if (wa.eval) {
+        if (w.live) lp_g[w.c] = lp = log_density_gradient(q, g, params);
+        __syncwarp();
+        stage_out(gr_g, sg, w.n, w.lane);
+    } else if (w.live) {
+        lp = lp_g[w.c];
+    }
+    for (int64_t t = 0; t < a.n_draws; ++t) {
+        bool acc = false;
+        T out = T(0);
+        if (w.live) {
+            T kin = T(0);
+#pragma unroll 2
+            for (int b = 0; b < NB; ++b) {
+                T z4[4];
+                normal4(a, a.C, w.c, t, b, z4);
+#pragma unroll
+                for (int i = 0; i < 4; ++i) {
+                    const int e = 4 * b + i;
+                    if (e >= D) break;
+                    const T z = z4[i];
+                    const T m = metric ? metric[e] : T(1);
+                    const T mg = metric ? A::mul(m, g[e]) : g[e];
+                    kin = A::add(kin, A::mul(z, metric ? A::mul(m, z) : z));
+                    T re = A::sub(z, A::mul(half_eps, mg));
+                    T qe = q[e];
+                    if (a.L > 0) {
+                        re = A::add(re, A::mul(eps, mg));
+                        qe = A::add(qe, A::mul(eps, re));
+                    }
+                    r[e * W] = re;
+                    q[e] = qe;
+                }
+            }
+            const T h0 = A::sub(lp, A::mul(T(0.5), kin));
+            T lpq = lp;
+            for (int s = 0; s < a.L; ++s) {
+                lpq = log_density_gradient(q, g, params);
+                if (s + 1 < a.L) {
+#pragma unroll 4
+                    for (int e = 0; e < D; ++e) {
+                        const T mg = metric ? A::mul(metric[e], g[e]) : g[e];
+                        const T re = A::add(r[e * W], A::mul(eps, mg));
+                        r[e * W] = re;
+                        q[e] = A::add(q[e], A::mul(eps, re));
+                    }
+                }
+            }
+            kin = T(0);
+#pragma unroll 4
+            for (int e = 0; e < D; ++e) {
+                const T m = metric ? metric[e] : T(1);
+                const T mg = metric ? A::mul(m, g[e]) : g[e];
+                const T re = A::add(r[e * W], A::mul(half_eps, mg));
+                kin = A::add(kin, A::mul(re, metric ? A::mul(m, re) : re));
+            }
+            const T h1 = A::sub(lpq, A::mul(T(0.5), kin));
+            acc = bk::log_u(accept_uniform(a, a.C, w.c, t, a.n_uniform != 1)) < A::sub(h1, h0);
+            if (acc) {
+                lp = lpq;
+                lp_g[w.c] = lp;
+            }
+            out = acc ? h1 : h0;
+        }
+        const unsigned am = __ballot_sync(0xffffffffu, acc);
+        __syncwarp();
+        commit<true>(am, sq, th_g, sg, gr_g, w.n, w.lane);
+        __syncwarp();
+        wide_emit(a, w, t, sq, out, acc);
+        __syncwarp();
+    }
+}
+
+// MALA: bk_user_mala with theta, the proposal and a gradient in shared rows.  At the start of a draw g holds
+// grad log p(theta); the user's function then overwrites it with the proposal's.  The forward proposal energy is
+// summed while the proposal is formed, before g is overwritten.
+extern "C" __global__ void __launch_bounds__(32) bk_user_wide_mala(const bk::UserWideArgs wa) {
+    using namespace bk::user;
+    extern __shared__ __align__(16) unsigned char bk_smem[];
+    const bk::UserRunArgs& a = wa.run;
+    const WideCta w(a.C);
+    const T* params = reinterpret_cast<const T*>(a.params);
+    const T eps = (T)a.eps, sd = (T)a.sd, coef = (T)a.coef;
+    T* sth = reinterpret_cast<T*>(bk_smem);
+    T* sq = sth + W * S;
+    T* sg = sq + W * S;
+    T* th = sth + w.lane * S;
+    T* q = sq + w.lane * S;
+    T* g = sg + w.lane * S;
+    T* th_g = reinterpret_cast<T*>(a.theta) + w.c0 * D;
+    T* gr_g = reinterpret_cast<T*>(wa.grad) + w.c0 * D;
+    T* lp_g = reinterpret_cast<T*>(wa.lp);
+    stage_in(sth, th_g, w.n, w.lane);
+    if (!wa.eval) stage_in(sg, gr_g, w.n, w.lane);
+    __syncwarp();
+    T lp = T(0);
+    if (wa.eval) {
+        if (w.live) lp_g[w.c] = lp = log_density_gradient(th, g, params);
+        __syncwarp();
+        stage_out(gr_g, sg, w.n, w.lane);
+    } else if (w.live) {
+        lp = lp_g[w.c];
+    }
+    for (int64_t t = 0; t < a.n_draws; ++t) {
+        bool acc = false;
+        if (w.live) {
+            T sf = T(0);
+#pragma unroll 2
+            for (int b = 0; b < NB; ++b) {
+                T z4[4];
+                normal4(a, a.C, w.c, t, b, z4);
+#pragma unroll
+                for (int i = 0; i < 4; ++i) {
+                    const int e = 4 * b + i;
+                    if (e >= D) break;
+                    const T qe = A::add(A::add(th[e], A::mul(eps, g[e])), A::mul(sd, z4[i]));
+                    const T df = A::sub(A::sub(qe, th[e]), A::mul(eps, g[e]));
+                    sf = A::add(sf, A::mul(df, df));
+                    q[e] = qe;
+                }
+            }
+            const T lpq = log_density_gradient(q, g, params);
+            T sr = T(0);
+#pragma unroll 4
+            for (int e = 0; e < D; ++e) {
+                const T dr = A::sub(A::sub(th[e], q[e]), A::mul(eps, g[e]));
+                sr = A::add(sr, A::mul(dr, dr));
+            }
+            const T fwd = A::mul(coef, sf), rev = A::mul(coef, sr);
+            acc = bk::log_u(accept_uniform(a, a.C, w.c, t, a.n_uniform != 1)) <
+                  A::add(A::sub(lpq, lp), A::sub(rev, fwd));
+            if (acc) {
+#pragma unroll 4
+                for (int e = 0; e < D; ++e) th[e] = q[e];
+                lp = lpq;
+                lp_g[w.c] = lp;
+            }
+        }
+        const unsigned am = __ballot_sync(0xffffffffu, acc);
+        __syncwarp();
+        commit<false>(am, sth, th_g, sg, gr_g, w.n, w.lane);
+        __syncwarp();
+        wide_emit(a, w, t, sth, lp, acc);
+        __syncwarp();
+    }
+}
+
+// Metropolis / MetropolisHastings with the Gaussian random walk: bk_user_mh with theta and the proposal in shared
+// rows.  The user's function writes its gradient to a thread-local array that is never read, so that those stores
+// die after inlining (stores to shared memory would not).
+extern "C" __global__ void __launch_bounds__(32) bk_user_wide_mh(const bk::UserWideArgs wa) {
+    using namespace bk::user;
+    extern __shared__ __align__(16) unsigned char bk_smem[];
+    const bk::UserRunArgs& a = wa.run;
+    const WideCta w(a.C);
+    const T* params = reinterpret_cast<const T*>(a.params);
+    const T scale = (T)a.scale, s2 = (T)a.s2;
+    T* sth = reinterpret_cast<T*>(bk_smem);
+    T* sq = sth + W * S;
+    T* th = sth + w.lane * S;
+    T* q = sq + w.lane * S;
+    T* th_g = reinterpret_cast<T*>(a.theta) + w.c0 * D;
+    T* lp_g = reinterpret_cast<T*>(wa.lp);
+    T unused[D];
+    stage_in(sth, th_g, w.n, w.lane);
+    __syncwarp();
+    T lp = T(0);
+    if (w.live) {
+        if (wa.eval) lp_g[w.c] = lp = log_density_gradient(th, unused, params);
+        else lp = lp_g[w.c];
+    }
+    for (int64_t t = 0; t < a.n_draws; ++t) {
+        bool acc = false;
+        if (w.live) {
+            T sf = T(0), sr = T(0);
+#pragma unroll 2
+            for (int b = 0; b < NB; ++b) {
+                T z4[4];
+                normal4(a, a.C, w.c, t, b, z4);
+#pragma unroll
+                for (int i = 0; i < 4; ++i) {
+                    const int e = 4 * b + i;
+                    if (e >= D) break;
+                    const T qe = A::add(th[e], A::mul(scale, z4[i]));
+                    if (a.hastings) {
+                        const T df = A::sub(qe, th[e]), dr = A::sub(th[e], qe);
+                        sf = A::add(sf, A::mul(df, df));
+                        sr = A::add(sr, A::mul(dr, dr));
+                    }
+                    q[e] = qe;
+                }
+            }
+            const T lpq = log_density_gradient(q, unused, params);
+            T ratio = A::sub(lpq, lp);
+            if (a.hastings) {
+                const T fwd = A::mul(T(-0.5), sf) / s2, rev = A::mul(T(-0.5), sr) / s2;
+                ratio = A::add(ratio, A::sub(rev, fwd));
+            }
+            acc = bk::log_u(accept_uniform(a, a.C, w.c, t, a.n_uniform != 1)) < ratio;
+            if (acc) {
+#pragma unroll 4
+                for (int e = 0; e < D; ++e) th[e] = q[e];
+                lp = lpq;
+                lp_g[w.c] = lp;
+            }
+        }
+        const unsigned am = __ballot_sync(0xffffffffu, acc);
+        __syncwarp();
+        commit<false>(am, sth, th_g, nullptr, nullptr, w.n, w.lane);
+        __syncwarp();
+        wide_emit(a, w, t, sth, lp, acc);
+        __syncwarp();
+    }
 }
 
 #endif  // BK_PROGRAM

@@ -18,8 +18,11 @@ class HMCDiag(ChainSampler):
     ``sample()`` returns ``(theta, joint_logp)`` exactly like hmc.py:55-63 (the
     JOINT log density ``log p(theta) - 0.5 rho.M.rho``).  One call advances all
     chains: a single fused kernel per call for iso/diagonal Gaussian plugins
-    (theta, rho in registers across the L leapfrog steps), a GEMM-gradient
-    pipeline for the dense / regression plugins.
+    (theta, rho in registers across the L leapfrog steps) and for a
+    ``CudaModel`` / ``CudaPriorLikModel`` up to 192 dims (registers up to 32,
+    the trajectory in shared memory above; the latter is compiled at
+    construction, ``compile_log`` holds ptxas's report, ``""`` on every other
+    engine), a GEMM-gradient pipeline for the dense / regression plugins.
 
     ``metric_diag``: the reference only works with None or a size-1 array
     (``metric_diag or np.ones(dim)``, hmc.py:22); a full [D] metric is accepted
@@ -43,6 +46,7 @@ class HMCDiag(ChainSampler):
             if m.numel() != self._dim:
                 raise ValueError(f"metric_diag must have {self._dim} entries")
             self._metric = m
+        self._prepare_wide("HMCDiag")
 
     def _launch(self, n, rng, out, c0=0, cn=None, cache_valid=None):
         lib = L.lib()

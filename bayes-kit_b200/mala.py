@@ -13,7 +13,9 @@ class MALA(ChainSampler):
     """``MALA(model, epsilon, init=None, seed=None)`` (mala.py:15-21).  Proposal
     ``theta + eps grad + sqrt(2 eps) z`` (mala.py:41-45), Hastings-corrected
     accept (mala.py:50-64); one gradient per draw with the current point's
-    (logp, grad) cached on device.  ``sample()`` returns ``(theta, log p(theta))``."""
+    (logp, grad) cached on device.  ``sample()`` returns ``(theta, log p(theta))``.  A ``CudaModel`` with
+    32 < dims <= 192 runs a kernel compiled at construction (``compile_log``: ptxas's report, ``""`` on every other
+    engine)."""
 
     def __init__(self, model, epsilon: float, init=None, seed=None, *,
                  chains: Optional[int] = None, chain_offset: int = 0):
@@ -21,6 +23,7 @@ class MALA(ChainSampler):
         self._epsilon = float(epsilon)
         if not self._epsilon > 0:
             raise ValueError(f"epsilon must be positive, got {epsilon}")
+        self._prepare_wide("MALA")
 
     def _launch(self, n, rng, out, c0=0, cn=None, cache_valid=None):
         lib = L.lib()

@@ -129,7 +129,9 @@ class MetropolisHastings(ChainSampler):
     """``MetropolisHastings(model, proposal_fn, transition_lp_fn, *, init=None,
     seed=None)`` (metropolis.py:80-99).  ``transition_lp_fn`` must be the
     proposal's own ``transition_lp`` (the Hastings terms are evaluated on
-    device; they cancel exactly for a symmetric proposal)."""
+    device; they cancel exactly for a symmetric proposal).  With ``GaussianRW`` and a ``CudaModel`` with
+    32 < dims <= 192 the sampler runs a kernel compiled at construction (``compile_log``: ptxas's report, ``""`` on
+    every other engine)."""
 
     _hastings = 1
 
@@ -153,6 +155,8 @@ class MetropolisHastings(ChainSampler):
             self.compile_log = compile_log(
                 lambda log, n: L.lib().bk_mh_cuda_prepare(self._model.handle, prop.handle, log, n),
                 "MetropolisHastings: NVRTC compilation of the model with the proposal failed:\n", self.device)
+        else:
+            self._prepare_wide(type(self).__name__)
 
     def _fuses_extras(self) -> bool:
         return not isinstance(self._proposal_fn, CudaProposal) and super()._fuses_extras()

@@ -179,9 +179,11 @@ BK_API int bk_model_log_prior_likelihood(uint64_t handle, const void* theta, int
  * the life of the process by (source, dims, dtype, prior/likelihood split) and never unloaded.  The handle works
  * everywhere a model handle does except the SMC, which needs the split (bk_model_create_cuda_prior_lik below):
  * HMCDiag, MALA and RW-Metropolis run one fused register-resident kernel per call for dims <= 32 (one thread per
- * chain; otherwise the generic engine), as do DrGhmcDiag and the Stretcher (see bk_drghmc_sample and
- * bk_stretch_move).  The fused kernels draw the same Philox words as every other engine; those of HMCDiag, MALA and
- * RW-Metropolis leave *cache_valid_host = 0.
+ * chain), as do DrGhmcDiag and the Stretcher (see bk_drghmc_sample and bk_stretch_move).  For 32 < dims <= 192
+ * HMCDiag, MALA and RW-Metropolis run one fused wide kernel per call (one thread per chain, the trajectory in shared
+ * memory, the state in lp_cache / grad_cache; see bk_user_wide_prepare); larger models run the generic engine.  The
+ * fused kernels draw the same Philox words as every other engine; the register-resident ones of HMCDiag, MALA and
+ * RW-Metropolis leave *cache_valid_host = 0, the wide ones keep the cache valid as the generic engine does.
  *
  * log_out [log_bytes] (may be NULL) receives NVRTC's log, truncated and NUL terminated; it includes ptxas's
  * register / spill report of every kernel.  Returns BK_E_INVALID on a bad argument or a compile error (the
@@ -207,6 +209,14 @@ BK_API int bk_model_create_cuda(const char* source, int64_t dims, int32_t dtype,
  * dims-element arrays). */
 BK_API int bk_model_create_cuda_prior_lik(const char* source, int64_t dims, int32_t dtype, const void* params,
                                           int64_t n_params, uint64_t* handle_out, char* log_out, size_t log_bytes);
+
+/* Compiles and loads the wide HMCDiag / MALA / RW-Metropolis program of a user model with 32 < dims <= 192
+ * (bk_user_wide_hmc / _mala / _mh, compiled from the model's source in a program of its own, once per process), so
+ * that the first bk_hmc_diag_sample / bk_mala_sample / bk_mh_rw_sample does not pay the NVRTC compile; log_out as
+ * bk_model_create_cuda's (ptxas's report of the three kernels).  BK_OK with an empty log for any other model,
+ * BK_E_HANDLE for an unknown handle, BK_E_INVALID on a compile error (with the log), BK_E_UNSUPPORTED without NVRTC.
+ * Source may test BK_WIDE (defined to 1 in this program). */
+BK_API int bk_user_wide_prepare(uint64_t model, char* log_out, size_t log_bytes);
 
 /* Initial states theta0 ~ N(0, I) (hmc.py:24-28, mala.py:26-30, metropolis.py:94-98; DrGhmcDiag's rho0,
  * drghmc.py:77): out [C, D] filled with device-Philox standard normals keyed by the GLOBAL chain id
