@@ -81,6 +81,8 @@ _SIGNATURES = {
     "bk_model_create_cuda_prior_lik": (C.c_int, [C.c_char_p, i64, i32, vp, i64, C.POINTER(u64), C.c_char_p, sz]),
     "bk_proposal_create_cuda": (C.c_int, [C.c_char_p, i64, i32, vp, i64, i32, i32, i32, C.POINTER(u64), C.c_char_p,
                                           sz]),
+    "bk_proposal_create_cuda_grad": (C.c_int, [C.c_char_p, i64, i32, vp, i64, i32, i32, i32, C.POINTER(u64),
+                                               C.c_char_p, sz]),
     "bk_proposal_destroy": (C.c_int, [u64]),
     "bk_user_wide_prepare": (C.c_int, [u64, C.c_char_p, sz]),
     "bk_mh_cuda_workspace_bytes": (sz, [u64, u64, i64]),

@@ -226,13 +226,22 @@ int mh_t(const Model& m, void* theta, void* lp, int32_t* valid, int64_t C, doubl
 }
 
 // ---- Metropolis / MetropolisHastings with a user proposal (bk_mh_cuda_*) ---------------------------------------------
-// fused: one bk_user_mhp launch per call (user model, dims and n_normals <= USER_FUSED_MAX_D); otherwise the generic
-// engine's ALGO_MHRW loop with bk_user_propose in place of k_mh_propose and its Hastings term in GenArgs::dh
+// fused: one bk_user_mhp (gradient proposals: bk_user_mhp_grad) launch per call (user model, dims and n_normals <=
+// USER_FUSED_MAX_D); otherwise the generic engine's ALGO_MHRW loop with bk_user_propose in place of k_mh_propose and
+// its Hastings term in GenArgs::dh (gradient proposals: bk_user_propose_grad, the model's evaluation with the gradient,
+// bk_user_dh_grad, k_mh_accept<T, true>)
 bool use_mhp_fused(const Model& m, const UserProposal& p) { return user_mhp_fusable(m, p) && !force_generic(); }
 
-// workspace of the three-launch path: [dh [C] | z, u scratch | generic engine]
+// the gradient cache of a gradient proposal on the three-launch path: grad log p(theta) [C, D] at the start of the
+// workspace, valid with lp_cache (bk.h)
+size_t proposal_grad_bytes(const Model& m, const UserProposal& p, int64_t C) {
+    return p.gradient ? align_up((size_t)C * m.d.dims * (m.d.dtype == BK_F64 ? 8 : 4), 256) : 0;
+}
+
+// workspace of the three-launch path: [grad [C, D] (gradient proposals) | dh [C] | z, u scratch | generic engine]
 size_t proposal_scratch_bytes(const Model& m, const UserProposal& p, int64_t C) {
-    return align_up((size_t)C * (m.d.dtype == BK_F64 ? 8 : 4), 256) + user_propose_ws_bytes(p, C);
+    return proposal_grad_bytes(m, p, C) + align_up((size_t)C * (m.d.dtype == BK_F64 ? 8 : 4), 256) +
+           user_propose_ws_bytes(p, C);
 }
 
 size_t mh_cuda_ws(const Model& m, const UserProposal& p, int64_t C) {
@@ -246,14 +255,32 @@ struct ProposeCtx {
     UserProposeArgs a;   // everything but theta, q, dh and t
 };
 
-int propose_hook(const void* ctx, const void* theta, void* q, void* dh, int64_t t, cudaStream_t st) {
+int propose_hook(const void* ctx, const void* theta, const void* grad, void* q, void* dh, int64_t t,
+                 cudaStream_t st) {
     const ProposeCtx* h = static_cast<const ProposeCtx*>(ctx);
     UserProposeArgs a = h->a;
     a.theta = theta;
     a.q = q;
     a.dh = dh;
     a.t = t;
-    return user_propose(*h->p, a, st);
+    if (!h->p->gradient) return user_propose(*h->p, a, st);
+    UserGradProposeArgs g;
+    memset(&g, 0, sizeof(g));
+    g.p = a;
+    g.grad = grad;
+    return user_propose_grad(*h->p, g, st);
+}
+
+int hastings_hook(const void* ctx, const void* theta, const void* q, const void* grad_q, void* dh, cudaStream_t st) {
+    const ProposeCtx* h = static_cast<const ProposeCtx*>(ctx);
+    UserGradProposeArgs g;
+    memset(&g, 0, sizeof(g));
+    g.p = h->a;
+    g.p.theta = theta;
+    g.p.q = const_cast<void*>(q);
+    g.p.dh = dh;
+    g.grad_q = grad_q;
+    return user_proposal_dh_grad(*h->p, g, st);
 }
 
 template <typename T>
@@ -271,6 +298,7 @@ int mh_cuda_t(const Model& m, const UserProposal& pr, void* theta, void* lp, int
     }
     BK_CHECK_ARG(lp, "bk_mh_cuda_sample: lp_cache is required for this model");
     Arena ar(ws, wsb);
+    T* grad = pr.gradient ? ar.take<T>((size_t)C * m.d.dims) : nullptr;
     T* dh = ar.take<T>(C);
     void* zbuf = ar.take<T>((size_t)C * pr.n_normals);
     void* ubuf = ar.take<T>((size_t)C * pr.n_uniforms);
@@ -294,9 +322,13 @@ int mh_cuda_t(const Model& m, const UserProposal& pr, void* theta, void* lp, int
     ctx.a.chain_offset = r.chain_offset;
     ctx.a.rng_mode = r.mode;
     ctx.a.n_uniform = r.n_uniform;
-    const MhProposeHook hook{propose_hook, &ctx};
+    MhProposeHook hook{propose_hook, &ctx};
+    if (pr.gradient) {
+        hook.gradient = true;
+        hook.hastings = hastings_hook;
+    }
     GenArgs<T> p;
-    fill_gen(p, m, theta, lp, nullptr, C, nullptr, n, &r, out);
+    fill_gen(p, m, theta, lp, grad, C, nullptr, n, &r, out);
     p.hastings = hastings;
     p.dh = hastings ? dh : nullptr;
     return run_generic<T>(m, p, ALGO_MHRW, valid, ar.base + ar.off, wsb - ar.off, st, &hook);

@@ -53,6 +53,7 @@ struct UserProposal {
     int64_t dims;
     int32_t dtype, n_normals, n_uniforms, has_transition;
     const void* params;          // [n_params] caller array, dtype, or NULL
+    int32_t gradient;            // bk_proposal_create_cuda_grad: propose / transition_log_density read grad log p
 };
 // returns nullptr (and sets the error) for an unknown handle
 const UserProposal* get_proposal(uint64_t handle);
@@ -96,6 +97,11 @@ int user_stretch_move(const Model& m, void* active, void* lp, bool eval_lp, cons
 // three-launch path: Philox scratch of bk_user_propose ([C, n_normals] and [C, n_uniforms]) and its launch
 size_t user_propose_ws_bytes(const UserProposal& p, int64_t C);
 int user_propose(const UserProposal& p, const UserProposeArgs& a, cudaStream_t st);
+// a gradient proposal's three-launch path: bk_user_propose_grad (q and the forward term) and, after the model's
+// evaluation of grad log p(q), bk_user_dh_grad (the Hastings term; proposals with a transition only)
+struct UserGradProposeArgs;
+int user_propose_grad(const UserProposal& p, const UserGradProposeArgs& a, cudaStream_t st);
+int user_proposal_dh_grad(const UserProposal& p, const UserGradProposeArgs& a, cudaStream_t st);
 
 size_t model_eval_ws_bytes(const Model& m, int64_t C);
 // true when model_eval(..., precise=false) is a genuinely cheaper (tensor-core) evaluation

@@ -200,7 +200,8 @@ __global__ void k_mh_propose(GenArgs<T> p, int64_t t) {
     }
 }
 
-template <typename T>
+// GRAD (gradient proposals): an accepted chain also takes grad log p(q) into the gradient cache
+template <typename T, bool GRAD = false>
 __global__ void k_mh_accept(GenArgs<T> p, int64_t t) {
     ROW_PROLOGUE();
     Row<T> row{p.rng, p.C, c, t, D, lane};
@@ -225,6 +226,7 @@ __global__ void k_mh_accept(GenArgs<T> p, int64_t t) {
         if (acc) {
             v = p.q[off + e];
             p.theta[off + e] = v;
+            if constexpr (GRAD) p.grad[off + e] = p.grad_q[off + e];
         } else {
             v = p.theta[off + e];
         }
@@ -276,7 +278,8 @@ int run_generic(const Model& m, GenArgs<T> p, int algo, int* cache_valid, void* 
     int rc = carve(m, p, ws, ws_bytes, &ews, &ebytes);
     if (rc) return rc;
     const unsigned blocks = (unsigned)((p.C * 32 + 255) / 256);
-    const bool need_grad = algo != ALGO_MHRW;
+    const bool gradient = propose && propose->gradient;   // a gradient proposal: ALGO_MHRW keeps grad too
+    const bool need_grad = algo != ALGO_MHRW || gradient;
     const bool fast = algo == ALGO_HMC && model_has_fast_path(m);
     if (!cache_valid || !*cache_valid) {
         if (fast) {   // same convention as inside the loop: tensor-core gradient, precise density
@@ -334,15 +337,23 @@ int run_generic(const Model& m, GenArgs<T> p, int algo, int* cache_valid, void* 
             BK_LAUNCH_CHECK();
         } else {
             if (propose) {
-                rc = propose->fn(propose->ctx, p.theta, p.q, p.dh, t, st);
+                rc = propose->fn(propose->ctx, p.theta, p.grad, p.q, p.dh, t, st);
                 if (rc) return rc;
             } else {
                 k_mh_propose<T><<<blocks, 256, 0, st>>>(p, t);
                 BK_LAUNCH_CHECK();
             }
-            rc = model_eval(m, p.q, p.C, p.lp_q, nullptr, ews, ebytes, st);
+            rc = model_eval(m, p.q, p.C, p.lp_q, gradient ? p.grad_q : nullptr, ews, ebytes, st);
             if (rc) return rc;
-            k_mh_accept<T><<<blocks, 256, 0, st>>>(p, t);
+            if (gradient) {
+                if (p.dh) {
+                    rc = propose->hastings(propose->ctx, p.theta, p.q, p.grad_q, p.dh, st);
+                    if (rc) return rc;
+                }
+                k_mh_accept<T, true><<<blocks, 256, 0, st>>>(p, t);
+            } else {
+                k_mh_accept<T><<<blocks, 256, 0, st>>>(p, t);
+            }
             BK_LAUNCH_CHECK();
         }
     }

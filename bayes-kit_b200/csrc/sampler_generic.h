@@ -29,11 +29,16 @@ struct GenArgs {
                 // place of the Gaussian random walk's; NULL: the built-in term (when hastings)
 };
 
-// Replaces k_mh_propose in run_generic's ALGO_MHRW loop (user proposals): writes q [C, D] from theta [C, D] for draw t
-// of the call, and dh [C] when dh is not NULL.
+// Replaces k_mh_propose in run_generic's ALGO_MHRW loop (user proposals): writes q [C, D] from theta [C, D] (and, for
+// a gradient proposal, grad [C, D] = grad log p(theta)) for draw t of the call, and dh [C] when dh is not NULL.
+// A gradient proposal (hastings not NULL) writes its forward term to dh; after the model's evaluation of q with its
+// gradient grad_q, hastings replaces it by the Hastings term.  The loop then keeps grad valid with lp.
 struct MhProposeHook {
-    int (*fn)(const void* ctx, const void* theta, void* q, void* dh, int64_t t, cudaStream_t st);
+    int (*fn)(const void* ctx, const void* theta, const void* grad, void* q, void* dh, int64_t t, cudaStream_t st);
     const void* ctx;
+    bool gradient = false;
+    int (*hastings)(const void* ctx, const void* theta, const void* q, const void* grad_q, void* dh,
+                    cudaStream_t st) = nullptr;
 };
 
 template <typename T>

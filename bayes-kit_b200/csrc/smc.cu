@@ -476,6 +476,11 @@ static int check_smc_proposal(const Model& m, const bk_smc_kernel& kn, const bk_
     }
     const UserProposal* p = get_proposal(kn.proposal);
     if (!p) return BK_E_HANDLE;
+    if (p->gradient) {
+        set_error("bk_smc: the proposal move does not take a gradient proposal (bk_proposal_create_cuda_grad): it "
+                  "would need the gradient of the tempered density; create the proposal with bk_proposal_create_cuda");
+        return BK_E_UNSUPPORTED;
+    }
     BK_CHECK_ARG(m.d.dims == p->dims && m.d.dtype == p->dtype,
                  "bk_smc: the proposal (dims %lld, dtype %d) does not match the model (dims %lld, dtype %d)",
                  (long long)p->dims, p->dtype, (long long)m.d.dims, m.d.dtype);

@@ -6,8 +6,10 @@
 // with -DBK_DIMS=D and -DBK_PROGRAM=<kind>, which selects one of the sections at the end of this file:
 //   BK_PROGRAM_MODEL            bk_user_eval; bk_user_hmc / mala / mh (D <= BK_USER_FUSED_MAX_D); prior/likelihood
 //                               models also bk_user_eval_pl and bk_user_smc_rw / mala / hmc
-//   BK_PROGRAM_PROPOSAL         bk_user_propose
-//   BK_PROGRAM_MODEL_PROPOSAL   bk_user_mhp; prior/likelihood models also bk_user_smc_mhp
+//   BK_PROGRAM_PROPOSAL         bk_user_propose; a gradient proposal (-DBK_PROPOSAL_GRADIENT=1) bk_user_propose_grad
+//                               and, with a transition, bk_user_dh_grad instead
+//   BK_PROGRAM_MODEL_PROPOSAL   bk_user_mhp; prior/likelihood models also bk_user_smc_mhp; a gradient proposal
+//                               bk_user_mhp_grad instead (no SMC kernel)
 //   BK_PROGRAM_DRGHMC           bk_user_drghmc (also compiled with -DBK_DRGHMC=1, which the model's source may test)
 //   BK_PROGRAM_STRETCH          bk_user_stretch (also compiled with -DBK_STRETCH=1, which the model's source may test)
 //   BK_PROGRAM_WIDE             bk_user_wide_hmc / mala / mh (BK_USER_FUSED_MAX_D < D <= BK_USER_WIDE_MAX_D; also
@@ -20,7 +22,8 @@
 //   __device__ bk_real log_prior_gradient(const bk_real* theta, bk_real* grad, const bk_real* params);
 //   __device__ bk_real log_likelihood_gradient(const bk_real* theta, bk_real* grad, const bk_real* params);
 // from which this file derives log_density_gradient = likelihood + prior.  A proposal's source defines propose() and,
-// with -DBK_PROPOSAL_TRANSITION=1, transition_log_density() (bk.h), for -DBK_PROPOSAL_NORMALS / _UNIFORMS streams.
+// with -DBK_PROPOSAL_TRANSITION=1, transition_log_density() (bk.h), for -DBK_PROPOSAL_NORMALS / _UNIFORMS streams;
+// with -DBK_PROPOSAL_GRADIENT=1 (bk_proposal_create_cuda_grad) both also read grad log p at their `from` point.
 //
 // bk_user_eval      one thread per chain on global rows: model_eval's case for this kind, through which the
 //                   generic HMC / MALA / RW-Metropolis engine, the lockstep DrGHMC engine and the Stretcher's
@@ -41,6 +44,11 @@
 //                   three-launch Metropolis(-Hastings) path.
 // bk_user_mhp       Metropolis / MetropolisHastings with a user proposal fused with a user model, one thread per
 //                   chain: bk_user_mh with propose() in place of the random walk.
+// bk_user_propose_grad / bk_user_dh_grad
+//                   the three-launch path of a gradient proposal: propose(theta, grad log p(theta)) with the forward
+//                   term log q(q | theta) in dh, and, after the model's evaluation of grad log p(q), dh = rev - fwd.
+// bk_user_mhp_grad  bk_user_mhp for a gradient proposal: bk_user_mala's state (theta, grad, log p in registers) with
+//                   propose() and transition_log_density() in place of the Langevin step and its Gaussian terms.
 // bk_user_smc_mhp   (prior/likelihood models) TemperedLikelihoodSMC's move + weight kernel with one
 //                   Metropolis(-Hastings) step of the user's proposal as the move: bk_user_smc_rw with propose() in
 //                   place of the random walk (BK_SMC_KERNEL_PROPOSAL).
@@ -155,6 +163,15 @@ struct UserProposeArgs {
     int64_t C, t;             // t: draw of this call
     uint64_t seed, draw_offset, chain_offset;
     int32_t rng_mode, n_uniform;
+};
+
+// Launch arguments of bk_user_propose_grad and bk_user_dh_grad (a gradient proposal's three-launch path): `p` as for
+// bk_user_propose, with p.dh the forward term log q(q | theta) written by the proposal launch (when not NULL) and
+// replaced by log q(theta | q) - log q(q | theta) in the second launch.
+struct UserGradProposeArgs {
+    UserProposeArgs p;
+    const void* grad;         // [C, D] grad log p(theta)
+    const void* grad_q;       // [C, D] grad log p(q): bk_user_dh_grad
 };
 
 #if !defined(__CUDACC_RTC__) || defined(BK_SMC_KERNELS)
@@ -341,6 +358,7 @@ __device__ __forceinline__ void proposal_streams(const S& s, const int64_t& C, i
     }
 }
 
+#ifndef BK_PROPOSAL_GRADIENT
 // log q(theta | q) - log q(q | theta), in MetropolisHastings's order: fwd = q(proposal | theta), rev = q(theta | proposal)
 __device__ __forceinline__ T proposal_dh(const T* th, const T* q, const T* pp) {
 #if BK_PROPOSAL_TRANSITION
@@ -351,6 +369,16 @@ __device__ __forceinline__ T proposal_dh(const T* th, const T* q, const T* pp) {
     return T(0);
 #endif
 }
+#elif BK_PROPOSAL_TRANSITION
+// a gradient proposal's terms: fwd = log q(q | theta) with g = grad log p(theta), rev = log q(theta | q) with
+// gq = grad log p(q); the Hastings term is A::sub(rev, fwd), as proposal_dh's
+__device__ __forceinline__ T proposal_fwd(const T* th, const T* g, const T* q, const T* pp) {
+    return bk_proposal::transition_log_density(q, th, g, pp);
+}
+__device__ __forceinline__ T proposal_rev(const T* th, const T* q, const T* gq, const T* pp) {
+    return bk_proposal::transition_log_density(th, q, gq, pp);
+}
+#endif
 
 }  // namespace user
 }  // namespace bk
@@ -721,6 +749,7 @@ extern "C" __global__ void __launch_bounds__(128) bk_user_smc_hmc(const bk::User
 // ---- BK_PROGRAM_PROPOSAL: a proposal's own program (bk_proposal_create_cuda) ----------------------------------------
 #elif BK_PROGRAM == BK_PROGRAM_PROPOSAL
 
+#ifndef BK_PROPOSAL_GRADIENT
 // One draw of the proposal for every chain: q = propose(theta, z, u) and, when dh is given, the Hastings term.
 extern "C" __global__ void __launch_bounds__(128) bk_user_propose(const bk::UserProposeArgs a) {
     using namespace bk::user;
@@ -745,6 +774,55 @@ extern "C" __global__ void __launch_bounds__(128) bk_user_propose(const bk::User
     if (a.dh) reinterpret_cast<T*>(a.dh)[c] = proposal_dh(th, q, pp);
 }
 
+#else  // BK_PROPOSAL_GRADIENT
+
+// One draw of a gradient proposal for every chain: q = propose(theta, grad, z, u), on bk_user_propose's streams, and,
+// when dh is given, the forward term log q(q | theta).
+extern "C" __global__ void __launch_bounds__(128) bk_user_propose_grad(const bk::UserGradProposeArgs ga) {
+    using namespace bk::user;
+    const bk::UserProposeArgs& a = ga.p;
+    const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= a.C) return;
+    const T* pp = reinterpret_cast<const T*>(a.params);
+    const T* th = reinterpret_cast<const T*>(a.theta) + c * (int64_t)D;
+    const T* g = reinterpret_cast<const T*>(ga.grad) + c * (int64_t)D;
+    T* q = reinterpret_cast<T*>(a.q) + c * (int64_t)D;
+    const T *z, *u;
+    if (a.rng_mode == 1) {   // BK_RNG_INJECTED: the proposal reads the rows in place
+        const int64_t r = a.t * a.C + c;
+        z = proposal_z(a, r);
+        u = proposal_u(a, r);
+    } else {   // Philox: through the scratch rows, so that a proposal of any size runs
+        T* zw = reinterpret_cast<T*>(a.zbuf) + c * NZ;
+        T* uw = reinterpret_cast<T*>(a.ubuf) + c * NU;
+        proposal_philox(a.seed, chain_word(a, c), draw_word(a, a.t), zw, uw);
+        z = zw;
+        u = uw;
+    }
+    bk_proposal::propose(th, g, q, z, u, pp);
+#if BK_PROPOSAL_TRANSITION
+    if (a.dh) reinterpret_cast<T*>(a.dh)[c] = proposal_fwd(th, g, q, pp);
+#endif
+}
+
+#if BK_PROPOSAL_TRANSITION
+// After the model's evaluation of grad log p(q): dh = log q(theta | q) - log q(q | theta), the forward term read from dh.
+extern "C" __global__ void __launch_bounds__(128) bk_user_dh_grad(const bk::UserGradProposeArgs ga) {
+    using namespace bk::user;
+    const bk::UserProposeArgs& a = ga.p;
+    const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= a.C) return;
+    const T* pp = reinterpret_cast<const T*>(a.params);
+    const T* th = reinterpret_cast<const T*>(a.theta) + c * (int64_t)D;
+    const T* q = reinterpret_cast<const T*>(a.q) + c * (int64_t)D;
+    const T* gq = reinterpret_cast<const T*>(ga.grad_q) + c * (int64_t)D;
+    T* dh = reinterpret_cast<T*>(a.dh) + c;
+    *dh = A::sub(proposal_rev(th, q, gq, pp), *dh);
+}
+#endif
+
+#endif  // BK_PROPOSAL_GRADIENT
+
 // ---- BK_PROGRAM_MODEL_PROPOSAL: a model's and a proposal's sources in one program, compiled on first use -----------
 #elif BK_PROGRAM == BK_PROGRAM_MODEL_PROPOSAL
 
@@ -753,6 +831,7 @@ extern "C" __global__ void __launch_bounds__(128) bk_user_propose(const bk::User
 extern "C" __global__ void __launch_bounds__(128) bk_user_smc_mhp(const bk::UserSmcArgs a) { bk::user::smc_move<3>(a); }
 #endif
 
+#ifndef BK_PROPOSAL_GRADIENT
 // Metropolis / MetropolisHastings with a user proposal, fused with the user's model: bk_user_mh with the random walk
 // replaced by propose() and its Gaussian Hastings sum by transition_log_density.  The model's gradient is dead code.
 extern "C" __global__ void __launch_bounds__(128) bk_user_mhp(const bk::UserRunArgs a) {
@@ -783,6 +862,47 @@ extern "C" __global__ void __launch_bounds__(128) bk_user_mhp(const bk::UserRunA
 #pragma unroll
     for (int e = 0; e < D; ++e) row[e] = th[e];
 }
+
+#else  // BK_PROPOSAL_GRADIENT
+
+// Metropolis / MetropolisHastings with a gradient proposal, fused with the user's model: bk_user_mala's state (theta,
+// grad log p(theta) and log p(theta) in registers across the draws) with propose(theta, grad) in place of the Langevin
+// step and transition_log_density(to, from, grad log p(from)) in place of its Gaussian terms.
+extern "C" __global__ void __launch_bounds__(128) bk_user_mhp_grad(const bk::UserRunArgs a) {
+    using namespace bk::user;
+    const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= a.C) return;
+    const T* params = reinterpret_cast<const T*>(a.params);
+    const T* pp = reinterpret_cast<const T*>(a.prop_params);
+    T* row = reinterpret_cast<T*>(a.theta) + c * (int64_t)D;
+    T th[D], g[D];
+    load_row(row, th);
+    T lp = log_density_gradient(th, g, params);
+    for (int64_t t = 0; t < a.n_draws; ++t) {
+        T q[D], gq[D], z[NZ1], u[NU1];
+        proposal_streams(a, a.C, c, t, z, u);
+        bk_proposal::propose(th, g, q, z, u, pp);
+        const T lpq = log_density_gradient(q, gq, params);
+        T ratio = A::sub(lpq, lp);
+#if BK_PROPOSAL_TRANSITION
+        if (a.hastings) ratio = A::add(ratio, A::sub(proposal_rev(th, q, gq, pp), proposal_fwd(th, g, q, pp)));
+#endif
+        const bool acc = bk::log_u(accept_uniform(a, a.C, c, t, a.n_uniform != 1)) < ratio;
+        if (acc) {
+#pragma unroll
+            for (int e = 0; e < D; ++e) {
+                th[e] = q[e];
+                g[e] = gq[e];
+            }
+            lp = lpq;
+        }
+        emit(a, c, t, th, lp, acc);
+    }
+#pragma unroll
+    for (int e = 0; e < D; ++e) row[e] = th[e];
+}
+
+#endif  // BK_PROPOSAL_GRADIENT
 
 // ---- BK_PROGRAM_DRGHMC: DrGhmcDiag on a model, compiled on first use ------------------------------------------------
 // One chain per thread follows its own retry / accept / ghost schedule (drghmc.py:348-446) and integrates only the

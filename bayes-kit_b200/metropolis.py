@@ -67,10 +67,24 @@ class CudaProposal:
     model's.  Pass the object as ``proposal_fn`` and its ``transition_lp`` as ``transition_lp_fn``.  With a
     ``CudaModel`` of ``dims <= 32`` (and ``normals <= 32``) the sampler runs one fused kernel per call, compiled at
     construction; otherwise three launches per draw (proposal, model, accept test).  A compile error raises
-    ``ValueError`` with NVRTC's log; ``compile_log`` holds the log of a successful compile."""
+    ``ValueError`` with NVRTC's log; ``compile_log`` holds the log of a successful compile.
+
+    With ``gradient=True`` the proposal also reads the gradient of the sampler's model (MALA, preconditioned MALA,
+    the Barker proposal, any drift-plus-noise move)::
+
+        __device__ void propose(const bk_real* theta, const bk_real* grad, bk_real* proposal, const bk_real* z,
+                                const bk_real* u, const bk_real* params);
+        __device__ bk_real transition_log_density(const bk_real* to, const bk_real* from, const bk_real* grad_from,
+                                                  const bk_real* params);
+
+    ``grad`` is ``grad log p(theta)`` and ``grad_from`` is ``grad log p(from)``; the Hastings term is
+    ``transition_log_density(theta, q, grad log p(q)) - transition_log_density(q, theta, grad log p(theta))``.  The
+    fused kernel keeps the gradient in registers; every other model runs four launches per draw (proposal, the
+    model's log density and gradient, the Hastings term, accept test), three without a Hastings term.  The SMC's
+    ``proposal_kernel`` does not take a gradient proposal."""
 
     def __init__(self, source: str, dims: int, params=None, normals=None, uniforms: int = 0, transition: bool = True,
-                 dtype=torch.float32, device="cuda"):
+                 dtype=torch.float32, device="cuda", gradient: bool = False):
         from .models import _load_nvrtc
         if not isinstance(source, str):
             raise TypeError("source must be a str of CUDA C++")
@@ -85,6 +99,7 @@ class CudaProposal:
         self.normals = self.dims if normals is None else int(normals)
         self.uniforms = int(uniforms)
         self.transition = bool(transition)
+        self.gradient = bool(gradient)
         self.params = None
         if params is not None:
             self.params = to_dev(params, dtype, self.device).reshape(-1)
@@ -93,10 +108,10 @@ class CudaProposal:
         n_params = 0 if self.params is None else self.params.numel()
         _load_nvrtc()
         h = L.u64(0)
+        create = L.lib().bk_proposal_create_cuda_grad if self.gradient else L.lib().bk_proposal_create_cuda
         self.compile_log = compile_log(
-            lambda log, n: L.lib().bk_proposal_create_cuda(source.encode(), self.dims, dtype_id(dtype), ptr(self.params),
-                                                           n_params, self.normals, self.uniforms, int(self.transition),
-                                                           C.byref(h), log, n),
+            lambda log, n: create(source.encode(), self.dims, dtype_id(dtype), ptr(self.params), n_params,
+                                  self.normals, self.uniforms, int(self.transition), C.byref(h), log, n),
             "CudaProposal: NVRTC compilation failed:\n", self.device)
         self._handle = h.value
 
@@ -151,6 +166,9 @@ class MetropolisHastings(ChainSampler):
                 raise ValueError(f"the proposal (dims {prop.dims}, {prop.dtype}) does not match the model "
                                  f"(dims {self._dim}, {self.dtype})")
             self._n_normal, self._n_uniform = prop.normals, 1 + prop.uniforms
+            # gradient proposals, three-launch path: the library caches grad log p(theta) in the workspace, for the
+            # rows of the last call; a call on other rows (sample_host's chunks) re-evaluates it
+            self._ws_grad_rows = None
             # compile the fused kernel now, not in the first sample(); its log, or "" (three launches)
             self.compile_log = compile_log(
                 lambda log, n: L.lib().bk_mh_cuda_prepare(self._model.handle, prop.handle, log, n),
@@ -164,10 +182,15 @@ class MetropolisHastings(ChainSampler):
     def _launch(self, n, rng, out, c0=0, cn=None, cache_valid=None):
         lib = L.lib()
         cn = self._C if cn is None else cn
-        cv = C.byref(self._cache_valid if cache_valid is None else cache_valid)
+        valid = self._cache_valid if cache_valid is None else cache_valid
+        cv = C.byref(valid)
         prop = self._proposal_fn
         if isinstance(prop, CudaProposal):
             wp, wn = self._ws.get(lib.bk_mh_cuda_workspace_bytes(self._model.handle, prop.handle, self._C))
+            if prop.gradient:
+                if self._ws_grad_rows != (c0, cn):
+                    valid.value = 0
+                self._ws_grad_rows = (c0, cn)
             L.check(lib.bk_mh_cuda_sample(
                 self._model.handle, prop.handle, self._theta[c0:].data_ptr(), self._lp[c0:].data_ptr(), cv, cn,
                 self._hastings, n, C.byref(rng), C.byref(out), wp, wn, stream_ptr(self.device)))

@@ -90,6 +90,9 @@ class ProposalKernel(_Kernel):
         if not isinstance(proposal, CudaProposal):
             raise TypeError("proposal_kernel needs a bayes_kit_b200.CudaProposal written in CUDA C++ "
                             f"(got {type(proposal).__name__})")
+        if proposal.gradient:
+            raise ValueError("proposal_kernel does not take a gradient proposal (CudaProposal(..., gradient=True)): "
+                             "the SMC's move would need the gradient of the tempered density")
         self.proposal = proposal          # keeps the handle alive as long as the kernel
 
     def desc(self) -> L.SmcKernel:

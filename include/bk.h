@@ -278,6 +278,22 @@ BK_API int bk_mh_rw_sample(uint64_t handle, void* theta, void* lp_cache, int32_t
 BK_API int bk_proposal_create_cuda(const char* source, int64_t dims, int32_t dtype, const void* params,
                                    int64_t n_params, int32_t n_normals, int32_t n_uniforms, int32_t has_transition,
                                    uint64_t* handle_out, char* log_out, size_t log_bytes);
+/* A gradient proposal: the same arguments, checks and returns, with a source that defines
+ *
+ *     __device__ void propose(const bk_real* theta, const bk_real* grad, bk_real* proposal, const bk_real* z,
+ *                             const bk_real* u, const bk_real* params);
+ *     __device__ bk_real transition_log_density(const bk_real* to, const bk_real* from, const bk_real* grad_from,
+ *                                               const bk_real* params);
+ *
+ * where grad = grad log p(theta) and grad_from = grad log p(from) of the sampler's model (e.g. MALA, preconditioned
+ * MALA or the Barker proposal).  Streams, limits and the injected layout are bk_proposal_create_cuda's; the
+ * Hastings term is transition_log_density(theta, theta', grad log p(theta')) - transition_log_density(theta', theta,
+ * grad log p(theta)).  The source is compiled with -DBK_PROPOSAL_GRADIENT=1.  bk_mh_cuda_* take the handle (below);
+ * the SMC's proposal move does not (BK_E_UNSUPPORTED). */
+BK_API int bk_proposal_create_cuda_grad(const char* source, int64_t dims, int32_t dtype, const void* params,
+                                        int64_t n_params, int32_t n_normals, int32_t n_uniforms,
+                                        int32_t has_transition, uint64_t* handle_out, char* log_out,
+                                        size_t log_bytes);
 BK_API int bk_proposal_destroy(uint64_t handle);
 /* Engines: a user model (bk_model_create_cuda*) with dims <= 32 and a proposal with n_normals <= 32 run one fused
  * kernel per call (bk_user_mhp: one thread per chain, theta and log p(theta) in registers across the draws; leaves
@@ -287,7 +303,13 @@ BK_API int bk_proposal_destroy(uint64_t handle);
  * lp_cache / cache_valid_host as there.  hastings != 0 adds transition_log_density(theta, theta') -
  * transition_log_density(theta', theta).  BK_E_INVALID when the model's and the proposal's dims or dtype differ,
  * when hastings != 0 and the proposal has no transition, or when INJECTED n_uniform != 1 + n_uniforms.  Draws are
- * [n_draws, C, D] only; streaming moments are folded from them. */
+ * [n_draws, C, D] only; streaming moments are folded from them.
+ * A gradient proposal (bk_proposal_create_cuda_grad) runs bk_user_mhp_grad on the fused engine (theta, grad log p and
+ * log p in registers) and, on every other model, four launches per draw (three without hastings): the proposal
+ * (bk_user_propose_grad), the model's evaluation of log p and its gradient, the Hastings term from grad log p(theta')
+ * (bk_user_dh_grad) and the accept test.  There grad log p(theta) [C, D] is cached in the first C * D elements of
+ * `ws`, kept valid with lp_cache: while *cache_valid_host is 1 the caller passes the same workspace, untouched, as
+ * on the previous call. */
 BK_API size_t bk_mh_cuda_workspace_bytes(uint64_t model, uint64_t proposal, int64_t C);
 BK_API int bk_mh_cuda_prepare(uint64_t model, uint64_t proposal, char* log_out, size_t log_bytes);
 BK_API int bk_mh_cuda_sample(uint64_t model, uint64_t proposal, void* theta, void* lp_cache,
