@@ -14,13 +14,13 @@ after 2 warm-up calls each):
   (c) the Barker proposal (one uniform per coordinate, so D <= 64) at the same D on the banana."""
 import json
 import os
-import re
-import subprocess
 import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
+
+from _user_cuda import BANANA, BARKER, MALA_G, card, ptxas_report  # noqa: E402
 
 C_ = 1 << 20
 N_DRAWS, WARM, REPS = 10, 2, 7
@@ -56,10 +56,9 @@ def timed(*samplers):
 
 def regs(log, kernel):
     """(registers, spill stores, spill loads) of `kernel` in a ptxas report."""
-    m = re.search("'" + kernel + r"'[\s\S]*?(\d+) bytes spill stores, (\d+) bytes spill loads[\s\S]*?Used (\d+) registers",
-                  log)
-    return None if m is None else {"registers": int(m.group(3)), "spill_stores": int(m.group(1)),
-                                   "spill_loads": int(m.group(2))}
+    r = ptxas_report(log).get(kernel)
+    return None if r is None else {"registers": r["registers"], "spill_stores": r["spill_store_bytes"],
+                                   "spill_loads": r["spill_load_bytes"]}
 
 
 def main(out_path):
@@ -67,10 +66,8 @@ def main(out_path):
     import torch
 
     import bayes_kit_b200 as bk
-    from test_user_grad_proposal_host import BANANA, BARKER, MALA_G
 
-    smi = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader", "-i", "0"],
-                         capture_output=True, text=True).stdout.strip()
+    smi = card()
     res = {"gpu": smi, "chains": C_, "draws_per_call": N_DRAWS, "dtype": "float32",
            "timing": f"two sides alternating call by call; median of {REPS} calls each after {WARM} warm-up calls "
                      "each, CUDA events", "ptxas": {}, "a_mala_user": {}, "b_mala_diag": {}, "c_barker": {}}

@@ -11,64 +11,24 @@ kernels above the library's dispatch threshold, the script links a variant of th
 with BK_USER_FUSED_MAX_D = 64 (the default build is left alone).  Per point: median of 7 timed calls after 2 warm-up
 calls; wall time by CUDA events, kernel time by bk_profile_read (fused: BK_PROF_SAMPLER; generic: the model
 evaluations, BK_PROF_GRAD) in separate calls."""
-import glob
 import json
 import os
-import re
-import subprocess
 import sys
 import tempfile
 import time
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-PKG = os.path.join(ROOT, "bayes-kit_b200")
+sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests"))
+
+from _user_cuda import BANANA, DIAG, build_variant, card, ptxas_report  # noqa: E402
+
 MAX_D = 64
-
-
-def build_variant(tmp):
-    sys.path.insert(0, PKG)
-    import build as b
-    b.build()
-    nvcc = b.NVCC
-    obj = os.path.join(tmp, "user_model.o")
-    subprocess.run([nvcc, *b.FLAGS, f"-DBK_USER_FUSED_MAX_D={MAX_D}", "-c", os.path.join(b.CSRC, "user_model.cu"),
-                    "-o", obj], check=True)
-    objs = [o for o in glob.glob(os.path.join(b.OBJ, "*.o")) if not o.endswith("user_model.o")] + [obj]
-    lib = os.path.join(tmp, "libbk_b200.so")
-    subprocess.run([nvcc, "-shared", "-o", lib, *objs, "-gencode", "arch=compute_100a,code=sm_100a", "-cudart",
-                    "static", "-Xcompiler", "-fPIC", "-ldl"], check=True)
-    return lib
-
-
-BANANA = """
-__device__ bk_real log_density_gradient(const bk_real* x, bk_real* g, const bk_real* params) {
-    const bk_real b = params[0], half = 0.5, two = 2;
-    const bk_real u = x[1] - b * x[0] * x[0];
-    bk_real lp = -half * (x[0] * x[0]) - half * (u * u);
-    g[0] = -x[0] + two * b * x[0] * u;
-    g[1] = -u;
-    for (int e = 2; e < BK_DIMS; ++e) { lp -= half * (x[e] * x[e]); g[e] = -x[e]; }
-    return lp;
-}
-"""
-DIAG = """
-__device__ bk_real log_density_gradient(const bk_real* x, bk_real* g, const bk_real* p) {
-    bk_real s = 0;
-    for (int e = 0; e < BK_DIMS; ++e) {
-        const bk_real d = x[e] - p[e];
-        const bk_real pd = p[BK_DIMS + e] * d;
-        s += d * pd;
-        g[e] = -pd;
-    }
-    return bk_real(-0.5) * s;
-}
-"""
 
 
 def main(out_path):
     tmp = tempfile.mkdtemp(prefix="bk_user_time_")
-    os.environ["BK_LIB"] = build_variant(tmp)
-    sys.path.insert(0, ROOT)
+    os.environ["BK_LIB"] = build_variant(tmp, f"BK_USER_FUSED_MAX_D={MAX_D}")
     import numpy as np
     import torch
 
@@ -76,8 +36,7 @@ def main(out_path):
     from bayes_kit_b200 import _lib as L
 
     lib = L.lib()
-    smi = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader", "-i", "0"],
-                         capture_output=True, text=True).stdout.strip()
+    smi = card()
     res = {"gpu": smi, "chains": 1 << 20, "steps_L": 10, "draws_per_call": 10, "dtype": "float32",
            "fused_max_d_of_variant": MAX_D, "compile_s": {}, "points": []}
 
@@ -123,14 +82,9 @@ def main(out_path):
                 "accept": acc}
 
     def regs(log):
-        out = {}
-        for k in ("bk_user_hmc", "bk_user_mala", "bk_user_mh", "bk_user_eval"):
-            m = re.search(rf"Function properties for {k}\n.*?(\d+) bytes spill stores, (\d+) bytes spill loads\n"
-                          rf".*?Used (\d+) registers", log, re.S)
-            if m:
-                out[k] = {"registers": int(m.group(3)), "spill_store_bytes": int(m.group(1)),
-                          "spill_load_bytes": int(m.group(2))}
-        return out
+        rep = ptxas_report(log)
+        return {k: {f: rep[k][f] for f in ("registers", "spill_store_bytes", "spill_load_bytes")}
+                for k in ("bk_user_hmc", "bk_user_mala", "bk_user_mh", "bk_user_eval") if k in rep}
 
     rng = np.random.default_rng(0)
     for D in (2, 8, 16, 32, 64):

@@ -15,65 +15,18 @@ warm-up calls, CUDA events around each call):
   (c) the log-normal walk and the independence sampler at D = 16 on the banana (fused)."""
 import json
 import os
-import re
 import subprocess
 import sys
 import time
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests"))
+
+from _user_cuda import BANANA, INDEP, LOGNORMAL_NO_HELPER, RW, card, ptxas_report  # noqa: E402
 
 C_ = 1 << 20
 N_DRAWS, WARM, REPS = 10, 2, 7
-
-BANANA = """
-__device__ bk_real log_density_gradient(const bk_real* x, bk_real* g, const bk_real* params) {
-    const bk_real b = params[0], half = 0.5, two = 2;
-    const bk_real u = x[1] - b * x[0] * x[0];
-    bk_real lp = -half * (x[0] * x[0]) - half * (u * u);
-    g[0] = -x[0] + two * b * x[0] * u;
-    g[1] = -u;
-    for (int e = 2; e < BK_DIMS; ++e) { lp -= half * (x[e] * x[e]); g[e] = -x[e]; }
-    return lp;
-}
-"""
-RW = """
-__device__ void propose(const bk_real* theta, bk_real* q, const bk_real* z, const bk_real* u, const bk_real* p) {
-    for (int e = 0; e < BK_DIMS; ++e) q[e] = theta[e] + p[0] * z[e];
-}
-__device__ bk_real transition_log_density(const bk_real* to, const bk_real* from, const bk_real* p) {
-    bk_real s = 0;
-    for (int e = 0; e < BK_DIMS; ++e) { const bk_real d = to[e] - from[e]; s += d * d; }
-    return bk_real(-0.5) * s / (p[0] * p[0]);
-}
-"""
-LOGNORMAL = """
-__device__ void propose(const bk_real* theta, bk_real* q, const bk_real* z, const bk_real* u, const bk_real* p) {
-    for (int e = 0; e < BK_DIMS; ++e) q[e] = theta[e] * exp(p[0] * z[e]);
-}
-__device__ bk_real transition_log_density(const bk_real* to, const bk_real* from, const bk_real* p) {
-    bk_real s = 0;
-    for (int e = 0; e < BK_DIMS; ++e) {
-        const bk_real d = (log(to[e]) - log(from[e])) / p[0];
-        s += bk_real(-0.5) * (d * d) - log(to[e]);
-    }
-    return s;
-}
-"""
-INDEP = """
-__device__ void propose(const bk_real* theta, bk_real* q, const bk_real* z, const bk_real* u, const bk_real* p) {
-    for (int e = 0; e < BK_DIMS; ++e) q[e] = p[e] + p[BK_DIMS + e] * z[e];
-}
-__device__ bk_real transition_log_density(const bk_real* to, const bk_real* from, const bk_real* p) {
-    bk_real s = 0;
-    for (int e = 0; e < BK_DIMS; ++e) {
-        const bk_real d = (to[e] - p[e]) / p[BK_DIMS + e];
-        s += bk_real(-0.5) * (d * d) - log(p[BK_DIMS + e]);
-    }
-    return s;
-}
-"""
-
 
 def timed(sampler):
     import torch
@@ -115,9 +68,9 @@ def child():
 
 def regs(log, kernel):
     """(registers, spill stores, spill loads) of `kernel` in a ptxas report."""
-    m = re.search(kernel + r"[\s\S]*?(\d+) bytes spill stores, (\d+) bytes spill loads[\s\S]*?Used (\d+) registers", log)
-    return None if m is None else {"registers": int(m.group(3)), "spill_stores": int(m.group(1)),
-                                   "spill_loads": int(m.group(2))}
+    r = ptxas_report(log).get(kernel)
+    return None if r is None else {"registers": r["registers"], "spill_stores": r["spill_store_bytes"],
+                                   "spill_loads": r["spill_load_bytes"]}
 
 
 def main(out_path):
@@ -126,8 +79,7 @@ def main(out_path):
 
     import bayes_kit_b200 as bk
 
-    smi = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader", "-i", "0"],
-                         capture_output=True, text=True).stdout.strip()
+    smi = card()
     res = {"gpu": smi, "chains": C_, "draws_per_call": N_DRAWS, "dtype": "float32",
            "timing": f"median of {REPS} calls after {WARM} warm-up calls, CUDA events", "compile": {}, "ptxas": {},
            "a_fused": {}, "b_three_launch": {}, "c_asymmetric": {}}
@@ -189,7 +141,7 @@ def main(out_path):
     D = 16
     model = bk.CudaModel(BANANA, D, params=[0.5])
     init = torch.rand(C_, D, device="cuda") + 0.5
-    p = bk.CudaProposal(LOGNORMAL, D, params=[0.3])
+    p = bk.CudaProposal(LOGNORMAL_NO_HELPER, D, params=[0.3])
     s = bk.MetropolisHastings(model, p, p.transition_lp, init=init, seed=1)
     res["c_asymmetric"]["lognormal_D16"] = timed(s)
     res["ptxas"]["bk_user_mhp_lognormal_D16"] = regs(s.compile_log, "bk_user_mhp")

@@ -11,30 +11,14 @@ run.  Also records the card name and power limit, the NVRTC compile + load time 
 and the registers / spill bytes of bk_user_smc_* per D from the compile log."""
 import json
 import os
-import re
-import subprocess
 import sys
 import time
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests"))
 
-GPL = """
-__device__ bk_real quad(const bk_real* x, bk_real* g, const bk_real* m, const bk_real* p) {
-    bk_real s = 0;
-    for (int e = 0; e < BK_DIMS; ++e) {
-        const bk_real d = x[e] - m[e], pd = p[e] * d;
-        s += pd * d;
-        g[e] = -pd;
-    }
-    return bk_real(-0.5) * s;
-}
-__device__ bk_real log_prior_gradient(const bk_real* x, bk_real* g, const bk_real* p) {
-    return quad(x, g, p + 2 * BK_DIMS, p + 3 * BK_DIMS);
-}
-__device__ bk_real log_likelihood_gradient(const bk_real* x, bk_real* g, const bk_real* p) {
-    return quad(x, g, p, p + BK_DIMS);
-}
-"""
+from _user_cuda import GPL, card, ptxas_report  # noqa: E402
 
 KERNELS = {"rw": 0.2, "mala": 0.05, "hmc": 0.1}
 DIMS = (2, 8, 16, 32, 50)
@@ -42,26 +26,19 @@ M, N, SEED, REPS = 1_000_000, 100, 1, 5
 
 
 def regs(log):
-    out = {}
-    for k in ("bk_user_smc_rw", "bk_user_smc_mala", "bk_user_smc_hmc", "bk_user_eval_pl"):
-        m = re.search(rf"Function properties for {k}\n.*?(\d+) bytes spill stores, (\d+) bytes spill loads\n"
-                      rf".*?Used (\d+) registers", log, re.S)
-        if m:
-            out[k] = {"registers": int(m.group(3)), "spill_store_bytes": int(m.group(1)),
-                      "spill_load_bytes": int(m.group(2))}
-    return out
+    rep = ptxas_report(log)
+    return {k: {f: rep[k][f] for f in ("registers", "spill_store_bytes", "spill_load_bytes")}
+            for k in ("bk_user_smc_rw", "bk_user_smc_mala", "bk_user_smc_hmc", "bk_user_eval_pl") if k in rep}
 
 
 def main(out_path):
-    sys.path.insert(0, ROOT)
     import numpy as np
     import torch
 
     import bayes_kit_b200 as bk
 
     assert torch.cuda.is_available(), "time_user_smc.py needs a CUDA device"
-    smi = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader", "-i", "0"],
-                         capture_output=True, text=True).stdout.strip()
+    smi = card()
     res = {"gpu": smi, "M": M, "N": N, "resample": "systematic", "dtype": "float32", "seed": SEED,
            "kernels": {"rw": {"scale": 0.2}, "mala": {"epsilon": 0.05}, "hmc": {"stepsize": 0.1, "steps": 5}},
            "runs_per_point": REPS, "compile_s": {}, "points": []}

@@ -15,90 +15,26 @@ bk_user_smc_rw from the compile logs."""
 import ctypes as C
 import json
 import os
-import re
-import subprocess
 import sys
 import time
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests"))
 
-GPL = """
-__device__ bk_real quad(const bk_real* x, bk_real* g, const bk_real* m, const bk_real* p) {
-    bk_real s = 0;
-    for (int e = 0; e < BK_DIMS; ++e) {
-        const bk_real d = x[e] - m[e], pd = p[e] * d;
-        s += pd * d;
-        g[e] = -pd;
-    }
-    return bk_real(-0.5) * s;
-}
-__device__ bk_real log_prior_gradient(const bk_real* x, bk_real* g, const bk_real* p) {
-    return quad(x, g, p + 2 * BK_DIMS, p + 3 * BK_DIMS);
-}
-__device__ bk_real log_likelihood_gradient(const bk_real* x, bk_real* g, const bk_real* p) {
-    return quad(x, g, p, p + BK_DIMS);
-}
-"""
-
-# Gamma(a, rate b) priors x Poisson likelihoods, params = [a, b, n, S (D)]
-GAMMA_POIS = """
-__device__ bk_real log_prior_gradient(const bk_real* x, bk_real* g, const bk_real* p) {
-    bk_real s = 0;
-    for (int e = 0; e < BK_DIMS; ++e) {
-        if (!(x[e] > 0)) return log(bk_real(0));
-        s += (p[0] - 1) * log(x[e]) - p[1] * x[e];
-        g[e] = (p[0] - 1) / x[e] - p[1];
-    }
-    return s;
-}
-__device__ bk_real log_likelihood_gradient(const bk_real* x, bk_real* g, const bk_real* p) {
-    bk_real s = 0;
-    for (int e = 0; e < BK_DIMS; ++e) {
-        if (!(x[e] > 0)) return log(bk_real(0));
-        s += p[3 + e] * log(x[e]) - p[2] * x[e];
-        g[e] = p[3 + e] / x[e] - p[2];
-    }
-    return s;
-}
-"""
-
-WALK = """
-__device__ void propose(const bk_real* theta, bk_real* q, const bk_real* z, const bk_real* u, const bk_real* p) {
-    for (int e = 0; e < BK_DIMS; ++e) q[e] = theta[e] + p[0] * z[e];
-}
-"""
-
-LOGNORMAL = """
-__device__ void propose(const bk_real* theta, bk_real* q, const bk_real* z, const bk_real* u, const bk_real* p) {
-    for (int e = 0; e < BK_DIMS; ++e) q[e] = theta[e] * exp(p[0] * z[e]);
-}
-__device__ bk_real transition_log_density(const bk_real* to, const bk_real* from, const bk_real* p) {
-    bk_real s = 0;
-    for (int e = 0; e < BK_DIMS; ++e) {
-        const bk_real d = (log(to[e]) - log(from[e])) / p[0];
-        s += bk_real(-0.5) * (d * d) - log(to[e]);
-    }
-    return s;
-}
-"""
+from _user_cuda import GAMMA_POIS, GPL, LOGNORMAL_NO_HELPER, WALK, card, ptxas_report  # noqa: E402
 
 DIMS = (2, 8, 16, 32, 50)
 M, N, SEED, REPS, SCALE = 1_000_000, 100, 1, 5, 0.2
 
 
 def regs(log, kernels):
-    out = {}
-    for k in kernels:
-        m = re.search(rf"Function properties for {k}\n.*?(\d+) bytes spill stores, (\d+) bytes spill loads\n"
-                      rf".*?Used (\d+) registers", log, re.S)
-        if m:
-            out[k] = {"registers": int(m.group(3)), "spill_store_bytes": int(m.group(1)),
-                      "spill_load_bytes": int(m.group(2))}
-    return out
+    rep = ptxas_report(log)
+    return {k: {f: rep[k][f] for f in ("registers", "spill_store_bytes", "spill_load_bytes")}
+            for k in kernels if k in rep}
 
 
 def main(out_path):
-    sys.path.insert(0, ROOT)
     import numpy as np
     import torch
 
@@ -106,8 +42,7 @@ def main(out_path):
     from bayes_kit_b200 import _lib as L
 
     assert torch.cuda.is_available(), "time_user_smc_proposal.py needs a CUDA device"
-    smi = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader", "-i", "0"],
-                         capture_output=True, text=True).stdout.strip()
+    smi = card()
     res = {"gpu": smi, "M": M, "N": N, "resample": "systematic", "dtype": "float32", "seed": SEED,
            "walk": {"scale": SCALE}, "lognormal": {"s": 0.4, "D": 16}, "runs_per_point": REPS, "prepare_s": {},
            "points": []}
@@ -171,7 +106,7 @@ def main(out_path):
     a, b, n = 2.0, 1.0, 4.0
     S = np.random.default_rng(16).integers(1, 10, D).astype(np.float64)
     model = bk.CudaPriorLikModel(GAMMA_POIS, D, params=np.concatenate([[a, b, n], S]))
-    kern = bk.proposal_kernel(bk.CudaProposal(LOGNORMAL, D, params=[0.4], transition=True))
+    kern = bk.proposal_kernel(bk.CudaProposal(LOGNORMAL_NO_HELPER, D, params=[0.4], transition=True))
     smc = bk.TemperedLikelihoodSMC(model, 4, 1, torch.ones(4, D, device="cuda"), kern)
     gamma = lambda D: torch.distributions.Gamma(torch.full((D,), a, device="cuda"), torch.full((D,), b, device="cuda")
                                                 ).sample((M,))

@@ -13,50 +13,26 @@ walker-moves/s, the accept rate over the timed sweeps, and the registers, stack 
 from ptxas."""
 import json
 import os
-import re
-import subprocess
 import sys
 import time
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests"))
 
-BANANA = """
-__device__ bk_real log_density_gradient(const bk_real* x, bk_real* g, const bk_real* params) {
-    const bk_real b = params[0], half = 0.5, two = 2;
-    const bk_real u = x[1] - b * x[0] * x[0];
-    bk_real lp = -half * (x[0] * x[0]) - half * (u * u);
-    g[0] = -x[0] + two * b * x[0] * u;
-    g[1] = -u;
-    for (int e = 2; e < BK_DIMS; ++e) { lp -= half * (x[e] * x[e]); g[e] = -x[e]; }
-    return lp;
-}
-"""
-DIAG = """
-__device__ bk_real log_density_gradient(const bk_real* x, bk_real* g, const bk_real* p) {
-    bk_real s = 0;
-    for (int e = 0; e < BK_DIMS; ++e) {
-        const bk_real d = x[e] - p[e];
-        const bk_real pd = p[BK_DIMS + e] * d;
-        s += d * pd;
-        g[e] = -pd;
-    }
-    return bk_real(-0.5) * s;
-}
-"""
+from _user_cuda import BANANA, DIAG, card, ptxas_report  # noqa: E402
+
 SWEEPS = 20
 
 
 def regs(log):
-    m = re.search(r"Function properties for bk_user_stretch\n.*?(\d+) bytes stack frame, (\d+) bytes spill stores, "
-                  r"(\d+) bytes spill loads\n.*?Used (\d+) registers", log, re.S)
-    if not m:
+    r = ptxas_report(log).get("bk_user_stretch")
+    if r is None:
         return None
-    return {"registers": int(m.group(4)), "stack_frame_bytes": int(m.group(1)), "spill_store_bytes": int(m.group(2)),
-            "spill_load_bytes": int(m.group(3))}
+    return {k: r[k] for k in ("registers", "stack_frame_bytes", "spill_store_bytes", "spill_load_bytes")}
 
 
 def main(out_path):
-    sys.path.insert(0, ROOT)
     import ctypes as C
 
     import numpy as np
@@ -66,8 +42,7 @@ def main(out_path):
     from bayes_kit_b200 import _lib as L
 
     lib = L.lib()
-    smi = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader", "-i", "0"],
-                         capture_output=True, text=True).stdout.strip()
+    smi = card()
     big = 1 << 20
     res = {"gpu": smi, "dtype": "float32", "a": 2.0, "sweeps_per_call": SWEEPS, "compile_s": {}, "points": []}
 

@@ -11,83 +11,26 @@ warm-up calls each, CUDA events), the accept rates of both, and ptxas's register
 three wide kernels; and one point at 4096 chains, a size bound by launches and the host.  Where the library's
 USER_WIDE_MAX_D is below 256 the script links a variant with BK_USER_WIDE_MAX_D = 256 in a temporary directory
 (the default build is left alone)."""
-import glob
 import json
 import os
-import re
-import subprocess
 import sys
 import tempfile
 import time
 
 ROOT = os.path.dirname(os.path.abspath(os.path.dirname(__file__)))
-PKG = os.path.join(ROOT, "bayes-kit_b200")
+sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests"))
+
+from _user_cuda import BANANA, DIAG, WIDE_MAX_D, build_variant, card, ptxas_report  # noqa: E402
+
 MAX_D = 256
 DIMS = (48, 64, 96, 128, 192, 256)
 
 
-def wide_max_d():
-    with open(os.path.join(PKG, "csrc", "model.h")) as f:
-        return int(re.search(r"#define BK_USER_WIDE_MAX_D (\d+)", f.read()).group(1))
-
-
-def build_variant(tmp):
-    sys.path.insert(0, PKG)
-    import build as b
-    b.build()
-    obj = os.path.join(tmp, "user_model.o")
-    subprocess.run([b.NVCC, *b.FLAGS, f"-DBK_USER_WIDE_MAX_D={MAX_D}", "-c", os.path.join(b.CSRC, "user_model.cu"),
-                    "-o", obj], check=True)
-    objs = [o for o in glob.glob(os.path.join(b.OBJ, "*.o")) if not o.endswith("user_model.o")] + [obj]
-    lib = os.path.join(tmp, "libbk_b200.so")
-    subprocess.run([b.NVCC, "-shared", "-o", lib, *objs, "-gencode", "arch=compute_100a,code=sm_100a", "-cudart",
-                    "static", "-Xcompiler", "-fPIC", "-ldl"], check=True)
-    return lib
-
-
-BANANA = """
-__device__ bk_real log_density_gradient(const bk_real* x, bk_real* g, const bk_real* params) {
-    const bk_real b = params[0], half = 0.5, two = 2;
-    const bk_real u = x[1] - b * x[0] * x[0];
-    bk_real lp = -half * (x[0] * x[0]) - half * (u * u);
-    g[0] = -x[0] + two * b * x[0] * u;
-    g[1] = -u;
-    for (int e = 2; e < BK_DIMS; ++e) { lp -= half * (x[e] * x[e]); g[e] = -x[e]; }
-    return lp;
-}
-"""
-DIAG = """
-__device__ bk_real log_density_gradient(const bk_real* x, bk_real* g, const bk_real* p) {
-    bk_real s = 0;
-    for (int e = 0; e < BK_DIMS; ++e) {
-        const bk_real d = x[e] - p[e];
-        const bk_real pd = p[BK_DIMS + e] * d;
-        s += d * pd;
-        g[e] = -pd;
-    }
-    return bk_real(-0.5) * s;
-}
-"""
-KERNELS = ("bk_user_wide_hmc", "bk_user_wide_mala", "bk_user_wide_mh")
-
-
-def ptxas(log):
-    out = {}
-    for k in KERNELS:
-        m = re.search(rf"Function properties for {k}\n.*?(\d+) bytes stack frame, (\d+) bytes spill stores, "
-                      rf"(\d+) bytes spill loads\n.*?Used (\d+) registers(.*?)\n", log, re.S)
-        if m:
-            out[k] = {"registers": int(m.group(4)), "stack_frame_bytes": int(m.group(1)),
-                      "spill_store_bytes": int(m.group(2)), "spill_load_bytes": int(m.group(3)),
-                      "ptxas_line": m.group(5).strip()}
-    return out
-
-
 def main(out_path):
     tmp = tempfile.mkdtemp(prefix="bk_user_wide_")
-    if wide_max_d() < MAX_D:
-        os.environ["BK_LIB"] = build_variant(tmp)
-    sys.path.insert(0, ROOT)
+    if WIDE_MAX_D < MAX_D:
+        os.environ["BK_LIB"] = build_variant(tmp, f"BK_USER_WIDE_MAX_D={MAX_D}")
     import ctypes as C
 
     import numpy as np
@@ -97,11 +40,10 @@ def main(out_path):
     from bayes_kit_b200 import _lib as L
 
     lib = L.lib()
-    smi = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader", "-i", "0"],
-                         capture_output=True, text=True).stdout.strip()
+    smi = card()
     Cn, n, Lsteps = 1 << 20, 10, 10
     res = {"gpu": smi, "chains": Cn, "hmc_steps_L": Lsteps, "draws_per_call": n, "dtype": "float32",
-           "library_wide_max_d": wide_max_d(), "timed_calls": 7, "warmup_calls": 2, "points": []}
+           "library_wide_max_d": WIDE_MAX_D, "timed_calls": 7, "warmup_calls": 2, "points": []}
     os.environ["BK_FORCE_GENERIC"] = "0"
 
     # NVRTC: the first prepare compiles and loads the wide program, the second finds it in the cache
@@ -162,7 +104,7 @@ def main(out_path):
                 r, log = measure(make, mod, Cn)
                 pt[f"{mname}_{sname}"] = r
                 if sname == "hmc":
-                    pt[f"ptxas_{mname}"] = ptxas(log)
+                    pt[f"ptxas_{mname}"] = ptxas_report(log)
                 print(json.dumps({"D": D, "model": mname, "sampler": sname,
                                   "wide": r["wide"]["chain_draws_per_s"], "generic": r["generic"]["chain_draws_per_s"],
                                   "ratio": r["wide_over_generic"], "acc": (r["wide"]["accept"],

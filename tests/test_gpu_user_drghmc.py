@@ -6,33 +6,11 @@ import pytest
 import torch
 
 from _dev import assert_traj, np_
+from _user_cuda import BANANA, BANANA_1, DIAG, GPL, NpBanana, binom, diag_params
 from conftest import golden
 from oracle import samplers as osm
-from test_gpu_user_model import BANANA, DIAG, _diag_params
-from test_gpu_user_smc import GPL, binom
 
 pytestmark = pytest.mark.gpu
-
-# the banana of test_gpu_user_model.py, also defined at D = 1 (then a standard normal); params = [b]
-BANANA_1 = """
-__device__ bk_real log_density_gradient(const bk_real* x, bk_real* g, const bk_real* params) {
-#if BK_DIMS == 1
-    g[0] = -x[0];
-    return bk_real(-0.5) * (x[0] * x[0]);
-#else
-    const bk_real b = params[0], half = 0.5, two = 2;
-    const bk_real u = x[1] - b * x[0] * x[0];
-    bk_real lp = -half * (x[0] * x[0]) - half * (u * u);
-    g[0] = -x[0] + two * b * x[0] * u;
-    g[1] = -u;
-    for (int e = 2; e < BK_DIMS; ++e) {
-        lp -= half * (x[e] * x[e]);
-        g[e] = -x[e];
-    }
-    return lp;
-#endif
-}
-"""
 
 # a standard normal truncated to x0 >= 0: log p = -inf on half the space
 HALF_NORMAL = """
@@ -45,30 +23,6 @@ __device__ bk_real log_density_gradient(const bk_real* x, bk_real* g, const bk_r
     return x[0] < 0 ? log(bk_real(0)) : bk_real(-0.5) * s;
 }
 """
-
-
-class NpBanana:
-    def __init__(self, D, b):
-        self.D, self.b = D, b
-
-    def dims(self):
-        return self.D
-
-    def log_density_gradient(self, x):
-        x = np.asarray(x, dtype=np.float64)
-        if self.D == 1:
-            return -0.5 * x[0] * x[0], -x.copy()
-        u = x[1] - self.b * x[0] * x[0]
-        lp = -0.5 * (x[0] * x[0]) - 0.5 * (u * u)
-        g = -x.copy()
-        g[0] = -x[0] + 2 * self.b * x[0] * u
-        g[1] = -u
-        for e in range(2, self.D):
-            lp -= 0.5 * (x[e] * x[e])
-        return lp, g
-
-    def log_density(self, x):
-        return self.log_density_gradient(x)[0]
 
 
 @pytest.fixture
@@ -227,7 +181,7 @@ def test_minus_inf_region_fused_equals_lockstep(bk, monkeypatch):
 # ---- 4. the built-in plugin's words -------------------------------------------------------------------------------
 @pytest.mark.parametrize("D", [3, 8])
 def test_user_diag_gauss_equals_builtin(bk, fused, D):
-    mu, pr = _diag_params(D)
+    mu, pr = diag_params(D)
     user = bk.CudaModel(DIAG, D, params=np.concatenate([mu, pr]), dtype=torch.float64)
     built = bk.DiagGauss(mu, pr, dtype=torch.float64)
     init = np.random.default_rng(D).normal(size=(64, D))

@@ -9,34 +9,12 @@ import pytest
 import torch
 
 from _dev import np_
+from _user_cuda import BANANA, BARKER, MALA_G, PRIOR_LIK, NpBanana
 from bayes_kit_b200 import _lib as L
 from oracle import models as om
 from oracle import proposals as opr
-from test_user_grad_proposal_host import BANANA, BARKER, MALA_G, PRIOR_LIK
 
 pytestmark = pytest.mark.gpu
-
-
-class NpBanana:
-    def __init__(self, D, b):
-        self.D, self.b = D, b
-
-    def dims(self):
-        return self.D
-
-    def log_density_gradient(self, x):
-        x = np.asarray(x, dtype=np.float64)
-        u = x[1] - self.b * x[0] * x[0]
-        lp = -0.5 * (x[0] * x[0]) - 0.5 * (u * u)
-        g = -x.copy()
-        g[0] = -x[0] + 2 * self.b * x[0] * u
-        g[1] = -u
-        for e in range(2, self.D):
-            lp -= 0.5 * (x[e] * x[e])
-        return lp, g
-
-    def log_density(self, x):
-        return self.log_density_gradient(x)[0]
 
 
 def np_barker(model, sigma):

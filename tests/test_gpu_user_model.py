@@ -6,42 +6,14 @@ import pytest
 import torch
 
 from _dev import np_
+from _user_cuda import (BANANA, DIAG, SCHOOLS_SIGMA, SCHOOLS_Y, NpSchools, banana, check, diag_params,
+                        streams_uniforms_first)
 from oracle import samplers as osm
 from oracle.models import DiagGauss as ODiag
 
 pytestmark = pytest.mark.gpu
 
 # ---- models ----------------------------------------------------------------------------------------------------
-# banana: x0 ~ N(0, 1), x1 - b x0^2 ~ N(0, 1), every further coordinate N(0, 1); params = [b]
-BANANA = """
-__device__ bk_real log_density_gradient(const bk_real* x, bk_real* g, const bk_real* params) {
-    const bk_real b = params[0], half = 0.5, two = 2;
-    const bk_real u = x[1] - b * x[0] * x[0];
-    bk_real lp = -half * (x[0] * x[0]) - half * (u * u);
-    g[0] = -x[0] + two * b * x[0] * u;
-    g[1] = -u;
-    for (int e = 2; e < BK_DIMS; ++e) {
-        lp -= half * (x[e] * x[e]);
-        g[e] = -x[e];
-    }
-    return lp;
-}
-"""
-
-# diagonal Gaussian, params = [mu (D), prec (D)]: the built-in DiagGauss restated
-DIAG = """
-__device__ bk_real log_density_gradient(const bk_real* x, bk_real* g, const bk_real* p) {
-    bk_real s = 0;
-    for (int e = 0; e < BK_DIMS; ++e) {
-        const bk_real d = x[e] - p[e];
-        const bk_real pd = p[BK_DIMS + e] * d;
-        s += d * pd;
-        g[e] = -pd;
-    }
-    return bk_real(-0.5) * s;
-}
-"""
-
 # non-centred eight schools: theta = (mu, log tau, eta[8]); y_j ~ N(mu + tau eta_j, sigma_j), eta ~ N(0, 1),
 # mu ~ N(0, 5^2), log tau ~ N(1, 1); params = [y (8), sigma (8)]
 SCHOOLS = """
@@ -67,65 +39,6 @@ __device__ bk_real log_density_gradient(const bk_real* th, bk_real* g, const bk_
     return lp;
 }
 """
-SCHOOLS_Y = np.array([28.0, 8.0, -3.0, 7.0, -1.0, 1.0, 18.0, 12.0])
-SCHOOLS_SIGMA = np.array([15.0, 10.0, 16.0, 11.0, 9.0, 11.0, 10.0, 18.0])
-
-
-class NpBanana:
-    def __init__(self, D, b):
-        self.D, self.b = D, b
-
-    def dims(self):
-        return self.D
-
-    def log_density_gradient(self, x):
-        x = np.asarray(x, dtype=np.float64)
-        u = x[1] - self.b * x[0] * x[0]
-        lp = -0.5 * (x[0] * x[0]) - 0.5 * (u * u)
-        g = -x.copy()
-        g[0] = -x[0] + 2 * self.b * x[0] * u
-        g[1] = -u
-        for e in range(2, self.D):
-            lp -= 0.5 * (x[e] * x[e])
-        return lp, g
-
-    def log_density(self, x):
-        return self.log_density_gradient(x)[0]
-
-
-class NpSchools:
-    def dims(self):
-        return 10
-
-    def log_density_gradient(self, th):
-        th = np.asarray(th, dtype=np.float64)
-        mu, lt = th[0], th[1]
-        tau = np.exp(lt)
-        lp = -0.5 * (mu * mu) / 25 - 0.5 * ((lt - 1) * (lt - 1))
-        g = np.empty(10)
-        gmu, glt = -mu / 25, -(lt - 1)
-        for j in range(8):
-            eta = th[2 + j]
-            d = SCHOOLS_Y[j] - mu - tau * eta
-            r = d / (SCHOOLS_SIGMA[j] * SCHOOLS_SIGMA[j])
-            lp += -0.5 * (eta * eta) - 0.5 * (d * r)
-            gmu += r
-            glt += r * tau * eta
-            g[2 + j] = -eta + r * tau
-        g[0], g[1] = gmu, glt
-        return lp, g
-
-    def log_density(self, th):
-        return self.log_density_gradient(th)[0]
-
-
-def banana(bk, D, b=0.5, dtype=torch.float64):
-    return bk.CudaModel(BANANA, D, params=[b], dtype=dtype), NpBanana(D, b)
-
-
-def _diag_params(D, seed=3):
-    rng = np.random.default_rng(seed)
-    return rng.normal(size=D), rng.uniform(0.5, 3.0, D)
 
 
 @pytest.fixture(params=["fused", "generic"])
@@ -141,7 +54,7 @@ def test_protocol_matches_numpy(bk, which):
     if which == "banana":
         dm, om = banana(bk, 5)
     elif which == "diag":
-        mu, pr = _diag_params(7)
+        mu, pr = diag_params(7)
         dm, om = bk.CudaModel(DIAG, 7, params=np.concatenate([mu, pr]), dtype=torch.float64), ODiag(mu, pr)
     else:
         dm = bk.CudaModel(SCHOOLS, 10, params=np.concatenate([SCHOOLS_Y, SCHOOLS_SIGMA]), dtype=torch.float64)
@@ -161,66 +74,53 @@ def test_protocol_matches_numpy(bk, which):
 
 
 # ---- 2. reference parity ---------------------------------------------------------------------------------------
-def _streams(C, D, n, seed, n_uniform=1):
-    rng = np.random.default_rng(seed)
-    u = rng.random((n, C)) if n_uniform == 1 else rng.random((n, C, n_uniform))
-    return rng.normal(size=(C, D)) * 0.7, rng.standard_normal((n, C, D)), u
-
-
-def _check(d, l, a, want):
-    wd, wl, wa = want
-    assert np.array_equal(np_(a).astype(bool), wa)
-    np.testing.assert_allclose(np_(d), wd, rtol=1e-10, atol=1e-10)
-    np.testing.assert_allclose(np_(l), wl, rtol=1e-10, atol=1e-10)
-
-
 @pytest.mark.parametrize("L", [0, 1, 7])
 @pytest.mark.parametrize("metric", [False, True])
 def test_hmc_matches_oracle(bk, engine, L, metric):
     C, D, n = 37, 3, 6
     dm, om = banana(bk, D)
-    th0, zs, us = _streams(C, D, n, L)
+    th0, zs, us = streams_uniforms_first(C, D, n, L)
     m = np.array([1.0, 0.5, 2.0]) if metric else None
     s = bk.HMCDiag(dm, 0.3, L, metric_diag=m, init=th0)
     d, l = s.sample_n(n, normals=zs, uniforms=us)
-    _check(d, l, s.last_accept, osm.hmc_diag_batch(om, th0, zs, us, 0.3, L, m))
+    check(d, l, s.last_accept, osm.hmc_diag_batch(om, th0, zs, us, 0.3, L, m))
     np.testing.assert_allclose(np_(s.theta), np_(d[-1]), rtol=0, atol=0)
 
 
 def test_mala_matches_oracle(bk, engine):
     C, D, n = 37, 4, 6
     dm, om = banana(bk, D)
-    th0, zs, us = _streams(C, D, n, 11)
+    th0, zs, us = streams_uniforms_first(C, D, n, 11)
     s = bk.MALA(dm, 0.2, init=th0)
     d, l = s.sample_n(n, normals=zs, uniforms=us)
-    _check(d, l, s.last_accept, osm.mala_batch(om, th0, zs, us, 0.2))
+    check(d, l, s.last_accept, osm.mala_batch(om, th0, zs, us, 0.2))
 
 
 @pytest.mark.parametrize("hastings", [False, True])
 def test_metropolis_matches_oracle(bk, engine, hastings):
     C, D, n = 37, 5, 6
     dm, om = banana(bk, D)
-    th0, zs, us = _streams(C, D, n, 12)
+    th0, zs, us = streams_uniforms_first(C, D, n, 12)
     prop = bk.GaussianRW(0.6)
     s = bk.MetropolisHastings(dm, prop, prop.transition_lp, init=th0) if hastings else bk.Metropolis(dm, prop, init=th0)
     d, l = s.sample_n(n, normals=zs, uniforms=us)
-    _check(d, l, s.last_accept, osm.metropolis_rw_batch(om, th0, zs, us, 0.6, hastings))
+    check(d, l, s.last_accept, osm.metropolis_rw_batch(om, th0, zs, us, 0.6, hastings))
 
 
 def test_schools_hmc_matches_oracle(bk, engine):
     C, D, n = 19, 10, 4
     dm = bk.CudaModel(SCHOOLS, 10, params=np.concatenate([SCHOOLS_Y, SCHOOLS_SIGMA]), dtype=torch.float64)
-    th0, zs, us = _streams(C, D, n, 13)
+    th0, zs, us = streams_uniforms_first(C, D, n, 13)
     s = bk.HMCDiag(dm, 0.1, 5, init=th0)
     d, l = s.sample_n(n, normals=zs, uniforms=us)
-    _check(d, l, s.last_accept, osm.hmc_diag_batch(NpSchools(), th0, zs, us, 0.1, 5))
+    check(d, l, s.last_accept, osm.hmc_diag_batch(NpSchools(), th0, zs, us, 0.1, 5))
 
 
 @pytest.mark.parametrize("K", [2, 3])
 def test_drghmc_matches_oracle(bk, K):
     C, D, n = 23, 3, 5
     dm, om = banana(bk, D)
-    th0, zs, us = _streams(C, D, n, 20 + K, n_uniform=2 * K)
+    th0, zs, us = streams_uniforms_first(C, D, n, 20 + K, n_uniform=2 * K)
     rho0 = np.random.default_rng(K).normal(size=(C, D))
     sizes, counts = [0.4, 0.2, 0.1][:K], [2, 4, 8][:K]
     s = bk.DrGhmcDiag(dm, K, sizes, counts, 0.5, init=th0)
@@ -249,7 +149,7 @@ def test_stretcher_matches_oracle(bk):
 # ---- 3. same RNG as the built-in plugins ---------------------------------------------------------------------------
 @pytest.mark.parametrize("D", [3, 8])
 def test_user_diag_gauss_equals_builtin(bk, D):
-    mu, pr = _diag_params(D)
+    mu, pr = diag_params(D)
     user = bk.CudaModel(DIAG, D, params=np.concatenate([mu, pr]), dtype=torch.float64)
     built = bk.DiagGauss(mu, pr, dtype=torch.float64)
     init = np.random.default_rng(D).normal(size=(64, D))

@@ -2,51 +2,20 @@
 written twice, in CUDA for the device and in NumPy for the oracle.  Engines: the fused bk_user_mhp (a user model with
 dims <= 32, compiled together with the proposal) and the three-launch path (bk_user_propose, the model's evaluation,
 the accept test) for every other model."""
-import ctypes as C
-
 import numpy as np
 import pytest
 import torch
 
 from _dev import np_
+from _user_cuda import (BANANA, DIAG, INDEP, LOGNORMAL, MIXTURE_WALK, RSCAN, RW, NpBanana, check, np_indep,
+                        np_lognormal, np_rscan, philox_streams)
 from bayes_kit_b200 import _lib as L
-from bayes_kit_b200._util import stream_ptr
 from oracle import models as om
-from oracle import philox as ph
 from oracle import proposals as opr
 
 pytestmark = pytest.mark.gpu
 
 # ---- models ----------------------------------------------------------------------------------------------------
-BANANA = """
-__device__ bk_real log_density_gradient(const bk_real* x, bk_real* g, const bk_real* params) {
-    const bk_real b = params[0], half = 0.5, two = 2;
-    const bk_real u = x[1] - b * x[0] * x[0];
-    bk_real lp = -half * (x[0] * x[0]) - half * (u * u);
-    g[0] = -x[0] + two * b * x[0] * u;
-    g[1] = -u;
-    for (int e = 2; e < BK_DIMS; ++e) {
-        lp -= half * (x[e] * x[e]);
-        g[e] = -x[e];
-    }
-    return lp;
-}
-"""
-
-# diagonal Gaussian, params = [mu (D), prec (D)]
-DIAG = """
-__device__ bk_real log_density_gradient(const bk_real* x, bk_real* g, const bk_real* p) {
-    bk_real s = 0;
-    for (int e = 0; e < BK_DIMS; ++e) {
-        const bk_real d = x[e] - p[e];
-        const bk_real pd = p[BK_DIMS + e] * d;
-        s += d * pd;
-        g[e] = -pd;
-    }
-    return bk_real(-0.5) * s;
-}
-"""
-
 # independent Gamma(a_e, rate b_e) coordinates, params = [a (D), b (D)].  Its helper `sq` has the name of the log-normal
 # proposal's: each source is compiled in a namespace of its own.
 GAMMA = """
@@ -61,123 +30,6 @@ __device__ bk_real log_density_gradient(const bk_real* x, bk_real* g, const bk_r
     return lp;
 }
 """
-
-
-class NpBanana:
-    def __init__(self, D, b):
-        self.D, self.b = D, b
-
-    def dims(self):
-        return self.D
-
-    def log_density(self, x):
-        x = np.asarray(x, dtype=np.float64)
-        u = x[1] - self.b * x[0] * x[0]
-        lp = -0.5 * (x[0] * x[0]) - 0.5 * (u * u)
-        for e in range(2, self.D):
-            lp -= 0.5 * (x[e] * x[e])
-        return lp
-
-
-# ---- proposals: CUDA and NumPy -------------------------------------------------------------------------------------
-# the Gaussian random walk restated, params = [scale]
-RW = """
-__device__ void propose(const bk_real* theta, bk_real* q, const bk_real* z, const bk_real* u, const bk_real* p) {
-    for (int e = 0; e < BK_DIMS; ++e) q[e] = theta[e] + p[0] * z[e];
-}
-__device__ bk_real transition_log_density(const bk_real* to, const bk_real* from, const bk_real* p) {
-    bk_real s = 0;
-    for (int e = 0; e < BK_DIMS; ++e) { const bk_real d = to[e] - from[e]; s += d * d; }
-    return bk_real(-0.5) * s / (p[0] * p[0]);
-}
-"""
-
-# independence sampler N(m, diag s^2), params = [m (D), s (D)]
-INDEP = """
-__device__ void propose(const bk_real* theta, bk_real* q, const bk_real* z, const bk_real* u, const bk_real* p) {
-    for (int e = 0; e < BK_DIMS; ++e) q[e] = p[e] + p[BK_DIMS + e] * z[e];
-}
-__device__ bk_real transition_log_density(const bk_real* to, const bk_real* from, const bk_real* p) {
-    bk_real s = 0;
-    for (int e = 0; e < BK_DIMS; ++e) {
-        const bk_real d = (to[e] - p[e]) / p[BK_DIMS + e];
-        s += bk_real(-0.5) * (d * d) - log(p[BK_DIMS + e]);
-    }
-    return s;
-}
-"""
-
-# multiplicative (log-normal) walk for positive parameters, params = [s]; the Jacobian -log(to) makes it asymmetric
-LOGNORMAL = """
-__device__ bk_real sq(bk_real x) { return x * x; }
-__device__ void propose(const bk_real* theta, bk_real* q, const bk_real* z, const bk_real* u, const bk_real* p) {
-    for (int e = 0; e < BK_DIMS; ++e) q[e] = theta[e] * exp(p[0] * z[e]);
-}
-__device__ bk_real transition_log_density(const bk_real* to, const bk_real* from, const bk_real* p) {
-    bk_real s = 0;
-    for (int e = 0; e < BK_DIMS; ++e) {
-        const bk_real d = (log(to[e]) - log(from[e])) / p[0];
-        s += bk_real(-0.5) * sq(d) - log(to[e]);
-    }
-    return s;
-}
-"""
-
-# random-scan single-site walk: u[0] picks the coordinate, z[0] is the step; params = [s]
-RSCAN = """
-__device__ void propose(const bk_real* theta, bk_real* q, const bk_real* z, const bk_real* u, const bk_real* p) {
-    for (int e = 0; e < BK_DIMS; ++e) q[e] = theta[e];
-    int j = (int)(u[0] * BK_DIMS);
-    if (j > BK_DIMS - 1) j = BK_DIMS - 1;
-    q[j] = theta[j] + p[0] * z[0];
-}
-__device__ bk_real transition_log_density(const bk_real* to, const bk_real* from, const bk_real* p) { return 0; }
-"""
-
-# a two-scale mixture walk with an extra small jitter: 2 D normals (more than D, so the stream skips the accept block)
-# and two uniforms; params = [s1, s2, w]
-MIXTURE = """
-__device__ void propose(const bk_real* theta, bk_real* q, const bk_real* z, const bk_real* u, const bk_real* p) {
-    const bk_real s = (u[0] < p[2] ? p[0] : p[1]) * (bk_real(0.5) + u[1]);
-    for (int e = 0; e < BK_DIMS; ++e) q[e] = theta[e] + s * z[e] + bk_real(0.01) * z[BK_DIMS + e];
-}
-"""
-
-
-def np_indep(m, s):
-    def propose(th, z, u):
-        return m + s * z
-
-    def tld(to, frm):
-        acc = 0.0
-        for e in range(to.shape[0]):
-            d = (to[e] - m[e]) / s[e]
-            acc += -0.5 * (d * d) - np.log(s[e])
-        return acc
-    return propose, tld
-
-
-def np_lognormal(s):
-    def propose(th, z, u):
-        return th * np.exp(s * z)
-
-    def tld(to, frm):
-        acc = 0.0
-        for e in range(to.shape[0]):
-            d = (np.log(to[e]) - np.log(frm[e])) / s
-            acc += -0.5 * (d * d) - np.log(to[e])
-        return acc
-    return propose, tld
-
-
-def np_rscan(s):
-    def propose(th, z, u):
-        D = th.shape[0]
-        q = th.copy()
-        j = min(int(u[0] * D), D - 1)
-        q[j] = th[j] + s * z[0]
-        return q
-    return propose, (lambda to, frm: 0.0)
 
 
 def _user(bk, src, D, params, dtype=torch.float64):
@@ -199,13 +51,6 @@ def _builtin(bk, kind, D, dtype=torch.float64):
         X, y = om.HierLogReg.c3_data(50, D - 2, seed=2)
         return bk.HierLogReg(X, y, dtype=dtype), om.HierLogReg(X, y)
     raise ValueError(kind)
-
-
-def _check(d, l, a, want):
-    wd, wl, wa = want
-    assert np.array_equal(np_(a).astype(bool), wa)
-    np.testing.assert_allclose(np_(d), wd, rtol=1e-10, atol=1e-10)
-    np.testing.assert_allclose(np_(l), wl, rtol=1e-10, atol=1e-10)
 
 
 def _launches(bk):
@@ -292,32 +137,14 @@ def test_matches_oracle(bk, which, mk):
     us = rng.random((n, C_, 1 + prop.uniforms))
     s = bk.MetropolisHastings(dev, prop, prop.transition_lp, init=th0)
     d, l = s.sample_n(n, normals=zs, uniforms=us)
-    _check(d, l, s.last_accept, opr.metropolis_hastings_batch(npm, th0, zs, us, propose, tld))
+    check(d, l, s.last_accept, opr.metropolis_hastings_batch(npm, th0, zs, us, propose, tld))
     if not asym:
         s = bk.Metropolis(dev, prop, init=th0)
         d, l = s.sample_n(n, normals=zs, uniforms=us)
-        _check(d, l, s.last_accept, opr.metropolis_hastings_batch(npm, th0, zs, us, propose))
+        check(d, l, s.last_accept, opr.metropolis_hastings_batch(npm, th0, zs, us, propose))
 
 
 # ---- 3. Philox equals the injected reconstruction (fp64) -------------------------------------------------------------
-def _philox_streams(bk, seed, chain_offset, C_, D, nz, nu, n, draw0):
-    """The proposal's Philox streams rebuilt outside the sampler: normals from bk_init_normal over enough element blocks
-    (the accept block's columns dropped), uniforms and the accept uniform from the NumPy restatement."""
-    blocks = opr.proposal_blocks(D, nz)
-    cols = [4 * b + i for b in blocks for i in range(4)][:nz]
-    Dp = 4 * (max(blocks) + 1)
-    Z = torch.empty(n, C_, nz, dtype=torch.float64, device="cuda")
-    U = np.empty((n, C_, 1 + nu))
-    ch = np.uint64(chain_offset) + np.arange(C_, dtype=np.uint64)
-    for t in range(n):
-        full = torch.empty(C_, Dp, dtype=torch.float64, device="cuda")
-        L.check(L.lib().bk_init_normal(full.data_ptr(), C_, Dp, L.BK_F64, seed, chain_offset, draw0 + t, stream_ptr()))
-        Z[t] = full[:, cols]
-        U[t, :, 0] = ph.accept_uniform(seed, ch, draw0 + t, D, np.float64)
-        U[t, :, 1:] = opr.proposal_uniforms(seed, chain_offset, draw0 + t, C_, nu)
-    return Z, U
-
-
 @pytest.mark.parametrize("offset", [0, 1000])
 @pytest.mark.parametrize("engine", ["fused", "three-launch"])
 @pytest.mark.parametrize("which", ["mixture", "rscan", "rw"])
@@ -328,7 +155,7 @@ def test_philox_equals_injected_reconstruction(bk, which, engine, offset):
     else:
         model = _builtin(bk, "diag", D)[0]
     if which == "mixture":
-        prop = bk.CudaProposal(MIXTURE, D, params=[0.3, 1.5, 0.4], normals=2 * D, uniforms=2, transition=False,
+        prop = bk.CudaProposal(MIXTURE_WALK, D, params=[0.3, 1.5, 0.4], normals=2 * D, uniforms=2, transition=False,
                                dtype=torch.float64)
     elif which == "rscan":
         prop = bk.CudaProposal(RSCAN, D, params=[0.8], normals=1, uniforms=1, dtype=torch.float64)
@@ -337,7 +164,7 @@ def test_philox_equals_injected_reconstruction(bk, which, engine, offset):
     init = np.random.default_rng(1).normal(size=(C_, D))
     a = bk.Metropolis(model, prop, init=init, seed=seed, chain_offset=offset)
     b = bk.Metropolis(model, prop, init=init, seed=seed, chain_offset=offset)
-    Z, U = _philox_streams(bk, seed, offset, C_, D, prop.normals, prop.uniforms, n, 0)
+    Z, U = philox_streams(bk, seed, offset, C_, D, prop.normals, prop.uniforms, n, 0)
     da, la = a.sample_n(n)
     db, lb = b.sample_n(n, normals=Z, uniforms=U)
     assert torch.equal(a.last_accept, b.last_accept)
@@ -441,7 +268,7 @@ def test_errors(bk):
         bk.Metropolis(model, bk.CudaProposal(RW, 4, params=[0.5]))
     with pytest.raises(ValueError, match="dims"):
         bk.Metropolis(model, bk.CudaProposal(RW, 3, params=[0.5], dtype=torch.float64))
-    sym = bk.CudaProposal(MIXTURE, 3, params=[0.3, 1.5, 0.4], normals=6, uniforms=2, transition=False)
+    sym = bk.CudaProposal(MIXTURE_WALK, 3, params=[0.3, 1.5, 0.4], normals=6, uniforms=2, transition=False)
     bk.Metropolis(model, sym)
     with pytest.raises(TypeError, match="transition"):
         bk.MetropolisHastings(model, sym, sym.transition_lp)

@@ -9,136 +9,12 @@ import pytest
 import torch
 
 from _dev import device_model, np_, smc_kernel
+from _user_cuda import GPL, MIX_MU, MIX_S, MIX_TAU, MIXTURE_MODEL, Mixture, binom, gpl, run_fake, user_twin
 from conftest import GOLDEN, golden
 from oracle import samplers as osm
 from oracle import models as om
 
 pytestmark = pytest.mark.gpu
-
-# ---- models ----------------------------------------------------------------------------------------------------
-# GaussPriorLik restated: params = [mu (D), pl (D), m0 (D), p0 (D)]
-GPL = """
-__device__ bk_real quad(const bk_real* x, bk_real* g, const bk_real* m, const bk_real* p) {
-    bk_real s = 0;
-    for (int e = 0; e < BK_DIMS; ++e) {
-        const bk_real d = x[e] - m[e], pd = p[e] * d;
-        s += pd * d;
-        g[e] = -pd;
-    }
-    return bk_real(-0.5) * s;
-}
-__device__ bk_real log_prior_gradient(const bk_real* x, bk_real* g, const bk_real* p) {
-    return quad(x, g, p + 2 * BK_DIMS, p + 3 * BK_DIMS);
-}
-__device__ bk_real log_likelihood_gradient(const bk_real* x, bk_real* g, const bk_real* p) {
-    return quad(x, g, p, p + BK_DIMS);
-}
-"""
-
-# the reference's beta-binomial on the logit scale restated: params = [alpha, beta, x, N, log C(N, x), log B(alpha, beta)]
-BINOM = """
-__device__ void logs(bk_real th, bk_real& lp1, bk_real& l1m, bk_real& p) {
-    const bk_real e = exp(-fabs(th)), l = log1p(e);
-    lp1 = th >= 0 ? -l : th - l;
-    l1m = th >= 0 ? -th - l : -l;
-    p = th >= 0 ? bk_real(1) / (1 + e) : e / (1 + e);
-}
-__device__ bk_real log_prior_gradient(const bk_real* x, bk_real* g, const bk_real* q) {
-    bk_real lp1, l1m, p;
-    logs(x[0], lp1, l1m, p);
-    g[0] = q[0] - (q[0] + q[1]) * p;
-    return (q[0] * lp1 + q[1] * l1m) - q[5];
-}
-__device__ bk_real log_likelihood_gradient(const bk_real* x, bk_real* g, const bk_real* q) {
-    bk_real lp1, l1m, p;
-    logs(x[0], lp1, l1m, p);
-    g[0] = q[2] - q[3] * p;
-    return (q[4] + q[2] * lp1) + (q[3] - q[2]) * l1m;
-}
-"""
-
-# no built-in counterpart: prior N(0, tau^2 I), likelihood 1/2 N(x; mu, s^2 I) + 1/2 N(x; -mu, s^2 I) (up to its
-# normalising constant), a bimodal posterior.  params = [mu (D), 1 / s^2, 1 / tau^2]
-MIXTURE = """
-__device__ bk_real log_prior_gradient(const bk_real* x, bk_real* g, const bk_real* p) {
-    const bk_real p0 = p[BK_DIMS + 1];
-    bk_real s = 0;
-    for (int e = 0; e < BK_DIMS; ++e) { s += x[e] * x[e]; g[e] = -p0 * x[e]; }
-    return bk_real(-0.5) * p0 * s;
-}
-__device__ bk_real log_likelihood_gradient(const bk_real* x, bk_real* g, const bk_real* p) {
-    const bk_real* mu = p;
-    const bk_real pl = p[BK_DIMS];
-    bk_real sa = 0, sb = 0;
-    for (int e = 0; e < BK_DIMS; ++e) {
-        const bk_real da = x[e] - mu[e], db = x[e] + mu[e];
-        sa += da * da;
-        sb += db * db;
-    }
-    const bk_real a = bk_real(-0.5) * pl * sa, b = bk_real(-0.5) * pl * sb;
-    const bk_real m = a > b ? a : b;
-    const bk_real ea = exp(a - m), eb = exp(b - m), z = ea + eb;
-    const bk_real wa = ea / z, wb = eb / z;
-    for (int e = 0; e < BK_DIMS; ++e) g[e] = -pl * (wa * (x[e] - mu[e]) + wb * (x[e] + mu[e]));
-    return m + log(bk_real(0.5) * z);
-}
-"""
-
-
-class Mixture:
-    """NumPy twin of MIXTURE."""
-
-    def __init__(self, mu, s, tau):
-        self.mu, self.pl, self.p0 = np.asarray(mu, dtype=np.float64), 1.0 / s ** 2, 1.0 / tau ** 2
-
-    def params(self):
-        return np.concatenate([self.mu, [self.pl, self.p0]])
-
-    def dims(self):
-        return self.mu.shape[0]
-
-    def log_prior(self, x):
-        return -0.5 * self.p0 * float(np.sum(x * x))
-
-    def log_prior_gradient(self, x):
-        return -self.p0 * x
-
-    def _ab(self, x):
-        return -0.5 * self.pl * float(np.sum((x - self.mu) ** 2)), -0.5 * self.pl * float(np.sum((x + self.mu) ** 2))
-
-    def log_likelihood(self, x):
-        a, b = self._ab(x)
-        m = max(a, b)
-        return m + math.log(0.5 * (math.exp(a - m) + math.exp(b - m)))
-
-    def log_likelihood_gradient(self, x):
-        a, b = self._ab(x)
-        m = max(a, b)
-        ea, eb = math.exp(a - m), math.exp(b - m)
-        wa, wb = ea / (ea + eb), eb / (ea + eb)
-        return -self.pl * (wa * (x - self.mu) + wb * (x + self.mu))
-
-    def log_density(self, x):
-        return self.log_likelihood(x) + self.log_prior(x)
-
-
-def gpl(bk, m0, p0, mu, pl, dtype=torch.float64):
-    return bk.CudaPriorLikModel(GPL, len(mu), params=np.concatenate([mu, pl, m0, p0]), dtype=dtype)
-
-
-def binom(bk, a, b, x, n, dtype=torch.float64):
-    lch = math.lgamma(n + 1) - math.lgamma(x + 1) - math.lgamma(n - x + 1)
-    lbe = math.lgamma(a) + math.lgamma(b) - math.lgamma(a + b)
-    return bk.CudaPriorLikModel(BINOM, 1, params=[a, b, x, n, lch, lbe], dtype=dtype)
-
-
-def user_twin(bk, z):
-    """The CUDA restatement of a golden fixture's built-in SMC model."""
-    kind = str(z["model_kind"])
-    if kind == "gpl":
-        return gpl(bk, z["model_m0"], z["model_p0"], z["model_mu"], z["model_pl"])
-    a, b, x, n = z["model_abxn"]
-    return binom(bk, float(a), float(b), int(x), int(n))
 
 
 def oracle_kernel(kind, scale, steps=5):
@@ -213,10 +89,6 @@ def test_smc_golden_through_the_user_model(bk, name):
 
 
 # ---- 3. a model with no built-in counterpart ---------------------------------------------------------------------
-MIX_MU = np.array([1.5, -1.5, 1.5, -1.5])
-MIX_S, MIX_TAU = 0.5, 2.0
-
-
 @pytest.mark.parametrize("kind,scale", [("rw", 0.3), ("mala", 0.05), ("hmc", 0.1)])
 @pytest.mark.parametrize("mode", ["systematic", "multinomial"])
 def test_mixture_vs_oracle(bk, kind, scale, mode):
@@ -226,7 +98,7 @@ def test_mixture_vs_oracle(bk, kind, scale, mode):
     th0 = rng.normal(size=(M, D)) * MIX_TAU
     zs, au, ru = rng.standard_normal((T, M, D)), rng.random((T, M)), rng.random((T, M))
     oth, oidx = osm.smc_tempered(nm, th0, zs, au, ru, scale, T, resample=mode, kernel=oracle_kernel(kind, scale))
-    dm = bk.CudaPriorLikModel(MIXTURE, D, params=nm.params(), dtype=torch.float64)
+    dm = bk.CudaPriorLikModel(MIXTURE_MODEL, D, params=nm.params(), dtype=torch.float64)
     smc = bk.TemperedLikelihoodSMC(dm, M, T, th0, device_kernel(bk, kind, scale), resample=mode)
     acc = []
     for n in range(1, T + 1):
@@ -241,7 +113,7 @@ def test_mixture_vs_oracle(bk, kind, scale, mode):
 
 def _mixture_stats(bk, kind, seed, M=1 << 16, T=40):
     nm = Mixture(MIX_MU, MIX_S, MIX_TAU)
-    dm = bk.CudaPriorLikModel(MIXTURE, 4, params=nm.params())
+    dm = bk.CudaPriorLikModel(MIXTURE_MODEL, 4, params=nm.params())
     th0 = torch.randn(M, 4, device="cuda", generator=torch.Generator(device="cuda").manual_seed(seed)) * MIX_TAU
     scale = {"rw": 0.3, "mala": 0.05, "hmc": 0.1}[kind]
     smc = bk.TemperedLikelihoodSMC(dm, M, T, th0, device_kernel(bk, kind, scale), resample="systematic", seed=seed)
@@ -294,28 +166,6 @@ def test_same_streams_as_the_builtin(bk, kind, scale):
 
 
 # ---- 5. sharding -------------------------------------------------------------------------------------------------
-def _run_fake(bk, world, make, T, streams):
-    """make(group) -> smc for that rank; streams(n, lo, hi, smc) -> (normals, acc_u, res_u) or Nones.
-    Returns (indices [T, M], thetas [M, D], ranks).  (The FakeWorld harness of test_gpu_sharded_smc.py.)"""
-    fw = bk.peer.FakeWorld(world)
-    ranks = [make(fw.rank(r)) for r in range(world)]
-    all_idx = []
-    for n in range(1, T + 1):
-        for s in ranks:
-            z, au, _ = streams(n, s._lo, s._hi, s)
-            s._move(n, z, au)
-        for ph in (1, 2):
-            for s in ranks:
-                _, _, ru = streams(n, s._lo, s._hi, s)
-                s._resample(n, ru, ph)
-        torch.cuda.synchronize()
-        all_idx.append(np.concatenate([np_(s.last_indices) for s in ranks]))
-    th = np.concatenate([np_(s.thetas) for s in ranks])
-    for s in ranks:
-        s._check()
-    return np.stack(all_idx), th, ranks
-
-
 @pytest.mark.parametrize("world", [1, 2, 3, 5])
 @pytest.mark.parametrize("mode", ["systematic", "multinomial"])
 def test_sharded_user_smc_equals_oracle(bk, world, mode):
@@ -325,7 +175,7 @@ def test_sharded_user_smc_equals_oracle(bk, world, mode):
     th0 = rng.normal(size=(M, D)) * MIX_TAU
     zs, au, ru = rng.standard_normal((T, M, D)), rng.random((T, M)), rng.random((T, M))
     oth, oidx = osm.smc_tempered(nm, th0, zs, au, ru, scale, T, resample=mode)
-    dm = bk.CudaPriorLikModel(MIXTURE, D, params=nm.params(), dtype=torch.float64)
+    dm = bk.CudaPriorLikModel(MIXTURE_MODEL, D, params=nm.params(), dtype=torch.float64)
 
     def make(group):
         return bk.TemperedLikelihoodSMC(dm, M, T, th0, bk.metropolis_kernel(scale), resample=mode, group=group)
@@ -334,7 +184,7 @@ def test_sharded_user_smc_equals_oracle(bk, world, mode):
         r = ru[n - 1, :1] if mode == "systematic" else ru[n - 1, lo:hi]
         return zs[n - 1, lo:hi], au[n - 1, lo:hi], r
 
-    idx, th, ranks = _run_fake(bk, world, make, T, streams)
+    idx, th, ranks = run_fake(bk, world, make, T, streams)
     assert np.array_equal(idx, oidx), f"indices differ (world={world}, {mode})"
     np.testing.assert_allclose(th, oth, rtol=1e-12, atol=1e-12)
     for s in ranks[1:]:
@@ -356,9 +206,9 @@ def test_sharded_user_smc_philox_invariant(bk, kind):
         return bk.TemperedLikelihoodSMC(dm, M, T, th0, kern, resample="systematic", seed=7, group=group)
 
     none = lambda n, lo, hi, s: (None, None, None)
-    idx1, th1, _ = _run_fake(bk, 1, make, T, none)
+    idx1, th1, _ = run_fake(bk, 1, make, T, none)
     for world in (3, 8):
-        idxg, thg, _ = _run_fake(bk, world, make, T, none)
+        idxg, thg, _ = run_fake(bk, world, make, T, none)
         assert np.array_equal(idx1, idxg), world
         assert np.array_equal(th1, thg), world
     single = bk.TemperedLikelihoodSMC(dm, M, T, th0, kern, resample="systematic", seed=7)
@@ -375,7 +225,7 @@ def test_user_smc_adaptive_vs_oracle(bk, thr):
     th0 = rng.normal(size=(M, D)) * MIX_TAU
     zs, au, ru = rng.standard_normal((T, M, D)), rng.random((T, M)), rng.random((T, M))
     oth, ologw, oflags = osm.smc_tempered_adaptive(nm, th0, zs, au, ru, scale, T, thr)
-    dm = bk.CudaPriorLikModel(MIXTURE, D, params=nm.params(), dtype=torch.float64)
+    dm = bk.CudaPriorLikModel(MIXTURE_MODEL, D, params=nm.params(), dtype=torch.float64)
     smc = bk.TemperedLikelihoodSMC(dm, M, T, th0, bk.metropolis_kernel(scale), resample="systematic",
                                    ess_threshold=thr)
     for n in range(1, T + 1):
@@ -405,7 +255,7 @@ __device__ bk_real log_density_gradient(const bk_real* x, bk_real* g, const bk_r
         bk.CudaPriorLikModel(GPL[:GPL.index("__device__ bk_real log_likelihood_gradient")], 3, params=np.ones(12))
     # run(), then transition() steps, then .thetas; last_accept [M_local] in {0, 1}
     nm = Mixture(MIX_MU, MIX_S, MIX_TAU)
-    dm = bk.CudaPriorLikModel(MIXTURE, 4, params=nm.params())
+    dm = bk.CudaPriorLikModel(MIXTURE_MODEL, 4, params=nm.params())
     assert "bk_user_smc_hmc" in dm.compile_log
     M, T = 1000, 8
     smc = bk.TemperedLikelihoodSMC(dm, M, T, lambda m: np.full(4, 0.1 * (m % 7)), bk.hmc_kernel(0.1, 3),

@@ -1,7 +1,8 @@
 """TemperedLikelihoodSMC with a user-written CudaProposal as the move (proposal_kernel): one Metropolis(-Hastings) step
 of the proposal on the tempered density, compiled together with a CudaPriorLikModel into one kernel
 (bk_user_smc_mhp).  Models and proposals are written in CUDA for the device and in NumPy for the restatement in
-tests/_smc_proposal_oracle.py; most of them are those of test_gpu_user_smc.py and test_gpu_user_proposal.py."""
+tests/_smc_proposal_oracle.py; most of them, shared with test_gpu_user_smc.py and test_gpu_user_proposal.py, are
+in tests/_user_cuda.py."""
 import math
 
 import numpy as np
@@ -10,70 +11,12 @@ import torch
 
 import _smc_proposal_oracle as sop
 from _dev import np_
+from _user_cuda import (GAMMA_POIS, GPL, INDEP, LOGNORMAL, MIX_MU, MIX_S, MIX_TAU, MIXTURE_MODEL, MIXTURE_WALK, RSCAN,
+                        RW, GammaPois, Mixture, binom, gpl, np_indep, np_lognormal, np_mixture_walk, np_rscan,
+                        philox_streams, run_fake, user_twin)
 from conftest import golden
-from test_gpu_user_proposal import INDEP, LOGNORMAL, RSCAN, RW, _philox_streams, np_indep, np_lognormal, np_rscan
-from test_gpu_user_proposal import MIXTURE as MIX_PROP
-from test_gpu_user_smc import GPL, MIX_MU, MIX_S, MIX_TAU, MIXTURE, Mixture, _run_fake, binom, gpl, user_twin
 
 pytestmark = pytest.mark.gpu
-
-# independent Gamma(a, rate b) priors and Poisson likelihoods on positive rates: coordinate e saw S_e events in
-# n intervals.  params = [a, b, n, S (D)]; the tempered posterior at t is Gamma(a + t S_e, b + t n).
-GAMMA_POIS = """
-__device__ bk_real log_prior_gradient(const bk_real* x, bk_real* g, const bk_real* p) {
-    bk_real s = 0;
-    for (int e = 0; e < BK_DIMS; ++e) {
-        if (!(x[e] > 0)) return log(bk_real(0));
-        s += (p[0] - 1) * log(x[e]) - p[1] * x[e];
-        g[e] = (p[0] - 1) / x[e] - p[1];
-    }
-    return s;
-}
-__device__ bk_real log_likelihood_gradient(const bk_real* x, bk_real* g, const bk_real* p) {
-    bk_real s = 0;
-    for (int e = 0; e < BK_DIMS; ++e) {
-        if (!(x[e] > 0)) return log(bk_real(0));
-        s += p[3 + e] * log(x[e]) - p[2] * x[e];
-        g[e] = p[3 + e] / x[e] - p[2];
-    }
-    return s;
-}
-"""
-
-
-class GammaPois:
-    """NumPy twin of GAMMA_POIS."""
-
-    def __init__(self, a, b, n, S):
-        self.a, self.b, self.n, self.S = float(a), float(b), float(n), np.asarray(S, dtype=np.float64)
-
-    def params(self):
-        return np.concatenate([[self.a, self.b, self.n], self.S])
-
-    def log_prior(self, x):
-        s = 0.0
-        for e in range(x.shape[0]):
-            if not x[e] > 0:
-                return -math.inf
-            s += (self.a - 1) * math.log(x[e]) - self.b * x[e]
-        return s
-
-    def log_likelihood(self, x):
-        s = 0.0
-        for e in range(x.shape[0]):
-            if not x[e] > 0:
-                return -math.inf
-            s += self.S[e] * math.log(x[e]) - self.n * x[e]
-        return s
-
-
-def np_mixprop(s1, s2, w):
-    """NumPy twin of test_gpu_user_proposal.MIXTURE (2 D normals, 2 uniforms, no transition)."""
-    def propose(th, z, u):
-        D = th.shape[0]
-        s = (s1 if u[0] < w else s2) * (0.5 + u[1])
-        return th + s * z[:D] + 0.01 * z[D:]
-    return propose
 
 
 def walk(bk, s, D, dtype, transition=False):
@@ -169,14 +112,15 @@ def _case(bk, which, dtype=torch.float64):
             p, t = np_indep(m, s)
         return dm, GP, prop, p, t, init
     nm = Mixture(MIX_MU, MIX_S, MIX_TAU)
-    dm = bk.CudaPriorLikModel(MIXTURE, 4, params=nm.params(), dtype=dtype)
+    dm = bk.CudaPriorLikModel(MIXTURE_MODEL, 4, params=nm.params(), dtype=dtype)
     init = lambda rng, M: rng.normal(size=(M, 4)) * MIX_TAU
     if which == "rscan":
         prop = bk.CudaProposal(RSCAN, 4, params=[0.8], normals=1, uniforms=1, dtype=dtype)
         p, t = np_rscan(0.8)
         return dm, nm, prop, p, t, init
-    prop = bk.CudaProposal(MIX_PROP, 4, params=[0.3, 1.2, 0.6], normals=8, uniforms=2, transition=False, dtype=dtype)
-    return dm, nm, prop, np_mixprop(0.3, 1.2, 0.6), None, init
+    prop = bk.CudaProposal(MIXTURE_WALK, 4, params=[0.3, 1.2, 0.6], normals=8, uniforms=2, transition=False,
+                           dtype=dtype)
+    return dm, nm, prop, np_mixture_walk(0.3, 1.2, 0.6), None, init
 
 
 def _streams(rng, T, M, prop):
@@ -221,11 +165,11 @@ def test_philox_equals_injected_reconstruction(bk, which):
     rs = np.random.default_rng(3).random((T, 1))
 
     def rebuilt(n, lo, hi, s):
-        Z, U = _philox_streams(bk, seed, lo, hi - lo, 4, prop.normals, prop.uniforms, 1, n)
+        Z, U = philox_streams(bk, seed, lo, hi - lo, 4, prop.normals, prop.uniforms, 1, n)
         return Z[0], U[0], rs[n - 1]
 
-    idx_p, th_p, ranks = _run_fake(bk, world, make, T, lambda n, lo, hi, s: (None, None, rs[n - 1]))
-    idx_i, th_i, _ = _run_fake(bk, world, make, T, rebuilt)
+    idx_p, th_p, ranks = run_fake(bk, world, make, T, lambda n, lo, hi, s: (None, None, rs[n - 1]))
+    idx_i, th_i, _ = run_fake(bk, world, make, T, rebuilt)
     assert np.array_equal(idx_p, idx_i)
     assert np.array_equal(th_p, th_i)
     assert 0 < float(ranks[0].last_accept.float().mean()) < 1
@@ -249,7 +193,7 @@ def test_sharded_equals_restatement(bk, world, mode):
         r = ru[n - 1, :1] if mode == "systematic" else ru[n - 1, lo:hi]
         return zs[n - 1, lo:hi], au[n - 1, lo:hi], r
 
-    idx, th, _ = _run_fake(bk, world, make, T, streams)
+    idx, th, _ = run_fake(bk, world, make, T, streams)
     assert np.array_equal(idx, oidx), f"indices differ (world={world}, {mode})"
     np.testing.assert_allclose(th, oth, rtol=1e-10, atol=1e-10)
 
@@ -261,17 +205,17 @@ def test_sharded_philox_invariant_fp32(bk):
     mu = torch.randn(D, device="cuda", generator=g)
     th0 = torch.randn(M, D, device="cuda", generator=g)
     dm = gpl(bk, np.zeros(D), np.ones(D), mu.cpu().numpy(), 4 * np.ones(D), dtype=torch.float32)
-    prop = bk.CudaProposal(MIX_PROP, D, params=[0.15, 0.4, 0.6], normals=2 * D, uniforms=2, transition=False)
+    prop = bk.CudaProposal(MIXTURE_WALK, D, params=[0.15, 0.4, 0.6], normals=2 * D, uniforms=2, transition=False)
     kern = bk.proposal_kernel(prop)
 
     def make(group):
         return bk.TemperedLikelihoodSMC(dm, M, T, th0, kern, resample="systematic", seed=7, group=group)
 
     none = lambda n, lo, hi, s: (None, None, None)
-    idx1, th1, r1 = _run_fake(bk, 1, make, T, none)
+    idx1, th1, r1 = run_fake(bk, 1, make, T, none)
     assert 0 < float(r1[0].last_accept.float().mean()) < 1
     for world in (3, 8):
-        idxg, thg, _ = _run_fake(bk, world, make, T, none)
+        idxg, thg, _ = run_fake(bk, world, make, T, none)
         assert np.array_equal(idx1, idxg), world
         assert np.array_equal(th1, thg), world
     single = bk.TemperedLikelihoodSMC(dm, M, T, th0, kern, resample="systematic", seed=7)

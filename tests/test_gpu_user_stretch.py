@@ -6,32 +6,12 @@ import pytest
 import torch
 
 from _dev import np_
+from _user_cuda import BANANA_1, SCHOOLS_SIGMA, SCHOOLS_Y, NpBanana, NpSchools
 from oracle import samplers as osm
 
 pytestmark = pytest.mark.gpu
 
 # ---- models ---------------------------------------------------------------------------------------------------------
-# banana: x0 ~ N(0, 1), x1 - b x0^2 ~ N(0, 1), every further coordinate N(0, 1); at D = 1 a standard normal; params = [b]
-BANANA = """
-__device__ bk_real log_density_gradient(const bk_real* x, bk_real* g, const bk_real* params) {
-#if BK_DIMS == 1
-    g[0] = -x[0];
-    return bk_real(-0.5) * (x[0] * x[0]);
-#else
-    const bk_real b = params[0], half = 0.5, two = 2;
-    const bk_real u = x[1] - b * x[0] * x[0];
-    bk_real lp = -half * (x[0] * x[0]) - half * (u * u);
-    g[0] = -x[0] + two * b * x[0] * u;
-    g[1] = -u;
-    for (int e = 2; e < BK_DIMS; ++e) {
-        lp -= half * (x[e] * x[e]);
-        g[e] = -x[e];
-    }
-    return lp;
-#endif
-}
-"""
-
 # non-centred eight schools: theta = (mu, log tau, eta[8]); y_j ~ N(mu + tau eta_j, sigma_j), eta ~ N(0, 1),
 # mu ~ N(0, 5^2), log tau ~ N(1, 1); params = [y (8), sigma (8)]
 SCHOOLS = """
@@ -53,9 +33,6 @@ __device__ bk_real log_density_gradient(const bk_real* th, bk_real* g, const bk_
     return lp;
 }
 """
-SCHOOLS_Y = np.array([28.0, 8.0, -3.0, 7.0, -1.0, 1.0, 18.0, 12.0])
-SCHOOLS_SIGMA = np.array([15.0, 10.0, 16.0, 11.0, 9.0, 11.0, 10.0, 18.0])
-
 # the banana split into a prior (x0 and x2.. standard normal) and a likelihood (x1 - b x0^2 standard normal), once as
 # a CudaPriorLikModel and once as a CudaModel that sums the two terms in the library's order (ll + prior)
 BANANA_TERMS = """
@@ -95,35 +72,6 @@ __device__ bk_real log_density_gradient(const bk_real* x, bk_real* g, const bk_r
 """
 
 
-class NpBanana:
-    def __init__(self, D, b):
-        self.D, self.b = D, b
-
-    def log_density(self, x):
-        x = np.asarray(x, dtype=np.float64)
-        if self.D == 1:
-            return -0.5 * x[0] * x[0]
-        u = x[1] - self.b * x[0] * x[0]
-        lp = -0.5 * (x[0] * x[0]) - 0.5 * (u * u)
-        for e in range(2, self.D):
-            lp -= 0.5 * (x[e] * x[e])
-        return lp
-
-
-class NpSchools:
-    def log_density(self, th):
-        th = np.asarray(th, dtype=np.float64)
-        mu, lt = th[0], th[1]
-        tau = np.exp(lt)
-        lp = -0.5 * (mu * mu) / 25 - 0.5 * ((lt - 1) * (lt - 1))
-        for j in range(8):
-            eta = th[2 + j]
-            d = SCHOOLS_Y[j] - mu - tau * eta
-            r = d / (SCHOOLS_SIGMA[j] * SCHOOLS_SIGMA[j])
-            lp += -0.5 * (eta * eta) - 0.5 * (d * r)
-        return lp
-
-
 @pytest.fixture
 def fused(monkeypatch):
     monkeypatch.setenv("BK_FORCE_GENERIC", "0")
@@ -131,7 +79,7 @@ def fused(monkeypatch):
 
 def _models(bk, which, D, dtype=torch.float64):
     if which == "banana":
-        return bk.CudaModel(BANANA, D, params=[0.5], dtype=dtype), NpBanana(D, 0.5)
+        return bk.CudaModel(BANANA_1, D, params=[0.5], dtype=dtype), NpBanana(D, 0.5)
     return bk.CudaModel(SCHOOLS, 10, params=np.concatenate([SCHOOLS_Y, SCHOOLS_SIGMA]), dtype=dtype), NpSchools()
 
 
@@ -156,7 +104,7 @@ def test_matches_oracle(bk, fused, which, D, W):
 # ---- 2. fused == three-launch engine, Philox ------------------------------------------------------------------------
 def _pair(bk, monkeypatch, dtype, D=6, W=64):
     monkeypatch.setenv("BK_FORCE_GENERIC", "0")
-    dm = bk.CudaModel(BANANA, D, params=[0.5], dtype=dtype)
+    dm = bk.CudaModel(BANANA_1, D, params=[0.5], dtype=dtype)
     init = np.random.default_rng(4).normal(size=(W, D))
     fu = bk.Stretcher(dm, walkers=W, init=init, seed=21)
     ge = bk.Stretcher(dm, walkers=W, init=init, seed=21)
@@ -254,7 +202,7 @@ def test_prior_lik_equals_model(bk, fused):
 def test_engine_choice_and_surface(bk, fused):
     lib = bk._lib.lib()
     for D, want_fused in ((32, True), (33, False)):
-        dm = bk.CudaModel(BANANA, D, params=[0.5])
+        dm = bk.CudaModel(BANANA_1, D, params=[0.5])
         model_log = dm.compile_log
         s = bk.Stretcher(dm, seed=1)
         assert dm.compile_log == model_log
@@ -277,7 +225,7 @@ def test_engine_choice_and_surface(bk, fused):
 # ---- 7. compile errors -------------------------------------------------------------------------------------------------
 def test_compile_error_raises_value_error(bk, fused):
     # compiles as a model; its Stretcher program (-DBK_STRETCH=1) does not
-    src = "#ifdef BK_STRETCH\n#error no stretch for this model\n#endif\n" + BANANA
+    src = "#ifdef BK_STRETCH\n#error no stretch for this model\n#endif\n" + BANANA_1
     dm = bk.CudaModel(src, 3, params=[0.5])
     with pytest.raises(ValueError, match="no stretch for this model") as e:
         bk.Stretcher(dm)
@@ -289,7 +237,7 @@ def test_banana_moments(bk, fused):
     """x1 has mean b and variance 1 + 2 b^2, every other coordinate is N(0, 1); within 4 MCSE (each walker's ESS from
     its own series, summed over walkers)."""
     b, D = 0.5, 8
-    dm = bk.CudaModel(BANANA, D, params=[b])
+    dm = bk.CudaModel(BANANA_1, D, params=[b])
     s = bk.Stretcher(dm, walkers=4096, seed=5)
     assert "bk_user_stretch" in s.compile_log
     for _ in range(500):

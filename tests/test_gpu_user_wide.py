@@ -2,132 +2,20 @@
 memory, state in the generic engine's cache).  Parity runs fp64 with injected streams against the NumPy oracle, and
 against the generic engine (BK_FORCE_GENERIC=1) and the built-in DiagGauss plugin on the same Philox words."""
 import ctypes as C
-import os
-import re
 
 import numpy as np
 import pytest
 import torch
 
 from _dev import np_
+from _user_cuda import (BANANA, DIAG, FUSED_MAX_D, PRIOR_LIK_WEIGHTED, WIDE_MAX_D, NpPriorLik, banana, check,
+                        diag_params, run_split, same, streams_uniforms_last)
 from oracle import samplers as osm
 from oracle.models import DiagGauss as ODiag
 
 pytestmark = pytest.mark.gpu
 
-with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), os.pardir, "bayes-kit_b200", "csrc",
-                       "model.h")) as _f:
-    _h = _f.read()
-FUSED_MAX_D = int(re.search(r"#define BK_USER_FUSED_MAX_D (\d+)", _h).group(1))
-WIDE_MAX_D = int(re.search(r"#define BK_USER_WIDE_MAX_D (\d+)", _h).group(1))
 DIMS = sorted({33, 64, WIDE_MAX_D})
-
-BANANA = """
-__device__ bk_real log_density_gradient(const bk_real* x, bk_real* g, const bk_real* params) {
-    const bk_real b = params[0], half = 0.5, two = 2;
-    const bk_real u = x[1] - b * x[0] * x[0];
-    bk_real lp = -half * (x[0] * x[0]) - half * (u * u);
-    g[0] = -x[0] + two * b * x[0] * u;
-    g[1] = -u;
-    for (int e = 2; e < BK_DIMS; ++e) {
-        lp -= half * (x[e] * x[e]);
-        g[e] = -x[e];
-    }
-    return lp;
-}
-"""
-
-DIAG = """
-__device__ bk_real log_density_gradient(const bk_real* x, bk_real* g, const bk_real* p) {
-    bk_real s = 0;
-    for (int e = 0; e < BK_DIMS; ++e) {
-        const bk_real d = x[e] - p[e];
-        const bk_real pd = p[BK_DIMS + e] * d;
-        s += d * pd;
-        g[e] = -pd;
-    }
-    return bk_real(-0.5) * s;
-}
-"""
-
-# prior N(0, I), likelihood N(1, diag(1 / w)) with weights params = [w (D)]
-PRIOR_LIK = """
-__device__ bk_real log_prior_gradient(const bk_real* x, bk_real* g, const bk_real* p) {
-    bk_real s = 0;
-    for (int e = 0; e < BK_DIMS; ++e) { s += x[e] * x[e]; g[e] = -x[e]; }
-    return bk_real(-0.5) * s;
-}
-__device__ bk_real log_likelihood_gradient(const bk_real* x, bk_real* g, const bk_real* p) {
-    bk_real s = 0;
-    for (int e = 0; e < BK_DIMS; ++e) { const bk_real d = x[e] - 1; s += p[e] * d * d; g[e] = -p[e] * d; }
-    return bk_real(-0.5) * s;
-}
-"""
-
-
-class NpBanana:
-    def __init__(self, D, b):
-        self.D, self.b = D, b
-
-    def dims(self):
-        return self.D
-
-    def log_density_gradient(self, x):
-        x = np.asarray(x, dtype=np.float64)
-        u = x[1] - self.b * x[0] * x[0]
-        lp = -0.5 * (x[0] * x[0]) - 0.5 * (u * u) - 0.5 * float(np.dot(x[2:], x[2:]))
-        g = -x.copy()
-        g[0] = -x[0] + 2 * self.b * x[0] * u
-        g[1] = -u
-        return lp, g
-
-    def log_density(self, x):
-        return self.log_density_gradient(x)[0]
-
-
-class NpPriorLik:
-    def __init__(self, w):
-        self.w = np.asarray(w, dtype=np.float64)
-
-    def dims(self):
-        return self.w.size
-
-    def log_density_gradient(self, x):
-        x = np.asarray(x, dtype=np.float64)
-        d = x - 1
-        return -0.5 * float(x @ x) - 0.5 * float(self.w @ (d * d)), -x - self.w * d
-
-    def log_density(self, x):
-        return self.log_density_gradient(x)[0]
-
-
-def banana(bk, D, b=0.5, dtype=torch.float64):
-    return bk.CudaModel(BANANA, D, params=[b], dtype=dtype), NpBanana(D, b)
-
-
-def _diag_params(D, seed=3):
-    rng = np.random.default_rng(seed)
-    return rng.normal(size=D), rng.uniform(0.5, 3.0, D)
-
-
-def _streams(C, D, n, seed):
-    rng = np.random.default_rng(seed)
-    return rng.normal(size=(C, D)) * 0.7, rng.standard_normal((n, C, D)), rng.random((n, C))
-
-
-def _run_split(s, zs, us, k):
-    """the n draws in two calls (the first evaluates the cache, the second starts from it)"""
-    d1, l1 = s.sample_n(k, normals=zs[:k], uniforms=us[:k])
-    a1 = s.last_accept.clone()
-    d2, l2 = s.sample_n(len(zs) - k, normals=zs[k:], uniforms=us[k:])
-    return torch.cat([d1, d2]), torch.cat([l1, l2]), torch.cat([a1, s.last_accept])
-
-
-def _check(d, l, a, want):
-    wd, wl, wa = want
-    assert np.array_equal(np_(a).astype(bool), wa)
-    np.testing.assert_allclose(np_(d), wd, rtol=1e-10, atol=1e-10)
-    np.testing.assert_allclose(np_(l), wl, rtol=1e-10, atol=1e-10)
 
 
 @pytest.fixture(autouse=True)
@@ -142,14 +30,14 @@ def _wide_engine(monkeypatch):
 @pytest.mark.parametrize("metric", [False, True])
 def test_hmc_matches_oracle(bk, C_, D, L, metric):
     n = 4
-    dm, om = banana(bk, D)
-    th0, zs, us = _streams(C_, D, n, D + L)
+    dm, om = banana(bk, D, dot=True)
+    th0, zs, us = streams_uniforms_last(C_, D, n, D + L)
     m = np.random.default_rng(D).uniform(0.5, 2.0, D) if metric else None
     eps = 0.6 / D ** 0.25
     s = bk.HMCDiag(dm, eps, L, metric_diag=m, init=th0)
     assert "bk_user_wide_hmc" in s.compile_log
-    d, l, a = _run_split(s, zs, us, 2)
-    _check(d, l, a, osm.hmc_diag_batch(om, th0, zs, us, eps, L, m))
+    d, l, a = run_split(s, zs, us, 2)
+    check(d, l, a, osm.hmc_diag_batch(om, th0, zs, us, eps, L, m))
     np.testing.assert_allclose(np_(s.theta), np_(d[-1]).reshape(np_(s.theta).shape), rtol=0, atol=0)
 
 
@@ -157,13 +45,13 @@ def test_hmc_matches_oracle(bk, C_, D, L, metric):
 @pytest.mark.parametrize("D", DIMS)
 def test_mala_matches_oracle(bk, C_, D):
     n = 6
-    dm, om = banana(bk, D)
-    th0, zs, us = _streams(C_, D, n, 11 + D)
+    dm, om = banana(bk, D, dot=True)
+    th0, zs, us = streams_uniforms_last(C_, D, n, 11 + D)
     eps = 0.4 / D ** (1 / 3)
     s = bk.MALA(dm, eps, init=th0)
     assert "bk_user_wide_mala" in s.compile_log
-    d, l, a = _run_split(s, zs, us, 3)
-    _check(d, l, a, osm.mala_batch(om, th0, zs, us, eps))
+    d, l, a = run_split(s, zs, us, 3)
+    check(d, l, a, osm.mala_batch(om, th0, zs, us, eps))
 
 
 @pytest.mark.parametrize("C_", [1, 37, 100])
@@ -171,29 +59,29 @@ def test_mala_matches_oracle(bk, C_, D):
 @pytest.mark.parametrize("hastings", [False, True])
 def test_metropolis_matches_oracle(bk, C_, D, hastings):
     n = 6
-    dm, om = banana(bk, D)
-    th0, zs, us = _streams(C_, D, n, 12 + D)
+    dm, om = banana(bk, D, dot=True)
+    th0, zs, us = streams_uniforms_last(C_, D, n, 12 + D)
     scale = 1.5 / D ** 0.5
     prop = bk.GaussianRW(scale)
     s = bk.MetropolisHastings(dm, prop, prop.transition_lp, init=th0) if hastings else bk.Metropolis(dm, prop, init=th0)
     assert "bk_user_wide_mh" in s.compile_log
-    d, l, a = _run_split(s, zs, us, 3)
-    _check(d, l, a, osm.metropolis_rw_batch(om, th0, zs, us, scale, hastings))
+    d, l, a = run_split(s, zs, us, 3)
+    check(d, l, a, osm.metropolis_rw_batch(om, th0, zs, us, scale, hastings))
 
 
 def test_prior_lik_matches_oracle(bk):
     C_, D, n = 37, 40, 5
     w = np.random.default_rng(4).uniform(0.5, 2.0, D)
-    dm = bk.CudaPriorLikModel(PRIOR_LIK, D, params=w, dtype=torch.float64)
+    dm = bk.CudaPriorLikModel(PRIOR_LIK_WEIGHTED, D, params=w, dtype=torch.float64)
     om = NpPriorLik(w)
-    th0, zs, us = _streams(C_, D, n, 31)
+    th0, zs, us = streams_uniforms_last(C_, D, n, 31)
     s = bk.HMCDiag(dm, 0.15, 5, init=th0)
     assert "bk_user_wide_hmc" in s.compile_log
-    d, l, a = _run_split(s, zs, us, 2)
-    _check(d, l, a, osm.hmc_diag_batch(om, th0, zs, us, 0.15, 5))
+    d, l, a = run_split(s, zs, us, 2)
+    check(d, l, a, osm.hmc_diag_batch(om, th0, zs, us, 0.15, 5))
     s = bk.MALA(dm, 0.05, init=th0)
-    d, l, a = _run_split(s, zs, us, 2)
-    _check(d, l, a, osm.mala_batch(om, th0, zs, us, 0.05))
+    d, l, a = run_split(s, zs, us, 2)
+    check(d, l, a, osm.mala_batch(om, th0, zs, us, 0.05))
 
 
 # ---- 2. against the generic engine and the built-in plugin, Philox ---------------------------------------------------
@@ -203,13 +91,6 @@ def _samplers(bk, D):
             lambda m, init: bk.Metropolis(m, bk.GaussianRW(1.5 / D ** 0.5), init=init, seed=17),
             lambda m, init: bk.MetropolisHastings(m, *(lambda p: (p, p.transition_lp))(bk.GaussianRW(1.5 / D ** 0.5)),
                                                   init=init, seed=17))
-
-
-def _same(a, b, da, db, la, lb):
-    assert torch.equal(a.last_accept, b.last_accept)
-    assert 0 < float(a.last_accept.float().mean()) < 1
-    np.testing.assert_allclose(np_(da), np_(db), rtol=1e-12, atol=1e-12)
-    np.testing.assert_allclose(np_(la), np_(lb), rtol=1e-12, atol=1e-12)
 
 
 @pytest.mark.parametrize("D", [64, WIDE_MAX_D])
@@ -223,7 +104,7 @@ def test_wide_equals_generic(bk, monkeypatch, D):
         monkeypatch.setenv("BK_FORCE_GENERIC", "1")
         b = make(dm, init)
         db, lb = b.sample_n(10)
-        _same(a, b, da, db, la, lb)
+        same(a, b, da, db, la, lb)
 
 
 def test_switching_engines_keeps_the_chains(bk, monkeypatch):
@@ -247,7 +128,7 @@ def test_switching_engines_keeps_the_chains(bk, monkeypatch):
 
 def test_user_diag_gauss_equals_builtin(bk):
     D = 64
-    mu, pr = _diag_params(D)
+    mu, pr = diag_params(D)
     user = bk.CudaModel(DIAG, D, params=np.concatenate([mu, pr]), dtype=torch.float64)
     built = bk.DiagGauss(mu, pr, dtype=torch.float64)
     init = np.random.default_rng(D).normal(size=(64, D))
@@ -255,7 +136,7 @@ def test_user_diag_gauss_equals_builtin(bk):
         a, b = make(user, init), make(built, init)
         da, la = a.sample_n(20)
         db, lb = b.sample_n(20)
-        _same(a, b, da, db, la, lb)
+        same(a, b, da, db, la, lb)
 
 
 def test_shard_invariant(bk):

@@ -1,44 +1,11 @@
 """bk_drghmc_cuda_prepare without a GPU: the entry point is exported and declared, rejects an unknown handle, and a
 model's own program does not contain DrGhmcDiag's kernel (that has a program of its own, compiled on first use)."""
 import ctypes as C
-import os
 
 import pytest
 
+from _user_cuda import HEADER, PLAIN, PRIOR_LIK, needs_nvrtc
 from bayes_kit_b200 import _lib
-from bayes_kit_b200.models import _load_nvrtc
-
-HEADER = os.path.join(os.path.dirname(__file__), os.pardir, "include", "bk.h")
-
-PLAIN = """
-__device__ bk_real log_density_gradient(const bk_real* x, bk_real* g, const bk_real* p) {
-    bk_real s = 0;
-    for (int e = 0; e < BK_DIMS; ++e) { s += x[e] * x[e]; g[e] = -x[e]; }
-    return bk_real(-0.5) * s;
-}
-"""
-
-PRIOR_LIK = """
-__device__ bk_real log_prior_gradient(const bk_real* x, bk_real* g, const bk_real* p) {
-    bk_real s = 0;
-    for (int e = 0; e < BK_DIMS; ++e) { s += x[e] * x[e]; g[e] = -x[e]; }
-    return bk_real(-0.5) * s;
-}
-__device__ bk_real log_likelihood_gradient(const bk_real* x, bk_real* g, const bk_real* p) {
-    bk_real s = 0;
-    for (int e = 0; e < BK_DIMS; ++e) { const bk_real d = x[e] - 1; s += d * d; g[e] = -d; }
-    return bk_real(-0.5) * s;
-}
-"""
-
-
-def _nvrtc_available():
-    _load_nvrtc()
-    try:
-        C.CDLL("libnvrtc.so.12")
-        return True
-    except OSError:
-        return False
 
 
 def test_prepare_is_exported_and_declared():
@@ -56,7 +23,7 @@ def test_prepare_rejects_an_unknown_handle():
     assert log.value == b""
 
 
-@pytest.mark.skipif(not _nvrtc_available(), reason="NVRTC (libnvrtc.so.12) cannot be loaded")
+@needs_nvrtc
 @pytest.mark.parametrize("create,source", [("bk_model_create_cuda", PLAIN),
                                            ("bk_model_create_cuda_prior_lik", PRIOR_LIK)])
 @pytest.mark.parametrize("dims", [2, 32])

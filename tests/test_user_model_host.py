@@ -4,32 +4,10 @@ import ctypes as C
 
 import pytest
 
+from _user_cuda import BANANA, needs_nvrtc
 from bayes_kit_b200 import _lib
-from bayes_kit_b200.models import _load_nvrtc
 
-BANANA = """
-__device__ bk_real log_density_gradient(const bk_real* x, bk_real* g, const bk_real* params) {
-    const bk_real b = params[0], half = 0.5, two = 2;
-    const bk_real u = x[1] - b * x[0] * x[0];
-    bk_real lp = -half * (x[0] * x[0]) - half * (u * u);
-    g[0] = -x[0] + two * b * x[0] * u;
-    g[1] = -u;
-    for (int e = 2; e < BK_DIMS; ++e) { lp -= half * (x[e] * x[e]); g[e] = -x[e]; }
-    return lp;
-}
-"""
-
-
-def _nvrtc_available():
-    _load_nvrtc()
-    try:
-        C.CDLL("libnvrtc.so.12")
-        return True
-    except OSError:
-        return False
-
-
-pytestmark = pytest.mark.skipif(not _nvrtc_available(), reason="NVRTC (libnvrtc.so.12) cannot be loaded")
+pytestmark = needs_nvrtc
 
 DUMMY_PTR = 256   # never dereferenced: validation and compilation do not touch params
 

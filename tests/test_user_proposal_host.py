@@ -8,36 +8,10 @@ import subprocess
 import numpy as np
 import pytest
 
+from _user_cuda import CSRC, RW, needs_nvrtc
 from bayes_kit_b200 import _lib
-from bayes_kit_b200.models import _load_nvrtc
 from oracle import philox as ph
 from oracle import proposals as opr
-
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-CSRC = os.path.join(ROOT, "bayes-kit_b200", "csrc")
-
-RW = """
-__device__ void propose(const bk_real* theta, bk_real* q, const bk_real* z, const bk_real* u, const bk_real* p) {
-    for (int e = 0; e < BK_DIMS; ++e) q[e] = theta[e] + p[0] * z[e];
-}
-__device__ bk_real transition_log_density(const bk_real* to, const bk_real* from, const bk_real* p) {
-    bk_real s = 0;
-    for (int e = 0; e < BK_DIMS; ++e) { const bk_real d = to[e] - from[e]; s += d * d; }
-    return bk_real(-0.5) * s / (p[0] * p[0]);
-}
-"""
-
-
-def _nvrtc_available():
-    _load_nvrtc()
-    try:
-        C.CDLL("libnvrtc.so.12")
-        return True
-    except OSError:
-        return False
-
-
-needs_nvrtc = pytest.mark.skipif(not _nvrtc_available(), reason="NVRTC (libnvrtc.so.12) cannot be loaded")
 
 DUMMY_PTR = 256   # never dereferenced: validation and compilation do not touch params
 

@@ -6,47 +6,10 @@ import os
 
 import pytest
 
+from _user_cuda import GPL, PLAIN, needs_nvrtc
 from bayes_kit_b200 import _lib
-from bayes_kit_b200.models import _load_nvrtc
 
-# GaussPriorLik restated, params = [mu (D), pl (D), m0 (D), p0 (D)]
-GPL = """
-__device__ bk_real quad(const bk_real* x, bk_real* g, const bk_real* m, const bk_real* p) {
-    bk_real s = 0;
-    for (int e = 0; e < BK_DIMS; ++e) {
-        const bk_real d = x[e] - m[e], pd = p[e] * d;
-        s += pd * d;
-        g[e] = -pd;
-    }
-    return bk_real(-0.5) * s;
-}
-__device__ bk_real log_prior_gradient(const bk_real* x, bk_real* g, const bk_real* p) {
-    return quad(x, g, p + 2 * BK_DIMS, p + 3 * BK_DIMS);
-}
-__device__ bk_real log_likelihood_gradient(const bk_real* x, bk_real* g, const bk_real* p) {
-    return quad(x, g, p, p + BK_DIMS);
-}
-"""
-
-PLAIN = """
-__device__ bk_real log_density_gradient(const bk_real* x, bk_real* g, const bk_real* p) {
-    bk_real s = 0;
-    for (int e = 0; e < BK_DIMS; ++e) { s += x[e] * x[e]; g[e] = -x[e]; }
-    return bk_real(-0.5) * s;
-}
-"""
-
-
-def _nvrtc_available():
-    _load_nvrtc()
-    try:
-        C.CDLL("libnvrtc.so.12")
-        return True
-    except OSError:
-        return False
-
-
-pytestmark = pytest.mark.skipif(not _nvrtc_available(), reason="NVRTC (libnvrtc.so.12) cannot be loaded")
+pytestmark = needs_nvrtc
 
 DUMMY_PTR = 256   # never dereferenced: validation and compilation do not touch params
 

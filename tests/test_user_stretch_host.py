@@ -1,14 +1,11 @@
 """bk_stretch_cuda_prepare without a GPU: the entry point is exported and declared, rejects an unknown handle, and a
 model's own program does not contain the Stretcher's kernel (that has a program of its own, compiled on first use)."""
 import ctypes as C
-import os
 
 import pytest
 
+from _user_cuda import HEADER, PLAIN, PRIOR_LIK, needs_nvrtc
 from bayes_kit_b200 import _lib
-from test_user_drghmc_host import PLAIN, PRIOR_LIK, _nvrtc_available
-
-HEADER = os.path.join(os.path.dirname(__file__), os.pardir, "include", "bk.h")
 
 
 def test_prepare_is_exported_and_declared():
@@ -26,7 +23,7 @@ def test_prepare_rejects_an_unknown_handle():
     assert log.value == b""
 
 
-@pytest.mark.skipif(not _nvrtc_available(), reason="NVRTC (libnvrtc.so.12) cannot be loaded")
+@needs_nvrtc
 @pytest.mark.parametrize("create,source", [("bk_model_create_cuda", PLAIN),
                                            ("bk_model_create_cuda_prior_lik", PRIOR_LIK)])
 def test_model_program_has_no_stretch_kernel(create, source):
