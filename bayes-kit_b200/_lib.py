@@ -16,6 +16,7 @@ BK_F32, BK_F64 = 0, 1
 MODEL_ISO, MODEL_DIAG, MODEL_DENSE, MODEL_HLR, MODEL_GPL, MODEL_BINOM, MODEL_USER = range(7)
 SMC_KERNEL_RW, SMC_KERNEL_MALA, SMC_KERNEL_HMC, SMC_KERNEL_PROPOSAL = 0, 1, 2, 3
 SMC_PROPOSAL_MAX_NORMALS = 512
+SMC_MAX_MOVES = 65535
 SMC_MAX_WORLD, SMC_MAILBOX_BYTES = 16, 4096
 RNG_PHILOX, RNG_INJECTED = 0, 1
 RESAMPLE_MULTINOMIAL, RESAMPLE_SYSTEMATIC = 0, 1
@@ -37,7 +38,7 @@ class Rng(C.Structure):
 
 
 class SmcKernel(C.Structure):
-    _fields_ = [("kind", i32), ("steps", i32), ("scale", f64), ("proposal", u64)]
+    _fields_ = [("kind", i32), ("steps", i32), ("scale", f64), ("proposal", u64), ("moves", i32)]
 
 
 class SmcShard(C.Structure):
@@ -124,6 +125,7 @@ _SIGNATURES = {
     "bk_smc_shard_run": (C.c_int, [u64, C.POINTER(SmcShard), vp, i32, i32, i32, C.POINTER(SmcKernel), C.POINTER(Rng), i32, f64,
                                    vp, vp, vp, sz, vp]),
     "bk_smc_cuda_prepare": (C.c_int, [u64, u64, C.c_char_p, sz]),
+    "bk_smc_moves_prepare": (C.c_int, [u64, C.POINTER(SmcKernel), C.c_char_p, sz]),
     "bk_smc_shard_gather": (C.c_int, [C.POINTER(SmcShard), i64, i32, vp, vp]),
     "bk_rank_normalize_workspace_bytes": (sz, [i64, i32]),
     "bk_rank_normalize": (C.c_int, [vp, i32, C.POINTER(SeriesLayout), vp, vp, vp, sz, vp]),

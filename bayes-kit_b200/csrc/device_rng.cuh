@@ -136,21 +136,22 @@ __device__ __forceinline__ void philox_normal4<double>(uint64_t seed, uint32_t b
 }
 
 // k-th uniform of (chain, draw)
+// (boff: added to the block counter word -- move j of an SMC temperature step draws at boff = 2^16 j, smc_move_block)
 template <typename T>
 __host__ __device__ __forceinline__ T philox_uniform(uint64_t seed, uint32_t k, uint32_t chain, uint32_t draw,
-                                                     uint32_t tag = TAG_UNIFORM);
+                                                     uint32_t tag = TAG_UNIFORM, uint32_t boff = 0);
 template <>
 __host__ __device__ __forceinline__ float philox_uniform<float>(uint64_t seed, uint32_t k, uint32_t chain,
-                                                                uint32_t draw, uint32_t tag) {
+                                                                uint32_t draw, uint32_t tag, uint32_t boff) {
     uint32_t r[4];
-    Philox::gen(seed, k >> 2, tag, chain, draw, r);
+    Philox::gen(seed, (k >> 2) + boff, tag, chain, draw, r);
     return u01(r[k & 3]);
 }
 template <>
 __host__ __device__ __forceinline__ double philox_uniform<double>(uint64_t seed, uint32_t k, uint32_t chain,
-                                                                  uint32_t draw, uint32_t tag) {
+                                                                  uint32_t draw, uint32_t tag, uint32_t boff) {
     uint32_t r[4];
-    Philox::gen(seed, k >> 1, tag, chain, draw, r);
+    Philox::gen(seed, (k >> 1) + boff, tag, chain, draw, r);
     return (k & 1) ? u01d(r[2], r[3]) : u01d(r[0], r[1]);
 }
 
@@ -166,11 +167,17 @@ __device__ __forceinline__ T uniform_of_words(uint32_t w0, uint32_t w1) {
     else return u01d(w0, w1);
 }
 template <typename T>
-__device__ __forceinline__ T philox_accept_uniform(uint64_t seed, uint32_t chain, uint32_t draw, int D) {
+__device__ __forceinline__ T philox_accept_uniform(uint64_t seed, uint32_t chain, uint32_t draw, int D, uint32_t boff = 0) {
     uint32_t r[4];
-    Philox::gen(seed, (uint32_t)accept_block(D), TAG_NORMAL, chain, draw, r);
+    Philox::gen(seed, (uint32_t)accept_block(D) + boff, TAG_NORMAL, chain, draw, r);
     return uniform_of_words<T>(r[0], r[1]);
 }
+
+// Several Markov moves per SMC temperature step (bk_smc_kernel.moves): move j draws exactly the words move 0 draws
+// (normals, accept uniform, fp64 TAG_NORMAL_HI words, a proposal's TAG_UNIFORM uniforms) with the element-block counter
+// word b replaced by b + 2^16 j.  Every block a move uses is below 2^16 (D <= 256, <= 512 proposal normals, <= 64
+// uniforms), so move 0 is the single-move stream and the moves' streams are disjoint.
+__host__ __device__ __forceinline__ uint32_t smc_move_block(int j) { return (uint32_t)j << 16; }
 
 // Normals of a user proposal (bk_proposal_create_cuda): normal k is element k % 4 of philox_normal4 on element block
 // proposal_normal_block(k, D) -- the blocks 0, 1, ... with accept_block(D) skipped, so the accept uniform never shares

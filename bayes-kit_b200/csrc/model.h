@@ -75,10 +75,12 @@ int user_wide_prepare(const Model& m, char* log_out, size_t log_bytes);
 int user_wide_sample(const Model& m, int algo, UserWideArgs& a, int32_t* cache_valid, cudaStream_t st);
 // prior/likelihood user models (bk_model_create_cuda_prior_lik): log_prior / log_likelihood of theta [C, D] (each
 // output nullable) and TemperedLikelihoodSMC's move + weight kernel (move: BK_SMC_KERNEL_*; the PROPOSAL move runs
-// bk_user_smc_mhp of the program of (m, p))
+// bk_user_smc_mhp of the program of (m, p)).  a.moves > 1 runs the *_moves kernel of the SMC_MOVES program of (m, p),
+// which user_smc_moves_prepare (or the first such move) compiles once per process.
 bool user_prior_lik(const Model& m);
 int user_log_prior_likelihood(const Model& m, const void* theta, int64_t C, void* lprior, void* llik, cudaStream_t st);
 int user_smc_move(const Model& m, const UserProposal* p, int move, const UserSmcArgs& a, cudaStream_t st);
+int user_smc_moves_prepare(const Model& m, const UserProposal* p, char* log_out, size_t log_bytes);
 // the fused bk_user_mhp serves (m, p): a user model with dims <= USER_FUSED_MAX_D and n_normals <= USER_FUSED_MAX_D
 bool user_mhp_fusable(const Model& m, const UserProposal& p);
 // The programs of (m, p) and of m's DrGHMC kernel are compiled (once per process) by these or on their first launch;

@@ -95,8 +95,9 @@ struct Lanes {
     // standard normals for (chain, draw); invalid slots are 0
     // raw2 (optional): the first two Philox words of element block `ub`, left in the lane that owns that block
     // (lane ub % G) -- the accept uniform of common.cuh's rule when the layout has a slot for it (ub < G * J)
+    // boff (Philox): added to every block's counter word (smc_move_block)
     __device__ __forceinline__ void normals(const bk_rng& rng, int64_t C, int64_t chain, int64_t t,
-                                            T (&z)[NE], uint32_t* raw2 = nullptr, int ub = -1) const {
+                                            T (&z)[NE], uint32_t* raw2 = nullptr, int ub = -1, uint32_t boff = 0) const {
         if (rng.mode == BK_RNG_INJECTED) {
             load(reinterpret_cast<const T*>(rng.normals) + (t * C + chain) * (int64_t)D, z, T(0));
         } else {
@@ -107,7 +108,7 @@ struct Lanes {
                 int blk = lane + G * j;
                 T q[4];
                 uint32_t w[2];
-                philox_normal4<T>(rng.seed, (uint32_t)blk, gc, gd, q, w);
+                philox_normal4<T>(rng.seed, (uint32_t)blk + boff, gc, gd, q, w);
                 if (raw2 && blk == ub) { raw2[0] = w[0]; raw2[1] = w[1]; }
                 if (4 * G * (j + 1) <= D) {   // warp-uniform: block j of EVERY lane is real -> no per-element masks
 #pragma unroll

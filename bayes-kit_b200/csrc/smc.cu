@@ -45,6 +45,7 @@ struct SmcArgs {
     T* llpr_out;
     const T* llpr_tab[BK_SMC_MAX_WORLD];
     int carry;
+    int moves;                 // Markov moves per particle visit (> 1: the k_smc_move_weight_moves instantiations)
 };
 
 // ---- per-lane views of the LogPriorLikelihoodModel plugins (typing.py:37-42) ------------------
@@ -127,9 +128,18 @@ struct BinomView {
 // VM: row access mode fixed at compile time (sep_common.cuh) for the hot layout; -1 = run-time flags.  (c4: 20.4 -> 17.8 ms.
 // Measured and dropped: the model's per-dimension parameters in shared memory instead of registers -- the same 17.8 ms
 // at 3 CTAs / SM, and 22.2 / 26.7 ms at 4 / 5 CTAs per SM, where the register cap spills.)
+// MOVE | SMC_MULTI: the visit applies the kernel a.moves times (bk_smc_kernel.moves) to the particle held in registers
+// -- theta and its (ll, prior) pair stay on chip between the moves; move j draws at element block b + 2^16 j
+// (smc_move_block), injected streams are read at draw j.  The loop is not unrolled (DESIGN 4.6: a doubled visit body
+// ran 10 % slower).  Without the flag the loop has one trip and folds away: the single-move instantiations are the
+// single-move kernel, instruction for instruction.  (The flag rides on MOVE so that those keep their names; a
+// __forceinline__ body shared by two kernels schedules them differently.)
+enum { SMC_MULTI = 16 };
 template <typename T, int G, int J, template <typename, int, int> class View, int MOVE, int OCC = 0, int VM = -1>
 __global__ void __launch_bounds__(128, OCC ? OCC : (J >= 4 && sizeof(T) == 4) ? 3 : (J == 2 && G == 8) ? 5 : 1) k_smc_move_weight(SmcArgs<T> a) {
     using A = Ar<T>;
+    constexpr bool MULTI = (MOVE & SMC_MULTI) != 0;
+    constexpr int KIND = MOVE & ~SMC_MULTI;
     constexpr int NE = 4 * J;
     const int64_t n_groups = (int64_t)gridDim.x * blockDim.x / G;
     const int64_t g0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) / G;
@@ -179,6 +189,7 @@ __global__ void __launch_bounds__(128, OCC ? OCC : (J >= 4 && sizeof(T) == 4) ? 
     if (n_it > 1) row_nn = row_of(particle(1));
     const T t0 = a.t0;
     auto tgrad = [&](const T (&x)[NE], int k) { return A::add(A::mul(md.gll(x, k), t0), md.gpr(x, k)); };
+    const int n_moves = MULTI ? a.moves : 1;
     for (int64_t it = 0; it < n_it; ++it) {
         const int64_t raw = g0 + it * n_groups;
         const bool active = raw < a.M;
@@ -193,92 +204,100 @@ __global__ void __launch_bounds__(128, OCC ? OCC : (J >= 4 && sizeof(T) == 4) ? 
             if (carry) { const T* lp2 = llpr_ptr(row_nn); nll = lp2[0]; npr = lp2[1]; }
         }
         if (it + 2 < n_it) row_nn = row_of(particle(it + 2));
-        uint32_t raw2[2] = {0u, 0u};
-        ln.normals(a.rng, a.M, m, 0, z, raw2, ub);
-        // accept uniform: when the lane layout has a slot for block ub, the pass above made its Philox words --
-        // one counter-mode call per lane and particle instead of two.  Otherwise one extra call (same block);
-        // injected streams: the recorded uniform.
-        T lu = T(0);
-        if (spare_block) {
-            if (ln.lane == ub % G) {
-                if constexpr (sizeof(T) == 4) lu = log_u(u01(raw2[0]));
-                else lu = log_u(u01d(raw2[0], raw2[1]));
-            }
-            lu = __shfl_sync(0xffffffffu, lu, ub % G, G);
-        } else {
-            if (ln.lane == 0)
-                lu = log_u(a.rng.mode == BK_RNG_PHILOX
-                               ? philox_accept_uniform<T>(a.rng.seed, (uint32_t)(a.rng.chain_offset + (uint64_t)m),
-                                                          (uint32_t)a.rng.draw_offset, a.D)
-                               : ln.uniform(a.rng, a.M, m, 0, 0));
-            lu = __shfl_sync(0xffffffffu, lu, 0, G);
-        }
-        T ll_s, pr_s;
-        if (!carry) md.terms(th, ll_c, pr_c);       // first step / replaced particles: nothing carried yet
-        const T lp_c = A::add(A::mul(ll_c, t0), pr_c);
+        int n_acc = 0;
         bool acc;
-        if constexpr (MOVE == BK_SMC_KERNEL_RW) {
-#pragma unroll
-            for (int k = 0; k < NE; ++k) st[k] = A::add(th[k], A::mul(a.scale, z[k]));  // smc.py:81
-            md.terms(st, ll_s, pr_s);
-            const T lp_s = A::add(A::mul(ll_s, t0), pr_s);
-            acc = lu < A::sub(lp_s, lp_c);  // smc.py:85
-        } else if constexpr (MOVE == BK_SMC_KERNEL_MALA) {
-            // one MALA transition on the tempered density (mala.py:40-66)
-            const T eps = a.scale, sd = A::sqrt_(A::mul(T(2), eps)), coef = T(-0.25) / eps;
-#pragma unroll
-            for (int k = 0; k < NE; ++k)
-                st[k] = ln.valid(k) ? A::add(A::add(th[k], A::mul(eps, tgrad(th, k))), A::mul(sd, z[k])) : T(0);
-            md.terms(st, ll_s, pr_s);
-            const T lp_s = A::add(A::mul(ll_s, t0), pr_s);
-            T sf = T(0), sr = T(0);
-#pragma unroll
-            for (int k = 0; k < NE; ++k) {
-                if (ln.valid(k)) {
-                    const T df = A::sub(A::sub(st[k], th[k]), A::mul(eps, tgrad(th, k)));
-                    const T dr = A::sub(A::sub(th[k], st[k]), A::mul(eps, tgrad(st, k)));
-                    sf = A::add(sf, A::mul(df, df));
-                    sr = A::add(sr, A::mul(dr, dr));
+#pragma unroll 1
+        for (int j = 0; j < n_moves; ++j) {
+            // move j: injected streams at draw j ([moves, M, .]), Philox words at element block b + 2^16 j
+            const int64_t tj = MULTI && a.rng.mode == BK_RNG_INJECTED ? j : 0;
+            const uint32_t boff = MULTI ? smc_move_block(j) : 0u;
+            uint32_t raw2[2] = {0u, 0u};
+            ln.normals(a.rng, a.M, m, tj, z, raw2, ub, boff);
+            // accept uniform: when the lane layout has a slot for block ub, the pass above made its Philox words --
+            // one counter-mode call per lane and particle instead of two.  Otherwise one extra call (same block);
+            // injected streams: the recorded uniform.
+            T lu = T(0);
+            if (spare_block) {
+                if (ln.lane == ub % G) {
+                    if constexpr (sizeof(T) == 4) lu = log_u(u01(raw2[0]));
+                    else lu = log_u(u01d(raw2[0], raw2[1]));
                 }
+                lu = __shfl_sync(0xffffffffu, lu, ub % G, G);
+            } else {
+                if (ln.lane == 0)
+                    lu = log_u(a.rng.mode == BK_RNG_PHILOX
+                                   ? philox_accept_uniform<T>(a.rng.seed, (uint32_t)(a.rng.chain_offset + (uint64_t)m),
+                                                              (uint32_t)a.rng.draw_offset, a.D, boff)
+                                   : ln.uniform(a.rng, a.M, m, tj, 0));
+                lu = __shfl_sync(0xffffffffu, lu, 0, G);
             }
-            const T fwd = A::mul(coef, group_sum<G>(sf)), rev = A::mul(coef, group_sum<G>(sr));
-            acc = lu < A::add(A::sub(lp_s, lp_c), A::sub(rev, fwd));   // metropolis.py:41-76
-        } else {
-            // one HMCDiag transition, identity metric, on the tempered density (hmc.py:40-63)
-            const T eps = a.scale, heps = A::mul(T(0.5), eps);
-            T kin = T(0);
+            T ll_s, pr_s;
+            if (!carry && j == 0) md.terms(th, ll_c, pr_c);   // first step / replaced particles: nothing carried yet
+            const T lp_c = A::add(A::mul(ll_c, t0), pr_c);
+            if constexpr (KIND == BK_SMC_KERNEL_RW) {
 #pragma unroll
-            for (int k = 0; k < NE; ++k) kin = A::add(kin, A::mul(z[k], z[k]));
-            const T h0 = A::sub(lp_c, A::mul(T(0.5), group_sum<G>(kin)));
+                for (int k = 0; k < NE; ++k) st[k] = A::add(th[k], A::mul(a.scale, z[k]));  // smc.py:81
+                md.terms(st, ll_s, pr_s);
+                const T lp_s = A::add(A::mul(ll_s, t0), pr_s);
+                acc = lu < A::sub(lp_s, lp_c);  // smc.py:85
+            } else if constexpr (KIND == BK_SMC_KERNEL_MALA) {
+                // one MALA transition on the tempered density (mala.py:40-66)
+                const T eps = a.scale, sd = A::sqrt_(A::mul(T(2), eps)), coef = T(-0.25) / eps;
 #pragma unroll
-            for (int k = 0; k < NE; ++k) {   // backward half kick (hmc.py:46)
-                st[k] = th[k];
-                z[k] = ln.valid(k) ? A::sub(z[k], A::mul(heps, tgrad(th, k))) : T(0);
-            }
-            for (int s = 0; s < a.steps; ++s) {   // hmc.py:47-50
+                for (int k = 0; k < NE; ++k)
+                    st[k] = ln.valid(k) ? A::add(A::add(th[k], A::mul(eps, tgrad(th, k))), A::mul(sd, z[k])) : T(0);
+                md.terms(st, ll_s, pr_s);
+                const T lp_s = A::add(A::mul(ll_s, t0), pr_s);
+                T sf = T(0), sr = T(0);
 #pragma unroll
                 for (int k = 0; k < NE; ++k) {
                     if (ln.valid(k)) {
-                        z[k] = A::add(z[k], A::mul(eps, tgrad(st, k)));
-                        st[k] = A::add(st[k], A::mul(eps, z[k]));
+                        const T df = A::sub(A::sub(st[k], th[k]), A::mul(eps, tgrad(th, k)));
+                        const T dr = A::sub(A::sub(th[k], st[k]), A::mul(eps, tgrad(st, k)));
+                        sf = A::add(sf, A::mul(df, df));
+                        sr = A::add(sr, A::mul(dr, dr));
                     }
                 }
-            }
-            kin = T(0);
+                const T fwd = A::mul(coef, group_sum<G>(sf)), rev = A::mul(coef, group_sum<G>(sr));
+                acc = lu < A::add(A::sub(lp_s, lp_c), A::sub(rev, fwd));   // metropolis.py:41-76
+            } else {
+                // one HMCDiag transition, identity metric, on the tempered density (hmc.py:40-63)
+                const T eps = a.scale, heps = A::mul(T(0.5), eps);
+                T kin = T(0);
 #pragma unroll
-            for (int k = 0; k < NE; ++k) {   // forward half kick (hmc.py:52)
-                if (ln.valid(k)) z[k] = A::add(z[k], A::mul(heps, tgrad(st, k)));
-                kin = A::add(kin, A::mul(z[k], z[k]));
-            }
-            md.terms(st, ll_s, pr_s);
-            const T h1 = A::sub(A::add(A::mul(ll_s, t0), pr_s), A::mul(T(0.5), group_sum<G>(kin)));
-            acc = lu < A::sub(h1, h0);   // hmc.py:60
-        }
-        if (acc) {
+                for (int k = 0; k < NE; ++k) kin = A::add(kin, A::mul(z[k], z[k]));
+                const T h0 = A::sub(lp_c, A::mul(T(0.5), group_sum<G>(kin)));
 #pragma unroll
-            for (int k = 0; k < NE; ++k) th[k] = st[k];
-            ll_c = ll_s;
-            pr_c = pr_s;
+                for (int k = 0; k < NE; ++k) {   // backward half kick (hmc.py:46)
+                    st[k] = th[k];
+                    z[k] = ln.valid(k) ? A::sub(z[k], A::mul(heps, tgrad(th, k))) : T(0);
+                }
+                for (int s = 0; s < a.steps; ++s) {   // hmc.py:47-50
+#pragma unroll
+                    for (int k = 0; k < NE; ++k) {
+                        if (ln.valid(k)) {
+                            z[k] = A::add(z[k], A::mul(eps, tgrad(st, k)));
+                            st[k] = A::add(st[k], A::mul(eps, z[k]));
+                        }
+                    }
+                }
+                kin = T(0);
+#pragma unroll
+                for (int k = 0; k < NE; ++k) {   // forward half kick (hmc.py:52)
+                    if (ln.valid(k)) z[k] = A::add(z[k], A::mul(heps, tgrad(st, k)));
+                    kin = A::add(kin, A::mul(z[k], z[k]));
+                }
+                md.terms(st, ll_s, pr_s);
+                const T h1 = A::sub(A::add(A::mul(ll_s, t0), pr_s), A::mul(T(0.5), group_sum<G>(kin)));
+                acc = lu < A::sub(h1, h0);   // hmc.py:60
+            }
+            if (acc) {
+#pragma unroll
+                for (int k = 0; k < NE; ++k) th[k] = st[k];
+                ll_c = ll_s;
+                pr_c = pr_s;
+            }
+            n_acc += acc ? 1 : 0;
         }
         // importance log-weight, both tempered densities in full (smc.py:67-70)
         const T lw = A::sub(A::add(A::mul(ll_c, a.t1), pr_c), A::add(A::mul(ll_c, a.t0), pr_c));
@@ -289,7 +308,7 @@ __global__ void __launch_bounds__(128, OCC ? OCC : (J >= 4 && sizeof(T) == 4) ? 
                 const T lw_tot = a.logw_prev ? A::add(a.logw_prev[m], lw) : lw;
                 a.logw[m] = lw_tot;
                 lw_max = fmax(lw_max, (double)lw_tot);
-                if (a.accept) a.accept[m] = acc ? 1 : 0;
+                if (a.accept) a.accept[m] = MULTI ? n_acc : acc ? 1 : 0;
             }
         }
     }
@@ -343,10 +362,15 @@ static int launch_smc3(const SmcArgs<T>& a, cudaStream_t st) {
     const int64_t need = (a.M + per_block - 1) / per_block;
     // persistent: exactly one wave -- as many CTAs of 128 threads as are resident at once (8 per SM at 62
     // registers, 3 for the 16-elements-per-lane layout); every B200 of a box has the same SM count
-    static int64_t cap = 0;
+    const bool multi = a.moves > 1;
+    static int64_t caps[2] = {0, 0};
+    int64_t& cap = caps[multi ? 1 : 0];
     if (!cap) {
         int nb = 0;
-        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_smc_move_weight<T, G, J, View, MOVE, OCC, VM>, 128, 0) != cudaSuccess || nb < 1) {
+        const cudaError_t e =
+            multi ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_smc_move_weight<T, G, J, View, MOVE | SMC_MULTI, OCC, VM>, 128, 0)
+                  : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_smc_move_weight<T, G, J, View, MOVE, OCC, VM>, 128, 0);
+        if (e != cudaSuccess || nb < 1) {
             cudaGetLastError();
             nb = 1;
         }
@@ -354,7 +378,8 @@ static int launch_smc3(const SmcArgs<T>& a, cudaStream_t st) {
     }
     int64_t blocks = need < cap ? need : cap;
     if (blocks > SMC_MAXPART) blocks = SMC_MAXPART;
-    k_smc_move_weight<T, G, J, View, MOVE, OCC, VM><<<(unsigned)blocks, 128, 0, st>>>(a);
+    if (multi) k_smc_move_weight<T, G, J, View, MOVE | SMC_MULTI, OCC, VM><<<(unsigned)blocks, 128, 0, st>>>(a);
+    else k_smc_move_weight<T, G, J, View, MOVE, OCC, VM><<<(unsigned)blocks, 128, 0, st>>>(a);
     BK_LAUNCH_CHECK();
     return BK_OK;
 }
@@ -406,6 +431,7 @@ static int smc_user(const Model& m, const SmcArgs<T>& a, const bk_smc_kernel& kn
     u.maxpart = a.maxpart;
     u.ticket = a.ticket;
     u.params = m.user_params;
+    u.moves = a.moves;
     const UserProposal* p = nullptr;
     if (kn.kind == BK_SMC_KERNEL_PROPOSAL) {   // check_smc_model resolved the handle
         p = get_proposal(kn.proposal);
@@ -418,6 +444,7 @@ static int smc_user(const Model& m, const SmcArgs<T>& a, const bk_smc_kernel& kn
 // fills the model / geometry part of the arguments and picks the lane layout
 template <typename T>
 static int smc_dispatch(const Model& m, SmcArgs<T>& a, const bk_smc_kernel& kn, cudaStream_t st) {
+    a.moves = kn.moves > 1 ? kn.moves : 1;
     if (m.d.kind == BK_MODEL_USER_CUDA) return smc_user<T>(m, a, kn, st);
     a.D = (int)m.d.dims;
     a.scale = (T)kn.scale;
@@ -502,6 +529,8 @@ static int check_smc_model(const Model& m, const bk_smc_kernel& kn, const bk_rng
                  (long long)m.d.dims);
     BK_CHECK_ARG(kn.kind >= BK_SMC_KERNEL_RW && kn.kind <= BK_SMC_KERNEL_PROPOSAL, "bk_smc: unknown kernel kind %d",
                  kn.kind);
+    BK_CHECK_ARG(kn.moves >= 0 && kn.moves <= BK_SMC_MAX_MOVES, "bk_smc: kernel moves must be in [0, %d] (got %d)",
+                 BK_SMC_MAX_MOVES, kn.moves);
     if (kn.kind == BK_SMC_KERNEL_PROPOSAL) return check_smc_proposal(m, kn, rng);
     BK_CHECK_ARG(kn.scale > 0, "bk_smc: kernel scale / step size must be positive (got %g)", kn.scale);
     BK_CHECK_ARG(kn.kind != BK_SMC_KERNEL_HMC || kn.steps >= 0, "bk_smc: HMC kernel needs steps >= 0");
@@ -1532,6 +1561,21 @@ int bk_smc_cuda_prepare(uint64_t model, uint64_t proposal, char* log_out, size_t
     bk_smc_kernel kn = {BK_SMC_KERNEL_PROPOSAL, 0, 0.0, proposal};
     if (int rc = check_smc_model(*m, kn)) return rc;
     return user_mhp_prepare(*m, *p, "bk_smc_cuda_prepare", log_out, log_bytes);
+}
+
+int bk_smc_moves_prepare(uint64_t model, const bk_smc_kernel* kernel, char* log_out, size_t log_bytes) {
+    if (log_out && log_bytes) log_out[0] = '\0';
+    const Model* m = get_model(model);
+    if (!m) return BK_E_HANDLE;
+    BK_CHECK_ARG(kernel, "bk_smc_moves_prepare: null kernel");
+    const UserProposal* p = nullptr;
+    if (kernel->kind == BK_SMC_KERNEL_PROPOSAL) {
+        p = get_proposal(kernel->proposal);
+        if (!p) return BK_E_HANDLE;
+    }
+    if (int rc = check_smc_model(*m, *kernel)) return rc;
+    if (m->d.kind != BK_MODEL_USER_CUDA) return BK_OK;   // built-in plugins: the library's own kernels
+    return user_smc_moves_prepare(*m, p, log_out, log_bytes);
 }
 
 int bk_smc_shard_gather(const bk_smc_shard* sh, int64_t D, int32_t dtype, void* out, void* stream) {

@@ -14,8 +14,10 @@
 //   BK_PROGRAM_STRETCH          bk_user_stretch (also compiled with -DBK_STRETCH=1, which the model's source may test)
 //   BK_PROGRAM_WIDE             bk_user_wide_hmc / mala / mh (BK_USER_FUSED_MAX_D < D <= BK_USER_WIDE_MAX_D; also
 //                               compiled with -DBK_WIDE=1, which the model's source may test)
-// -DBK_SMC_KERNELS=1 marks the programs that carry SMC kernels (prior/likelihood models, kinds MODEL and
-// MODEL_PROPOSAL): exactly those into which smc_mailbox.cuh is spliced.
+//   BK_PROGRAM_SMC_MOVES        bk_user_smc_rw_moves / mala_moves / hmc_moves (prior/likelihood models); with a
+//                               proposal's source bk_user_smc_mhp_moves instead
+// -DBK_SMC_KERNELS=1 marks the programs that carry SMC kernels (prior/likelihood models, kinds MODEL,
+// MODEL_PROPOSAL and SMC_MOVES): exactly those into which smc_mailbox.cuh is spliced.
 // A model's source defines either
 //   __device__ bk_real log_density_gradient(const bk_real* theta, bk_real* grad, const bk_real* params);
 // or (bk_model_create_cuda_prior_lik: compiled with -DBK_PRIOR_LIK=1) the pair
@@ -52,6 +54,10 @@
 // bk_user_smc_mhp   (prior/likelihood models) TemperedLikelihoodSMC's move + weight kernel with one
 //                   Metropolis(-Hastings) step of the user's proposal as the move: bk_user_smc_rw with propose() in
 //                   place of the random walk (BK_SMC_KERNEL_PROPOSAL).
+// bk_user_smc_*_moves
+//                   bk_user_smc_rw / mala / hmc / mhp with bk_smc_kernel.moves > 1 Markov moves per particle visit: the
+//                   particle, its (ll, prior) pair and (MALA, HMC) its tempered gradient stay in registers between the
+//                   moves; move j draws at element block b + 2^16 j (smc_move_block, device_rng.cuh).
 // bk_user_drghmc    DrGhmcDiag, one thread per chain: k_drghmc (drghmc.cu) on the arithmetic and streams of the
 //                   lockstep engine (drghmc_generic.cu).
 // bk_user_stretch   one half-step of the Stretcher, one thread per active walker: k_stretch_propose, the density of
@@ -71,6 +77,7 @@
 #define BK_PROGRAM_DRGHMC 4
 #define BK_PROGRAM_STRETCH 5
 #define BK_PROGRAM_WIDE 6
+#define BK_PROGRAM_SMC_MOVES 7
 
 namespace bk {
 
@@ -187,8 +194,8 @@ struct UserSmcArgs {
     int32_t steps;                         // HMC: leapfrog steps
     int32_t rng_mode, n_uniform;           // bk_rng
     uint64_t seed, draw_offset, chain_offset;
-    const void* normals;                   // injected [M, D]
-    const void* uniforms;                  // injected [M, n_uniform]
+    const void* normals;                   // injected [M, D] (the *_moves kernels: [moves, M, D])
+    const void* uniforms;                  // injected [M, n_uniform] ([moves, M, n_uniform])
     void* logw;                            // [M] out
     const void* logw_prev;                 // [M] carried log-weights or NULL
     int32_t* accept;                       // [M] or NULL
@@ -204,6 +211,7 @@ struct UserSmcArgs {
     unsigned* ticket;
     const void* params;                    // [n_params] or NULL
     const void* prop_params;               // bk_user_smc_mhp: the proposal's [n_params] or NULL
+    int32_t moves;                         // the *_moves kernels: Markov moves per particle (> 1)
 };
 #endif
 
@@ -308,7 +316,9 @@ __device__ __forceinline__ void emit(const UserRunArgs& a, int64_t c, int64_t t,
 }  // namespace bk
 
 // ---- what a proposal's programs share -------------------------------------------------------------------------------
-#if BK_PROGRAM == BK_PROGRAM_PROPOSAL || BK_PROGRAM == BK_PROGRAM_MODEL_PROPOSAL
+#if BK_PROGRAM == BK_PROGRAM_PROPOSAL || BK_PROGRAM == BK_PROGRAM_MODEL_PROPOSAL || \
+    (BK_PROGRAM == BK_PROGRAM_SMC_MOVES && defined(BK_PROPOSAL_NORMALS))
+#define BK_HAS_PROPOSAL 1
 
 namespace bk {
 namespace user {
@@ -327,18 +337,19 @@ __device__ __forceinline__ const T* proposal_u(const S& s, int64_t row) {
 }
 
 // the proposal's Philox streams of (global chain, draw): z[k] from block proposal_normal_block(k, D), u[k] the k-th
-// TAG_UNIFORM uniform
-__device__ __forceinline__ void proposal_philox(uint64_t seed, uint32_t chain, uint32_t draw, T* z, T* u) {
+// TAG_UNIFORM uniform; boff is added to every block (smc_move_block)
+__device__ __forceinline__ void proposal_philox(uint64_t seed, uint32_t chain, uint32_t draw, T* z, T* u,
+                                                uint32_t boff = 0) {
 #pragma unroll
     for (int b = 0; 4 * b < NZ; ++b) {
         T z4[4];
-        philox_normal4<T>(seed, (uint32_t)proposal_normal_block(4 * b, D), chain, draw, z4);
+        philox_normal4<T>(seed, (uint32_t)proposal_normal_block(4 * b, D) + boff, chain, draw, z4);
 #pragma unroll
         for (int i = 0; i < 4; ++i)
             if (4 * b + i < NZ) z[4 * b + i] = z4[i];
     }
 #pragma unroll
-    for (int k = 0; k < NU; ++k) u[k] = philox_uniform<T>(seed, (uint32_t)k, chain, draw);
+    for (int k = 0; k < NU; ++k) u[k] = philox_uniform<T>(seed, (uint32_t)k, chain, draw, TAG_UNIFORM, boff);
 }
 
 // the proposal's z / u into local arrays: copied from the injected rows or drawn from Philox
@@ -400,8 +411,34 @@ __device__ __forceinline__ void tempered(const T (&x)[D], T t, const T* params, 
     for (int e = 0; e < D; ++e) g[e] = A::add(A::mul(g[e], t), gp[e]);
 }
 
+// The random streams of move j of a particle visit: MULTI (the *_moves kernels) reads the injected rows of draw j
+// ([moves, M, .]) and the Philox words of draw 0 at element block b + 2^16 j (smc_move_block); without MULTI the
+// single-move kernels' calls, unchanged.
+template <bool MULTI>
+__device__ __forceinline__ void smc_normal4(const UserSmcArgs& a, int64_t m, int j, int b, T (&z)[4]) {
+    if constexpr (!MULTI) normal4(a, a.M, m, 0, b, z);
+    else if (a.rng_mode == 1) normal4(a, a.M, m, j, b, z);
+    else philox_normal4<T>(a.seed, (uint32_t)b + smc_move_block(j), chain_word(a, m), draw_word(a, 0), z);
+}
+template <bool MULTI>
+__device__ __forceinline__ T smc_accept_uniform(const UserSmcArgs& a, int64_t m, int j) {
+    if constexpr (!MULTI) return accept_uniform(a, a.M, m, 0);
+    else if (a.rng_mode == 1) return accept_uniform(a, a.M, m, j);
+    else return philox_accept_uniform<T>(a.seed, chain_word(a, m), draw_word(a, 0), D, smc_move_block(j));
+}
+#ifdef BK_HAS_PROPOSAL
+template <bool MULTI>
+__device__ __forceinline__ void smc_proposal_streams(const UserSmcArgs& a, int64_t m, int j, T (&z)[NZ1], T (&u)[NU1]) {
+    if constexpr (!MULTI) proposal_streams(a, a.M, m, 0, z, u);   // injected: normals [M, NZ], uniforms [M, 1 + NU]
+    else if (a.rng_mode == 1) proposal_streams(a, a.M, m, j, z, u);
+    else proposal_philox(a.seed, chain_word(a, m), draw_word(a, 0), z, u, smc_move_block(j));
+}
+#endif
+
 // k_smc_move_weight with one lane per particle.  MOVE: BK_SMC_KERNEL_RW / _MALA / _HMC / _PROPOSAL (bk.h: 0 .. 3).
-template <int MOVE>
+// MULTI: a.moves Markov moves per visit (the loop is not unrolled); theta, (ll_c, pr_c) and, for MALA and HMC, the
+// tempered gradient at theta (gc) stay in registers, so after move 0 the model is evaluated at proposals only.
+template <int MOVE, bool MULTI = false>
 __device__ __forceinline__ void smc_move(const UserSmcArgs& a) {
     const T* params = reinterpret_cast<const T*>(a.params);
     const T t0 = (T)a.t0, t1 = (T)a.t1;
@@ -415,6 +452,7 @@ __device__ __forceinline__ void smc_move(const UserSmcArgs& a) {
         __syncthreads();
     }
     double lw_max = (double)neg_inf<float>();
+    const int n_moves = MULTI ? a.moves : 1;
     const int64_t stride = (int64_t)gridDim.x * blockDim.x;
     for (int64_t m = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; m < a.M; m += stride) {
         const int64_t gid = a.src_idx ? a.src_idx[m] : m;
@@ -432,103 +470,133 @@ __device__ __forceinline__ void smc_move(const UserSmcArgs& a) {
         }
         T th[D], st[D], z[D];
         load_row(row, th);
-        // proposal normals: the words Lanes<T, G, J>::normals consumes for blocks 0 .. ceil(D / 4) - 1 (the user's
-        // proposal draws its own streams below).  The loop is normals()'s, spelled out: through normals() ptxas
-        // allocates the fp64 RW kernel's registers differently.
-#pragma unroll
-        for (int b = 0; b < (MOVE == 3 ? 0 : NB); ++b) {
-            T z4[4];
-            normal4(a, a.M, m, 0, b, z4);
-#pragma unroll
-            for (int i = 0; i < 4; ++i)
-                if (4 * b + i < D) z[4 * b + i] = z4[i];
-        }
-        const T lu = log_u(accept_uniform(a, a.M, m, 0));
         T ll_c, pr_c, ll_s, pr_s;
-        if (carry) { ll_c = llpr[0]; pr_c = llpr[1]; }
+        T gc[D];   // MULTI, MALA / HMC: the tempered gradient at th
         bool acc;
-        if constexpr (MOVE == 0) {   // RW (smc.py:79-89); the gradients are dead code after inlining
-            T unused[D];
-            if (!carry) tempered(th, t0, params, ll_c, pr_c, unused);
-            const T lp_c = A::add(A::mul(ll_c, t0), pr_c);
+        int n_acc = 0;
+#pragma unroll 1
+        for (int j = 0; j < n_moves; ++j) {
+            // proposal normals: the words Lanes<T, G, J>::normals consumes for blocks 0 .. ceil(D / 4) - 1 (the user's
+            // proposal draws its own streams below).  The loop is normals()'s, spelled out: through normals() ptxas
+            // allocates the fp64 RW kernel's registers differently.
 #pragma unroll
-            for (int e = 0; e < D; ++e) st[e] = A::add(th[e], A::mul((T)a.scale, z[e]));   // smc.py:81
-            tempered(st, t0, params, ll_s, pr_s, unused);
-            const T lp_s = A::add(A::mul(ll_s, t0), pr_s);
-            acc = lu < A::sub(lp_s, lp_c);   // smc.py:85
-        } else if constexpr (MOVE == 1) {   // one MALA transition on the tempered density (mala.py:40-66)
-            const T eps = (T)a.scale, sd = A::sqrt_(A::mul(T(2), eps)), coef = T(-0.25) / eps;
-            T g[D], gs[D], ll_e, pr_e;
-            tempered(th, t0, params, ll_e, pr_e, g);
-            if (!carry) { ll_c = ll_e; pr_c = pr_e; }
-            const T lp_c = A::add(A::mul(ll_c, t0), pr_c);
+            for (int b = 0; b < (MOVE == 3 ? 0 : NB); ++b) {
+                T z4[4];
+                smc_normal4<MULTI>(a, m, j, b, z4);
 #pragma unroll
-            for (int e = 0; e < D; ++e) st[e] = A::add(A::add(th[e], A::mul(eps, g[e])), A::mul(sd, z[e]));
-            tempered(st, t0, params, ll_s, pr_s, gs);
-            const T lp_s = A::add(A::mul(ll_s, t0), pr_s);
-            T sf = T(0), sr = T(0);
-#pragma unroll
-            for (int e = 0; e < D; ++e) {
-                const T df = A::sub(A::sub(st[e], th[e]), A::mul(eps, g[e]));
-                const T dr = A::sub(A::sub(th[e], st[e]), A::mul(eps, gs[e]));
-                sf = A::add(sf, A::mul(df, df));
-                sr = A::add(sr, A::mul(dr, dr));
+                for (int i = 0; i < 4; ++i)
+                    if (4 * b + i < D) z[4 * b + i] = z4[i];
             }
-            const T fwd = A::mul(coef, sf), rev = A::mul(coef, sr);
-            acc = lu < A::add(A::sub(lp_s, lp_c), A::sub(rev, fwd));   // metropolis.py:41-76
-#if BK_PROGRAM == BK_PROGRAM_MODEL_PROPOSAL
-        } else if constexpr (MOVE == 3) {   // the RW branch with the user's proposal: bk_user_mhp's step
-            const T* pp = reinterpret_cast<const T*>(a.prop_params);
-            T zp[NZ1], up[NU1], unused[D];
-            proposal_streams(a, a.M, m, 0, zp, up);   // injected: normals [M, NZ], uniforms [M, 1 + NU]
-            if (!carry) tempered(th, t0, params, ll_c, pr_c, unused);
-            const T lp_c = A::add(A::mul(ll_c, t0), pr_c);
-            bk_proposal::propose(th, st, zp, up, pp);
-            tempered(st, t0, params, ll_s, pr_s, unused);
-            const T lp_s = A::add(A::mul(ll_s, t0), pr_s);
-            T ratio = A::sub(lp_s, lp_c);
-#if BK_PROPOSAL_TRANSITION
-            ratio = A::add(ratio, proposal_dh(th, st, pp));
-#endif
-            acc = lu < ratio;
-#endif
-        } else {   // one HMCDiag transition, identity metric, on the tempered density (hmc.py:40-63)
-            const T eps = (T)a.scale, heps = A::mul(T(0.5), eps);
-            T g[D];
-            tempered(th, t0, params, ll_s, pr_s, g);   // (ll_s, pr_s): the terms at st, which starts at th
-            if (!carry) { ll_c = ll_s; pr_c = pr_s; }
-            const T lp_c = A::add(A::mul(ll_c, t0), pr_c);
-            T kin = T(0);
+            const T lu = log_u(smc_accept_uniform<MULTI>(a, m, j));
+            if (carry && j == 0) { ll_c = llpr[0]; pr_c = llpr[1]; }
+            if constexpr (MOVE == 0) {   // RW (smc.py:79-89); the gradients are dead code after inlining
+                T unused[D];
+                if (!carry && j == 0) tempered(th, t0, params, ll_c, pr_c, unused);
+                const T lp_c = A::add(A::mul(ll_c, t0), pr_c);
 #pragma unroll
-            for (int e = 0; e < D; ++e) kin = A::add(kin, A::mul(z[e], z[e]));
-            const T h0 = A::sub(lp_c, A::mul(T(0.5), kin));
+                for (int e = 0; e < D; ++e) st[e] = A::add(th[e], A::mul((T)a.scale, z[e]));   // smc.py:81
+                tempered(st, t0, params, ll_s, pr_s, unused);
+                const T lp_s = A::add(A::mul(ll_s, t0), pr_s);
+                acc = lu < A::sub(lp_s, lp_c);   // smc.py:85
+            } else if constexpr (MOVE == 1) {   // one MALA transition on the tempered density (mala.py:40-66)
+                const T eps = (T)a.scale, sd = A::sqrt_(A::mul(T(2), eps)), coef = T(-0.25) / eps;
+                T g[D], gs[D], ll_e, pr_e;
+                if (j == 0) {
+                    tempered(th, t0, params, ll_e, pr_e, g);
+                    if (!carry) { ll_c = ll_e; pr_c = pr_e; }
+                } else {
 #pragma unroll
-            for (int e = 0; e < D; ++e) {   // backward half kick (hmc.py:46)
-                st[e] = th[e];
-                z[e] = A::sub(z[e], A::mul(heps, g[e]));
-            }
-            for (int s = 0; s < a.steps; ++s) {   // hmc.py:47-50
+                    for (int e = 0; e < D; ++e) g[e] = gc[e];
+                }
+                const T lp_c = A::add(A::mul(ll_c, t0), pr_c);
+#pragma unroll
+                for (int e = 0; e < D; ++e) st[e] = A::add(A::add(th[e], A::mul(eps, g[e])), A::mul(sd, z[e]));
+                tempered(st, t0, params, ll_s, pr_s, gs);
+                const T lp_s = A::add(A::mul(ll_s, t0), pr_s);
+                T sf = T(0), sr = T(0);
 #pragma unroll
                 for (int e = 0; e < D; ++e) {
-                    z[e] = A::add(z[e], A::mul(eps, g[e]));
-                    st[e] = A::add(st[e], A::mul(eps, z[e]));
+                    const T df = A::sub(A::sub(st[e], th[e]), A::mul(eps, g[e]));
+                    const T dr = A::sub(A::sub(th[e], st[e]), A::mul(eps, gs[e]));
+                    sf = A::add(sf, A::mul(df, df));
+                    sr = A::add(sr, A::mul(dr, dr));
                 }
-                tempered(st, t0, params, ll_s, pr_s, g);
-            }
-            kin = T(0);
+                const T fwd = A::mul(coef, sf), rev = A::mul(coef, sr);
+                acc = lu < A::add(A::sub(lp_s, lp_c), A::sub(rev, fwd));   // metropolis.py:41-76
+                if constexpr (MULTI) {
 #pragma unroll
-            for (int e = 0; e < D; ++e) {   // forward half kick (hmc.py:52)
-                z[e] = A::add(z[e], A::mul(heps, g[e]));
-                kin = A::add(kin, A::mul(z[e], z[e]));
-            }
-            const T h1 = A::sub(A::add(A::mul(ll_s, t0), pr_s), A::mul(T(0.5), kin));
-            acc = lu < A::sub(h1, h0);   // hmc.py:60
-        }
-        if (acc) {
+                    for (int e = 0; e < D; ++e) gc[e] = acc ? gs[e] : g[e];
+                }
+#ifdef BK_HAS_PROPOSAL
+            } else if constexpr (MOVE == 3) {   // the RW branch with the user's proposal: bk_user_mhp's step
+                const T* pp = reinterpret_cast<const T*>(a.prop_params);
+                T zp[NZ1], up[NU1], unused[D];
+                smc_proposal_streams<MULTI>(a, m, j, zp, up);
+                if (!carry && j == 0) tempered(th, t0, params, ll_c, pr_c, unused);
+                const T lp_c = A::add(A::mul(ll_c, t0), pr_c);
+                bk_proposal::propose(th, st, zp, up, pp);
+                tempered(st, t0, params, ll_s, pr_s, unused);
+                const T lp_s = A::add(A::mul(ll_s, t0), pr_s);
+                T ratio = A::sub(lp_s, lp_c);
+#if BK_PROPOSAL_TRANSITION
+                ratio = A::add(ratio, proposal_dh(th, st, pp));
+#endif
+                acc = lu < ratio;
+#endif
+            } else {   // one HMCDiag transition, identity metric, on the tempered density (hmc.py:40-63)
+                const T eps = (T)a.scale, heps = A::mul(T(0.5), eps);
+                T g[D];
+                if (j == 0) {
+                    tempered(th, t0, params, ll_s, pr_s, g);   // (ll_s, pr_s): the terms at st, which starts at th
+                    if (!carry) { ll_c = ll_s; pr_c = pr_s; }
+                } else {
+                    ll_s = ll_c;
+                    pr_s = pr_c;
 #pragma unroll
-            for (int e = 0; e < D; ++e) th[e] = st[e];
-            ll_c = ll_s;
-            pr_c = pr_s;
+                    for (int e = 0; e < D; ++e) g[e] = gc[e];
+                }
+                const T lp_c = A::add(A::mul(ll_c, t0), pr_c);
+                if constexpr (MULTI) {
+#pragma unroll
+                    for (int e = 0; e < D; ++e) gc[e] = g[e];
+                }
+                T kin = T(0);
+#pragma unroll
+                for (int e = 0; e < D; ++e) kin = A::add(kin, A::mul(z[e], z[e]));
+                const T h0 = A::sub(lp_c, A::mul(T(0.5), kin));
+#pragma unroll
+                for (int e = 0; e < D; ++e) {   // backward half kick (hmc.py:46)
+                    st[e] = th[e];
+                    z[e] = A::sub(z[e], A::mul(heps, g[e]));
+                }
+                for (int s = 0; s < a.steps; ++s) {   // hmc.py:47-50
+#pragma unroll
+                    for (int e = 0; e < D; ++e) {
+                        z[e] = A::add(z[e], A::mul(eps, g[e]));
+                        st[e] = A::add(st[e], A::mul(eps, z[e]));
+                    }
+                    tempered(st, t0, params, ll_s, pr_s, g);
+                }
+                kin = T(0);
+#pragma unroll
+                for (int e = 0; e < D; ++e) {   // forward half kick (hmc.py:52)
+                    z[e] = A::add(z[e], A::mul(heps, g[e]));
+                    kin = A::add(kin, A::mul(z[e], z[e]));
+                }
+                const T h1 = A::sub(A::add(A::mul(ll_s, t0), pr_s), A::mul(T(0.5), kin));
+                acc = lu < A::sub(h1, h0);   // hmc.py:60
+                if constexpr (MULTI) {
+#pragma unroll
+                    for (int e = 0; e < D; ++e) gc[e] = acc ? g[e] : gc[e];
+                }
+            }
+            if (acc) {
+#pragma unroll
+                for (int e = 0; e < D; ++e) th[e] = st[e];
+                ll_c = ll_s;
+                pr_c = pr_s;
+            }
+            n_acc += acc ? 1 : 0;
         }
         // importance log-weight, both tempered densities in full (smc.py:67-70)
         const T lw = A::sub(A::add(A::mul(ll_c, t1), pr_c), A::add(A::mul(ll_c, t0), pr_c));
@@ -543,7 +611,7 @@ __device__ __forceinline__ void smc_move(const UserSmcArgs& a) {
         const T lw_tot = a.logw_prev ? A::add(reinterpret_cast<const T*>(a.logw_prev)[m], lw) : lw;
         reinterpret_cast<T*>(a.logw)[m] = lw_tot;
         lw_max = fmax(lw_max, (double)lw_tot);
-        if (a.accept) a.accept[m] = acc ? 1 : 0;
+        if (a.accept) a.accept[m] = MULTI ? n_acc : acc ? 1 : 0;
     }
     if (a.maxpart) smc_post_max(lw_max, a.maxpart, a.ticket, a.sh, a.mail_tab, a.epoch);
 }
@@ -1445,6 +1513,26 @@ extern "C" __global__ void __launch_bounds__(32) bk_user_wide_mh(const bk::UserW
         __syncwarp();
     }
 }
+
+// ---- BK_PROGRAM_SMC_MOVES: the SMC's move + weight kernel with several moves per temperature, compiled on prepare ----
+// (a model's program and its (model, proposal) program keep the single-move kernels only)
+#elif BK_PROGRAM == BK_PROGRAM_SMC_MOVES
+
+#ifdef BK_HAS_PROPOSAL
+extern "C" __global__ void __launch_bounds__(128) bk_user_smc_mhp_moves(const bk::UserSmcArgs a) {
+    bk::user::smc_move<3, true>(a);
+}
+#else
+extern "C" __global__ void __launch_bounds__(128) bk_user_smc_rw_moves(const bk::UserSmcArgs a) {
+    bk::user::smc_move<0, true>(a);
+}
+extern "C" __global__ void __launch_bounds__(128) bk_user_smc_mala_moves(const bk::UserSmcArgs a) {
+    bk::user::smc_move<1, true>(a);
+}
+extern "C" __global__ void __launch_bounds__(128) bk_user_smc_hmc_moves(const bk::UserSmcArgs a) {
+    bk::user::smc_move<2, true>(a);
+}
+#endif
 
 #endif  // BK_PROGRAM
 #endif  // __CUDACC_RTC__

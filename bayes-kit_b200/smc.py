@@ -45,8 +45,8 @@ class _Kernel:
         if not self.scale > 0:
             raise ValueError(f"{what} must be positive, got {scale}")
 
-    def desc(self) -> L.SmcKernel:
-        return L.SmcKernel(self.kind, self.steps, self.scale)
+    def desc(self, moves: int = 1) -> L.SmcKernel:
+        return L.SmcKernel(self.kind, self.steps, self.scale, 0, moves)
 
     def stream_widths(self, D: int):
         """(normals, uniforms) per particle of the injected streams."""
@@ -95,8 +95,8 @@ class ProposalKernel(_Kernel):
                              "the SMC's move would need the gradient of the tempered density")
         self.proposal = proposal          # keeps the handle alive as long as the kernel
 
-    def desc(self) -> L.SmcKernel:
-        return L.SmcKernel(self.kind, 0, 0.0, self.proposal.handle)
+    def desc(self, moves: int = 1) -> L.SmcKernel:
+        return L.SmcKernel(self.kind, 0, 0.0, self.proposal.handle, moves)
 
     def stream_widths(self, D: int):
         return self.proposal.normals, 1 + self.proposal.uniforms
@@ -140,12 +140,20 @@ class TemperedLikelihoodSMC:
       smc.py:60) or a fraction in (0, 1]: resample only when the importance-weight
       ESS drops below ``ess_threshold * M``, carrying the log-weights otherwise
       (``log_weights``, ``resampled``); the decision is taken on device.
+    * ``moves``: applications of the kernel per particle and temperature (1 <= moves <= 65535), all targeting
+      time(n-1), before the reweighting to time(n) and the resampling: the reference run with the composed kernel
+      ``K(K(...K(theta)))``.  The moves run inside the one move + weight kernel, on the particle held in registers;
+      ``last_accept`` counts the accepted moves of each particle.  On a ``CudaPriorLikModel`` the program of these
+      kernels is compiled at construction when moves > 1 (``compile_log``).
     With torch.distributed initialised (or ``group=`` given), M is the GLOBAL particle
     count and each rank owns a contiguous slice.
     """
 
     def __init__(self, model, M: int, N: int, sample_initial, kernel, *, resample: str = "multinomial",
-                 ess_threshold: Optional[float] = None, seed=None, group=None):
+                 ess_threshold: Optional[float] = None, seed=None, group=None, moves: int = 1):
+        if isinstance(moves, bool) or not isinstance(moves, (int, np.integer)) or not 1 <= moves <= L.SMC_MAX_MOVES:
+            raise ValueError(f"moves must be an int in [1, {L.SMC_MAX_MOVES}], got {moves!r}")
+        self.moves = int(moves)
         self._model = require_plugin(model)
         if not isinstance(self._model, (GaussPriorLik, Binomial, CudaPriorLikModel)):
             raise TypeError("TemperedLikelihoodSMC needs a model plugin with log_prior/log_likelihood "
@@ -154,9 +162,12 @@ class TemperedLikelihoodSMC:
             raise TypeError("kernel must be bayes_kit_b200.metropolis_kernel(scale) (or mala_kernel / hmc_kernel / "
                             "proposal_kernel): arbitrary Python kernels cannot run per particle on the GPU and there is "
                             "no CPU fallback")
+        self.kernel = kernel
         self.compile_log = ""
         if isinstance(kernel, ProposalKernel):
             self._prepare(kernel.proposal)
+        elif self.moves > 1 and isinstance(self._model, CudaPriorLikModel):
+            self._prepare_moves()
         if resample not in ("multinomial", "systematic"):
             raise ValueError("resample must be 'multinomial' or 'systematic'")
         if ess_threshold is not None and not 0 < ess_threshold <= 1:
@@ -165,7 +176,6 @@ class TemperedLikelihoodSMC:
             raise ValueError("ess_threshold needs resample='systematic'")
         self.ess_threshold = ess_threshold      # None: resample at every temperature (smc.py:60)
         self.M, self.N = int(M), int(N)
-        self.kernel = kernel
         self.resample = resample
         self._mode = L.RESAMPLE_MULTINOMIAL if resample == "multinomial" else L.RESAMPLE_SYSTEMATIC
         self.device, self.dtype = self._model.device, self._model.dtype
@@ -222,9 +232,19 @@ class TemperedLikelihoodSMC:
         if prop.dims != self._model.dims() or prop.dtype != self._model.dtype:
             raise ValueError(f"the proposal (dims {prop.dims}, {prop.dtype}) does not match the model "
                              f"(dims {self._model.dims()}, {self._model.dtype})")
+        if self.moves > 1:
+            self._prepare_moves()
+            return
         self.compile_log = compile_log(
             lambda log, n: L.lib().bk_smc_cuda_prepare(self._model.handle, prop.handle, log, n),
             "TemperedLikelihoodSMC: NVRTC compilation of the model with the proposal failed:\n", self._model.device)
+
+    def _prepare_moves(self) -> None:
+        """Compile the program of the user model's (and proposal's) kernels of several moves per temperature now."""
+        kn = self.kernel.desc(self.moves)
+        self.compile_log = compile_log(
+            lambda log, n: L.lib().bk_smc_moves_prepare(self._model.handle, C.byref(kn), log, n),
+            f"TemperedLikelihoodSMC: NVRTC compilation of the {self.moves}-move kernel failed:\n", self._model.device)
 
     # ---- plumbing --------------------------------------------------------------------
     def _sh(self) -> L.SmcShard:
@@ -296,7 +316,7 @@ class TemperedLikelihoodSMC:
         self._epoch += 1                       # epoch of step n_from
         self._acc = torch.empty(Ml, dtype=torch.int32, device=self.device)
         rng = make_rng(self._seed, n_from, self._lo, None, None, 1)
-        kn = self.kernel.desc()
+        kn = self.kernel.desc(self.moves)
         src = None if self._pending else self._src_local.data_ptr()
         thr = float(self.ess_threshold) * self.M if self.ess_threshold is not None else 0.0
         with torch.cuda.device(self.device):
@@ -345,7 +365,10 @@ class TemperedLikelihoodSMC:
         reference's recorded legacy-RNG streams (parity mode): proposal normals
         [M_local, D], accept uniforms [M_local], resampling uniforms [M_local] (systematic: [1]).
         With ``proposal_kernel``: normals [M_local, normals] and acc_uniforms [M_local, 1 + uniforms] (column 0 the
-        accept uniform, columns 1.. the proposal's u; [M_local] when it draws no uniforms)."""
+        accept uniform, columns 1.. the proposal's u; [M_local] when it draws no uniforms).
+        With ``moves`` > 1 each particle's streams are in the order its moves consume them: normals
+        [M_local, moves, D] and acc_uniforms [M_local, moves] (``proposal_kernel``: [M_local, moves, normals] and
+        [M_local, moves, 1 + uniforms])."""
         self._move(n, normals, acc_uniforms)
         self._resample(n, res_uniforms, 0)
 
@@ -357,7 +380,18 @@ class TemperedLikelihoodSMC:
         self._epoch += 1
         self._acc = torch.empty(Ml, dtype=torch.int32, device=self.device)
         nz, nu = self.kernel.stream_widths(self.D)
-        if normals is not None and isinstance(self.kernel, ProposalKernel):
+        if normals is not None and self.moves > 1:
+            # the reference's order [M_local, moves, .] -> the ABI's one draw per move [moves, M_local, .]
+            k = self.moves
+            normals = to_dev(normals, self.dtype, self.device)
+            acc_uniforms = to_dev(acc_uniforms, self.dtype, self.device)
+            if normals.numel() != Ml * k * nz or acc_uniforms.numel() != Ml * k * nu:
+                raise ValueError(f"injected streams of {k} moves: normals [{Ml}, {k}, {nz}] and acc_uniforms "
+                                 f"[{Ml}, {k}{'' if nu == 1 else f', {nu}'}] (got {tuple(normals.shape)} and "
+                                 f"{tuple(acc_uniforms.shape)})")
+            normals = normals.reshape(Ml, k, nz).transpose(0, 1).contiguous()
+            acc_uniforms = acc_uniforms.reshape(Ml, k, nu).transpose(0, 1).contiguous()
+        elif normals is not None and isinstance(self.kernel, ProposalKernel):
             normals = to_dev(normals, self.dtype, self.device)
             acc_uniforms = to_dev(acc_uniforms, self.dtype, self.device)
             if normals.numel() != Ml * nz or acc_uniforms.numel() != Ml * nu:
@@ -369,7 +403,7 @@ class TemperedLikelihoodSMC:
             acc_uniforms = to_dev(acc_uniforms, self.dtype, self.device).reshape(Ml)
         self._inj = (normals, acc_uniforms)     # keep the injected streams alive until the kernel ran
         rng = make_rng(self._seed, n, self._lo, normals, acc_uniforms, nu)
-        kn = self.kernel.desc()
+        kn = self.kernel.desc(self.moves)
         src = None if self._pending else self._src_local.data_ptr()
         accumulate = 1 if (self.ess_threshold is not None and self._epoch > 1) else 0
         with torch.cuda.device(self.device):

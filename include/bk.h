@@ -436,9 +436,28 @@ BK_API int bk_gather_rows(const void* src, const int64_t* idx, int64_t M, int64_
  *             restate GAUSS_PRIOR_LIK / BINOMIAL_LOGIT as one): BK_E_UNSUPPORTED otherwise.  The proposal's dims
  *             and dtype must be the model's and n_normals <= BK_SMC_PROPOSAL_MAX_NORMALS; INJECTED streams need
  *             n_uniform = 1 + n_uniforms (layout: the note after bk_rng).  `scale` and `steps` are not read.
- * `proposal` is read only by the PROPOSAL kind: initialisers such as {BK_SMC_KERNEL_RW, 0, scale} leave it 0. */
+ * `proposal` is read only by the PROPOSAL kind: initialisers such as {BK_SMC_KERNEL_RW, 0, scale} leave it 0.
+ * `moves`: applications of the kernel per particle and temperature, all targeting time(n-1), before the particle is
+ * reweighted to time(n) and resampled (the reference with the composed kernel K(K(...K(theta))) ).  0 and 1 both mean
+ * one move, so existing initialisers keep their meaning; at most BK_SMC_MAX_MOVES, else BK_E_INVALID.  The moves run
+ * in one kernel on the particle held in registers: the row read (with the resample gather), the (ll, prior) carry,
+ * the row write, the log-weight and the max message happen once per temperature.  Streams of move j (0-based):
+ *   PHILOX    exactly move 0's words with the element-block counter word b replaced by b + 2^16 j (proposal
+ *             normals, the accept uniform, the fp64 TAG_NORMAL_HI words, a proposal's TAG_UNIFORM uniforms); every
+ *             block a move uses is below 2^16, so move 0 is the single-move stream.  TAG_RESAMPLE is untouched.
+ *   INJECTED  one "draw" per move: normals [moves, M_local, D] (PROPOSAL: [moves, M_local, n_normals]) and
+ *             uniforms [moves, M_local, n_uniform].
+ * accept_out then counts the accepted moves of each particle (0 .. moves).  User models run moves > 1 through the
+ * program bk_smc_moves_prepare compiles. */
 enum { BK_SMC_KERNEL_RW = 0, BK_SMC_KERNEL_MALA = 1, BK_SMC_KERNEL_HMC = 2, BK_SMC_KERNEL_PROPOSAL = 3 };
-typedef struct bk_smc_kernel { int32_t kind; int32_t steps; double scale; uint64_t proposal; } bk_smc_kernel;
+typedef struct bk_smc_kernel {
+    int32_t kind;
+    int32_t steps;
+    double scale;
+    uint64_t proposal;
+    int32_t moves;
+} bk_smc_kernel;
+#define BK_SMC_MAX_MOVES 65535
 /* one thread per particle keeps the proposal's normals in local memory: the bound keeps that array small */
 #define BK_SMC_PROPOSAL_MAX_NORMALS 512
 /* Checks (model, proposal) as bk_smc_shard_move does for the PROPOSAL kind and compiles their fused program
@@ -447,6 +466,12 @@ typedef struct bk_smc_kernel { int32_t kind; int32_t steps; double scale; uint64
  * on a bad argument or a compile error (with the log), BK_E_UNSUPPORTED for a model the proposal move does not
  * serve. */
 BK_API int bk_smc_cuda_prepare(uint64_t model, uint64_t proposal, char* log_out, size_t log_bytes);
+/* Checks (model, kernel) as bk_smc_shard_move does and, for a user model, compiles the program of its moves > 1
+ * kernels (bk_user_smc_{rw,mala,hmc}_moves; with a PROPOSAL kernel bk_user_smc_mhp_moves of the (model, proposal)
+ * pair) once per process, so that the first move does not pay the NVRTC compile; log_out as bk_model_create_cuda's
+ * (ptxas's report).  Built-in plugins: BK_OK without compiling.  BK_E_HANDLE for an unknown model or proposal handle
+ * (before any device call), BK_E_INVALID / BK_E_UNSUPPORTED as bk_smc_cuda_prepare. */
+BK_API int bk_smc_moves_prepare(uint64_t model, const bk_smc_kernel* kernel, char* log_out, size_t log_bytes);
 #define BK_SMC_MAX_WORLD 16
 #define BK_SMC_MAILBOX_BYTES 4096
 typedef struct bk_smc_shard {
@@ -489,7 +514,7 @@ BK_API int bk_smc_shard_resample(const bk_smc_shard* sh, int32_t dtype, int32_t 
  * ~60 us of device time, less than two Python-level calls cost).  sh->epoch is the epoch of step n_from and
  * advances by one per step (the caller continues with epoch + n_to - n_from + 1); Philox only (rng->mode),
  * rng->draw_offset is ignored: step n draws with draw_offset = n, like the step-wise calls.
- * stats_out: [n_to - n_from + 1, 4] doubles or NULL; accept_out: flags of the LAST step or NULL. */
+ * stats_out: [n_to - n_from + 1, 4] doubles or NULL; accept_out: accepted moves of the LAST step or NULL. */
 BK_API int bk_smc_shard_run(uint64_t handle, const bk_smc_shard* sh, const void* src_local, int32_t n_from,
                      int32_t n_to, int32_t T, const bk_smc_kernel* kernel, const bk_rng* rng, int32_t mode,
                      double ess_threshold, double* stats_out, int32_t* accept_out, void* ws, size_t ws_bytes,
